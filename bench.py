@@ -57,7 +57,14 @@ def parse():
     ap.add_argument("--probe-queries", type=int, default=256, help="random queries checked against the f64 oracle after the run")
     ap.add_argument("--seconds", type=float, default=3600.0, help="configs 2 / 5: seconds of synthetic audio")
     ap.add_argument("--mode", default="dtw", choices=["dtw", "cosine"], help="config 5: matcher")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="configs 3 / 4: write the match result of the last timed step to DIR/*.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config not in (3, 4)):
+        ap.error("--dump-outputs is available for --impl ours with --config 3 or 4")
+    return args
 
 
 class ClockSampler:
@@ -157,6 +164,25 @@ def algorithmic_bytes(doff, qoff, s0, s1):
     lq = int(qoff[-1])
     nq, nd = len(qoff) - 1, s1 - s0
     return (nd * lq + nq * ld) * C * 4
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, idx, dist):
+    """Writes a match result as the caller of ss_dict_match_dev receives it, in float64: indices.npy (u32 segment indices,
+    0xFFFFFFFF = empty slot) and distances.npy, both [queries, k], and query_ids.npy, the query each row belongs to.
+    A result larger than DUMP_BYTES is cut to a fixed, seeded sample of queries, so that two builds run with the same
+    arguments write the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    nq, k = idx.shape
+    row_bytes = 8 * (2 * k + 1)
+    rows = np.arange(nq)
+    if nq * row_bytes > DUMP_BYTES - 3 * 4096:  # room for the three .npy headers
+        rows = np.sort(np.random.default_rng(2026).choice(nq, size=(DUMP_BYTES - 3 * 4096) // row_bytes, replace=False))
+    np.save(os.path.join(out_dir, "query_ids.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "indices.npy"), idx[rows].astype(np.float64))
+    np.save(os.path.join(out_dir, "distances.npy"), dist[rows].astype(np.float64))
 
 
 def cpu_sample(d, doff, q, qoff, nsample, threads):
@@ -335,6 +361,8 @@ def run_match(args):
         scan_ms = float(lib.ss_dict_last_scan_ms(shard.h))
         tc_fallback, exhaustive, uncert = shard.last_tc_fallback, shard.last_exhaustive, shard.last_uncertified
         clocks = sampler.stop() if rank == 0 else None
+        if args.dump_outputs and rank == 0:  # every rank holds the merged result of the last timed step
+            dump_outputs(args.dump_outputs, o_idx.cpu().numpy().view(np.uint32), o_dist.cpu().numpy())
         for _ in range(2):
             step_e2e()
         # e2e blocks on the host every step (the call returns results in host memory): wall clock == device time here

@@ -16,6 +16,7 @@ Each oracle output was cross-checked against oracle/numpy_twin.py by tests/test_
 import json
 import os
 import sys
+import zipfile
 
 import numpy as np
 
@@ -27,6 +28,15 @@ from soundsym_b200 import synth  # noqa: E402
 
 REF = "/root/reference/tests"
 OUT = os.path.dirname(os.path.abspath(__file__))
+
+
+def savez_lzma(path, **arrays):
+    """np.savez with LZMA-compressed members, which np.load reads like any .npz: the PCM of the two WAV fixtures
+    compresses to under 1 MB per file this way (deflate leaves sample_excerpt.npz at 1.2 MB)."""
+    with zipfile.ZipFile(path, "w", zipfile.ZIP_LZMA) as z:
+        for name, a in arrays.items():
+            with z.open(name + ".npy", "w", force_zip64=True) as f:
+                np.lib.format.write_array(f, np.asanyarray(a))
 
 
 def cut(mfcc, seg_lens_samples, hop=256):
@@ -52,7 +62,7 @@ def main():
         votes = O.cast_votes(sym71, depth)
         g["votes_d%d" % depth] = votes
         g["splits_d%dt%d" % (depth, thr)] = O.split(votes, len(sym71), thr) * np.uint64(256)
-    np.savez_compressed(os.path.join(OUT, "section71.npz"), **g)
+    savez_lzma(os.path.join(OUT, "section71.npz"), **g)
 
     # ---- sample.wav excerpt : config 1 ----------------------------------------------------------------------------
     s, sr, bits, pcm = T.read_wav(os.path.join(REF, "sample.wav"))
@@ -74,19 +84,19 @@ def main():
     samp_off = np.zeros(len(g["splits_d3t4"]) + 1, dtype=np.uint64)
     samp_off[1:] = np.cumsum(g["splits_d3t4"])
     resyn = O.resynth(s71, samp_off, cos_idx, splits_ex)
-    np.savez_compressed(os.path.join(OUT, "sample_excerpt.npz"), pcm=pcm_ex.astype(np.int32), bits=np.int32(bits),
-                        sample_rate=np.float64(sr), mfcc=m_ex, max_power=np.float64(O.max_power(s_ex)), symbols=sym_ex,
-                        splits_d3t4=splits_ex, q_max_power=q_pow, cos_idx=cos_idx, cos_dist=cos_dist, dtw_idx=dtw_idx,
-                        dtw_dist=dtw_dist, resynth_head=resyn[:65536], resynth_sum=np.float64(resyn.sum()),
-                        resynth_len=np.uint64(len(resyn)))
+    savez_lzma(os.path.join(OUT, "sample_excerpt.npz"), pcm=pcm_ex.astype(np.int32), bits=np.int32(bits),
+               sample_rate=np.float64(sr), mfcc=m_ex, max_power=np.float64(O.max_power(s_ex)), symbols=sym_ex,
+               splits_d3t4=splits_ex, q_max_power=q_pow, cos_idx=cos_idx, cos_dist=cos_dist, dtw_idx=dtw_idx,
+               dtw_dist=dtw_dist, resynth_head=resyn[:65536], resynth_sum=np.float64(resyn.sum()),
+               resynth_len=np.uint64(len(resyn)))
 
     # ---- synthetic small : config-3 generator ----------------------------------------------------------------------
     d, doff = synth.segments(600, 13, seed=1234)
     q, qoff = synth.segments(48, 13, seed=5678)
     di, dd = O.dtw_topk(d, doff, q, qoff, 13, k=4)
     ci, cd = O.cosine_match(d, doff, q, qoff, 13)
-    np.savez_compressed(os.path.join(OUT, "synthetic_small.npz"), dtw_idx=di, dtw_dist=dd, cos_idx=ci, cos_dist=cd,
-                        dict_checksum=np.float64(d.sum()), q_checksum=np.float64(q.sum()))
+    savez_lzma(os.path.join(OUT, "synthetic_small.npz"), dtw_idx=di, dtw_dist=dd, cos_idx=ci, cos_dist=cd,
+               dict_checksum=np.float64(d.sum()), q_checksum=np.float64(q.sum()))
 
     kats = {
         "decode_24bit_max_abs_sample_wav": {"value": full_max_abs, "expected": 0.6503654301602161, "tol": 1e-9,

@@ -48,6 +48,44 @@ def test_bench_sharding_and_algorithmic_bytes():
         assert sum(bench.algorithmic_bytes(doff, qoff, a, b) for a, b in zip(cuts, cuts[1:])) == whole
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 .npy files that round-trip the u32 indices exactly; past the size cap, the same
+    seeded sample of queries on every run; --steps 0 and unsupported configurations are refused."""
+    import importlib.util
+    import os
+    import sys
+    import numpy as np
+    import pytest
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rng = np.random.default_rng(5)
+    idx = rng.integers(0, 100000, size=(1000, 4)).astype(np.uint32)
+    idx[3, 2:] = 0xFFFFFFFF
+    dist = rng.uniform(0.0, 50.0, size=(1000, 4))
+    bench.dump_outputs(str(tmp_path / "all"), idx, dist)
+    out = {n: np.load(str(tmp_path / "all" / (n + ".npy"))) for n in ("query_ids", "indices", "distances")}
+    assert all(a.dtype == np.float64 for a in out.values())
+    assert np.array_equal(out["query_ids"], np.arange(1000)) and np.array_equal(out["distances"], dist)
+    assert np.array_equal(out["indices"].astype(np.uint32), idx) and out["indices"][3, 3] == 0xFFFFFFFF
+    monkeypatch.setattr(bench, "DUMP_BYTES", 3 * 4096 + 72 * 100)  # room for 100 rows of k = 4
+    samples = []
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), idx, dist)
+        ids = np.load(str(tmp_path / run / "query_ids.npy")).astype(np.int64)
+        assert len(ids) == 100 and np.all(np.diff(ids) > 0)
+        assert np.array_equal(np.load(str(tmp_path / run / "indices.npy")).astype(np.uint32), idx[ids])
+        assert np.array_equal(np.load(str(tmp_path / run / "distances.npy")), dist[ids])
+        samples.append(ids)
+    assert np.array_equal(samples[0], samples[1])
+    for argv in (["--steps", "0"], ["--config", "5", "--dump-outputs", str(tmp_path)],
+                 ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+        with pytest.raises(SystemExit):
+            bench.parse()
+
+
 def test_synth_is_seeded():
     import numpy as np
     from soundsym_b200 import synth
