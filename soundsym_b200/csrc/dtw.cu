@@ -10,7 +10,7 @@
 //                     contraction on packed FFMA2 (fma.rn.f32x2); DP step = FMNMX3 + FADD. Every thread keeps its KP
 //                     best candidates in registers.
 //   2. k_dtw_merge    per query, merges the per-slice candidate lists.
-//   3. k_dtw_rescore  f64, direct (a-b)^2, unfused — the oracle's arithmetic — on the KP candidates only.
+//   3. k_dtw_rescore_warp  f64, direct (a-b)^2, unfused — the oracle's arithmetic — on the KP candidates only.
 //   4. k_dtw_finalize sorts by (distance, index), writes the top-k, and certifies that no pair outside the candidate
 //                     list could have entered it given the scan's error bound.
 #include <algorithm>
@@ -382,9 +382,11 @@ __global__ void k_dtw_merge(const unsigned long long* __restrict__ partial, uint
 namespace ss {
 int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, double eps,
                          const float* d_max_na, const float* d_max_nb, const float* d_slot_max_na, int bound_mode, uint8_t* d_uncert_flag,
-                         bool fill, uint32_t* d_out_idx, double* d_out_dist);
-int dtw_tc_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist, bool* used);
-int dtw_h2_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist, bool* used, int kp_override = 0);
+                         uint32_t* d_out_idx, double* d_out_dist);
+bool dtw_tc_applies(const ss_dict* d, const ss_queries* q);
+int dtw_tc_match_dev(ss_dict* d, ss_queries* q, int k, bool timed, uint32_t* d_out_idx, double* d_out_dist);
+bool dtw_h2_applies(const ss_dict* d, const ss_queries* q);
+int dtw_h2_match_dev(ss_dict* d, ss_queries* q, int k, bool wide, bool second_chance, bool timed, uint32_t* d_out_idx, double* d_out_dist);
 int dtw_exhaustive_match(ss_dict* d, ss_queries* q, int k, const std::vector<uint32_t>& subset, uint32_t* d_out_idx, double* d_out_dist);
 }
 
@@ -451,19 +453,14 @@ int dtw_dict_build(ss_dict* d) {
     return SS_OK;
 }
 
-int dtw_queries_build(ss_queries* q, const std::vector<uint32_t>* subset) {
+int dtw_queries_build(ss_queries* q) {
     ss_ctx* ctx = q->ctx;
-    if (q->lane_built && !subset) return SS_OK;
+    if (q->lane_built) return SS_OK;
     // sort query ids by length, longest first (heavy CTAs are scheduled first); zero-length queries get no lane
     std::vector<uint32_t> order;
     order.reserve(q->nq);
-    if (subset) {
-        for (uint32_t i : *subset)
-            if (q->h_off[i + 1] > q->h_off[i]) order.push_back(i);
-    } else {
-        for (size_t i = 0; i < q->nq; i++)
-            if (q->h_off[i + 1] > q->h_off[i]) order.push_back((uint32_t)i);
-    }
+    for (size_t i = 0; i < q->nq; i++)
+        if (q->h_off[i + 1] > q->h_off[i]) order.push_back((uint32_t)i);
     auto len_of = [&](uint32_t i) { return (uint32_t)(q->h_off[i + 1] - q->h_off[i]); };
     std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return len_of(x) > len_of(y); });
     std::vector<uint32_t> glen, gbase, gqid;
@@ -499,278 +496,41 @@ int dtw_queries_build(ss_queries* q, const std::vector<uint32_t>* subset) {
         SS_LAUNCHED(ctx);
     }
     // (the group tables are staged by cudaMemcpyAsync before it returns: no synchronisation needed for the host vectors)
-    q->lane_built = !subset;  // a subset layout is transient
+    q->lane_built = true;
     return SS_OK;
 }
 
-template <int RB, int KP>
-static int launch_scan(ss_ctx* ctx, const ScanParams& p, uint32_t grid) {
-    SS_CUDA(ctx, cudaFuncSetAttribute(k_dtw_scan<RB, KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, kScanSmemBytes));
-    k_dtw_scan<RB, KP><<<grid, kWarpsPerCta * 32, kScanSmemBytes, ctx->stream>>>(p);
+constexpr int kScanRB = 4;     // query rows per pass of k_dtw_scan (DESIGN.md §3.1c)
+constexpr int kScanWaves = 8;  // the fp32 scan's grid: about this many waves at 4 CTAs / SM
+
+template <int KP>
+static int launch_scan_merge(ss_dict* d, const ScanParams& p, uint32_t grid, uint32_t nslots, bool timed) {
+    ss_ctx* ctx = d->ctx;
+    if (timed) SS_CUDA(ctx, cudaEventRecord(d->ev_scan0, ctx->stream));
+    SS_CUDA(ctx, cudaFuncSetAttribute(k_dtw_scan<kScanRB, KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, kScanSmemBytes));
+    k_dtw_scan<kScanRB, KP><<<grid, kWarpsPerCta * 32, kScanSmemBytes, ctx->stream>>>(p);
+    SS_LAUNCHED(ctx);
+    if (timed) {
+        SS_CUDA(ctx, cudaEventRecord(d->ev_scan1, ctx->stream));
+        d->scan_timed = true;
+    }
+    k_dtw_merge<KP><<<ceil_div(nslots, 128), 128, 0, ctx->stream>>>(d->d_partial.p, p.nslices, nslots, d->d_cand_idx.p, d->d_cand_adist.p);
     SS_LAUNCHED(ctx);
     return SS_OK;
 }
 
-
-static int dtw_fp32_match(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist, const std::vector<uint32_t>* subset);
-
-// Sequences of more than 32 frames have no cheap second filter (the fp32-DP tensor-core scan stops at 32 frames, the CUDA-core
-// scan of ONE long query is a single warp's serial walk: 16 ms at config 5): below 2e8 cells the exhaustive stage is the
-// fastest way to finish (f64, measured 9e10 cells / s: 2 ms); a dozen such queries first take the second packed-half pass.
-static bool exhaustive_is_cheaper(const ss_dict* d, const ss_queries* q, const std::vector<uint32_t>& subset) {
-    if (d->max_len <= 32 && q->max_len <= 32) return false;
-    uint64_t rows = 0;
-    for (uint32_t i : subset) rows += q->h_off[i + 1] - q->h_off[i];
-    return rows * d->total_frames <= 200000000ull;
-}
-
-// which queries the last stage could not certify (synchronous; only called once the counter said there are some)
-static int uncertified_subset(ss_dict* d, ss_queries* q, std::vector<uint32_t>* subset) {
+// the fp32 CUDA-core scan of batch q, its f64 refine and certification (any sequence length)
+static int dtw_fp32_match(ss_dict* d, ss_queries* q, int k, bool timed, uint32_t* d_out_idx, double* d_out_dist) {
     ss_ctx* ctx = d->ctx;
-    subset->clear();
-    std::vector<uint8_t> flags(q->nq);
-    SS_CUDA(ctx, cudaMemcpyAsync(flags.data(), q->d_uncert_flag.p, q->nq, cudaMemcpyDeviceToHost, ctx->stream));
-    SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    for (size_t i = 0; i < q->nq; i++)
-        if (flags[i]) subset->push_back((uint32_t)i);
-    return SS_OK;
-}
-
-// the uncertified count of the stage that just ran travels to pinned host memory behind it; ev_done marks its arrival
-static int post_counters(ss_dict* d) {
-    ss_ctx* ctx = d->ctx;
-    if (!d->h_counters) {
-        if (!ctx->pinned_free.empty()) {  // (a block a destroyed dictionary of this ctx handed back)
-            d->h_counters = static_cast<unsigned long long*>(ctx->pinned_free.back());
-            ctx->pinned_free.pop_back();
-        } else {
-            SS_CUDA(ctx, cudaHostAlloc((void**)&d->h_counters, 4 * sizeof(unsigned long long), cudaHostAllocDefault));
-        }
-        SS_CUDA(ctx, cudaEventCreateWithFlags(&d->ev_done, cudaEventDisableTiming));
-    }
-    SS_CUDA(ctx, d->d_counters.reserve(4));
-    SS_CUDA(ctx, cudaMemcpyAsync(d->h_counters, d->d_counters.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
-    SS_CUDA(ctx, cudaEventRecord(d->ev_done, ctx->stream));
-    return SS_OK;
-}
-
-// Three stages, each only for the queries the previous one could not certify:
-//   1. tensor-core scan (fp16 products)          dtw_h2.cu (packed-half DP) or dtw_tc.cu (fp32 DP)
-//                                                              bound: triangle inequality on the rounded frames
-//   2. fp32 scan                                 k_dtw_scan    bound: 4e-6 (max|a|^2 + max|b|^2)
-//   3. exhaustive f64 DTW against every segment  exact.cu      exact by construction
-// Stage 3 only triggers when more than KP segments are closer to each other than the fp32 scan can resolve (e.g. many
-// near-identical dictionary entries); it guarantees that what ss_dict_match returns is THE f64 top-k.
-//
-// dtw_match_dev enqueues the first applicable stage and returns without a host round trip: the whole step (layout kernel,
-// scan, merge, refine) is in the stream before the GPU has started on it. Whether a later stage is needed is only known
-// once the refine has run; dtw_match_finish waits for that (one event), and runs stages 2 / 3 synchronously for the few
-// queries concerned. Every reader of the results or of the last_* counters goes through dtw_match_finish first.
-int dtw_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist) {
-    ss_ctx* ctx = d->ctx;
-    if (k < 1 || k > SS_MAX_TOPK) return set_error(ctx, SS_ERR_INVALID, "k must be in 1..%d (got %d)", SS_MAX_TOPK, k);
-    SS_TRY(dtw_match_finish(d));  // the previous match shares this dictionary's workspaces
-    SS_CUDA(ctx, q->d_uncert_flag.reserve(std::max<size_t>(q->nq, 1)));
-    SS_CUDA(ctx, cudaMemsetAsync(q->d_uncert_flag.p, 0, std::max<size_t>(q->nq, 1), ctx->stream));
-    d->last_tc_fallback = 0;
-    d->last_exhaustive = 0;
-    d->last_uncertified = 0;
-    bool used = false;
-    SS_TRY(dtw_h2_match_dev(d, q, k, d_out_idx, d_out_dist, &used));                 // packed-half tensor-core scan
-    d->pending.h2 = used;
-    d->last_scan_kind = used ? 1 : 0;
-    if (!used) {
-        SS_TRY(dtw_tc_match_dev(d, q, k, d_out_idx, d_out_dist, &used));  // fp32-DP tensor-core scan
-        d->last_scan_kind = used ? 2 : 3;
-    }
-    if (!used) SS_TRY(dtw_fp32_match(d, q, k, d_out_idx, d_out_dist, nullptr));
-    SS_TRY(post_counters(d));
-    d->pending.active = true;
-    d->pending.stage = used ? 1 : 2;
-    d->pending.q = q;
-    d->pending.k = k;
-    d->pending.d_out_idx = d_out_idx;
-    d->pending.d_out_dist = d_out_dist;
-    return SS_OK;
-}
-
-// ---- re-running a few queries through the slower stages -------------------------------------------------------------------
-// The queries a first stage could not certify are gathered (on the device) into a small batch of their own, which then runs
-// the remaining stages - fp32-DP tensor-core scan, fp32 CUDA-core scan, exhaustive f64 - synchronously; their rows are
-// scattered back into the caller's result arrays. At config 4 this is ~50 of the 10 000 queries: one group of 128 for the
-// fp32-DP tensor-core scan (~0.6 ms) instead of a CUDA-core scan of the whole dictionary for them (~43 ms).
-__global__ void k_gather_query_rows(const double* __restrict__ src, const uint64_t* __restrict__ src_off, const uint32_t* __restrict__ ids,
-                                    const uint64_t* __restrict__ dst_off, int c, double* __restrict__ dst) {
-    const uint32_t i = blockIdx.x;
-    const double* from = src + src_off[ids[i]] * c;
-    double* to = dst + dst_off[i] * c;
-    const size_t n = (size_t)(dst_off[i + 1] - dst_off[i]) * c;
-    for (size_t e = threadIdx.x; e < n; e += blockDim.x) to[e] = from[e];
-}
-__global__ void k_scatter_topk(const uint32_t* __restrict__ sub_idx, const double* __restrict__ sub_dist, const uint32_t* __restrict__ ids, uint32_t nsub,
-                               int k, uint32_t* __restrict__ out_idx, double* __restrict__ out_dist) {
-    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= nsub * (uint32_t)k) return;
-    const uint32_t i = t / (uint32_t)k, s = t % (uint32_t)k;
-    out_idx[(size_t)ids[i] * k + s] = sub_idx[t];
-    out_dist[(size_t)ids[i] * k + s] = sub_dist[t];
-}
-
-// stages 1b (fp32-DP tensor-core scan, if it applies), 2 and 3 on a whole batch, synchronously; results are exact on return
-static int dtw_match_remaining_stages(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist, uint64_t* n_exhaustive,
-                                      bool allow_h2) {
-    ss_ctx* ctx = d->ctx;
-    SS_CUDA(ctx, q->d_uncert_flag.reserve(std::max<size_t>(q->nq, 1)));
-    SS_CUDA(ctx, cudaMemsetAsync(q->d_uncert_flag.p, 0, std::max<size_t>(q->nq, 1), ctx->stream));
-    bool used = false, h2_ran = false;
-    std::vector<uint32_t> subset;
-    TraceTimer tt(ctx);
-    // 1a'. the packed-half scan once more with 32 candidates per query: the queries that reach this point had more than 8
-    // segments inside the filter's margin; almost all of them have fewer than 32 (one group of 128 lanes: ~0.1 - 0.5 ms)
-    if (allow_h2) {
-        SS_TRY(dtw_h2_match_dev(d, q, k, d_out_idx, d_out_dist, &used, 32));
-        if (used) {
-            SS_TRY(post_counters(d));
-            SS_CUDA(ctx, cudaEventSynchronize(d->ev_done));
-            tt.lap("  packed-half stage, 32 candidates");
-            if (dtw_trace()) fprintf(stderr, "[ss dtw trace]   -> %llu of %zu still uncertified\n", d->h_counters[0], q->nq);
-            if (!d->h_counters[0]) return SS_OK;
-            h2_ran = true;
-            used = false;
-        }
-    }
-    SS_TRY(dtw_tc_match_dev(d, q, k, d_out_idx, d_out_dist, &used));
-    if (used) {
-        SS_TRY(post_counters(d));
-        SS_CUDA(ctx, cudaEventSynchronize(d->ev_done));
-        tt.lap("  fp32-DP tensor-core stage");
-        if (dtw_trace()) fprintf(stderr, "[ss dtw trace]   -> %llu of %zu still uncertified\n", d->h_counters[0], q->nq);
-        if (!d->h_counters[0]) return SS_OK;
-        SS_TRY(uncertified_subset(d, q, &subset));
-        SS_TRY(dtw_fp32_match(d, q, k, d_out_idx, d_out_dist, &subset));
-    } else {
-        if (h2_ran) {  // what the second packed-half pass left
-            SS_TRY(uncertified_subset(d, q, &subset));
-            if (exhaustive_is_cheaper(d, q, subset)) {
-                *n_exhaustive += subset.size();
-                return dtw_exhaustive_match(d, q, k, subset, d_out_idx, d_out_dist);
-            }
-        }
-        SS_TRY(dtw_fp32_match(d, q, k, d_out_idx, d_out_dist, h2_ran ? &subset : nullptr));
-    }
-    SS_TRY(post_counters(d));
-    SS_CUDA(ctx, cudaEventSynchronize(d->ev_done));
-    tt.lap("  fp32 CUDA-core stage");
-    if (dtw_trace()) fprintf(stderr, "[ss dtw trace]   -> %llu still uncertified\n", d->h_counters[0]);
-    if (!d->h_counters[0]) return SS_OK;
-    SS_TRY(uncertified_subset(d, q, &subset));
-    *n_exhaustive += subset.size();
-    return dtw_exhaustive_match(d, q, k, subset, d_out_idx, d_out_dist);
-}
-
-static int dtw_rerun_subset(ss_dict* d, ss_queries* q, int k, const std::vector<uint32_t>& subset, uint32_t* d_out_idx, double* d_out_dist) {
-    ss_ctx* ctx = d->ctx;
-    TraceTimer tt(ctx);
-    if (!d->sub_q) {
-        d->sub_q = new (std::nothrow) ss_queries();
-        if (!d->sub_q) return set_error(ctx, SS_ERR_NOMEM, "out of host memory");
-        d->sub_q->ctx = ctx;
-        d->sub_q->c = d->c;
-    }
-    ss_queries* sub = d->sub_q;
-    const size_t ns = subset.size();
-    std::vector<uint64_t> off(ns + 1, 0);
-    for (size_t i = 0; i < ns; i++) off[i + 1] = off[i] + (q->h_off[subset[i] + 1] - q->h_off[subset[i]]);
-    SS_TRY(queries_prepare(sub, off.data(), ns));
-    SS_TRY(upload(ctx, sub->d_off, sub->h_off.data(), ns + 1));
-    SS_TRY(upload(ctx, d->d_sub_ids, subset.data(), ns));
-    SS_CUDA(ctx, sub->d_mfcc.reserve(std::max<size_t>((size_t)sub->total_frames * sub->c, 1)));
-    k_gather_query_rows<<<(unsigned)ns, 128, 0, ctx->stream>>>(q->d_mfcc.p, q->d_off.p, d->d_sub_ids.p, sub->d_off.p, q->c, sub->d_mfcc.p);
-    SS_LAUNCHED(ctx);
-    SS_TRY(dtw_tc_queries_group(sub));
-    tt.lap("rerun: gather + group");
-    SS_CUDA(ctx, d->d_sub_idx.reserve(ns * (size_t)k));
-    SS_CUDA(ctx, d->d_sub_dist.reserve(ns * (size_t)k));
-    const uint64_t work = d->last_work;  // the stages below account their own (partial) work: keep the whole match's figure
-    // (a second packed-half pass with 32 candidates certifies all of them too, but measured slower than going straight to the
-    // fp32-DP tensor-core scan: 1.95 vs 1.52 ms for the 47 queries of config 4 - one group of 128 lanes padded to 32 rows)
-    // Sequences of more than 32 frames have no fp32-DP tensor-core scan: there the second packed-half pass (32 per-pair
-    // lower-bound keys per query) stands between the first pass and the CUDA-core scan.
-    const bool long_seqs = d->max_len > 32 || sub->max_len > 32;
-    SS_TRY(dtw_match_remaining_stages(d, sub, k, d->d_sub_idx.p, d->d_sub_dist.p, &d->last_exhaustive, /*allow_h2=*/long_seqs));
-    d->last_work = work;
-    tt.lap("rerun: remaining stages");
-    k_scatter_topk<<<ceil_div((long long)ns * k, 128), 128, 0, ctx->stream>>>(d->d_sub_idx.p, d->d_sub_dist.p, d->d_sub_ids.p, (uint32_t)ns, k, d_out_idx,
-                                                                              d_out_dist);
-    SS_LAUNCHED(ctx);
-    SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return SS_OK;
-}
-
-int dtw_match_finish(ss_dict* d) {
-    if (!d->pending.active) return SS_OK;
-    ss_ctx* ctx = d->ctx;
-    d->pending.active = false;
-    ss_queries* q = d->pending.q;
-    const int k = d->pending.k;
-    TraceTimer tt(ctx);
-    SS_CUDA(ctx, cudaEventSynchronize(d->ev_done));
-    tt.lap("first stage (wait)");
-    unsigned long long n_unc = d->h_counters[0];
-    std::vector<uint32_t> subset;
-    struct Guard {  // the stages below are fallbacks: they do not touch the first stage's scan-time events
-        ss_dict* d;
-        explicit Guard(ss_dict* dd) : d(dd) { d->in_fallback = true; }
-        ~Guard() { d->in_fallback = false; }
-    } guard(d);
-    if (d->pending.stage == 1 && n_unc) {
-        SS_TRY(uncertified_subset(d, q, &subset));
-        d->last_tc_fallback = subset.size();
-        if (exhaustive_is_cheaper(d, q, subset)) {
-            // a handful of long queries: the f64 DTW against every segment, one warp per pair, costs less than any further filter
-            // pass (a scan's CTA walks all rows of a group of 128 lanes whatever the number of live queries)
-            d->last_exhaustive += subset.size();
-            SS_TRY(dtw_exhaustive_match(d, q, k, subset, d->pending.d_out_idx, d->pending.d_out_dist));
-            tt.lap("exhaustive f64 (few long queries)");
-            n_unc = 0;
-        } else if (d->pending.h2) {
-            // the packed-half filter leaves a fraction of a percent of the queries: a small batch of their own
-            SS_TRY(dtw_rerun_subset(d, q, k, subset, d->pending.d_out_idx, d->pending.d_out_dist));
-            n_unc = 0;
-        } else {
-            SS_TRY(dtw_fp32_match(d, q, k, d->pending.d_out_idx, d->pending.d_out_dist, &subset));
-            SS_TRY(post_counters(d));
-            SS_CUDA(ctx, cudaEventSynchronize(d->ev_done));
-            n_unc = d->h_counters[0];
-        }
-    }
-    if (n_unc) {
-        SS_TRY(uncertified_subset(d, q, &subset));
-        d->last_exhaustive += subset.size();
-        SS_TRY(dtw_exhaustive_match(d, q, k, subset, d->pending.d_out_idx, d->pending.d_out_dist));
-        n_unc = 0;  // everything is exact now
-    }
-    d->last_uncertified = n_unc;
-    return SS_OK;
-}
-
-static int dtw_fp32_match(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist, const std::vector<uint32_t>* subset) {
-    ss_ctx* ctx = d->ctx;
-    SS_TRY(dtw_queries_build(q, subset));
+    SS_TRY(dtw_queries_build(q));
     const int kp = k <= 2 ? 4 : (k <= 6 ? 8 : 16);  // candidates kept per query by the scan
     const uint32_t nslots = q->ngroups * 32;
-    d->last_work = d->total_frames * q->total_frames;
-    d->last_uncertified = 0;
 
     // ---- slices: contiguous tile ranges starting at segment boundaries, balanced by frames ------------------------
     const uint32_t nqb = (q->ngroups + kWarpsPerCta - 1) / kWarpsPerCta;
     uint32_t nslices = 1;
     if (nqb && d->ntiles) {
-        static const int waves = [] {  // (initialised once, thread-safe)
-            const char* e = getenv("SS_DTW_WAVES");
-            return e ? std::max(1, atoi(e)) : 8;
-        }();
-        const uint32_t target_ctas = (uint32_t)ctx->sm_count * 4 * waves;  // ~`waves` waves at 4 CTAs / SM
+        const uint32_t target_ctas = (uint32_t)ctx->sm_count * 4 * kScanWaves;
         nslices = std::max<uint32_t>(1, std::min<uint32_t>(d->ntiles, (target_ctas + nqb - 1) / nqb));
     }
     std::vector<uint32_t>& st = d->h_slice_tile;
@@ -793,11 +553,6 @@ static int dtw_fp32_match(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx,
     SS_CUDA(ctx, d->d_cand_adist.reserve(std::max<size_t>((size_t)nslots * kp, 1)));
 
     if (nqb) {
-        static const int g_scan_rb = [] {  // rows per pass; tools may override through SS_DTW_RB (read once, thread-safe)
-            const char* e = getenv("SS_DTW_RB");
-            const int v = e ? atoi(e) : 4;
-            return (v == 1 || v == 2) ? v : 4;
-        }();
         const uint32_t grid = nqb * nslices;
         ScanParams p;
         p.qlane = q->d_lane.p;
@@ -821,32 +576,235 @@ static int dtw_fp32_match(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx,
             SS_CUDA(ctx, cudaEventCreate(&d->ev_scan0));
             SS_CUDA(ctx, cudaEventCreate(&d->ev_scan1));
         }
-#define SS_SCAN_CASE(RBV, KPV)                                       \
-    if (g_scan_rb == RBV && kp == KPV) {                              \
-        if (!d->in_fallback) SS_CUDA(ctx, cudaEventRecord(d->ev_scan0, ctx->stream)); \
-        SS_TRY((launch_scan<RBV, KPV>(ctx, p, grid)));                \
-        if (!d->in_fallback) {                                        \
-            SS_CUDA(ctx, cudaEventRecord(d->ev_scan1, ctx->stream));  \
-            d->scan_timed = true;                                     \
-        }                                                             \
-        k_dtw_merge<KPV><<<ceil_div(nslots, 128), 128, 0, ctx->stream>>>(d->d_partial.p, nslices, nslots, d->d_cand_idx.p, \
-                                                                        d->d_cand_adist.p);                                \
-        SS_LAUNCHED(ctx);                                             \
-    }
-        SS_SCAN_CASE(1, 4)
-        SS_SCAN_CASE(2, 4)
-        SS_SCAN_CASE(4, 4)
-        SS_SCAN_CASE(4, 8)
-        SS_SCAN_CASE(4, 16)
-        SS_SCAN_CASE(2, 8)
-        SS_SCAN_CASE(2, 16)
-        SS_SCAN_CASE(1, 8)
-        SS_SCAN_CASE(1, 16)
-#undef SS_SCAN_CASE
+        if (kp == 4) SS_TRY(launch_scan_merge<4>(d, p, grid, nslots, timed));
+        else if (kp == 8) SS_TRY(launch_scan_merge<8>(d, p, grid, nslots, timed));
+        else SS_TRY(launch_scan_merge<16>(d, p, grid, nslots, timed));
     }
     // fp32 scan: |error| of a normalised distance <= 4e-6 (max|a|^2 + max|b|^2)  (14 roundings of 2^-24 on terms <= 2(|a|^2+|b|^2))
     return dtw_rescore_finalize(d, q, k, kp, nslots, q->d_group_qid.p, 4e-6, q->d_max_norm.p, d->d_max_norm.p, nullptr, 0, q->d_uncert_flag.p,
-                                /*fill=*/subset == nullptr, d_out_idx, d_out_dist);
+                                d_out_idx, d_out_dist);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// the stage cascade
+// ---------------------------------------------------------------------------------------------------------------
+// Each stage only runs for the queries the previous one could not certify; its bound decides which:
+//   H2          packed-half tensor-core scan + second chance   dtw_h2.cu   bound: triangle inequality on the rounded frames
+//   H2_WIDE     the same scan with 32 candidates per query      dtw_h2.cu
+//   TC          fp32-DP tensor-core scan (<= 32 x <= 32 frames) dtw_tc.cu   bound: as H2
+//   FP32        fp32 CUDA-core scan (any length)                k_dtw_scan  bound: 4e-6 (max|a|^2 + max|b|^2)
+//   EXHAUSTIVE  f64 DTW against every segment                   exact.cu    exact by construction
+// EXHAUSTIVE only triggers when more than KP segments are closer to each other than the scans can resolve (e.g. many
+// near-identical dictionary entries); it guarantees that what ss_dict_match returns is THE f64 top-k.
+//
+// dtw_match_dev enqueues the first stage and returns without a host round trip: the whole step (layout kernel, scan, merge,
+// refine) is in the stream before the GPU has started on it. Whether a later stage is needed is only known once the refine
+// has run; dtw_match_finish waits for that (one event) and runs the later stages synchronously for the few queries
+// concerned. Every reader of the results or of the last_* counters goes through dtw_match_finish first.
+
+static const char* stage_name(DtwStage s) {
+    static const char* const names[] = {"packed-half", "packed-half, 32 candidates", "fp32-DP tensor-core", "fp32 CUDA-core", "exhaustive f64"};
+    return names[(int)s];
+}
+
+// The first stage: the ss_dict_set_scan preference, then what applies to the shapes
+static DtwStage first_stage(const ss_dict* d, const ss_queries* q) {
+    if ((d->scan_pref == 0 || d->scan_pref == 3) && dtw_h2_applies(d, q)) return DtwStage::H2;
+    if (d->scan_pref != 2 && dtw_tc_applies(d, q)) return DtwStage::TC;
+    return DtwStage::FP32;
+}
+
+// Whether later stage s applies to the uncertified queries (gathered into sub) after stage prev ran. H2_WIDE is only ever
+// tried right after H2, and it replaces TC: it is for sequences of more than 32 frames, which TC does not take.
+static bool later_stage_applies(const ss_dict* d, const ss_queries* sub, DtwStage prev, DtwStage s) {
+    if (s == DtwStage::H2_WIDE) return dtw_h2_applies(d, sub) && (d->max_len > 32 || sub->max_len > 32);
+    if (s == DtwStage::TC) return prev != DtwStage::H2_WIDE && dtw_tc_applies(d, sub);
+    return true;
+}
+
+// runs one filter stage on batch q: scan, merge, f64 refine, certification (q->d_uncert_flag, d_counters[0]); only the
+// first stage of a match records the scan-time events
+static int run_stage(ss_dict* d, ss_queries* q, int k, DtwStage s, bool timed, uint32_t* d_out_idx, double* d_out_dist) {
+    const bool second_chance = d->scan_pref != 3;
+    switch (s) {
+    case DtwStage::H2: return dtw_h2_match_dev(d, q, k, /*wide=*/false, second_chance, timed, d_out_idx, d_out_dist);
+    case DtwStage::H2_WIDE: return dtw_h2_match_dev(d, q, k, /*wide=*/true, second_chance, timed, d_out_idx, d_out_dist);
+    case DtwStage::TC: return dtw_tc_match_dev(d, q, k, timed, d_out_idx, d_out_dist);
+    default: return dtw_fp32_match(d, q, k, timed, d_out_idx, d_out_dist);
+    }
+}
+
+// Sequences of more than 32 frames have no cheap second filter (the fp32-DP tensor-core scan stops at 32 frames, the CUDA-core
+// scan of ONE long query is a single warp's serial walk: 16 ms at config 5): below 2e8 cells the exhaustive stage is the
+// fastest way to finish (f64, measured 9e10 cells / s: 2 ms); a dozen such queries first take the wide packed-half pass.
+// ran_max_len: the longest query of the batch the last stage ran on; u: the uncertified queries of q.
+static bool exhaustive_is_cheaper(const ss_dict* d, uint32_t ran_max_len, const ss_queries* q, const std::vector<uint32_t>& u) {
+    if (d->max_len <= 32 && ran_max_len <= 32) return false;
+    uint64_t rows = 0;
+    for (uint32_t i : u) rows += q->h_off[i + 1] - q->h_off[i];
+    return rows * d->total_frames <= 200000000ull;
+}
+
+// the uncertified count of the stage that just ran travels to pinned host memory behind it; ev_done marks its arrival
+static int post_counters(ss_dict* d) {
+    ss_ctx* ctx = d->ctx;
+    if (!d->h_counters) {
+        if (!ctx->pinned_free.empty()) {  // (a block a destroyed dictionary of this ctx handed back)
+            d->h_counters = static_cast<unsigned long long*>(ctx->pinned_free.back());
+            ctx->pinned_free.pop_back();
+        } else {
+            SS_CUDA(ctx, cudaHostAlloc((void**)&d->h_counters, 4 * sizeof(unsigned long long), cudaHostAllocDefault));
+        }
+        SS_CUDA(ctx, cudaEventCreateWithFlags(&d->ev_done, cudaEventDisableTiming));
+    }
+    SS_CUDA(ctx, d->d_counters.reserve(4));
+    SS_CUDA(ctx, cudaMemcpyAsync(d->h_counters, d->d_counters.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    SS_CUDA(ctx, cudaEventRecord(d->ev_done, ctx->stream));
+    return SS_OK;
+}
+
+// The queries batch `ran` could not certify, as ids of the caller's batch: ids[i] for query i of `ran` (i itself when ids
+// is null). Called once ev_done has been reached; synchronous when there are any.
+static int read_uncertified(ss_dict* d, const ss_queries* ran, const std::vector<uint32_t>* ids, std::vector<uint32_t>* out) {
+    ss_ctx* ctx = d->ctx;
+    std::vector<uint32_t> u;
+    if (d->h_counters[0]) {
+        std::vector<uint8_t> flags(ran->nq);
+        SS_CUDA(ctx, cudaMemcpyAsync(flags.data(), ran->d_uncert_flag.p, ran->nq, cudaMemcpyDeviceToHost, ctx->stream));
+        SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        for (size_t i = 0; i < ran->nq; i++)
+            if (flags[i]) u.push_back(ids ? (*ids)[i] : (uint32_t)i);
+    }
+    out->swap(u);
+    return SS_OK;
+}
+
+int dtw_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist) {
+    ss_ctx* ctx = d->ctx;
+    if (k < 1 || k > SS_MAX_TOPK) return set_error(ctx, SS_ERR_INVALID, "k must be in 1..%d (got %d)", SS_MAX_TOPK, k);
+    SS_TRY(dtw_match_finish(d));  // the previous match shares this dictionary's workspaces
+    SS_CUDA(ctx, q->d_uncert_flag.reserve(std::max<size_t>(q->nq, 1)));
+    SS_CUDA(ctx, cudaMemsetAsync(q->d_uncert_flag.p, 0, std::max<size_t>(q->nq, 1), ctx->stream));
+    const DtwStage first = first_stage(d, q);
+    d->last_scan_kind = first == DtwStage::H2 ? 1 : (first == DtwStage::TC ? 2 : 3);
+    d->last_work = d->total_frames * q->total_frames;
+    d->last_tc_fallback = 0;
+    d->last_exhaustive = 0;
+    d->last_uncertified = q->nq;  // no row is final before dtw_match_finish
+    SS_TRY(run_stage(d, q, k, first, /*timed=*/true, d_out_idx, d_out_dist));
+    SS_TRY(post_counters(d));
+    d->pending.active = true;
+    d->pending.first = first;
+    d->pending.q = q;
+    d->pending.k = k;
+    d->pending.d_out_idx = d_out_idx;
+    d->pending.d_out_dist = d_out_dist;
+    return SS_OK;
+}
+
+// ---- running a few queries through the later stages -----------------------------------------------------------------------
+// The queries a stage could not certify are gathered (on the device) into a small batch of their own for the next stage;
+// their rows are scattered back into the caller's result arrays. At config 4 without the second chance this is ~50 of the
+// 10 000 queries: one group of 128 for the fp32-DP tensor-core scan (~0.6 ms) instead of a scan of the whole batch.
+__global__ void k_gather_query_rows(const double* __restrict__ src, const uint64_t* __restrict__ src_off, const uint32_t* __restrict__ ids,
+                                    const uint64_t* __restrict__ dst_off, int c, double* __restrict__ dst) {
+    const uint32_t i = blockIdx.x;
+    const double* from = src + src_off[ids[i]] * c;
+    double* to = dst + dst_off[i] * c;
+    const size_t n = (size_t)(dst_off[i + 1] - dst_off[i]) * c;
+    for (size_t e = threadIdx.x; e < n; e += blockDim.x) to[e] = from[e];
+}
+__global__ void k_scatter_topk(const uint32_t* __restrict__ sub_idx, const double* __restrict__ sub_dist, const uint32_t* __restrict__ ids, uint32_t nsub,
+                               int k, uint32_t* __restrict__ out_idx, double* __restrict__ out_dist) {
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= nsub * (uint32_t)k) return;
+    const uint32_t i = t / (uint32_t)k, s = t % (uint32_t)k;
+    out_idx[(size_t)ids[i] * k + s] = sub_idx[t];
+    out_dist[(size_t)ids[i] * k + s] = sub_dist[t];
+}
+
+// queries `ids` of q -> the dictionary's sub-batch d->sub_q (refilled: no layout of its previous contents is kept), ids in
+// d_sub_ids, room for its results in d_sub_idx / d_sub_dist
+static int gather_queries(ss_dict* d, ss_queries* q, const std::vector<uint32_t>& ids, int k) {
+    ss_ctx* ctx = d->ctx;
+    if (!d->sub_q) {
+        d->sub_q = new (std::nothrow) ss_queries();
+        if (!d->sub_q) return set_error(ctx, SS_ERR_NOMEM, "out of host memory");
+        d->sub_q->ctx = ctx;
+        d->sub_q->c = d->c;
+    }
+    ss_queries* sub = d->sub_q;
+    const size_t ns = ids.size();
+    std::vector<uint64_t> off(ns + 1, 0);
+    for (size_t i = 0; i < ns; i++) off[i + 1] = off[i] + (q->h_off[ids[i] + 1] - q->h_off[ids[i]]);
+    SS_TRY(queries_prepare(sub, off.data(), ns));
+    SS_TRY(upload(ctx, sub->d_off, sub->h_off.data(), ns + 1));
+    SS_TRY(upload(ctx, d->d_sub_ids, ids.data(), ns));
+    SS_CUDA(ctx, sub->d_mfcc.reserve(std::max<size_t>((size_t)sub->total_frames * sub->c, 1)));
+    k_gather_query_rows<<<(unsigned)ns, 128, 0, ctx->stream>>>(q->d_mfcc.p, q->d_off.p, d->d_sub_ids.p, sub->d_off.p, q->c, sub->d_mfcc.p);
+    SS_LAUNCHED(ctx);
+    SS_TRY(dtw_tc_queries_group(sub));
+    SS_CUDA(ctx, sub->d_uncert_flag.reserve(ns));
+    SS_CUDA(ctx, cudaMemsetAsync(sub->d_uncert_flag.p, 0, ns, ctx->stream));
+    SS_CUDA(ctx, d->d_sub_idx.reserve(ns * (size_t)k));
+    SS_CUDA(ctx, d->d_sub_dist.reserve(ns * (size_t)k));
+    return SS_OK;
+}
+
+// The later stages of the pending match. d->last_uncertified follows the number of queries whose rows are not final, so
+// that it is right also when a stage fails.
+static int run_later_stages(ss_dict* d) {
+    ss_ctx* ctx = d->ctx;
+    ss_queries* q = d->pending.q;
+    const int k = d->pending.k;
+    uint32_t* out_idx = d->pending.d_out_idx;
+    double* out_dist = d->pending.d_out_dist;
+    DtwStage s = d->pending.first;
+    uint32_t ran_max_len = q->max_len;
+    std::vector<uint32_t> u;  // the queries of q whose rows are not final
+    TraceTimer tt(ctx);
+    auto trace = [&](DtwStage st) {
+        tt.lap(stage_name(st));
+        if (dtw_trace()) fprintf(stderr, "[ss dtw trace]   -> %zu of %zu still uncertified\n", u.size(), q->nq);
+    };
+    SS_CUDA(ctx, cudaEventSynchronize(d->ev_done));
+    SS_TRY(read_uncertified(d, q, nullptr, &u));
+    trace(s);
+    d->last_uncertified = u.size();
+    if (s != DtwStage::FP32) d->last_tc_fallback = u.size();
+    while (!u.empty()) {
+        if (s == DtwStage::FP32 || exhaustive_is_cheaper(d, ran_max_len, q, u)) {
+            d->last_exhaustive += u.size();
+            SS_TRY(dtw_exhaustive_match(d, q, k, u, out_idx, out_dist));
+            u.clear();
+            trace(DtwStage::EXHAUSTIVE);
+            break;
+        }
+        SS_TRY(gather_queries(d, q, u, k));
+        ss_queries* sub = d->sub_q;
+        const DtwStage prev = s;
+        do s = (DtwStage)((int)s + 1);
+        while (!later_stage_applies(d, sub, prev, s));
+        SS_TRY(run_stage(d, sub, k, s, /*timed=*/false, d->d_sub_idx.p, d->d_sub_dist.p));
+        k_scatter_topk<<<ceil_div((long long)u.size() * k, 128), 128, 0, ctx->stream>>>(d->d_sub_idx.p, d->d_sub_dist.p, d->d_sub_ids.p,
+                                                                                      (uint32_t)u.size(), k, out_idx, out_dist);
+        SS_LAUNCHED(ctx);
+        SS_TRY(post_counters(d));
+        SS_CUDA(ctx, cudaEventSynchronize(d->ev_done));
+        SS_TRY(read_uncertified(d, sub, &u, &u));
+        ran_max_len = sub->max_len;
+        trace(s);
+        d->last_uncertified = u.size();
+    }
+    d->last_uncertified = 0;
+    return SS_OK;
+}
+
+int dtw_match_finish(ss_dict* d) {
+    if (!d->pending.active) return SS_OK;
+    const int rc = run_later_stages(d);
+    d->pending = ss_dict::Pending();  // (after a failure too: the next match can run, and last_uncertified is not 0)
+    return rc;
 }
 
 }  // namespace ss

@@ -38,7 +38,7 @@ namespace ss {
 
 int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, double eps,
                          const float* d_max_na, const float* d_max_nb, const float* d_slot_max_na, int bound_mode, uint8_t* d_uncert_flag,
-                         bool fill, uint32_t* d_out_idx, double* d_out_dist);
+                         uint32_t* d_out_idx, double* d_out_dist);
 
 int dtw_second_chance(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, const unsigned long long* d_partial,
                       uint32_t nlists, const unsigned long long* d_thr, double eps, const float* d_max_na, const float* d_max_nb,
@@ -1053,12 +1053,13 @@ struct H2Plan {
     size_t smem;
     bool use_long;  // segments or queries of more than 32 frames: k_dtw_scan_h2_long (strips, streamed A block, deflated keys)
 };
+constexpr int kH2Waves = 16;  // CTAs per SM over the launches of one scan
+// Candidates kept per query for k <= 2. Measured at config 4 (profiles/bench/r2_h2_kp_sweep.json): 8 leaves 47 of the 10 000
+// queries uncertified by the merged list, but the scan itself is 3 ms faster than with 16.
+constexpr int kH2Kp = 8;
+
 static int h2_plan(ss_dict* d, ss_queries* q, int kp, H2Plan* plan) {
     ss_ctx* ctx = d->ctx;
-    static const int waves = [] {
-        const char* e = getenv("SS_DTW_H2_WAVES");
-        return e ? std::max(1, atoi(e)) : 16;
-    }();
     const uint32_t nslots = q->tc_ngroups * kTcM;
     if (d->h2_slices.size() > 64 && !d->h2_slices.count(q->tc_ngroups)) {  // (many different batch sizes: start over)
         SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1067,9 +1068,9 @@ static int h2_plan(ss_dict* d, ss_queries* q, int kp, H2Plan* plan) {
     std::unique_ptr<ss_dict::H2Slices>& sl = d->h2_slices[q->tc_ngroups];
     if (!sl) {
         sl.reset(new ss_dict::H2Slices());
-        // about `waves` CTAs per SM, but never slices of fewer than ~12 tiles: a small batch (nq = 1: one group) would
+        // about kH2Waves CTAs per SM, but never slices of fewer than ~12 tiles: a small batch (nq = 1: one group) would
         // otherwise pay a CTA's fixed cost (TMEM allocation, the A-block copy, list merge) two thousand times
-        const uint32_t want = std::max<uint32_t>(1, std::min<uint32_t>(((uint32_t)ctx->sm_count * waves + q->tc_ngroups - 1) / q->tc_ngroups,
+        const uint32_t want = std::max<uint32_t>(1, std::min<uint32_t>(((uint32_t)ctx->sm_count * kH2Waves + q->tc_ngroups - 1) / q->tc_ngroups,
                                                                        std::max<uint32_t>((uint32_t)ctx->sm_count, d->h2_ntiles / 12)));
         std::vector<uint32_t> st;
         uint64_t total = 0;
@@ -1158,63 +1159,48 @@ static int h2_launch_all(ss_ctx* ctx, const H2Plan& plan) {
     return plan.use_long ? h2_launch_kinds<KP, DBG, true>(ctx, plan) : h2_launch_kinds<KP, DBG, false>(ctx, plan);
 }
 
-static bool h2_enabled() {
-    static const int enabled = [] {
-        const char* e = getenv("SS_DTW_H2");
-        return e ? atoi(e) : 1;
-    }();
-    return enabled != 0;
+// the packed-half scan takes segments and queries of at most kH2MaxLong frames
+bool dtw_h2_applies(const ss_dict* d, const ss_queries* q) {
+    return d->h2_ready && q->max_len <= (uint32_t)kH2MaxLong && q->total_frames > 0;
 }
 
-
-// kp_override > 0: candidates kept per query (the re-run of the queries a first pass could not certify uses 32)
-int dtw_h2_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist, bool* used, int kp_override) {
+// The scan of batch q (dtw_h2_applies), its f64 refine and certification. wide: 32 candidates per query whatever k (the re-run
+// of queries an earlier pass could not certify); second_chance: refine the union of the per-slice lists for the queries the
+// merged list leaves uncertified.
+int dtw_h2_match_dev(ss_dict* d, ss_queries* q, int k, bool wide, bool second_chance, bool timed, uint32_t* d_out_idx, double* d_out_dist) {
     ss_ctx* ctx = d->ctx;
-    *used = false;
-    if (!h2_enabled() || (d->scan_pref != 0 && d->scan_pref != 3) || !d->h2_ready || q->max_len > (uint32_t)kH2MaxLong || q->total_frames == 0) return SS_OK;
     TraceTimer tt(ctx);
     SS_TRY(h2_queries_build(d, q));
     tt.lap("  h2: query A blocks");
-    if (!q->tc_ngroups) return SS_OK;
     // k > 2: the k-th and the kp-th neighbour must be further apart than the filter's ~4 % margin: a longer list
-    // SS_DTW_H2_KP=8|16|32: candidates kept per query for k <= 2. Measured at config 4 (profiles/bench/r2_h2_kp_sweep.json): 8 leaves
-    // 47 of the 10 000 queries to the fallback (+1.5 ms for their re-run) but the scan itself is 3 ms faster than with 16.
-    static const int kp_small = [] {
-        const char* e = getenv("SS_DTW_H2_KP");
-        const int v = e ? atoi(e) : 8;
-        return v == 16 || v == 32 ? v : 8;
-    }();
-    const int kp = kp_override > 0 ? kp_override : (k <= 2 ? kp_small : 32);
-    d->last_work = d->total_frames * q->total_frames;
-    d->last_uncertified = 0;
+    const int kp = wide || k > 2 ? 32 : kH2Kp;
     H2Plan plan;
     SS_TRY(h2_plan(d, q, kp, &plan));
     tt.lap("  h2: plan (slices, workspaces)");
-    if (getenv("SS_DTW_H2_TIMELINE") && !plan.use_long) {
+    const char* timeline = timed && !plan.use_long ? getenv("SS_DTW_H2_TIMELINE") : nullptr;  // (set and unset between matches)
+    if (timeline) {
         const size_t n = (size_t)plan.p.ngroups * plan.p.nslices * 8;
         SS_CUDA(ctx, d->d_h2_timeline.reserve(n));
         SS_CUDA(ctx, cudaMemsetAsync(d->d_h2_timeline.p, 0, n * sizeof(unsigned long long), ctx->stream));
         plan.p.timeline = d->d_h2_timeline.p;
     }
-    if (!d->in_fallback) SS_CUDA(ctx, cudaEventRecord(d->ev_scan0, ctx->stream));
-    if (kp == 8) SS_TRY((h2_launch_all<8, false>(ctx, plan)));
-    else if (kp == 16) SS_TRY((h2_launch_all<16, false>(ctx, plan)));
+    if (timed) SS_CUDA(ctx, cudaEventRecord(d->ev_scan0, ctx->stream));
+    if (kp == kH2Kp) SS_TRY((h2_launch_all<kH2Kp, false>(ctx, plan)));
     else SS_TRY((h2_launch_all<32, false>(ctx, plan)));
-    if (!d->in_fallback) {  // a fallback re-run keeps the first pass's scan time
+    if (timed) {
         SS_CUDA(ctx, cudaEventRecord(d->ev_scan1, ctx->stream));
         d->scan_timed = true;
     }
-    if (kp == 8) k_tc_merge<8><<<ceil_div(plan.nslots, 8), 256, 0, ctx->stream>>>(d->d_tc_partial.p, plan.p.nslices, plan.nslots, d->d_cand_idx.p, d->d_cand_adist.p);
-    else if (kp == 16) k_tc_merge<16><<<ceil_div(plan.nslots, 8), 256, 0, ctx->stream>>>(d->d_tc_partial.p, plan.p.nslices, plan.nslots, d->d_cand_idx.p, d->d_cand_adist.p);
+    if (kp == kH2Kp) k_tc_merge<kH2Kp><<<ceil_div(plan.nslots, 8), 256, 0, ctx->stream>>>(d->d_tc_partial.p, plan.p.nslices, plan.nslots, d->d_cand_idx.p, d->d_cand_adist.p);
     else k_tc_merge<32><<<ceil_div(plan.nslots, 8), 256, 0, ctx->stream>>>(d->d_tc_partial.p, plan.p.nslices, plan.nslots, d->d_cand_idx.p, d->d_cand_adist.p);
     SS_LAUNCHED(ctx);
     tt.lap("  h2: scan + merge");
-    if (plan.p.timeline) {  // SS_DTW_H2_TIMELINE: one line per CTA (measurement only; synchronises)
+    if (timeline) {  // SS_DTW_H2_TIMELINE: one line per CTA (measurement only; synchronises)
         const size_t n = (size_t)plan.p.ngroups * plan.p.nslices;
         std::vector<unsigned long long> h(n * 8);
         SS_CUDA(ctx, cudaMemcpyAsync(h.data(), plan.p.timeline, n * 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
         SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        if (FILE* f = fopen(getenv("SS_DTW_H2_TIMELINE"), "w")) {
+        if (FILE* f = fopen(timeline, "w")) {
             fprintf(f, "# cta start_ns setup_ns dp_done_ns end_ns smid kind group L ntiles dp_cycles half_ns\n");
             for (size_t i = 0; i < n; i++)
                 fprintf(f, "%zu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu\n", i, h[i * 8], h[i * 8 + 1], h[i * 8 + 2], h[i * 8 + 3],
@@ -1227,30 +1213,24 @@ int dtw_h2_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, doub
     // bound_mode 3 (strip kernel): the keys are per-pair lower bounds already; eta and the longest segment go into the cap.
     d->h2_bound_inv_s = 1.0 / (double)d->h2_s;
     SS_TRY(dtw_rescore_finalize(d, q, k, kp, plan.nslots, q->d_tc_qid.p, h2_eta(d), q->d_tc_max_norm.p, d->d_tc_max_norm.p, q->d_tc_slot_max_na.p,
-                                plan.use_long ? 3 : 2, q->d_uncert_flag.p, /*fill=*/true, d_out_idx, d_out_dist));
+                                plan.use_long ? 3 : 2, q->d_uncert_flag.p, d_out_idx, d_out_dist));
     tt.lap("  h2: f64 refine + certification");
     // the queries the merged list could not certify: refine what the union of the per-slice lists still holds below the scan's
     // own insertion threshold, and certify against that threshold (exact.cu, k_dtw_second_chance)
-    static const bool second = [] {
-        const char* e = getenv("SS_DTW_SECOND_CHANCE");
-        return e ? atoi(e) != 0 : true;
-    }();
-    if (second && d->scan_pref != 3) {
+    if (second_chance) {
         SS_TRY(dtw_second_chance(d, q, k, kp, plan.nslots, q->d_tc_qid.p, d->d_tc_partial.p, plan.p.nslices, d->d_h2_thr.p, h2_eta(d), q->d_tc_max_norm.p,
                                  d->d_tc_max_norm.p, q->d_tc_slot_max_na.p, plan.use_long ? 3 : 2, q->d_uncert_flag.p, d_out_idx, d_out_dist));
         tt.lap("  h2: second chance (union of the slice lists)");
     }
-    *used = true;
     return SS_OK;
 }
 
 // ss_dict_debug_tc_scan's half-precision counterpart: the raw scan distance of every pair (see dtw_tc_debug_scan)
 int dtw_h2_debug_scan(ss_dict* d, ss_queries* q, float* d_out, std::vector<uint32_t>* slot_qid, double* mu16, float* scale, float* s_out) {
     ss_ctx* ctx = d->ctx;
-    if (!h2_enabled() || !d->h2_ready || q->max_len > (uint32_t)kH2MaxLong || q->total_frames == 0)
-        return set_error(ctx, SS_ERR_INVALID, "debug_h2_scan: the packed-half scan does not apply (segments / queries > %d frames, or disabled)", kH2MaxLong);
+    if (!dtw_h2_applies(d, q))
+        return set_error(ctx, SS_ERR_INVALID, "debug_h2_scan: the packed-half scan does not apply (segments / queries > %d frames, or no frame)", kH2MaxLong);
     SS_TRY(h2_queries_build(d, q));
-    if (!q->tc_ngroups) return set_error(ctx, SS_ERR_INVALID, "debug_h2_scan: no non-empty query");
     H2Plan plan;
     SS_TRY(h2_plan(d, q, 8, &plan));
     plan.p.dbg = d_out;

@@ -37,7 +37,7 @@ namespace ss {
 
 int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, double eps,
                          const float* d_max_na, const float* d_max_nb, const float* d_slot_max_na, int bound_mode, uint8_t* d_uncert_flag,
-                         bool fill, uint32_t* d_out_idx, double* d_out_dist);
+                         uint32_t* d_out_idx, double* d_out_dist);
 
 // ---------------------------------------------------------------------------------------------------------------
 // layout builders
@@ -656,15 +656,11 @@ int dtw_tc_dict_build(ss_dict* d) {
     // A tile has 4 slots of 32 columns. A segment longer than 16 frames takes a slot of its own; shorter ones share a slot
     // two by two (the second at column 16), so that the per-step hand-off is paid once for both. Per slot the descriptor is
     // {segment A, length A, segment B, length B}, B = -1 when absent.
-    static const int pairing = [] {  // read once, thread-safe (C++11 static initialisation)
-        const char* e = getenv("SS_DTW_TC_PAIR");
-        return e ? atoi(e) : 1;
-    }();
     std::vector<int4> desc;
     d->tc_first_pair_tile = 0xFFFFFFFFu;
     d->h_tc_tile_frames.clear();  // per tile: an instruction-count estimate of one pipeline step (slice balancing)
     for (size_t o = 0; o < order.size();) {
-        const bool pair = pairing && len_of(order[o]) <= kTcPairCol;
+        const bool pair = len_of(order[o]) <= kTcPairCol;
         const size_t take = std::min<size_t>(order.size() - o, pair ? 2 * kTcSlots : kTcSlots);
         uint32_t cost = 0;
         for (int sidx = 0; sidx < 4; sidx++) {
@@ -795,11 +791,12 @@ static int tc_launch_kind(ss_ctx* ctx, TcParams p, uint32_t slice_begin, uint32_
 }
 // slices [0, nsingle) hold single-segment tiles, [nsingle, nslices) paired ones
 template <int KP>
-static int tc_launch(ss_ctx* ctx, const TcParams& p, uint32_t nsingle, uint32_t nslices, size_t smem, uint32_t nlists, uint32_t nslots, ss_dict* d) {
-    if (!d->in_fallback) SS_CUDA(ctx, cudaEventRecord(d->ev_scan0, ctx->stream));
+static int tc_launch(ss_ctx* ctx, const TcParams& p, uint32_t nsingle, uint32_t nslices, size_t smem, uint32_t nlists, uint32_t nslots, ss_dict* d,
+                     bool timed) {
+    if (timed) SS_CUDA(ctx, cudaEventRecord(d->ev_scan0, ctx->stream));
     SS_TRY((tc_launch_kind<KP, false>(ctx, p, 0, nsingle, smem, false)));
     SS_TRY((tc_launch_kind<KP, true>(ctx, p, nsingle, nslices - nsingle, smem, nsingle != 0)));
-    if (!d->in_fallback) {  // the fallback stages of a match keep the first stage's scan time
+    if (timed) {
         SS_CUDA(ctx, cudaEventRecord(d->ev_scan1, ctx->stream));
         d->scan_timed = true;
     }
@@ -808,16 +805,10 @@ static int tc_launch(ss_ctx* ctx, const TcParams& p, uint32_t nsingle, uint32_t 
     return SS_OK;
 }
 
-static bool tc_enabled() {
-    static const int enabled = [] {
-        const char* e = getenv("SS_DTW_TC");
-        return e ? atoi(e) : 1;
-    }();
-    return enabled != 0;
-}
+constexpr int kTcWaves = 16;  // CTAs per SM over the two launches of one scan
 
 // slices (contiguous tile ranges of ONE kind - single-segment tiles come first, paired tiles after - balanced by the
-// tiles' step-cost estimate; about `waves` CTAs per SM over the two launches, 1 resident per SM), workspaces and the
+// tiles' step-cost estimate; about kTcWaves CTAs per SM over the two launches, 1 resident per SM), workspaces and the
 // kernel parameters of one scan of query batch q against dictionary d with candidate lists of kp entries
 struct TcPlan {
     TcParams p;
@@ -826,15 +817,11 @@ struct TcPlan {
 };
 static int tc_plan(ss_dict* d, ss_queries* q, int kp, TcPlan* plan) {
     ss_ctx* ctx = d->ctx;
-    static const int waves = [] {
-        const char* e = getenv("SS_DTW_TC_WAVES");
-        return e ? std::max(1, atoi(e)) : 16;
-    }();
     const uint32_t nslots = q->tc_ngroups * kTcM;
     if (d->slice_for_groups != q->tc_ngroups) {  // the slice table only depends on the dictionary and the number of query groups
-        // about `waves` CTAs per SM, but never slices of fewer than ~12 tiles: a small batch (nq = 1: one group) would
+        // about kTcWaves CTAs per SM, but never slices of fewer than ~12 tiles: a small batch (nq = 1: one group) would
         // otherwise pay a CTA's fixed cost (TMEM allocation, the A-block copy, list merge) two thousand times
-        const uint32_t want = std::max<uint32_t>(1, std::min<uint32_t>(((uint32_t)ctx->sm_count * waves + q->tc_ngroups - 1) / q->tc_ngroups,
+        const uint32_t want = std::max<uint32_t>(1, std::min<uint32_t>(((uint32_t)ctx->sm_count * kTcWaves + q->tc_ngroups - 1) / q->tc_ngroups,
                                                                        std::max<uint32_t>((uint32_t)ctx->sm_count, d->tc_ntiles / 12)));
         std::vector<uint32_t> st;  // (staged by cudaMemcpyAsync before it returns)
         uint64_t total = 0;
@@ -887,24 +874,23 @@ static int tc_plan(ss_dict* d, ss_queries* q, int kp, TcPlan* plan) {
     return SS_OK;
 }
 
-int dtw_tc_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist, bool* used) {
+// the fp32-DP tensor-core scan takes segments and queries of at most kTcMaxLen frames
+bool dtw_tc_applies(const ss_dict* d, const ss_queries* q) {
+    return d->tc_ready && q->max_len <= (uint32_t)kTcMaxLen && q->total_frames > 0;
+}
+
+// the scan of batch q (dtw_tc_applies), its f64 refine and certification
+int dtw_tc_match_dev(ss_dict* d, ss_queries* q, int k, bool timed, uint32_t* d_out_idx, double* d_out_dist) {
     ss_ctx* ctx = d->ctx;
-    *used = false;
-    if (!tc_enabled() || d->scan_pref == 2 || !d->tc_ready || q->max_len > (uint32_t)kTcMaxLen || q->total_frames == 0) return SS_OK;
     SS_TRY(tc_queries_build(d, q));
-    if (!q->tc_ngroups) return SS_OK;
     const int kp = k <= 2 ? 8 : 16;  // fp16 products are noisier than the fp32 scan: keep a longer candidate list
-    d->last_work = d->total_frames * q->total_frames;
-    d->last_uncertified = 0;
     TcPlan plan;
     SS_TRY(tc_plan(d, q, kp, &plan));
-    if (kp == 8) SS_TRY(tc_launch<8>(ctx, plan.p, plan.nsingle, plan.nslices, plan.smem, plan.nslices, plan.nslots, d));
-    else SS_TRY(tc_launch<16>(ctx, plan.p, plan.nsingle, plan.nslices, plan.smem, plan.nslices, plan.nslots, d));
+    if (kp == 8) SS_TRY(tc_launch<8>(ctx, plan.p, plan.nsingle, plan.nslices, plan.smem, plan.nslices, plan.nslots, d, timed));
+    else SS_TRY(tc_launch<16>(ctx, plan.p, plan.nsingle, plan.nslices, plan.smem, plan.nslices, plan.nslots, d, timed));
     // certification bound for fp16 inputs: see k_dtw_finalize (bound_mode 1)
-    SS_TRY(dtw_rescore_finalize(d, q, k, kp, plan.nslots, q->d_tc_qid.p, 0.0, q->d_tc_max_norm.p, d->d_tc_max_norm.p, q->d_tc_slot_max_na.p, 1,
-                                q->d_uncert_flag.p, /*fill=*/true, d_out_idx, d_out_dist));
-    *used = true;
-    return SS_OK;
+    return dtw_rescore_finalize(d, q, k, kp, plan.nslots, q->d_tc_qid.p, 0.0, q->d_tc_max_norm.p, d->d_tc_max_norm.p, q->d_tc_slot_max_na.p, 1,
+                                q->d_uncert_flag.p, d_out_idx, d_out_dist);
 }
 
 // ss_dict_debug_tc_scan: the tensor-core scan's raw (filter-stage) distance of EVERY (query, segment) pair, plus the mean
@@ -913,10 +899,9 @@ int dtw_tc_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, doub
 // DBG store compiled in; returns SS_ERR_INVALID if these inputs would not take the tensor-core path.
 int dtw_tc_debug_scan(ss_dict* d, ss_queries* q, float* d_out, std::vector<uint32_t>* slot_qid, double* mu16, float* scale) {
     ss_ctx* ctx = d->ctx;
-    if (!tc_enabled() || !d->tc_ready || q->max_len > (uint32_t)kTcMaxLen || q->total_frames == 0)
-        return set_error(ctx, SS_ERR_INVALID, "debug_tc_scan: the tensor-core scan does not apply (segments / queries > %d frames, or disabled)", kTcMaxLen);
+    if (!dtw_tc_applies(d, q))
+        return set_error(ctx, SS_ERR_INVALID, "debug_tc_scan: the tensor-core scan does not apply (segments / queries > %d frames, or no frame)", kTcMaxLen);
     SS_TRY(tc_queries_build(d, q));
-    if (!q->tc_ngroups) return set_error(ctx, SS_ERR_INVALID, "debug_tc_scan: no non-empty query");
     TcPlan plan;
     SS_TRY(tc_plan(d, q, 8, &plan));
     plan.p.dbg = d_out;

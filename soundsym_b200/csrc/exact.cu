@@ -713,13 +713,11 @@ __device__ __forceinline__ double scan_lower_bound(float scan, double na, double
     return make_scan_bound(na, nb, eps, bound_mode, la, inv_s, ld_max).lower(scan);
 }
 
-// Thread t of the launch handles candidate s_begin + t % s_count of slot t / s_count. Two launches per match:
+// Pair t of a k_dtw_rescore_warp launch is candidate s_begin + t % s_count of slot t / s_count. Two launches per match:
 //   (s_begin, s_count) = (0, k):       the k best candidates by scan distance, unconditionally;
 //   (s_begin, s_count) = (k, kp - k):  the rest, but only those whose scan distance does not already PROVE (by the scan's
 //                                      error bound) that they are farther than the k-th exact distance found in the first
 //                                      launch - such a candidate cannot enter the top-k and is recorded as +inf.
-// SMEM_ROWS: segments of <= 32 frames keep the DP row in shared memory ([column][thread], conflict-free) instead of the
-// global scratch.
 struct RescoreBound {
     const float* cand_adist;   // scan distances of the candidates (nullptr: rescore unconditionally)
     const float* max_na;       // [0] max |a|^2 over the queries
@@ -730,77 +728,10 @@ struct RescoreBound {
     double inv_s;  // bound_mode 2 / 3: 1 / S
     int ld_max;    // bound_mode 3: the dictionary's longest segment
 };
-template <bool SMEM_ROWS>
-__global__ void __launch_bounds__(128)
-k_dtw_rescore(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ qmfcc,
-              const uint64_t* __restrict__ qoff, int c, const uint32_t* __restrict__ group_qid, const uint32_t* __restrict__ cand_idx,
-              uint32_t t_begin, uint32_t t_end, int kp, int s_begin, int s_count, RescoreBound rb, double* __restrict__ rows,
-              uint32_t row_pairs, double* __restrict__ exact, unsigned long long* __restrict__ counters) {
-    __shared__ double srow[SMEM_ROWS ? 32 * 128 : 1];
-    const uint32_t local = blockIdx.x * blockDim.x + threadIdx.x;
-    const uint32_t t = t_begin + local;
-    if (t >= t_end) return;
-    const uint32_t slot = t / (uint32_t)s_count;
-    const uint32_t pair = slot * (uint32_t)kp + (uint32_t)s_begin + t % (uint32_t)s_count;
-    const uint32_t qid = group_qid[slot];
-    const uint32_t idx = cand_idx[pair];
-    if (qid == 0xFFFFFFFFu || idx == 0xFFFFFFFFu) {
-        exact[pair] = kInf;
-        return;
-    }
-    if (rb.cand_adist) {
-        // k-th smallest exact distance among the slot's first k candidates
-        double kth = 0.0;
-        for (int s = 0; s < rb.k; s++) {
-            double e = exact[(size_t)slot * kp + s];
-            if (!(e < kInf)) e = kInf;  // empty slot / NaN: nothing can be ruled out
-            kth = fmax(kth, e);
-        }
-        const double na = rb.slot_max_na ? (double)rb.slot_max_na[slot] : (double)rb.max_na[0];
-        const int lq = (int)(qoff[qid + 1] - qoff[qid]);
-        if (scan_lower_bound(rb.cand_adist[pair], na, (double)rb.max_nb[0], rb.eps, rb.bound_mode, lq, rb.inv_s, rb.ld_max) > kth) {
-            exact[pair] = kInf;  // provably outside the top-k
-            return;
-        }
-        atomicAdd(&counters[1], 1ull);
-    }
-    const double* a = qmfcc + qoff[qid] * c;
-    const double* b = dmfcc + doff[idx] * c;
-    const uint32_t la = (uint32_t)(qoff[qid + 1] - qoff[qid]), lb = (uint32_t)(doff[idx + 1] - doff[idx]);
-    double* row = SMEM_ROWS ? srow + threadIdx.x : rows + local;
-    const size_t rstride = SMEM_ROWS ? 128 : row_pairs;
-    double last = kInf;
-    for (uint32_t i = 0; i < la; i++) {
-        double ar[SS_MAX_NCOEFFS];
-#pragma unroll
-        for (int k = 0; k < SS_MAX_NCOEFFS; k++) ar[k] = k < c ? a[(size_t)i * c + k] : 0.0;
-        double left = kInf, diag = kInf;  // D(i, j-1), D(i-1, j-1)
-        for (uint32_t j = 0; j < lb; j++) {
-            double cost = 0.0;
-#pragma unroll
-            for (int k = 0; k < SS_MAX_NCOEFFS; k++)
-                if (k < c) {
-                    const double dlt = ar[k] - b[(size_t)j * c + k];
-                    cost = cost + dlt * dlt;
-                }
-            const double up = i ? row[(size_t)j * rstride] : kInf;  // D(i-1, j)
-            double m;
-            if (i == 0 && j == 0) m = 0.0;
-            else m = fmin(fmin(up, left), diag);
-            const double cur = cost + m;
-            row[(size_t)j * rstride] = cur;
-            diag = up;
-            left = cur;
-        }
-        last = left;
-    }
-    exact[pair] = (la && lb) ? last / (double)(la + lb) : kInf;
-}
-
 // ---------------------------------------------------------------------------------------------------------------
 // The whole refine of one query slot by ONE warp (sequences of <= 32 frames on both sides): the k best candidates by scan
 // distance unconditionally, the other kp - k only if the scan's error bound cannot rule them out against the k-th exact
-// distance, then the (distance, index) sort, the top-k store and the certification - what k_dtw_rescore (twice) and
+// distance, then the (distance, index) sort, the top-k store and the certification - what k_dtw_rescore_warp (twice) and
 // k_dtw_finalize do in three launches for longer sequences, with the same arithmetic per cell. Lane j owns dictionary column
 // j; the pair's local costs go to shared memory first (39 f64 operations per cell on 32 busy lanes), then the recurrence runs
 // as an anti-diagonal wavefront: at step t lane j computes cell (t - j, j) from its own previous value (up), its left
@@ -924,7 +855,7 @@ k_dtw_refine_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// The same exact recurrence for sequences of ANY length, one warp per pair (k_dtw_rescore's interface; a single thread needs
+// The same exact recurrence for sequences of ANY length, one warp per pair (a single thread needs
 // ~80 ms for a pair of 383 x 383 frames, which was most of config 5's match). The dictionary segment is cut into strips of 32
 // columns, lane j owning column 32 s + j of strip s with its frame in registers. Per strip the warp alternates
 //   A. local costs of the next 32 query rows against the strip's 32 columns -> a shared-memory ring of 64 rows (the row's
@@ -1010,7 +941,7 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
     return result / (double)(la + lb);
 }
 
-// k_dtw_rescore with one WARP per (slot, candidate) pair (grid-stride over the pairs; bnd: one row of bnd_stride doubles per warp)
+// one WARP per (slot, candidate) pair (grid-stride over the pairs; bnd: one row of bnd_stride doubles per warp)
 __global__ void __launch_bounds__(64)
 k_dtw_rescore_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ qmfcc,
                    const uint64_t* __restrict__ qoff, int c, const uint32_t* __restrict__ group_qid, const uint32_t* __restrict__ cand_idx,
@@ -1351,10 +1282,10 @@ __global__ void k_dtw_finalize(const uint32_t* __restrict__ cand_idx, const floa
 
 int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, double eps,
                          const float* d_max_na, const float* d_max_nb, const float* d_slot_max_na, int bound_mode, uint8_t* d_uncert_flag,
-                         bool fill, uint32_t* d_out_idx, double* d_out_dist) {
+                         uint32_t* d_out_idx, double* d_out_dist) {
     ss_ctx* ctx = d->ctx;
     // queries without a frame never reach a slot: their rows keep (inf, 0xFFFFFFFF). Only launched when such queries exist.
-    if (q->nq && fill && q->nonempty < q->nq) {
+    if (q->nq && q->nonempty < q->nq) {
         k_fill_result<<<ceil_div((long long)q->nq * k, 256), 256, 0, ctx->stream>>>(d_out_idx, d_out_dist, q->nq * (size_t)k,
                                                                                    0xFFFFFFFFu, kInf);
         SS_LAUNCHED(ctx);
@@ -1362,8 +1293,7 @@ int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslo
     SS_CUDA(ctx, d->d_counters.reserve(4));
     SS_CUDA(ctx, cudaMemsetAsync(d->d_counters.p, 0, 4 * sizeof(unsigned long long), ctx->stream));
     if (!nslots || !d->ntiles) return SS_OK;
-    const uint32_t max_ld = std::max<uint32_t>(d->max_len, 1);
-    if (max_ld <= 32 && q->max_len <= 32) {  // one warp per query slot does the whole refine
+    if (d->max_len <= 32 && q->max_len <= 32) {  // one warp per query slot does the whole refine
         k_dtw_refine_warp<<<ceil_div(nslots, 4), 128, 0, ctx->stream>>>(d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d_slot_qid,
                                                                         d->d_cand_idx.p, d->d_cand_adist.p, nslots, kp, std::min(k, kp), d->index_base,
                                                                         d_max_na, d_max_nb, eps, d_slot_max_na, bound_mode, d->h2_bound_inv_s,
@@ -1371,59 +1301,26 @@ int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslo
         SS_LAUNCHED(ctx);
         return SS_OK;
     }
-    const uint32_t npairs = nslots * (uint32_t)kp;
-    SS_CUDA(ctx, d->d_cand_exact.reserve(npairs));
-    static const bool thread_rescore = [] {  // SS_DTW_THREAD_RESCORE=1: the thread-per-pair kernels (A/B measurements)
-        const char* e = getenv("SS_DTW_THREAD_RESCORE");
-        return e && atoi(e) != 0;
-    }();
-    if (!thread_rescore) {
-        // one warp per pair: the k best of every slot, then the others unless the scan's bound rules them out, then the sort
-        const uint32_t stride = (std::max<uint32_t>(q->max_len, 1) + 15) & ~15u;
-        const uint32_t max_ctas = (uint32_t)ctx->sm_count * 6;  // 33 KB of shared memory each
-        SS_CUDA(ctx, d->d_rescore_rows.reserve((size_t)max_ctas * 2 * stride));
-        for (int phase = 0; phase < 2; phase++) {
-            const int s_begin = phase ? std::min(k, kp) : 0, s_count = phase ? kp - std::min(k, kp) : std::min(k, kp);
-            if (s_count <= 0) continue;
-            RescoreBound rb = {phase ? d->d_cand_adist.p : nullptr, d_max_na, d_max_nb, d_slot_max_na, eps, bound_mode, std::min(k, kp), d->h2_bound_inv_s,
-                               (int)d->max_len};
-            const uint32_t nt = nslots * (uint32_t)s_count;
-            k_dtw_rescore_warp<<<std::min<uint32_t>(max_ctas, ceil_div(nt, 2)), 64, 0, ctx->stream>>>(d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c,
-                                                                                                  d_slot_qid, d->d_cand_idx.p, nt, kp, s_begin, s_count, rb,
-                                                                                                  d->d_rescore_rows.p, stride, d->d_cand_exact.p,
-                                                                                                  d->d_counters.p);
-            SS_LAUNCHED(ctx);
-        }
-        k_dtw_finalize<<<ceil_div(nslots, 128), 128, 0, ctx->stream>>>(d->d_cand_idx.p, d->d_cand_adist.p, d->d_cand_exact.p, d_slot_qid, nslots, kp, k,
-                                                                      d->index_base, d_max_na, d_max_nb, eps, d_slot_max_na, bound_mode, d->h2_bound_inv_s,
-                                                                      (int)d->max_len, q->d_off.p, d_uncert_flag, d_out_idx, d_out_dist, d->d_counters.p);
-        SS_LAUNCHED(ctx);
-        return SS_OK;
-    }
-    const uint64_t budget = 32ull << 20;  // doubles of DP-row scratch (256 MB)
-    const uint32_t batch = (uint32_t)std::min<uint64_t>(npairs, std::max<uint64_t>(1024, budget / max_ld));
-    SS_CUDA(ctx, d->d_rescore_rows.reserve((size_t)batch * max_ld));
-    auto kern = max_ld <= 32 ? k_dtw_rescore<true> : k_dtw_rescore<false>;
-    // the candidate lists are ascending in scan distance: the first k unconditionally, the others only if the scan's error
-    // bound cannot already rule them out against the k-th exact distance of the first launch
+    SS_CUDA(ctx, d->d_cand_exact.reserve(nslots * (uint32_t)kp));
+    // one warp per pair: the k best of every slot, then the others unless the scan's bound rules them out, then the sort
+    const uint32_t stride = (std::max<uint32_t>(q->max_len, 1) + 15) & ~15u;
+    const uint32_t max_ctas = (uint32_t)ctx->sm_count * 6;  // 33 KB of shared memory each
+    SS_CUDA(ctx, d->d_rescore_rows.reserve((size_t)max_ctas * 2 * stride));
     for (int phase = 0; phase < 2; phase++) {
         const int s_begin = phase ? std::min(k, kp) : 0, s_count = phase ? kp - std::min(k, kp) : std::min(k, kp);
         if (s_count <= 0) continue;
         RescoreBound rb = {phase ? d->d_cand_adist.p : nullptr, d_max_na, d_max_nb, d_slot_max_na, eps, bound_mode, std::min(k, kp), d->h2_bound_inv_s,
                            (int)d->max_len};
         const uint32_t nt = nslots * (uint32_t)s_count;
-        for (uint32_t tb = 0; tb < nt; tb += batch) {
-            const uint32_t te = std::min<uint32_t>(nt, tb + batch);
-            kern<<<ceil_div(te - tb, 128), 128, 0, ctx->stream>>>(d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d_slot_qid,
-                                                                   d->d_cand_idx.p, tb, te, kp, s_begin, s_count, rb, d->d_rescore_rows.p,
-                                                                   batch, d->d_cand_exact.p, d->d_counters.p);
-            SS_LAUNCHED(ctx);
-        }
+        k_dtw_rescore_warp<<<std::min<uint32_t>(max_ctas, ceil_div(nt, 2)), 64, 0, ctx->stream>>>(d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c,
+                                                                                              d_slot_qid, d->d_cand_idx.p, nt, kp, s_begin, s_count, rb,
+                                                                                              d->d_rescore_rows.p, stride, d->d_cand_exact.p,
+                                                                                              d->d_counters.p);
+        SS_LAUNCHED(ctx);
     }
-    k_dtw_finalize<<<ceil_div(nslots, 128), 128, 0, ctx->stream>>>(d->d_cand_idx.p, d->d_cand_adist.p, d->d_cand_exact.p,
-                                                                  d_slot_qid, nslots, kp, k, d->index_base, d_max_na, d_max_nb, eps,
-                                                                  d_slot_max_na, bound_mode, d->h2_bound_inv_s, (int)d->max_len, q->d_off.p,
-                                                                  d_uncert_flag, d_out_idx, d_out_dist, d->d_counters.p);
+    k_dtw_finalize<<<ceil_div(nslots, 128), 128, 0, ctx->stream>>>(d->d_cand_idx.p, d->d_cand_adist.p, d->d_cand_exact.p, d_slot_qid, nslots, kp, k,
+                                                                  d->index_base, d_max_na, d_max_nb, eps, d_slot_max_na, bound_mode, d->h2_bound_inv_s,
+                                                                  (int)d->max_len, q->d_off.p, d_uncert_flag, d_out_idx, d_out_dist, d->d_counters.p);
     SS_LAUNCHED(ctx);
     return SS_OK;
 }

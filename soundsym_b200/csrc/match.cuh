@@ -20,6 +20,9 @@ constexpr int kStages = 3;        // tile ring depth
 constexpr int kWarpsPerCta = 4;
 constexpr int kMaxKeep = 32;      // largest candidate list per query kept by a scan
 
+// the stages of an SS_DTW match, in cascade order (dtw.cu)
+enum class DtwStage { H2, H2_WIDE, TC, FP32, EXHAUSTIVE };
+
 struct StripDesc {  // 16 B, read as int4
     uint32_t frame_begin;  // first frame of the strip in the shard's frame stream
     uint32_t seg;          // local segment index
@@ -66,14 +69,14 @@ struct ss_dict {
     ss::DevBuf<double> d_second_bnd;  // boundary rows of the long second-chance kernel (exact.cu)
     ss::DevBuf<unsigned long long> d_counters;  // [0] uncertified
     std::vector<uint32_t> h_slice_tile;
-    uint64_t last_work = 0, last_uncertified = 0;
-    uint64_t last_tc_fallback = 0;  // queries of the last match that the tensor-core scan handed to the fp32 scan
-    uint64_t last_exhaustive = 0;   // queries that neither scan could certify and that were matched exhaustively in f64
+    uint64_t last_work = 0;         // work of the last match (SS_DTW: dictionary frames x query frames, the first stage's cells)
+    uint64_t last_uncertified = 0;  // queries of the last match whose rows are not final (0 unless a stage failed)
+    uint64_t last_tc_fallback = 0;  // queries of the last match that its first stage, a tensor-core scan, left uncertified
+    uint64_t last_exhaustive = 0;   // queries of the last match sent to the exhaustive f64 stage
     ss::DevBuf<double> d_exh_dist;
     ss::DevBuf<uint32_t> d_exh_qid;
-    cudaEvent_t ev_scan0 = nullptr, ev_scan1 = nullptr;  // around the dominant kernel of the last match
+    cudaEvent_t ev_scan0 = nullptr, ev_scan1 = nullptr;  // around the first stage's scan of the last match
     bool scan_timed = false;
-    bool in_fallback = false;  // set while dtw_match_finish runs later stages
     int last_scan_kind = 0;    // first-stage scan of the last match: 1 packed-half tensor-core, 2 fp32-DP tensor-core, 3 fp32 CUDA-core, 4 cosine-ref
     // tensor-core scan (dtw_tc.cu): fp16 UMMA tiles of 4 segment slots x 32 columns, segments sorted by length
     bool tc_ready = false;
@@ -115,11 +118,10 @@ struct ss_dict {
     ss::DevBuf<unsigned long long> d_h2_thr;   // per query slot: running bound on the global KP-th key (dtw_h2.cu)
     int scan_pref = 0;  // test / A-B hook (ss_dict_set_scan): 0 = packed-half scan first, 1 = start at the fp32 tensor-core scan, 2 = fp32 CUDA-core scan, 3 = packed-half scan without its second chance
     // the last SS_DTW match is asynchronous up to its fallback decision: ss::dtw_match_finish waits for ev_done, reads the
-    // uncertified count from pinned memory and runs the fallback stages for the queries that need them
+    // uncertified count from pinned memory and runs the later stages for the queries that need them
     struct Pending {
         bool active = false;
-        int stage = 0;  // 1 = a tensor-core scan ran, 2 = the fp32 scan ran (for every query)
-        bool h2 = false;  // stage 1 was the packed-half scan
+        ss::DtwStage first = ss::DtwStage::FP32;  // the stage dtw_match_dev ran on the whole batch
         struct ss_queries* q = nullptr;
         int k = 0;
         uint32_t* d_out_idx = nullptr;
@@ -130,7 +132,7 @@ struct ss_dict {
     ss::DevBuf<uint32_t> d_tc_slice_tile;       // the tensor-core scan's own slice table (cached)
     uint32_t slice_for_groups = 0xFFFFFFFFu;  // tc_ngroups the cached slice table (d_slice_tile / h_slice_tile) was built for
     uint32_t tc_nsingle = 0, tc_nslices = 0;
-    // the few queries a first stage could not certify, as a batch of their own (dtw.cu dtw_rerun_subset)
+    // the few queries a stage could not certify, as a batch of their own for the next stage (dtw.cu gather_queries)
     struct ss_queries* sub_q = nullptr;
     ss::DevBuf<uint32_t> d_sub_ids, d_sub_idx;
     ss::DevBuf<double> d_sub_dist;
@@ -182,7 +184,7 @@ struct ss_queries {
     ss::DevBuf<unsigned char> d_tc_a;
     ss::DevBuf<float> d_tc_max_norm;                // [0] = max |fp16(a - mu)|^2
     ss::DevBuf<float> d_tc_slot_max_na;             // per query slot: max over its rows of |fp16(a - mu)|^2
-    ss::DevBuf<uint8_t> d_uncert_flag;              // per query: 1 if the tensor-core scan could not certify its top-k
+    ss::DevBuf<uint8_t> d_uncert_flag;              // per query: 1 if the last stage run on the batch could not certify its top-k
 };
 
 inline ss_dict::~ss_dict() {
@@ -198,7 +200,7 @@ inline ss_dict::~ss_dict() {
 }
 
 namespace ss {
-// SS_DTW_TRACE=1: wall-clock of the fallback path's steps on stderr (each step is followed by a stream synchronisation)
+// SS_DTW_TRACE=1: wall-clock of a match's steps and the stages it takes, on stderr (each step is followed by a stream synchronisation)
 inline bool dtw_trace() {
     static const bool on = [] {
         const char* e = getenv("SS_DTW_TRACE");
@@ -221,7 +223,7 @@ struct TraceTimer {
 
 int dtw_dict_build(ss_dict* d);       // builds the fp32 stream + strip / tile tables (dtw.cu)
 int dtw_tc_dict_build(ss_dict* d);    // builds the fp16 UMMA tiles (dtw_tc.cu)
-int dtw_queries_build(ss_queries* q, const std::vector<uint32_t>* subset = nullptr); // builds the lane layout (dtw.cu)
+int dtw_queries_build(ss_queries* q); // builds the lane layout (dtw.cu)
 int dtw_tc_queries_group(ss_queries* q);  // length-sorted groups of 128 for the tensor-core scan (dtw_tc.cu); no-op for long queries
 // asynchronous on the ctx stream up to the fallback decision; dtw_match_finish completes it (a no-op when nothing is pending)
 int dtw_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist);

@@ -274,11 +274,21 @@ def test_tensor_core_scan_fallback_on_near_duplicates(ctx):
     check_dtw(idx, dist, oidx, odist, 4)
     assert list(idx[0, :3]) == [3, 104, 105] and dist[0, 0] == 0.0
     assert dev.last_tc_fallback >= 1 and dev.last_exhaustive >= 1 and dev.last_uncertified == 0
+    # from the other first stages: fp32-DP tensor-core scan -> fp32 CUDA-core scan -> exhaustive, and fp32 CUDA-core scan ->
+    # exhaustive; here neither scan certifies either query of the batch
+    for first_stage, scan_kind, tc_fallback, exhaustive in ((1, 2, 2, 2), (2, 3, 0, 2)):
+        dev.set_scan(first_stage)
+        idx, dist = dev.match(q, qoff, SS_DTW, 4)
+        check_dtw(idx, dist, oidx, odist, 4)
+        assert list(idx[0, :3]) == [3, 104, 105] and dist[0, 0] == 0.0
+        assert dev.last_scan_kind == scan_kind
+        assert (dev.last_tc_fallback, dev.last_exhaustive, dev.last_uncertified) == (tc_fallback, exhaustive, 0)
 
 
 def test_fp32_scan_forced_matches_tensor_core_scan(ctx):
-    """SS_DTW_TC=0 is read once per process, so the fp32 scan is exercised here through shapes the tensor-core scan
-    declines (a 33-frame segment in the dictionary) on otherwise identical data."""
+    """One 33-frame segment in the dictionary (far from everything: never a candidate) rules out the fp32-DP tensor-core
+    scan and moves the packed-half scan to its strip kernel; on otherwise identical data the results must not change.
+    (ss_dict_set_scan(2) forces the fp32 CUDA-core scan itself: see the config-1 and config-3 tests.)"""
     d, doff = synth.segments(300, 13, seed=31)
     q, qoff = synth.segments(70, 13, seed=32)
     tc = api.DeviceDictionary(ctx, d, doff)
