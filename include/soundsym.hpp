@@ -380,6 +380,14 @@ class SoundDictionary {
         match_indices({other}, {distance}, 1, &idx, &dist);
         return sounds[idx[0]];
     }
+    /// SoundSequence::from_distances' chain for SS_COSINE_REF on the device (ss_dict_walk): step t matches the sound step
+    /// t - 1 returned (step 0: start) at distances[t]
+    void walk(const Sound& start, const std::vector<double>& distances, std::vector<uint32_t>* idx, std::vector<double>* dist) {
+        ss_dict* d = device();
+        idx->assign(distances.size(), 0);
+        dist->assign(distances.size(), 0.0);
+        ctx_->check(ss_dict_walk(d, start.mfccs().data(), start.num_frames(), distances.data(), distances.size(), idx->data(), dist->data()));
+    }
     /// SoundDictionary::match_sound (src/sound.rs:346-348)
     std::shared_ptr<Sound> match_sound(const std::shared_ptr<Sound>& other) { return at_distance(1.0, other); }
     Context& context() const { return *ctx_; }
@@ -449,10 +457,18 @@ class SoundSequence {
         for (uint32_t i : idx) out.push_back(dict.sounds[i]);
         return SoundSequence(std::move(out), *ctx_);
     }
-    /// SoundSequence::from_distances (src/sound.rs:405-417): sequential chain of nq = 1 matches
+    /// SoundSequence::from_distances (src/sound.rs:405-417): a chain, step t matches the sound step t - 1 returned.
+    /// SS_COSINE_REF runs it on the device in one call; SS_DTW (whose at_distance ignores the target) keeps the nq = 1 loop.
     static SoundSequence from_distances(const std::vector<double>& distances, std::shared_ptr<Sound> start, SoundDictionary& dict) {
         std::vector<std::shared_ptr<Sound>> sounds{std::move(start)};
-        for (double d : distances) sounds.push_back(dict.at_distance(d, sounds.back()));
+        if (!distances.empty() && dict.mode == SS_COSINE_REF) {
+            std::vector<uint32_t> idx;
+            std::vector<double> dist;
+            dict.walk(*sounds[0], distances, &idx, &dist);
+            for (uint32_t i : idx) sounds.push_back(dict.sounds[i]);
+        } else {
+            for (double d : distances) sounds.push_back(dict.at_distance(d, sounds.back()));
+        }
         return SoundSequence(std::move(sounds), dict.context());
     }
 

@@ -168,6 +168,17 @@ void ss_queries_destroy(ss_queries* q);
 int ss_dict_match_dev(ss_dict* dict, ss_queries* q, int mode, const double* d_targets, int k, uint32_t* d_out_idx,
                       double* d_out_dist);
 int ss_dict_match_finish(ss_dict* dict);
+/* SoundSequence::from_distances (src/sound.rs:405-417) for SS_COSINE_REF, on the device: step t matches the previous
+ * step's dictionary segment (step 0: the start query) at target distances[t]. Host buffers, one blocking point.
+ * Every step's (out_idx[t], out_dist[t]) equals ss_dict_match(dict, query, 1, SS_COSINE_REF, &distances[t], 1, ...) bit for
+ * bit, indices include index_base. A pending SS_DTW match completes first; the ss_dict_last_* readers still describe the
+ * last MATCH (a walk changes none of them). nsteps == 0 returns SS_OK and launches nothing. */
+int ss_dict_walk(ss_dict* dict, const double* start_mfcc, size_t start_frames, const double* distances, size_t nsteps,
+                 uint32_t* out_idx, double* out_dist);
+/* the same on device pointers, asynchronous on the ctx stream (nsteps + 1 kernel launches, no host synchronisation);
+ * `start` holds exactly one query */
+int ss_dict_walk_dev(ss_dict* dict, ss_queries* start, const double* d_distances, size_t nsteps, uint32_t* d_out_idx,
+                     double* d_out_dist);
 int ss_topk_merge_dev(ss_ctx* ctx, const uint32_t* d_idx, const double* d_dist, int nlists, size_t nq, int k,
                       uint32_t* d_out_idx, double* d_out_dist);
 /* drops the cached device layouts of a query batch so that the next match rebuilds them (bench.py calls this every

@@ -248,6 +248,17 @@ class DeviceDictionary:
         self.ctx.check(self.ctx.lib.ss_dict_match(self.h, _ptr(q), _ptr(qo), nq, int(mode), _ptr(t), int(k), _ptr(idx), _ptr(dist)))
         return idx, dist
 
+    def walk(self, start_mfcc, distances):
+        """ss_dict_walk: SoundSequence::from_distances for SS_COSINE_REF on the device -> (idx u32 [n], dist f64 [n]); step t
+        matches the segment step t - 1 returned (step 0: start_mfcc, frames x ncoeffs) at target distances[t]."""
+        s = np.ascontiguousarray(start_mfcc, dtype=np.float64).reshape(-1, self.ncoeffs)
+        t = np.ascontiguousarray(distances, dtype=np.float64).reshape(-1)
+        n = t.shape[0]
+        idx = np.empty(n, dtype=np.uint32)
+        dist = np.empty(n, dtype=np.float64)
+        self.ctx.check(self.ctx.lib.ss_dict_walk(self.h, _ptr(s), s.shape[0], _ptr(t), n, _ptr(idx), _ptr(dist)))
+        return idx, dist
+
     def debug_tc_scan(self, q_flat, q_frame_offsets):
         """ss_dict_debug_tc_scan: raw tensor-core scan distance of every (query, segment) pair -> (scan f32 [nq, nseg],
         mean frame f64 [16], norm scale)."""
@@ -720,10 +731,16 @@ class SoundSequence:
 
     @classmethod
     def from_distances(cls, distances, start, dictionary):
-        """src/sound.rs:405-417: inherently sequential chain of nq = 1 matches."""
+        """src/sound.rs:405-417: a chain, step t matches the sound step t - 1 returned. SS_COSINE_REF runs it on the device
+        in one call (ss_dict_walk); in SS_DTW mode at_distance ignores the target, so that mode keeps the nq = 1 loop."""
         sounds = [start]
-        for d in distances:
-            sounds.append(dictionary.at_distance(d, sounds[-1]))
+        distances = list(distances)
+        if distances and dictionary.mode == SS_COSINE_REF:
+            idx, _ = dictionary._device().walk(start.mfcc_arrays(), distances)
+            sounds += [dictionary.sounds[int(i)] for i in idx]
+        else:
+            for d in distances:
+                sounds.append(dictionary.at_distance(d, sounds[-1]))
         return cls(sounds)
 
     def to_sound(self):

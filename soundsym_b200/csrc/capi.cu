@@ -315,6 +315,56 @@ int ss_dict_match(ss_dict* d, const double* q_mfcc, const uint64_t* q_frame_offs
     return rc;
 }
 
+// SoundSequence::from_distances for SS_COSINE_REF. Like the cosine match, the walk first completes a pending asynchronous
+// SS_DTW match; it has its own workspaces and leaves the ss_dict_last_* counters as the last match left them.
+int ss_dict_walk_dev(ss_dict* d, ss_queries* start, const double* d_distances, size_t nsteps, uint32_t* d_out_idx, double* d_out_dist) {
+    if (!d) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
+    ss_ctx* ctx = d->ctx;
+    if (nsteps && (!d_distances || !d_out_idx || !d_out_dist)) return set_error(ctx, SS_ERR_INVALID, "distance / output pointers are NULL");
+    if (d->nseg == 0) return set_error(ctx, SS_ERR_EMPTY_DICT, "walk over an empty dictionary");
+    if (!start) return set_error(ctx, SS_ERR_INVALID, "start is NULL");
+    if (start->ctx != ctx) return set_error(ctx, SS_ERR_INVALID, "dict and start belong to different contexts");
+    if (start->c != d->c) return set_error(ctx, SS_ERR_INVALID, "ncoeffs mismatch: dict %d, start %d", d->c, start->c);
+    if (start->nq != 1) return set_error(ctx, SS_ERR_INVALID, "start must hold exactly one query (got %zu)", start->nq);
+    if (nsteps > 0xFFFFFFFFull) return set_error(ctx, SS_ERR_INVALID, "too many steps");
+    if (!nsteps) return SS_OK;
+    SS_CUDA(ctx, cudaSetDevice(ctx->device));
+    SS_TRY(dtw_match_finish(d));  // a pending SS_DTW match completes first, as before a cosine match
+    return cosine_walk_dev(d, start->d_mfcc.p, start->d_off.p, d_distances, nsteps, d_out_idx, d_out_dist);
+}
+
+int ss_dict_walk(ss_dict* d, const double* start_mfcc, size_t start_frames, const double* distances, size_t nsteps, uint32_t* out_idx,
+                 double* out_dist) {
+    if (!d) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
+    ss_ctx* ctx = d->ctx;
+    if (nsteps && (!distances || !out_idx || !out_dist)) return set_error(ctx, SS_ERR_INVALID, "distance / output pointers are NULL");
+    if (d->nseg == 0) return set_error(ctx, SS_ERR_EMPTY_DICT, "walk over an empty dictionary");
+    if (start_frames && !start_mfcc) return set_error(ctx, SS_ERR_INVALID, "start_mfcc is NULL");
+    if (start_frames > 0x7FFFFFFFull / (uint64_t)d->c) return set_error(ctx, SS_ERR_INVALID, "start sound too long");
+    if (nsteps > 0xFFFFFFFFull) return set_error(ctx, SS_ERR_INVALID, "too many steps");
+    if (!nsteps) return SS_OK;
+    SS_CUDA(ctx, cudaSetDevice(ctx->device));
+    auto body = [&]() -> int {
+        SS_TRY(dtw_match_finish(d));
+        d->h_walk_off[0] = 0;
+        d->h_walk_off[1] = start_frames;
+        SS_TRY(upload(ctx, d->d_walk_start, start_mfcc, start_frames * (size_t)d->c));
+        SS_TRY(upload(ctx, d->d_walk_off, d->h_walk_off, 2));
+        SS_TRY(upload(ctx, d->d_walk_targets, distances, nsteps));
+        SS_CUDA(ctx, d->d_walk_idx.reserve(nsteps));
+        SS_CUDA(ctx, d->d_walk_dist.reserve(nsteps));
+        SS_TRY(cosine_walk_dev(d, d->d_walk_start.p, d->d_walk_off.p, d->d_walk_targets.p, nsteps, d->d_walk_idx.p, d->d_walk_dist.p));
+        // ONE blocking point per call
+        SS_CUDA(ctx, cudaMemcpyAsync(out_idx, d->d_walk_idx.p, nsteps * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+        SS_CUDA(ctx, cudaMemcpyAsync(out_dist, d->d_walk_dist.p, nsteps * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        return SS_OK;
+    };
+    const int rc = body();
+    if (rc != SS_OK) cudaStreamSynchronize(ctx->stream);
+    return rc;
+}
+
 int ss_dict_set_scan(ss_dict* d, int first_stage) {
     if (!d) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
     if (first_stage < 0 || first_stage > 3) return set_error(d->ctx, SS_ERR_INVALID, "first_stage must be 0, 1, 2 or 3");

@@ -653,6 +653,165 @@ int cosine_match_dev(ss_dict* d, ss_queries* q, const double* d_targets, uint32_
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// SoundSequence::from_distances (src/sound.rs:405-417) on the device: step t is at_distance(distances[t], previous), and
+// from step 1 on the query IS a dictionary segment already in HBM, so the whole chain runs as one launch per step with
+// no host decision in between. k_cosine_scan puts 32 queries on the lanes; with one query that lights one lane in 32, so
+// this kernel turns the mapping around: DICTIONARY SEGMENTS on lanes, the one query broadcast from shared memory.
+//
+// kWalkLanes = 8 lanes per segment, lane u owning rulinalg's partial sum p_u (elements u, u + 8, ...): a group reads 64
+// contiguous bytes of its segment per chunk. The combine is cos_finish's, through shuffles into lane 0 of the group:
+// 0.0 + (p0 + p4), + (p1 + p5), + (p2 + p6), + (p3 + p7), then the <= 7 tail elements in order, then
+// sum / (norm_d * norm_q) - the same operations in the same order as k_cosine_scan, so every (idx, dist) is the bits of
+// ss_dict_match(nq = 1). A warp's four groups take four consecutive positions of the (length, index) walk order, so they
+// almost always run the same number of chunks. Each CTA leaves its (distance, index) minimum in a partial; the last CTA
+// to finish (atomic ticket) reduces the partials, writes step t's result and the local index the next step queries, and
+// resets the ticket. No CTA ever waits for another.
+constexpr int kWalkThreads = 256;                        // 32 segments in flight per CTA
+constexpr int kWalkLanes = 8;                            // lanes per dictionary segment (rulinalg's 8 partial sums)
+constexpr int kWalkGroups = kWalkThreads / kWalkLanes;
+constexpr int kWalkCtasPerSm = 6;                        // all resident at 40 registers a thread: one wave
+constexpr uint32_t kWalkQCap = 2048;                     // query doubles staged in shared memory (beyond: global memory)
+
+// (distance, index) minimum with the fold's seed (2.0, none): a smaller distance wins, an equal one only with a smaller
+// index than a winner already found - never against the seed, so a distance of exactly 2.0 never beats it (src/sound.rs:362);
+// NaN never wins. Every candidate that replaces the seed is < 2.0, so partials merge with the same rule.
+__device__ __forceinline__ void walk_min(double& bd, uint32_t& bi, double d, uint32_t i) {
+    if (d < bd || (d == bd && i < bi && bi != kCosNone)) {
+        bd = d;
+        bi = i;
+    }
+}
+
+__device__ __forceinline__ void walk_block_min(double& bd, uint32_t& bi) {
+    __shared__ double sd[kWalkThreads / 32];
+    __shared__ uint32_t si[kWalkThreads / 32];
+#pragma unroll
+    for (int o = 16; o; o >>= 1) walk_min(bd, bi, __shfl_xor_sync(0xffffffffu, bd, o), __shfl_xor_sync(0xffffffffu, bi, o));
+    __syncthreads();  // (sd / si are reused by the last CTA's second reduction)
+    if ((threadIdx.x & 31) == 0) sd[threadIdx.x >> 5] = bd, si[threadIdx.x >> 5] = bi;
+    __syncthreads();
+    if (threadIdx.x == 0)
+        for (int w = 1; w < kWalkThreads / 32; w++) walk_min(bd, bi, sd[w], si[w]);
+}
+
+__global__ void __launch_bounds__(kWalkThreads)
+k_cosine_walk_step(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ dnorm,
+                   const uint4* __restrict__ cseg, const double* __restrict__ cnorm, uint32_t nseg, int c, uint32_t max_kd,
+                   const double* __restrict__ start, const uint64_t* __restrict__ start_off, const double* __restrict__ start_norm,
+                   const double* __restrict__ targets, uint32_t step, uint32_t index_base, double* __restrict__ part_dist,
+                   uint32_t* __restrict__ part_idx, uint32_t* __restrict__ state /* [0] ticket, [1] query of the next step */,
+                   uint32_t* __restrict__ out_idx, double* __restrict__ out_dist) {
+    __shared__ double sq[kWalkQCap];
+    __shared__ bool last;
+    // the query: the start sound at step 0, else the segment the previous step returned (written by its last CTA)
+    const double* qp;
+    uint32_t kq;
+    double nq;
+    if (step == 0) {
+        qp = start + start_off[0] * c;
+        kq = (uint32_t)(start_off[1] - start_off[0]) * (uint32_t)c;
+        nq = start_norm[0];
+    } else {
+        const uint32_t s = state[1];
+        qp = dmfcc + doff[s] * c;
+        kq = (uint32_t)(doff[s + 1] - doff[s]) * (uint32_t)c;
+        nq = dnorm[s];
+    }
+    const double target = targets[step];
+    const uint32_t nstage = min(min(kq, max_kd), kWalkQCap);  // no segment reads past max_kd
+    for (uint32_t e = threadIdx.x; e < nstage; e += kWalkThreads) sq[e] = qp[e];
+    __syncthreads();
+
+    const uint32_t u = threadIdx.x % kWalkLanes;
+    const uint32_t lane = threadIdx.x & 31;
+    const uint32_t gmask = 0xFFu << (lane & ~(kWalkLanes - 1));  // this group's 8 lanes
+    double bd = 2.0;              // fold((0, 2.0)), src/sound.rs:361
+    uint32_t bi = kCosNone;
+    for (uint32_t base = blockIdx.x * kWalkGroups; base < nseg; base += gridDim.x * kWalkGroups) {  // warp-uniform
+        const uint32_t pos = base + threadIdx.x / kWalkLanes;
+        if (pos >= nseg) break;  // (whole groups leave together: the shuffles below only span a group)
+        const uint4 dsc = __ldg(&cseg[pos]);
+        const double* x = dmfcc + (((uint64_t)dsc.y << 32) | dsc.x) * c;
+        const uint32_t kd = dsc.z * (uint32_t)c;
+        const uint32_t len = kd < kq ? kd : kq;
+        const uint32_t nch = len / kWalkLanes;
+        const uint32_t nch_s = min(nch, kWalkQCap / kWalkLanes);  // chunks whose query values are staged
+        double p = 0.0;
+        uint32_t ch = 0;
+#pragma unroll 4
+        for (; ch < nch_s; ch++) {
+            const uint32_t e = ch * kWalkLanes + u;
+            p = p + __ldg(x + e) * sq[e];
+        }
+        for (; ch < nch; ch++) {
+            const uint32_t e = ch * kWalkLanes + u;
+            p = p + __ldg(x + e) * qp[e];
+        }
+        // (p0 + p4), (p1 + p5), (p2 + p6), (p3 + p7) on lanes 0..3 of the group, then summed in that order on lane 0
+        const double pair = p + __shfl_down_sync(gmask, p, 4, kWalkLanes);
+        const double pr1 = __shfl_sync(gmask, pair, 1, kWalkLanes);
+        const double pr2 = __shfl_sync(gmask, pair, 2, kWalkLanes);
+        const double pr3 = __shfl_sync(gmask, pair, 3, kWalkLanes);
+        if (u == 0) {
+            double sum = 0.0 + pair;
+            sum = sum + pr1;
+            sum = sum + pr2;
+            sum = sum + pr3;
+            for (uint32_t e = nch * kWalkLanes; e < len; e++) sum = sum + __ldg(x + e) * (e < kWalkQCap ? sq[e] : qp[e]);
+            const double sim = sum / (__ldg(&cnorm[pos]) * nq);  // src/sound.rs:30-32
+            walk_min(bd, bi, fabs(sim - target), dsc.w);         // src/sound.rs:359-366
+        }
+    }
+    walk_block_min(bd, bi);
+    if (threadIdx.x == 0) {
+        part_dist[blockIdx.x] = bd;
+        part_idx[blockIdx.x] = bi;
+        __threadfence();
+        last = atomicAdd(&state[0], 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (!last) return;
+    // the last CTA: every other CTA's partial is visible (its fence came before its ticket)
+    __threadfence();
+    bd = 2.0;
+    bi = kCosNone;
+    for (uint32_t b = threadIdx.x; b < gridDim.x; b += kWalkThreads) walk_min(bd, bi, __ldcg(&part_dist[b]), __ldcg(&part_idx[b]));
+    walk_block_min(bd, bi);
+    if (threadIdx.x == 0) {
+        const uint32_t s = bi != kCosNone ? bi : 0;  // nothing < 2.0: index 0, as the fold's seed (src/sound.rs:369)
+        out_idx[step] = s + index_base;
+        out_dist[step] = bd;
+        state[1] = s;
+        state[0] = 0;
+    }
+}
+
+int cosine_walk_dev(ss_dict* d, const double* d_start, const uint64_t* d_start_off, const double* d_targets, size_t nsteps,
+                    uint32_t* d_out_idx, double* d_out_dist) {
+    ss_ctx* ctx = d->ctx;
+    if (!nsteps) return SS_OK;
+    const uint32_t nseg = (uint32_t)d->nseg;
+    const uint32_t grid = (uint32_t)std::min<long long>(ceil_div(nseg, kWalkGroups), (long long)ctx->sm_count * kWalkCtasPerSm);
+    SS_CUDA(ctx, d->d_walk_part_dist.reserve(grid));
+    SS_CUDA(ctx, d->d_walk_part_idx.reserve(grid));
+    SS_CUDA(ctx, d->d_walk_state.reserve(2));
+    SS_CUDA(ctx, d->d_walk_qnorm.reserve(1));
+    SS_CUDA(ctx, cudaMemsetAsync(d->d_walk_state.p, 0, 2 * sizeof(uint32_t), ctx->stream));
+    // the start query's norm by the same kernel as every query's and segment's (src/sound.rs:36-38)
+    k_seg_norm<<<1, 32, 0, ctx->stream>>>(d_start, d_start_off, 1, d->c, d->d_walk_qnorm.p);
+    SS_LAUNCHED(ctx);
+    const uint32_t max_kd = d->max_len * (uint32_t)d->c;
+    for (size_t t = 0; t < nsteps; t++) {
+        k_cosine_walk_step<<<grid, kWalkThreads, 0, ctx->stream>>>(d->d_mfcc.p, d->d_off.p, d->d_norm.p, d->d_cos_seg.p, d->d_cos_norm.p, nseg, d->c,
+                                                                   max_kd, d_start, d_start_off, d->d_walk_qnorm.p, d_targets, (uint32_t)t,
+                                                                   d->index_base, d->d_walk_part_dist.p, d->d_walk_part_idx.p,
+                                                                   d->d_walk_state.p, d_out_idx, d_out_dist);
+        SS_LAUNCHED(ctx);
+    }
+    return SS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // DTW refine: exact f64 recurrence on the candidates. One thread per (query slot, candidate); the DP row lives in a
 // global scratch laid out [column][pair] so that neighbouring threads touch neighbouring addresses.
 // ---------------------------------------------------------------------------------------------------------------

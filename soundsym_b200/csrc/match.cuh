@@ -140,6 +140,14 @@ struct ss_dict {
     struct ss_queries* scratch_q = nullptr;
     ss::DevBuf<uint32_t> d_res_idx;
     ss::DevBuf<double> d_res_dist, d_res_targets;
+    // ss_dict_walk (exact.cu cosine_walk_dev): its own buffers, so that a walk never touches a match's workspaces or the
+    // last_* counters. state = {ticket of the last-CTA reduction, local index of the next step's query}
+    ss::DevBuf<double> d_walk_part_dist, d_walk_qnorm;
+    ss::DevBuf<uint32_t> d_walk_part_idx, d_walk_state;
+    ss::DevBuf<double> d_walk_start, d_walk_targets, d_walk_dist;  // host-buffer entry point: start frames, targets, results
+    ss::DevBuf<uint64_t> d_walk_off;
+    ss::DevBuf<uint32_t> d_walk_idx;
+    uint64_t h_walk_off[2] = {0, 0};
     ~ss_dict();
 };
 
@@ -238,6 +246,9 @@ int fill_result(ss_ctx* ctx, uint32_t* d_idx, double* d_dist, size_t n);  // (in
 int cosine_dict_build(ss_dict* d);    // per-segment norms (cosine.cu)
 int cosine_queries_build(ss_queries* q);
 int cosine_match_dev(ss_dict* d, ss_queries* q, const double* d_targets, uint32_t* d_out_idx, double* d_out_dist);
+// SoundSequence::from_distances for SS_COSINE_REF: nsteps + 1 launches on the ctx stream, no host synchronisation (exact.cu)
+int cosine_walk_dev(ss_dict* d, const double* d_start, const uint64_t* d_start_off, const double* d_targets, size_t nsteps,
+                    uint32_t* d_out_idx, double* d_out_dist);
 int topk_merge_dev(ss_ctx* ctx, const uint32_t* d_idx, const double* d_dist, int nlists, size_t nq, int k,
                    uint32_t* d_out_idx, double* d_out_dist);
 }  // namespace ss
