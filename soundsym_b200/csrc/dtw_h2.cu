@@ -28,8 +28,13 @@
 // bands of 2 interleaved segments each - NB = 1 (segments of 17..32 frames), 2 (9..16) or 4 (<= 8): every step is
 // 2 rows x 64 columns = 128 cells per thread whatever the segment length, so the hand-off cost per cell is the same for
 // short and long segments (the fp32 scan's paired tiles spent 4.5 instructions per cell on short segments).
+// With 8 candidates per query (k <= 2) the NB = 1 and NB = 2 tiles run k_dtw_scan_h2_2p instead: the same geometry twice in
+// one CTA, two pipelines of 8 DP warps + 1 producer warp that each own one 2-row TMEM buffer and take every other tile of the
+// slice, so that one pipeline's warps issue while the other's wait for their MMAs or close a tile (640 threads, setmaxnreg:
+// DP 112 registers, each step's columns pulled in two chunks).
 #include <algorithm>
 #include <atomic>
+#include <type_traits>
 
 #include "match.cuh"
 #include "tc_common.cuh"
@@ -53,6 +58,14 @@ constexpr int kH2DescInt4 = 4;                        // per (tile, slot): {seg 
 constexpr int kH2In = 1, kH2Out = 2;                   // strip flags: boundary column comes in from / goes out to the neighbouring strip
 constexpr int kH2ARing = 32;                          // rows of the A block resident at a time when a query group is longer (4 pieces of 8)
 constexpr int kH2MaxLong = 2048;                      // longest segment / query the strip kernel takes (boundary scratch: %nsmid x rows x 1 KB)
+// k_dtw_scan_h2_2p: two independent pipelines of 8 DP warps per CTA, each with its own 2-row TMEM buffer and producer warp
+constexpr int kH2Pipes = 2;
+constexpr int kH2PDpWarps = kH2Pipes * kH2DpWarps;       // 16; warp w: lane quadrant w % 4, slot (w >> 2) & 1, pipeline w >> 3
+constexpr int kH2PDpThreads = kH2PDpWarps * 32;          // 512
+constexpr int kH2PThreads = (kH2PDpWarps + 4) * 32;      // 640: warps 16, 17 = the producers, 18, 19 = idle register donors
+// setmaxnreg: 640 threads launch with 96 registers; DP 112 / producer warpgroup 32 is the whole pool (512 x 112 + 128 x 32)
+constexpr int kH2PRegsDp = 112, kH2PRegsProd = 32;
+static_assert(kH2PDpThreads * kH2PRegsDp + 128 * kH2PRegsProd == kH2PThreads * 96, "setmaxnreg budget must match the launch pool");
 
 struct H2Params {
     const unsigned char* a_blocks;
@@ -234,29 +247,106 @@ __device__ __forceinline__ void h2_band_row(const __half2 (&tm)[4 * NG], __half2
     }
 }
 
+// columns [J0, J1) of h2_band, the carries (left0, diag0, left1) passed in and out: the same operations in the same order,
+// so a band split into column chunks gives the bits of the whole band (tm0 / tm1 hold columns J0 ..)
+template <int NG, int J0, int J1>
+__device__ __forceinline__ void h2_band_cols(const __half2* tm0, const __half2* tm1, __half2 (&d)[4 * NG], __half2& left0, __half2& diag0,
+                                             __half2& left1, __half2 (&c0l)[4]) {
+#pragma unroll
+    for (int j = J0; j < J1; j++) {
+        const __half2 up0 = d[j];
+        const __half2 c0 = __hadd2(tm0[j - J0], h2_min3(left0, up0, diag0));
+        const __half2 c1 = __hadd2(tm1[j - J0], h2_min3(left1, c0, left0));
+        diag0 = up0;
+        left0 = c0;
+        left1 = c1;
+        d[j] = c1;
+        if (j >= 4 * (NG - 1)) c0l[j - 4 * (NG - 1)] = c0;
+    }
+}
+
+// consumer side of one pipeline's single 2-row TMEM buffer (k_dtw_scan_h2_2p): its "empty" barrier sits 16 bytes above its
+// "full" barrier, as in TcCursor, but the buffer and the barriers never change - only the parity flips
+struct H2PipeCursor {
+    uint32_t par, full, taddr;
+    __device__ __forceinline__ void wait() const {
+        mb_wait_addr(full, par);
+        tc_fence_after();
+    }
+    __device__ __forceinline__ void release() {
+        tc_fence_before();
+        mb_arrive_elect(full + 16);
+        par ^= 1u;
+    }
+};
+
 // one pipeline step for one thread: wait for the step's MMAs, pull the NB bands' columns of both rows, hand the buffer back,
-// advance the bands
-template <int NB, int NG>
-__device__ __forceinline__ void h2_step2(TcCursor& cur, __half2 (&d)[NB][4 * NG], __half2 dinit, __half2 (&c0l)[NB][4]) {
+// advance the bands. With the single-buffer cursor (112 registers) the columns come in two chunks of at most 32 registers:
+// the first 16 registers of each row (NB = 1) or the first half of the bands, then the rest; the buffer goes back after the
+// second chunk's loads.
+template <int NB, int NG, class Cur>
+__device__ __forceinline__ void h2_step2(Cur& cur, __half2 (&d)[NB][4 * NG], __half2 dinit, __half2 (&c0l)[NB][4]) {
     constexpr int kBandCols = kH2SlotCols / NB;
     cur.wait();
     const uint32_t taddr = cur.taddr;
-    __half2 tm0[NB][4 * NG], tm1[NB][4 * NG];
+    if constexpr (std::is_same<Cur, H2PipeCursor>::value && NB == 1) {
+        static_assert(NG >= 5, "NB = 1 tiles have 5..8 column groups");
+        __half2 left0 = h2_inf(), diag0 = dinit, left1 = h2_inf();
+        {
+            __half2 a0[16], a1[16];
+            h2_ld_row<4>(taddr, a0);
+            h2_ld_row<4>(taddr + kTcN, a1);
+            tc_wait_ld();
+            h2_band_cols<NG, 0, 16>(a0, a1, d[0], left0, diag0, left1, c0l[0]);
+        }
+        __half2 b0[4 * (NG - 4)], b1[4 * (NG - 4)];
+        h2_ld_row<NG - 4>(taddr + 32, b0);
+        h2_ld_row<NG - 4>(taddr + kTcN + 32, b1);
+        tc_wait_ld();
+        cur.release();
+        h2_band_cols<NG, 16, 4 * NG>(b0, b1, d[0], left0, diag0, left1, c0l[0]);
+    } else if constexpr (std::is_same<Cur, H2PipeCursor>::value) {
+        constexpr int H = NB / 2;
+        {
+            __half2 tm0[H][4 * NG], tm1[H][4 * NG];
 #pragma unroll
-    for (int b = 0; b < NB; b++) {
-        h2_ld_row<NG>(taddr + b * kBandCols, tm0[b]);
-        h2_ld_row<NG>(taddr + kTcN + b * kBandCols, tm1[b]);
+            for (int b = 0; b < H; b++) {
+                h2_ld_row<NG>(taddr + b * kBandCols, tm0[b]);
+                h2_ld_row<NG>(taddr + kTcN + b * kBandCols, tm1[b]);
+            }
+            tc_wait_ld();
+#pragma unroll
+            for (int b = 0; b < H; b++) h2_band<NG>(tm0[b], tm1[b], d[b], dinit, c0l[b]);
+        }
+        __half2 tm0[H][4 * NG], tm1[H][4 * NG];
+#pragma unroll
+        for (int b = 0; b < H; b++) {
+            h2_ld_row<NG>(taddr + (H + b) * kBandCols, tm0[b]);
+            h2_ld_row<NG>(taddr + kTcN + (H + b) * kBandCols, tm1[b]);
+        }
+        tc_wait_ld();
+        cur.release();
+#pragma unroll
+        for (int b = 0; b < H; b++) h2_band<NG>(tm0[b], tm1[b], d[H + b], dinit, c0l[H + b]);
+    } else {
+        __half2 tm0[NB][4 * NG], tm1[NB][4 * NG];
+#pragma unroll
+        for (int b = 0; b < NB; b++) {
+            h2_ld_row<NG>(taddr + b * kBandCols, tm0[b]);
+            h2_ld_row<NG>(taddr + kTcN + b * kBandCols, tm1[b]);
+        }
+        tc_wait_ld();
+        cur.release();
+#pragma unroll
+        for (int b = 0; b < NB; b++) h2_band<NG>(tm0[b], tm1[b], d[b], dinit, c0l[b]);
     }
-    tc_wait_ld();
-    cur.release();
-#pragma unroll
-    for (int b = 0; b < NB; b++) h2_band<NG>(tm0[b], tm1[b], d[b], dinit, c0l[b]);
 }
 
 // One dictionary tile for one thread (= one query x one slot = 2 NB segments). ra / rb: position of column len - 1 inside the
 // last 4-column group, for the band's first (low halves) and second (high halves) segment. res[b] = D(Lm - 1, len - 1) of both.
-template <int NB, int NG>
-__device__ __forceinline__ void h2_tile(uint32_t L, uint32_t lmin, uint32_t Lm, const int4& sc, TcCursor& cur, __half2 (&res)[NB]) {
+// Cur: TcCursor (two TMEM buffers, k_dtw_scan_h2 / _long) or H2PipeCursor (one buffer per pipeline, k_dtw_scan_h2_2p).
+template <int NB, int NG, class Cur>
+__device__ __forceinline__ void h2_tile(uint32_t L, uint32_t lmin, uint32_t Lm, const int4& sc, Cur& cur, __half2 (&res)[NB]) {
     __half2 d[NB][4 * NG];
 #pragma unroll
     for (int b = 0; b < NB; b++) {
@@ -268,33 +358,43 @@ __device__ __forceinline__ void h2_tile(uint32_t L, uint32_t lmin, uint32_t Lm, 
     const uint32_t nfull = L >> 1;                       // steps that carry two rows
     const uint32_t ncap = min((lmin - 1) >> 1, nfull);   // steps before any query of the group can end
     uint32_t st = 0;
-    // steps [0, ncap): no query of the group ends; two per iteration on buffers 0, 1 with loop-invariant addresses
-    if (st < ncap && cur.buf) {
-        __half2 c0l[NB][4];
-        h2_step2<NB, NG>(cur, d, dinit, c0l);
-        dinit = h2_inf();
-        st++;
-    }
-    if (st + 2 <= ncap) {
-        const uint32_t full0 = cur.full, taddr0 = cur.taddr;
-        uint32_t par = cur.par;
+    if constexpr (std::is_same<Cur, H2PipeCursor>::value) {
+        // steps [0, ncap): no query of the group ends; one buffer, so every step has the same addresses
 #pragma unroll 1
-        for (; st + 2 <= ncap; st += 2) {
+        for (; st < ncap; st++) {
             __half2 c0l[NB][4];
-            TcCursor c0 = {0u, par, full0, taddr0, cur.full_sum, cur.taddr_sum};
-            h2_step2<NB, NG>(c0, d, dinit, c0l);
-            TcCursor c1 = {1u, par, full0 + 8u, taddr0 + (uint32_t)kTcBufCols, cur.full_sum, cur.taddr_sum};
-            h2_step2<NB, NG>(c1, d, h2_inf(), c0l);
+            h2_step2<NB, NG>(cur, d, dinit, c0l);
             dinit = h2_inf();
-            par ^= 1u;
         }
-        cur.par = par;
-    }
-    if (st < ncap) {
-        __half2 c0l[NB][4];
-        h2_step2<NB, NG>(cur, d, dinit, c0l);
-        dinit = h2_inf();
-        st++;
+    } else {
+        // steps [0, ncap): no query of the group ends; two per iteration on buffers 0, 1 with loop-invariant addresses
+        if (st < ncap && cur.buf) {
+            __half2 c0l[NB][4];
+            h2_step2<NB, NG>(cur, d, dinit, c0l);
+            dinit = h2_inf();
+            st++;
+        }
+        if (st + 2 <= ncap) {
+            const uint32_t full0 = cur.full, taddr0 = cur.taddr;
+            uint32_t par = cur.par;
+#pragma unroll 1
+            for (; st + 2 <= ncap; st += 2) {
+                __half2 c0l[NB][4];
+                TcCursor c0 = {0u, par, full0, taddr0, cur.full_sum, cur.taddr_sum};
+                h2_step2<NB, NG>(c0, d, dinit, c0l);
+                TcCursor c1 = {1u, par, full0 + 8u, taddr0 + (uint32_t)kTcBufCols, cur.full_sum, cur.taddr_sum};
+                h2_step2<NB, NG>(c1, d, h2_inf(), c0l);
+                dinit = h2_inf();
+                par ^= 1u;
+            }
+            cur.par = par;
+        }
+        if (st < ncap) {
+            __half2 c0l[NB][4];
+            h2_step2<NB, NG>(cur, d, dinit, c0l);
+            dinit = h2_inf();
+            st++;
+        }
     }
 #pragma unroll 1
     for (; st < nfull; st++) {  // only the last step or two of a tile: some query of the group can end here
@@ -584,6 +684,211 @@ __global__ void __launch_bounds__(kH2Threads, 1) k_dtw_scan_h2(const H2Params p)
     tc_fence_before();
     __syncthreads();
     if (warp == kH2DpWarps) {
+        tc_fence_after();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    }
+    if (tl && threadIdx.x == 0) tl[3] = h2_now();
+}
+
+// ---- the same scan with TWO PIPELINES per CTA (KP = 8, the first stage for k <= 2). In k_dtw_scan_h2 all 8 DP warps wait
+// for the same buffer, load it, hand it back and reach the end of a tile together, so nothing covers those latencies (ncu:
+// 2.25 eligible warps per scheduler, issue 47 %). Here pipeline p = 0, 1 walks the tiles t0 + p, t0 + p + 2, .. of the
+// slice with its own 8 DP warps, its own 2-row TMEM buffer (columns [256 p, 256 p + 256)), its own producer warp with its
+// own B ring and barriers: the two run out of phase, and while one waits for its MMAs or closes a tile the other's warps
+// issue. The A block is copied once (producer 0) and both producers wait for it. MMA shape, operands and the band code are
+// those of k_dtw_scan_h2, so every pair's scan value has the same bits. The 4 lists of a query (2 slots x 2 pipelines) are
+// merged before the partial write.
+template <int KP, int NB, bool DBG = false>
+__global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Params p) {
+    extern __shared__ unsigned char smem_raw[];
+    // [A tiles: max_len x 4 KB][B rings: 2 pipelines x 4 x 4 KB][barriers][candidate lists [KP][512]], 128-byte aligned
+    unsigned char* smem = smem_raw + ((128u - (s32(smem_raw) & 127u)) & 127u);
+    unsigned char* sA = smem;
+    unsigned char* sB = smem + (size_t)p.max_len * kTcATileBytes;
+    // barriers (u64): a_full | b_full[4], b_empty[4] of pipeline 0 | the same of pipeline 1 | t_full[2] | t_empty[2]
+    uint64_t* bars = reinterpret_cast<uint64_t*>(sB + kH2Pipes * kTcStages * kTcBTileBytes);
+    uint64_t* a_full = bars;
+    uint64_t* t_full = bars + 1 + 2 * kH2Pipes * kTcStages;  // 17
+    uint64_t* t_empty = t_full + kH2Pipes;                   // = t_full + 16 bytes (H2PipeCursor::release)
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(t_empty + kH2Pipes);
+    unsigned long long* topk = reinterpret_cast<unsigned long long*>(bars + 32);  // [KP][512]
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    // CTA order as in k_dtw_scan_h2: the first slice of every group, then the others
+    uint32_t g, slice;
+    if (blockIdx.x < p.ngroups) {
+        g = blockIdx.x, slice = p.slice_begin;
+    } else {
+        const uint32_t r = blockIdx.x - p.ngroups;
+        g = r / (p.nslices - 1), slice = p.slice_begin + 1 + r % (p.nslices - 1);
+    }
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // the next tile kind's launch may start filling SMs
+    const uint32_t glen = p.group_len[g];
+    const uint32_t L = glen & 0xFFFFu, lmin = glen >> 16;
+    const uint32_t t0 = p.slice_tile[slice], t1 = p.slice_tile[slice + 1];
+    const uint32_t ntiles = t1 - t0;
+    unsigned long long* tl = p.timeline ? p.timeline + ((size_t)(p.slice_begin * p.ngroups) + blockIdx.x) * 8 : nullptr;
+    if (tl && threadIdx.x == 0) {
+        unsigned smid;
+        asm("mov.u32 %0, %%smid;" : "=r"(smid));
+        tl[0] = h2_now(), tl[4] = smid | ((unsigned long long)NB << 16) | ((unsigned long long)g << 32), tl[7] = ((unsigned long long)L << 32) | ntiles;
+    }
+
+    if (threadIdx.x == 0) {
+        mb_init(a_full, 1);
+        for (int s = 0; s < 2 * kH2Pipes * kTcStages; s++) mb_init(&bars[1 + s], 1);
+        for (int s = 0; s < kH2Pipes; s++) mb_init(&t_full[s], 1), mb_init(&t_empty[s], kH2DpWarps);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == kH2PDpWarps) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(512u) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = *tmem_slot;
+    if (tl && threadIdx.x == 0) tl[1] = h2_now(), tl[5] = clock64();
+    if (warp >= kH2PDpWarps) {
+        asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kH2PRegsProd));
+        const uint32_t pipe = (uint32_t)(warp - kH2PDpWarps);
+        const uint32_t ntp = ntiles > pipe ? (ntiles - pipe + 1) >> 1 : 0u;  // this pipeline's tiles: t0 + pipe, t0 + pipe + 2, ..
+        if (pipe < (uint32_t)kH2Pipes && lane == 0 && ntp) {
+            // ---- producer of pipeline `pipe`: its B ring (TMA), its MMAs; producer 0 also copies the A block ---------------
+            const uint32_t bars_s = s32(bars), sA_s = s32(sA), sB_s = s32(sB) + pipe * (kTcStages * kTcBTileBytes);
+            const uint32_t a_full_s = bars_s, b_full_s = bars_s + 8 + pipe * (16 * kTcStages), b_empty_s = b_full_s + 8 * kTcStages,
+                           t_full_s = s32(t_full) + 8 * pipe, t_empty_s = t_full_s + 16;
+            if (pipe == 0) {
+                mbs_expect_tx(a_full_s, L * kTcATileBytes);
+                tmas_g2s(sA_s, p.a_blocks + p.group_off[g], L * kTcATileBytes, a_full_s);
+            }
+            constexpr size_t kStride = (size_t)kH2Pipes * kTcBTileBytes;  // this pipeline's next tile
+            const unsigned char* tile_src = p.tiles + (size_t)(t0 + pipe) * kTcBTileBytes;
+            for (uint32_t n = 0; n < ntp && n < (uint32_t)kTcStages; n++) {
+                mbs_expect_tx(b_full_s + 8 * n, kTcBTileBytes);
+                tmas_g2s(sB_s + n * kTcBTileBytes, tile_src + n * kStride, kTcBTileBytes, b_full_s + 8 * n);
+            }
+            tile_src += kTcStages * kStride;
+            mbs_wait_sleep(a_full_s, 0);
+            // f16 x f16 -> F16 accumulator (c_format = 0), K-major both, N = 128, M = 128
+            const uint32_t idesc = (0u << 4) | ((uint32_t)(kTcN >> 3) << 17) | ((uint32_t)(kTcM >> 4) << 24);
+            const uint64_t adesc0 = tc_smem_desc_s<kTcM>(sA_s);
+            const uint32_t tm = tmem_base + pipe * kTcBufCols;
+            uint32_t cnt = 0, stage = 0, sphase = 0;
+            for (uint32_t n = 0; n < ntp; n++) {
+                mbs_wait_sleep(b_full_s + 8 * stage, sphase);
+                const uint64_t bdesc = tc_smem_desc_s<kTcN>(sB_s + stage * kTcBTileBytes);
+                uint64_t adesc = adesc0;
+                for (uint32_t row = 0; row < L; row += 2, cnt++) {
+                    if (cnt >= 1) mbs_wait_sleep(t_empty_s, (cnt - 1) & 1);  // the pipeline's 8 DP warps have pulled the last step
+                    tc_fence_after();
+                    tc_mma_f16(tm, adesc, bdesc, idesc);
+                    if (row + 1 < L) tc_mma_f16(tm + kTcN, adesc + (kTcATileBytes >> 4), bdesc, idesc);
+                    tcs_commit(t_full_s);
+                    adesc += 2 * (kTcATileBytes >> 4);
+                }
+                tcs_commit(b_empty_s + 8 * stage);
+                if (n + kTcStages < ntp) {
+                    mbs_wait_sleep(b_empty_s + 8 * stage, sphase);
+                    mbs_expect_tx(b_full_s + 8 * stage, kTcBTileBytes);
+                    tmas_g2s(sB_s + stage * kTcBTileBytes, tile_src, kTcBTileBytes, b_full_s + 8 * stage);
+                    tile_src += kStride;
+                }
+                if (++stage == (uint32_t)kTcStages) stage = 0, sphase ^= 1;
+            }
+        }
+    } else {
+        // ---- DP warps ---------------------------------------------------------------------------------------------------
+        asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kH2PRegsDp));
+        const int q = warp & 3, slot = (warp >> 2) & 1, pipe = warp >> 3;
+        const int m = q * 32 + lane;
+        unsigned long long* list = topk + threadIdx.x;  // [KP][512] keys, this thread's column
+#pragma unroll
+        for (int s = 0; s < KP; s++) list[s * kH2PDpThreads] = 0xFFFFFFFFFFFFFFFFull;
+        const unsigned long long thr0 = __ldcg(p.thr + g * kTcM + m);  // (L2: other CTAs update it)
+        unsigned long long worst = thr0;
+        int cnt = 0, wpos = 0;  // unsorted list while the slice is scanned, as in k_dtw_scan_h2
+        const uint32_t Lm = p.slot_len[g * kTcM + m];  // this lane's own query length
+        H2PipeCursor cur = {0u, s32(t_full + pipe), tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(pipe * kTcBufCols + slot * kH2SlotCols)};
+        const uint32_t ntp = ntiles > (uint32_t)pipe ? (ntiles - pipe + 1) >> 1 : 0u;
+        // the NEXT tile's descriptors are fetched while the current tile is processed
+        const int4* dp = p.desc + ((size_t)(t0 + pipe) * kH2Slots + slot) * kH2DescInt4;
+        int4 na = make_int4(0, 0, 0, 0), nb = na, nc = na;
+        if (ntp) na = __ldg(dp), nb = __ldg(dp + 1), nc = __ldg(dp + 2);
+        for (uint32_t n = 0; n < ntp; n++) {
+            const int4 sa = na, sb = nb, sc = nc;
+            dp += kH2Pipes * kH2Slots * kH2DescInt4;
+            if (n + 1 < ntp) na = __ldg(dp), nb = __ldg(dp + 1), nc = __ldg(dp + 2);
+            const int ng = sc.z;
+            __half2 res[NB];
+            if constexpr (NB == 1) {
+                switch (ng) {
+                    case 5: h2_tile<1, 5>(L, lmin, Lm, sc, cur, res); break;
+                    case 6: h2_tile<1, 6>(L, lmin, Lm, sc, cur, res); break;
+                    case 7: h2_tile<1, 7>(L, lmin, Lm, sc, cur, res); break;
+                    default: h2_tile<1, 8>(L, lmin, Lm, sc, cur, res); break;
+                }
+            } else if constexpr (NB == 2) {
+                if (ng == 3) h2_tile<2, 3>(L, lmin, Lm, sc, cur, res);
+                else h2_tile<2, 4>(L, lmin, Lm, sc, cur, res);
+            } else {
+                if (ng == 1) h2_tile<4, 1>(L, lmin, Lm, sc, cur, res);
+                else h2_tile<4, 2>(L, lmin, Lm, sc, cur, res);
+            }
+            if (tl && threadIdx.x == 0 && n + 1 == (ntp + 1) / 2) tl[6] = h2_now();  // (measurement: half of pipeline 0's tiles)
+            if (Lm) {
+#pragma unroll
+                for (int b = 0; b < NB; b++) {
+#pragma unroll
+                    for (int hsel = 0; hsel < 2; hsel++) {
+                        const int e = 2 * b + hsel;
+                        const int seg = h2_seg_of(sa, sb, e);
+                        if (seg >= 0) {
+                            const float v = hsel ? __high2float(res[b]) : __low2float(res[b]);
+                            const float dist = __fdividef(v * p.inv_s, (float)(Lm + (uint32_t)h2_len_of(sc, e)));
+                            const unsigned long long key = ((unsigned long long)tc_f2ord(dist) << 32) | (uint32_t)seg;
+                            if (key < worst && dist == dist) {
+                                const bool full = cnt == KP;
+                                list[(full ? wpos : cnt) * kH2PDpThreads] = key;
+                                cnt += full ? 0 : 1;
+                                if (cnt == KP) {
+                                    tc_list_max<KP, kH2PDpThreads>(list, worst, wpos);
+                                    worst = worst < thr0 ? worst : thr0;
+                                }
+                            }
+                            if constexpr (DBG) p.dbg[(size_t)(g * kTcM + m) * p.dbg_nseg + seg] = dist;
+                        }
+                    }
+                }
+            }
+        }
+        tc_sort_list<KP, kH2PDpThreads>(list, cnt);  // (the places beyond cnt still hold the initial +inf keys)
+        worst = list[(KP - 1) * kH2PDpThreads];
+        worst = worst < thr0 ? worst : thr0;
+        // the four lists of query m (threads m + 128 s, s = slot + 2 pipeline) are merged by thread m
+        asm volatile("bar.sync 1, %0;" ::"n"(kH2PDpThreads) : "memory");
+        if (tl && threadIdx.x == 0) tl[2] = h2_now(), tl[5] = clock64() - tl[5];  // SM cycles of the DP phase (-> the SM clock under load)
+        if (threadIdx.x < kTcM) {
+            for (int o = 1; o < kH2Pipes * kH2Slots; o++) {
+                const unsigned long long* other = list + o * kTcM;
+                for (int s = 0; s < KP; s++) {  // ascending: stop at the first key that does not make the cut
+                    const unsigned long long key = other[s * kH2PDpThreads];
+                    if (key >= worst) break;
+                    tc_insert_key<KP, kH2PDpThreads>(list, worst, key);
+                    worst = worst < thr0 ? worst : thr0;
+                }
+            }
+            const unsigned long long kept_worst = list[(KP - 1) * kH2PDpThreads];
+            if (kept_worst != 0xFFFFFFFFFFFFFFFFull && kept_worst < thr0) atomicMin(p.thr + g * kTcM + m, kept_worst);
+            unsigned long long* out = p.partial + ((size_t)slice * p.ngroups * kTcM + (size_t)g * kTcM + m) * KP;
+#pragma unroll
+            for (int s = 0; s < KP; s++) out[s] = list[s * kH2PDpThreads];
+        }
+    }
+    if constexpr (NB != 1) asm volatile("griddepcontrol.wait;" ::: "memory");  // see k_dtw_scan_tc: not complete before the launch ahead is
+    tc_fence_before();
+    __syncthreads();
+    if (warp == kH2PDpWarps) {
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
     }
@@ -1021,16 +1326,32 @@ static int h2_queries_build(ss_dict* d, ss_queries* q) {
     return SS_OK;
 }
 
+// Candidates kept per query for k <= 2. Measured at config 4 (profiles/bench/r2_h2_kp_sweep.json): 8 leaves 47 of the 10 000
+// queries uncertified by the merged list, but the scan itself is 3 ms faster than with 16.
+constexpr int kH2Kp = 8;
+
 template <int KP, int NB, bool DBG, bool LONG>
 static int h2_launch_kind(ss_ctx* ctx, H2Params p, uint32_t slice_begin, uint32_t nslices, size_t smem, bool dependent) {
     if (!nslices) return SS_OK;
     p.slice_begin = slice_begin;
     p.nslices = nslices;
-    auto kern = LONG ? k_dtw_scan_h2_long<KP, NB, DBG> : k_dtw_scan_h2<KP, NB, DBG>;
+    // KP = 8 (k <= 2) runs the two-pipeline kernel for NB = 1 and 2. Its 32-entry lists (H2_WIDE, k > 2) would need 128 KB of
+    // shared memory, and NB = 4 does not fit its 112 DP registers without spilling: both keep the one-pipeline kernel.
+    void (*kern)(H2Params);
+    unsigned threads = kH2Threads;
+    if constexpr (LONG) {
+        kern = k_dtw_scan_h2_long<KP, NB, DBG>;
+    } else if constexpr (KP == kH2Kp && NB != 4) {
+        kern = k_dtw_scan_h2_2p<KP, NB, DBG>;
+        threads = kH2PThreads;
+        smem = (size_t)p.max_len * kTcATileBytes + kH2Pipes * kTcStages * kTcBTileBytes + 32 * 8 + (size_t)KP * kH2PDpThreads * 8 + 1024;
+    } else {
+        kern = k_dtw_scan_h2<KP, NB, DBG>;
+    }
     SS_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(p.ngroups * nslices);
-    cfg.blockDim = dim3(kH2Threads);
+    cfg.blockDim = dim3(threads);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = ctx->stream;
     cudaLaunchAttribute attr[1];
@@ -1054,9 +1375,6 @@ struct H2Plan {
     bool use_long;  // segments or queries of more than 32 frames: k_dtw_scan_h2_long (strips, streamed A block, deflated keys)
 };
 constexpr int kH2Waves = 16;  // CTAs per SM over the launches of one scan
-// Candidates kept per query for k <= 2. Measured at config 4 (profiles/bench/r2_h2_kp_sweep.json): 8 leaves 47 of the 10 000
-// queries uncertified by the merged list, but the scan itself is 3 ms faster than with 16.
-constexpr int kH2Kp = 8;
 
 static int h2_plan(ss_dict* d, ss_queries* q, int kp, H2Plan* plan) {
     ss_ctx* ctx = d->ctx;
