@@ -388,6 +388,30 @@ class SoundDictionary {
         dist->assign(distances.size(), 0.0);
         ctx_->check(ss_dict_walk(d, start.mfccs().data(), start.num_frames(), distances.data(), distances.size(), idx->data(), dist->data()));
     }
+    /// DTW warping path (ss_dict_align) of queries[p] against sounds[indices[p]] (indices as match_indices returns them;
+    /// 0xFFFFFFFF -> empty path, inf): (*paths)[p] holds (frame of the query, frame of the dictionary sound) pairs in order.
+    /// Works in either mode: the path is the SS_DTW one whatever matcher chose the indices.
+    void align(const std::vector<std::shared_ptr<Sound>>& queries, const std::vector<uint32_t>& indices,
+               std::vector<std::vector<std::pair<uint32_t, uint32_t>>>* paths, std::vector<double>* dist) {
+        if (indices.size() != queries.size()) ctx_->check(SS_ERR_INVALID);
+        ss_dict* d = device();
+        std::vector<uint64_t> off(queries.size() + 1, 0);
+        std::vector<double> flat;
+        size_t cap = 0;
+        for (size_t i = 0; i < queries.size(); i++) {
+            off[i + 1] = off[i] + queries[i]->num_frames();
+            flat.insert(flat.end(), queries[i]->mfccs().begin(), queries[i]->mfccs().end());
+            if (indices[i] < sounds.size() && queries[i]->num_frames() && sounds[indices[i]]->num_frames())
+                cap += queries[i]->num_frames() + sounds[indices[i]]->num_frames() - 1;
+        }
+        std::vector<uint32_t> cells(2 * std::max<size_t>(cap, 1));
+        std::vector<uint64_t> poff(queries.size() + 1);
+        dist->assign(queries.size(), 0.0);
+        ctx_->check(ss_dict_align(d, flat.data(), off.data(), queries.size(), indices.data(), cells.data(), cap, poff.data(), dist->data()));
+        paths->assign(queries.size(), {});
+        for (size_t p = 0; p < queries.size(); p++)
+            for (uint64_t e = poff[p]; e < poff[p + 1]; e++) (*paths)[p].emplace_back(cells[2 * e], cells[2 * e + 1]);
+    }
     /// SoundDictionary::match_sound (src/sound.rs:346-348)
     std::shared_ptr<Sound> match_sound(const std::shared_ptr<Sound>& other) { return at_distance(1.0, other); }
     Context& context() const { return *ctx_; }

@@ -179,6 +179,24 @@ int ss_dict_walk(ss_dict* dict, const double* start_mfcc, size_t start_frames, c
  * `start` holds exactly one query */
 int ss_dict_walk_dev(ss_dict* dict, ss_queries* start, const double* d_distances, size_t nsteps, uint32_t* d_out_idx,
                      double* d_out_dist);
+/* DTW warping path of query p against dictionary segment seg_idx[p] (an index as ss_dict_match
+ * reports it, index_base included; 0xFFFFFFFF -> empty path, inf). out_path: (i, j) uint32 pairs, compacted; path p is
+ * out_path[out_path_offsets[p] .. out_path_offsets[p+1]) (nq + 1 offsets, in pairs). out_dist[p] is bit-equal to ss_dict_match's
+ * SS_DTW distance; an empty side or a distance that is not finite gives an empty path and inf. The path runs from (0, 0) to
+ * (Lq-1, Ld-1); backtracking through the DTW matrix D, each step takes the smallest D of diag (i-1, j-1), up (i-1, j), left
+ * (i, j-1), ties in that order, NaN as +inf (DESIGN.md §3.1e). path_capacity is in cells:
+ * at least the sum over the pairs with both sides non-empty of (Lq + Ld - 1); less, or an index out of range, returns
+ * SS_ERR_INVALID. Works whatever mode the dictionary was last matched in. A pending SS_DTW match completes first; the
+ * ss_dict_last_* readers still describe the last MATCH. Host buffers, stream-synchronised on return. */
+int ss_dict_align(ss_dict* dict, const double* q_mfcc, const uint64_t* q_frame_offsets, size_t nq, const uint32_t* seg_idx,
+                  uint32_t* out_path, size_t path_capacity, uint64_t* out_path_offsets, double* out_dist);
+/* the same on device pointers, asynchronous on the ctx stream (no host synchronisation besides completing a pending SS_DTW match),
+ * so that it can take ss_dict_match_dev's d_out_idx (k = 1) as d_seg_idx directly. path_capacity >= the sum over non-empty queries of
+ * (Lq + Ld_max - 1), Ld_max = the longest segment (checked on the host); an index out of range, which only the device sees, gives an
+ * empty path and NaN. Launches: 3 + one per wave of pairs with a side longer than 32 frames (waves are sized on the host from the
+ * query lengths and Ld_max, so the count is known before the call); nq == 0 launches nothing. */
+int ss_dict_align_dev(ss_dict* dict, ss_queries* q, const uint32_t* d_seg_idx, uint32_t* d_out_path, size_t path_capacity,
+                      uint64_t* d_out_path_offsets, double* d_out_dist);
 int ss_topk_merge_dev(ss_ctx* ctx, const uint32_t* d_idx, const double* d_dist, int nlists, size_t nq, int k,
                       uint32_t* d_out_idx, double* d_out_dist);
 /* drops the cached device layouts of a query batch so that the next match rebuilds them (bench.py calls this every

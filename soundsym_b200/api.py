@@ -219,6 +219,7 @@ class DeviceDictionary:
         if ncoeffs is None:
             ncoeffs = mfcc_flat.shape[1]
         self.ncoeffs = int(ncoeffs)
+        self.max_len = int(np.max(np.diff(off))) if off.shape[0] > 1 else 0
         h = C.c_void_p()
         ctx.check(ctx.lib.ss_dict_create(ctx.h, _ptr(mfcc_flat), _ptr(off), off.shape[0] - 1, self.ncoeffs, int(index_base), C.byref(h)))
         self.h = h
@@ -258,6 +259,23 @@ class DeviceDictionary:
         dist = np.empty(n, dtype=np.float64)
         self.ctx.check(self.ctx.lib.ss_dict_walk(self.h, _ptr(s), s.shape[0], _ptr(t), n, _ptr(idx), _ptr(dist)))
         return idx, dist
+
+    def align(self, q_flat, q_frame_offsets, seg_idx):
+        """ss_dict_align: the DTW warping path (DESIGN.md §3.1e) of query p against segment seg_idx[p] (an index as
+        match reports it; 0xFFFFFFFF -> empty path, inf) -> (paths: list of uint32 [n, 2] arrays of (i, j), dist f64 [nq])."""
+        q = np.ascontiguousarray(q_flat, dtype=np.float64)
+        qo = np.ascontiguousarray(q_frame_offsets, dtype=np.uint64)
+        seg = np.ascontiguousarray(seg_idx, dtype=np.uint32).reshape(-1)
+        nq = qo.shape[0] - 1
+        if seg.shape[0] != nq:
+            raise SoundsymError(_lib.SS_ERR_INVALID, "one segment index per query (%d queries, %d indices)" % (nq, seg.shape[0]))
+        lq = np.diff(qo).astype(np.int64)
+        cap = int(np.sum(lq[lq > 0] + max(self.max_len, 1) - 1))  # >= the sum of Lq + Ld - 1 the call requires
+        path = np.empty((max(cap, 1), 2), dtype=np.uint32)
+        poff = np.empty(nq + 1, dtype=np.uint64)
+        dist = np.empty(nq, dtype=np.float64)
+        self.ctx.check(self.ctx.lib.ss_dict_align(self.h, _ptr(q), _ptr(qo), nq, _ptr(seg), _ptr(path), cap, _ptr(poff), _ptr(dist)))
+        return [path[int(poff[p]):int(poff[p + 1])].copy() for p in range(nq)], dist
 
     def debug_tc_scan(self, q_flat, q_frame_offsets):
         """ss_dict_debug_tc_scan: raw tensor-core scan distance of every (query, segment) pair -> (scan f32 [nq, nseg],
@@ -647,6 +665,16 @@ class SoundDictionary:
         off[1:] = np.cumsum(lens)
         flat = np.concatenate([s.mfcc_arrays() for s in sounds], axis=0) if int(off[-1]) else np.zeros((0, NCOEFFS))
         return self._device().match(flat, off, self.mode, k, targets)
+
+    def align(self, sounds, indices):
+        """the DTW warping path of every sound against the dictionary sound of the same position in `indices` (as
+        match_indices returns them) -> (paths: list of uint32 [n, 2] arrays of (frame of the sound, frame of the dictionary
+        sound), dist f64). Works in either mode: the path is the SS_DTW one whatever matcher chose the indices."""
+        lens = np.array([s.num_frames() for s in sounds], dtype=np.uint64)
+        off = np.zeros(len(lens) + 1, dtype=np.uint64)
+        off[1:] = np.cumsum(lens)
+        flat = np.concatenate([s.mfcc_arrays() for s in sounds], axis=0) if int(off[-1]) else np.zeros((0, NCOEFFS))
+        return self._device().align(flat, off, indices)
 
     def at_distance(self, distance, other):
         """src/sound.rs:351-370 (always Some)."""

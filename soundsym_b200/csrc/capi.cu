@@ -365,6 +365,82 @@ int ss_dict_walk(ss_dict* d, const double* start_mfcc, size_t start_frames, cons
     return rc;
 }
 
+// DTW warping paths (DESIGN.md §3.1e). Alignment takes indices, not a matcher: it works whatever mode the dictionary was last
+// matched in. Like a walk it first completes a pending SS_DTW match, has its own workspaces and leaves the ss_dict_last_*
+// counters as the last match left them.
+static size_t align_capacity_dev(const ss_dict* d, const uint64_t* h_qoff, size_t nq) {
+    const uint64_t wpad = std::max<uint32_t>(d->max_len, 1) - 1;
+    size_t cells = 0;
+    for (size_t p = 0; p < nq; p++)
+        if (h_qoff[p + 1] > h_qoff[p]) cells += h_qoff[p + 1] - h_qoff[p] + wpad;
+    return cells;
+}
+
+int ss_dict_align_dev(ss_dict* d, ss_queries* q, const uint32_t* d_seg_idx, uint32_t* d_out_path, size_t path_capacity,
+                      uint64_t* d_out_path_offsets, double* d_out_dist) {
+    if (!d || !q) return set_error(d ? d->ctx : nullptr, SS_ERR_INVALID, "dict / queries is NULL");
+    ss_ctx* ctx = d->ctx;
+    if (q->ctx != ctx) return set_error(ctx, SS_ERR_INVALID, "dict and queries belong to different contexts");
+    if (q->c != d->c) return set_error(ctx, SS_ERR_INVALID, "ncoeffs mismatch: dict %d, queries %d", d->c, q->c);
+    if (!d_out_path_offsets) return set_error(ctx, SS_ERR_INVALID, "d_out_path_offsets is NULL");
+    if (q->nq && (!d_seg_idx || !d_out_dist)) return set_error(ctx, SS_ERR_INVALID, "index / distance pointers are NULL");
+    const size_t need = align_capacity_dev(d, q->h_off.data(), q->nq);
+    if (path_capacity < need)
+        return set_error(ctx, SS_ERR_INVALID, "path_capacity %zu < %zu cells (sum of Lq + Ld_max - 1 over non-empty queries)", path_capacity, need);
+    if (need && !d_out_path) return set_error(ctx, SS_ERR_INVALID, "d_out_path is NULL");
+    SS_CUDA(ctx, cudaSetDevice(ctx->device));
+    SS_TRY(dtw_match_finish(d));  // a pending SS_DTW match completes first (its d_out_idx may be this call's d_seg_idx)
+    return dtw_align_dev(d, q->d_mfcc.p, q->d_off.p, q->h_off.data(), q->nq, d_seg_idx, d_out_path, d_out_path_offsets, d_out_dist);
+}
+
+int ss_dict_align(ss_dict* d, const double* q_mfcc, const uint64_t* q_frame_offsets, size_t nq, const uint32_t* seg_idx, uint32_t* out_path,
+                  size_t path_capacity, uint64_t* out_path_offsets, double* out_dist) {
+    if (!d) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
+    ss_ctx* ctx = d->ctx;
+    if (!out_path_offsets) return set_error(ctx, SS_ERR_INVALID, "out_path_offsets is NULL");
+    if (nq && (!seg_idx || !out_dist)) return set_error(ctx, SS_ERR_INVALID, "index / distance pointers are NULL");
+    SS_TRY(queries_check(ctx, q_mfcc, q_frame_offsets, nq, d->c));
+    std::vector<uint64_t> off(nq + 1, 0);
+    size_t need = 0;
+    for (size_t p = 0; p < nq; p++) {
+        off[p + 1] = q_frame_offsets[p + 1] - q_frame_offsets[0];
+        if (seg_idx[p] == 0xFFFFFFFFu) continue;
+        const uint32_t s = seg_idx[p] - d->index_base;
+        if (seg_idx[p] < d->index_base || s >= d->nseg)
+            return set_error(ctx, SS_ERR_INVALID, "seg_idx[%zu] = %u is outside [%u, %u)", p, seg_idx[p], d->index_base,
+                             (uint32_t)(d->index_base + d->nseg));
+        const uint64_t lq = off[p + 1] - off[p], ld = d->h_off[s + 1] - d->h_off[s];
+        if (lq && ld) need += lq + ld - 1;
+    }
+    if (path_capacity < need)
+        return set_error(ctx, SS_ERR_INVALID, "path_capacity %zu < %zu cells (sum of Lq + Ld - 1 over the pairs)", path_capacity, need);
+    if (need && !out_path) return set_error(ctx, SS_ERR_INVALID, "out_path is NULL");
+    SS_CUDA(ctx, cudaSetDevice(ctx->device));
+    auto body = [&]() -> int {
+        SS_TRY(dtw_match_finish(d));
+        SS_TRY(upload(ctx, d->d_align_q, q_mfcc ? q_mfcc + q_frame_offsets[0] * d->c : nullptr, (size_t)off[nq] * d->c));
+        SS_TRY(upload(ctx, d->d_align_qoff, off.data(), nq + 1));
+        SS_TRY(upload(ctx, d->d_align_seg, seg_idx, nq));
+        SS_CUDA(ctx, d->d_align_path.reserve(2 * align_capacity_dev(d, off.data(), nq)));
+        SS_CUDA(ctx, d->d_align_off.reserve(nq + 1));
+        SS_CUDA(ctx, d->d_align_dist.reserve(nq));
+        SS_TRY(dtw_align_dev(d, d->d_align_q.p, d->d_align_qoff.p, off.data(), nq, d->d_align_seg.p, d->d_align_path.p, d->d_align_off.p,
+                             d->d_align_dist.p));
+        SS_CUDA(ctx, cudaMemcpyAsync(out_path_offsets, d->d_align_off.p, (nq + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        if (nq) SS_CUDA(ctx, cudaMemcpyAsync(out_dist, d->d_align_dist.p, nq * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        const uint64_t cells = out_path_offsets[nq];  // <= need: every path is at most Lq + Ld - 1 cells
+        if (cells) {
+            SS_CUDA(ctx, cudaMemcpyAsync(out_path, d->d_align_path.p, cells * 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+            SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        }
+        return SS_OK;
+    };
+    const int rc = body();
+    if (rc != SS_OK) cudaStreamSynchronize(ctx->stream);
+    return rc;
+}
+
 int ss_dict_set_scan(ss_dict* d, int first_stage) {
     if (!d) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
     if (first_stage < 0 || first_stage > 3) return set_error(d->ctx, SS_ERR_INVALID, "first_stage must be 0, 1, 2 or 3");

@@ -4,6 +4,9 @@
 //   cosine-ref matcher   cosine_sim / norm / at_distance, src/sound.rs:23-38, 351-370 (+ rulinalg::utils::dot [RECALL A9])
 //   DTW refine           the oracle's f64 recurrence (ASSUMPTIONS.h A8) on the candidates the fp32 scan kept
 //   top-k merge          (distance, index) lexicographic merge of per-shard lists
+//   DTW alignment        the refine's recurrence with the direction of every cell kept, then the backtrack (DESIGN.md §3.1e)
+#include <cub/cub.cuh>
+
 #include <algorithm>
 
 #include "match.cuh"
@@ -1610,6 +1613,341 @@ int topk_merge_dev(ss_ctx* ctx, const uint32_t* d_idx, const double* d_dist, int
     if (k < 1 || k > SS_MAX_TOPK || nlists < 1) return set_error(ctx, SS_ERR_INVALID, "topk_merge: bad k / nlists");
     if (!nq) return SS_OK;
     k_topk_merge<<<ceil_div((long long)nq, 128), 128, 0, ctx->stream>>>(d_idx, d_dist, nlists, nq, k, d_out_idx, d_out_dist);
+    SS_LAUNCHED(ctx);
+    return SS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// DTW alignment (ss_dict_align, spec in DESIGN.md §3.1e): the warping path of query p against dictionary segment seg_idx[p].
+// The recurrences below are warp_dtw_exact / warp_dtw_exact_long with one addition: every cell also records which of its
+// three neighbours the min chose, as 2 bits (0 diag, 1 up, 2 left; ties in that order), compared against the very value
+// fmin(fmin(up, left), diag) returned. D's bits are the refine's, so the path is the oracle's path cell for cell.
+//   <= 32 x <= 32 (k_dtw_align_warp): lane j owns column j, whose 32 rows of directions fit in one u64 register; the
+//     backtrack is <= 63 steps of one shuffle of the current column's word.
+//   longer (k_dtw_align_long, waves of pairs): per strip, lane j packs 32 rows of its column into a u64 and stores it to the
+//     pair's direction block [strip][row / 32][lane], coalesced, once the whole warp has finished those rows. The backtrack
+//     loads one 32 x 32 tile (one coalesced u64 per lane) whenever the path enters it, then shuffles within it.
+// Paths are found from the end: cell s from the end goes to stage[last - s] of the pair's staging slot (last = its end),
+// so a path lands in forward order without knowing its length first. A scan of the lengths then gives the offsets and
+// k_dtw_align_compact packs the paths. Nothing is read back to the host.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr uint32_t kAlignNone = 0xFFFFFFFFu;
+constexpr uint64_t kAlignDirBudget = 256ull << 20;  // direction blocks + boundary rows of one wave of long pairs
+
+struct AlignArgs {
+    const double* dmfcc;
+    const uint64_t* doff;
+    uint32_t nseg, index_base;
+    const double* qmfcc;
+    const uint64_t* qoff;
+    uint32_t nq;
+    int c;
+    const uint32_t* seg_idx;
+    uint32_t wpad;  // max(longest segment, 1) - 1: pair p stages its path in [qoff[p] + p wpad, + Lq + wpad)
+    uint2* stage;
+    uint64_t* len;
+    double* out_dist;
+};
+
+// the pair's two sides; false (the pair's empty result written) when there is nothing to align
+__device__ __forceinline__ bool align_pair(const AlignArgs& A, uint32_t p, int lane, int* la, int* lb, uint32_t* s) {
+    const uint32_t idx = A.seg_idx[p];
+    *s = idx - A.index_base;
+    const bool known = idx != kAlignNone && *s < A.nseg;
+    *la = (int)(A.qoff[p + 1] - A.qoff[p]);
+    *lb = known ? (int)(A.doff[*s + 1] - A.doff[*s]) : 0;
+    if (known && *la && *lb) return true;
+    if (lane == 0) {
+        A.len[p] = 0;
+        A.out_dist[p] = (idx == kAlignNone || known) ? kInf : __longlong_as_double(0x7ff8000000000000ll);  // out of range: NaN
+    }
+    return false;
+}
+
+__device__ __forceinline__ uint64_t align_dir(double up, double left, double diag, double m) {
+    return diag == m ? 0ull : (up == m ? 1ull : 2ull);
+}
+
+// warp_dtw_exact (same loads, same operations in the same order) + the directions of lane `lane`'s column in *dirs
+__device__ __forceinline__ double warp_dtw_align(const double* __restrict__ sa, int la, const double* __restrict__ b, int lb, int c, double* cst,
+                                                 int lane, uint64_t* dirs) {
+    double br[SS_MAX_NCOEFFS];
+#pragma unroll
+    for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = (k < c && lane < lb) ? b[(size_t)lane * c + k] : 0.0;
+    for (int i = 0; i < la; i++) {
+        double cost = 0.0;
+#pragma unroll
+        for (int k = 0; k < SS_MAX_NCOEFFS; k++)
+            if (k < c) {
+                const double dlt = sa[i * c + k] - br[k];
+                cost = cost + dlt * dlt;
+            }
+        cst[i * 32 + lane] = cost;
+    }
+    __syncwarp();
+    double cur = kInf, recv_prev = kInf, result = kInf;
+    uint64_t w = 0;
+    for (int step = 0; step < la + lb - 1; step++) {
+        const double recv = __shfl_up_sync(0xffffffffu, cur, 1);
+        const int i = step - lane;
+        const bool active = lane < lb && i >= 0 && i < la;
+        if (active) {
+            const double up = cur;
+            const double left = lane ? recv : kInf;
+            const double diag = lane ? recv_prev : kInf;
+            double m;
+            if (i == 0 && lane == 0) m = 0.0;
+            else m = fmin(fmin(up, left), diag);
+            w |= align_dir(up, left, diag, m) << (2 * i);
+            cur = cst[i * 32 + lane] + m;
+            if (i == la - 1 && lane == lb - 1) result = cur;
+        }
+        recv_prev = recv;
+    }
+    *dirs = w;
+    result = __shfl_sync(0xffffffffu, result, lb - 1);
+    return result / (double)(la + lb);
+}
+
+// one warp per pair, both sides <= 32 frames (the other pairs are k_dtw_align_long's)
+__global__ void __launch_bounds__(128) k_dtw_align_warp(AlignArgs A) {
+    __shared__ double scost[4][32 * 32];
+    __shared__ double squery[4][32 * SS_MAX_NCOEFFS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t p = blockIdx.x * 4 + warp;
+    if (p >= A.nq) return;  // warp-uniform from here on
+    int la, lb;
+    uint32_t s;
+    if (!align_pair(A, p, lane, &la, &lb, &s) || la > 32 || lb > 32) return;
+    const int c = A.c;
+    const double* a = A.qmfcc + A.qoff[p] * c;
+    for (int e = lane; e < la * c; e += 32) squery[warp][e] = a[e];
+    __syncwarp();
+    uint64_t dirs;
+    const double dist = warp_dtw_align(squery[warp], la, A.dmfcc + A.doff[s] * c, lb, c, scost[warp], lane, &dirs);
+    if (!(dist < kInf)) {  // NaN or inf: no path
+        if (lane == 0) A.len[p] = 0, A.out_dist[p] = kInf;
+        return;
+    }
+    // backtrack: lane (n & 31) keeps cell n from the end (n < 32 in keep0, else keep1)
+    int i = la - 1, j = lb - 1, n = 0;
+    uint2 keep0 = make_uint2(0, 0), keep1 = keep0;
+    for (;;) {
+        if (lane == (n & 31)) (n < 32 ? keep0 : keep1) = make_uint2((uint32_t)i, (uint32_t)j);
+        n++;
+        if (i == 0 && j == 0) break;
+        const uint64_t w = __shfl_sync(0xffffffffu, dirs, j);
+        const uint32_t dir = i == 0 ? 2u : j == 0 ? 1u : (uint32_t)(w >> (2 * i)) & 3u;
+        i -= dir != 2u;
+        j -= dir != 1u;
+    }
+    uint2* last = A.stage + A.qoff[p] + (uint64_t)p * A.wpad + (uint64_t)la + A.wpad - 1;
+    if (lane < n) *(last - lane) = keep0;
+    if (lane + 32 < n) *(last - 32 - lane) = keep1;
+    if (lane == 0) A.len[p] = (uint64_t)n, A.out_dist[p] = dist;
+}
+
+// warp_dtw_exact_long (same loads, same operations in the same order) + the direction block `dir`, [strip][row / 32][lane]
+__device__ __forceinline__ double warp_dtw_align_long(const double* __restrict__ a, int la, const double* __restrict__ b, int lb, int c,
+                                                      double* __restrict__ ring, double* bnd, uint64_t* __restrict__ dir, int lane) {
+    double result = kInf;
+    const int nstrips = (lb + 31) >> 5, nrb = (la + 31) >> 5;
+    const int nsteps = la + 31;
+    for (int s = 0; s < nstrips; s++) {
+        const int col = 32 * s + lane;
+        const bool colv = col < lb, first = s == 0, last = s == nstrips - 1;
+        double br[SS_MAX_NCOEFFS];
+#pragma unroll
+        for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = (k < c && colv) ? b[(size_t)col * c + k] : 0.0;
+        double cur = kInf, recv_prev = kInf, bl_prev = kInf;
+        // at step t0 + r lane j is on row t0 + r - j: row block t0 / 32 - 1 (wprev) or t0 / 32 (wcur)
+        uint64_t wprev = 0, wcur = 0;
+        uint64_t* sdir = dir + (size_t)s * nrb * 32 + lane;
+        __syncwarp();
+        for (int t0 = 0; t0 < nsteps; t0 += 32) {
+            const int rows = min(32, la - t0);
+            int r = 0;
+            for (; r + 4 <= rows; r += 4) {
+                const double* ar = a + (size_t)(t0 + r) * c;
+                double c0 = 0.0, c1 = 0.0, c2 = 0.0, c3 = 0.0;
+#pragma unroll
+                for (int k = 0; k < SS_MAX_NCOEFFS; k++)
+                    if (k < c) {
+                        const double d0 = ar[k] - br[k], d1 = ar[c + k] - br[k], d2 = ar[2 * c + k] - br[k], d3 = ar[3 * c + k] - br[k];
+                        c0 = c0 + d0 * d0;
+                        c1 = c1 + d1 * d1;
+                        c2 = c2 + d2 * d2;
+                        c3 = c3 + d3 * d3;
+                    }
+                double* dst = ring + ((t0 + r) & 63) * 32 + lane;
+                dst[0] = c0, dst[32] = c1, dst[64] = c2, dst[96] = c3;
+            }
+            for (; r < rows; r++) {
+                const double* ar = a + (size_t)(t0 + r) * c;
+                double cost = 0.0;
+#pragma unroll
+                for (int k = 0; k < SS_MAX_NCOEFFS; k++)
+                    if (k < c) {
+                        const double dlt = ar[k] - br[k];
+                        cost = cost + dlt * dlt;
+                    }
+                ring[((t0 + r) & 63) * 32 + lane] = cost;
+            }
+            __syncwarp();
+            const int steps = min(32, nsteps - t0);
+            double left_in = (lane == 0 && !first && t0 < la) ? bnd[t0] : kInf;
+            for (int r = 0; r < steps; r++) {
+                const int t = t0 + r;
+                const double recv = __shfl_up_sync(0xffffffffu, cur, 1);
+                const double left_now = left_in;
+                if (r + 1 < steps) left_in = (lane == 0 && !first && t + 1 < la) ? bnd[t + 1] : kInf;
+                const int i = t - lane;
+                const bool active = colv && i >= 0 && i < la;
+                if (active) {
+                    const double up = cur;
+                    const double left = lane ? recv : left_now;
+                    const double diag = lane ? recv_prev : bl_prev;
+                    double m;
+                    if (first && i == 0 && lane == 0) m = 0.0;
+                    else m = fmin(fmin(up, left), diag);
+                    const uint64_t bits = align_dir(up, left, diag, m) << (2 * (i & 31));
+                    if (i < t0) wprev |= bits;
+                    else wcur |= bits;
+                    cur = ring[(i & 63) * 32 + lane] + m;
+                    if (last && i == la - 1 && col == lb - 1) result = cur;
+                    if (!last && lane == 31) bnd[i] = cur;
+                }
+                bl_prev = left_now;
+                recv_prev = recv;
+            }
+            __syncwarp();
+            if (t0 >= 32) sdir[(size_t)((t0 >> 5) - 1) * 32] = wprev;  // every lane is past that row block
+            wprev = wcur;
+            wcur = 0;
+        }
+        const int rb_last = (nsteps - 1) >> 5;
+        if (rb_last < nrb) sdir[(size_t)rb_last * 32] = wprev;
+    }
+    result = __shfl_sync(0xffffffffu, result, (lb - 1) & 31);
+    return result / (double)(la + lb);
+}
+
+// one warp per pair of the wave [p0, p0 + np) that has a side longer than 32 frames; the pair's direction block and
+// boundary row are its own (dir_stride u64 words, bnd_stride doubles)
+__global__ void __launch_bounds__(64) k_dtw_align_long(AlignArgs A, uint32_t p0, uint32_t np, uint64_t* __restrict__ dir, uint64_t dir_stride,
+                                                       double* __restrict__ bnd, uint32_t bnd_stride) {
+    __shared__ double ring[2][64 * 32];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t t = blockIdx.x * 2 + warp;
+    if (t >= np) return;
+    const uint32_t p = p0 + t;
+    int la, lb;
+    uint32_t s;
+    if (!align_pair(A, p, -1, &la, &lb, &s) || (la <= 32 && lb <= 32)) return;  // (lane -1: k_dtw_align_warp wrote those)
+    const int c = A.c;
+    uint64_t* my_dir = dir + (size_t)t * dir_stride;
+    const double dist = warp_dtw_align_long(A.qmfcc + A.qoff[p] * c, la, A.dmfcc + A.doff[s] * c, lb, c, ring[warp],
+                                            bnd + (size_t)t * bnd_stride, my_dir, lane);
+    if (!(dist < kInf)) {
+        if (lane == 0) A.len[p] = 0, A.out_dist[p] = kInf;
+        return;
+    }
+    const int nrb = (la + 31) >> 5;
+    uint2* last = A.stage + A.qoff[p] + (uint64_t)p * A.wpad + (uint64_t)la + A.wpad - 1;
+    int i = la - 1, j = lb - 1, ts = -1, trb = -1;
+    uint32_t n = 0;
+    uint64_t w = 0;
+    uint2 keep = make_uint2(0, 0);
+    for (;;) {
+        if (lane == (int)(n & 31)) keep = make_uint2((uint32_t)i, (uint32_t)j);
+        n++;
+        if ((n & 31) == 0) *(last - (n - 32) - lane) = keep;  // lane l holds cell n - 32 + l from the end
+        if (i == 0 && j == 0) break;
+        if ((j >> 5) != ts || (i >> 5) != trb) {  // the path enters another 32 x 32 tile (warp-uniform)
+            ts = j >> 5;
+            trb = i >> 5;
+            w = my_dir[((size_t)ts * nrb + trb) * 32 + lane];  // this lane's own store
+        }
+        const uint64_t wc = __shfl_sync(0xffffffffu, w, j & 31);
+        const uint32_t d = i == 0 ? 2u : j == 0 ? 1u : (uint32_t)(wc >> (2 * (i & 31))) & 3u;
+        i -= d != 2u;
+        j -= d != 1u;
+    }
+    const uint32_t rem = n & 31;
+    if ((uint32_t)lane < rem) *(last - (n - rem) - lane) = keep;
+    if (lane == 0) A.len[p] = (uint64_t)n, A.out_dist[p] = dist;
+}
+
+// one warp per pair: its path from the end of its staging slot to out_path[out_off[p] ..), as (i, j) uint32 pairs
+__global__ void __launch_bounds__(256) k_dtw_align_compact(const uint2* __restrict__ stage, const uint64_t* __restrict__ qoff, uint32_t nq,
+                                                           uint32_t wpad, const uint64_t* __restrict__ out_off, uint32_t* __restrict__ out) {
+    const int lane = threadIdx.x & 31;
+    const uint32_t p = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (p >= nq) return;
+    const uint64_t o = out_off[p], n = out_off[p + 1] - o;
+    const uint2* src = stage + qoff[p] + (uint64_t)p * wpad + (qoff[p + 1] - qoff[p]) + wpad - n;
+    for (uint64_t e = lane; e < n; e += 32) {
+        const uint2 v = src[e];
+        out[2 * (o + e)] = v.x;
+        out[2 * (o + e) + 1] = v.y;
+    }
+}
+
+int dtw_align_dev(ss_dict* d, const double* d_qmfcc, const uint64_t* d_qoff, const uint64_t* h_qoff, size_t nq, const uint32_t* d_seg_idx,
+                  uint32_t* d_out_path, uint64_t* d_out_off, double* d_out_dist) {
+    ss_ctx* ctx = d->ctx;
+    SS_CUDA(ctx, cudaMemsetAsync(d_out_off, 0, sizeof(uint64_t), ctx->stream));
+    if (!nq) return SS_OK;
+    const uint32_t ld_max = std::max<uint32_t>(d->max_len, 1), wpad = ld_max - 1;
+    uint32_t lq_max = 0;
+    for (size_t p = 0; p < nq; p++) lq_max = std::max<uint32_t>(lq_max, (uint32_t)(h_qoff[p + 1] - h_qoff[p]));
+    SS_CUDA(ctx, d->d_align_stage.reserve(h_qoff[nq] + nq * (size_t)wpad)  /* (offsets start at 0) */);
+    SS_CUDA(ctx, d->d_align_len.reserve(nq));
+    AlignArgs A{d->d_mfcc.p, d->d_off.p, (uint32_t)d->nseg, d->index_base, d_qmfcc, d_qoff, (uint32_t)nq, d->c, d_seg_idx, wpad,
+                d->d_align_stage.p, d->d_align_len.p, d_out_dist};
+    // waves of long pairs, sized from host-known bounds only: (the wave's longest query) x (the longest segment)
+    struct Wave {
+        uint32_t p0, np, lq;
+    };
+    std::vector<Wave> waves;
+    if (lq_max > 32 || ld_max > 32) {
+        const uint64_t nsb = (ld_max + 31) / 32;
+        auto bytes_of = [&](uint64_t lq) { return (lq + 31) / 32 * nsb * 32 * sizeof(uint64_t) + lq * sizeof(double); };
+        for (size_t p0 = 0; p0 < nq;) {
+            uint32_t lq = 0;
+            size_t p1 = p0;
+            for (; p1 < nq; p1++) {
+                const uint32_t m = std::max<uint32_t>(lq, (uint32_t)(h_qoff[p1 + 1] - h_qoff[p1]));
+                if (p1 > p0 && (p1 - p0 + 1) * bytes_of(m) > kAlignDirBudget) break;  // (one pair alone may exceed the budget)
+                lq = m;
+            }
+            if (lq > 32 || (lq > 0 && ld_max > 32)) waves.push_back({(uint32_t)p0, (uint32_t)(p1 - p0), lq});
+            p0 = p1;
+        }
+        size_t dir_words = 0, bnd_rows = 0;
+        for (const Wave& w : waves) {
+            dir_words = std::max<size_t>(dir_words, (size_t)w.np * ((w.lq + 31) / 32) * nsb * 32);
+            bnd_rows = std::max<size_t>(bnd_rows, (size_t)w.np * w.lq);
+        }
+        if (!waves.empty()) {
+            SS_CUDA(ctx, d->d_align_dir.reserve(dir_words));
+            SS_CUDA(ctx, d->d_align_bnd.reserve(bnd_rows));
+        }
+    }
+    size_t cub_bytes = 0;
+    SS_CUDA(ctx, cub::DeviceScan::InclusiveSum(nullptr, cub_bytes, d->d_align_len.p, d_out_off + 1, (int)nq, ctx->stream));
+    SS_CUDA(ctx, d->d_align_cub.reserve(cub_bytes));
+
+    k_dtw_align_warp<<<ceil_div((long long)nq, 4), 128, 0, ctx->stream>>>(A);
+    SS_LAUNCHED(ctx);
+    for (const Wave& w : waves) {
+        const uint64_t dir_stride = (uint64_t)((w.lq + 31) / 32) * ((ld_max + 31) / 32) * 32;
+        k_dtw_align_long<<<ceil_div(w.np, 2), 64, 0, ctx->stream>>>(A, w.p0, w.np, d->d_align_dir.p, dir_stride, d->d_align_bnd.p, w.lq);
+        SS_LAUNCHED(ctx);
+    }
+    SS_CUDA(ctx, cub::DeviceScan::InclusiveSum(d->d_align_cub.p, cub_bytes, d->d_align_len.p, d_out_off + 1, (int)nq, ctx->stream));
+    ctx->launches++;
+    k_dtw_align_compact<<<ceil_div((long long)nq, 8), 256, 0, ctx->stream>>>(d->d_align_stage.p, d_qoff, (uint32_t)nq, wpad, d_out_off, d_out_path);
     SS_LAUNCHED(ctx);
     return SS_OK;
 }

@@ -148,6 +148,15 @@ struct ss_dict {
     ss::DevBuf<uint64_t> d_walk_off;
     ss::DevBuf<uint32_t> d_walk_idx;
     uint64_t h_walk_off[2] = {0, 0};
+    // ss_dict_align (exact.cu dtw_align_dev): staging slots of the paths, path lengths, direction blocks and boundary rows of
+    // the long pairs, the scan's temporary storage; then the host-buffer entry point's inputs and outputs
+    ss::DevBuf<uint2> d_align_stage;
+    ss::DevBuf<uint64_t> d_align_len, d_align_dir;
+    ss::DevBuf<double> d_align_bnd;
+    ss::DevBuf<unsigned char> d_align_cub;
+    ss::DevBuf<double> d_align_q, d_align_dist;
+    ss::DevBuf<uint64_t> d_align_qoff, d_align_off;
+    ss::DevBuf<uint32_t> d_align_seg, d_align_path;
     ~ss_dict();
 };
 
@@ -249,6 +258,11 @@ int cosine_match_dev(ss_dict* d, ss_queries* q, const double* d_targets, uint32_
 // SoundSequence::from_distances for SS_COSINE_REF: nsteps + 1 launches on the ctx stream, no host synchronisation (exact.cu)
 int cosine_walk_dev(ss_dict* d, const double* d_start, const uint64_t* d_start_off, const double* d_targets, size_t nsteps,
                     uint32_t* d_out_idx, double* d_out_dist);
+// the DTW warping path (DESIGN.md §3.1e) of query p (frames d_qoff[p] .. d_qoff[p+1], h_qoff its host copy) against segment
+// d_seg_idx[p]: 1 + (waves of long pairs) + 2 launches on the ctx stream, no host synchronisation (exact.cu). d_out_path must
+// hold sum over non-empty queries of (Lq + max(longest segment, 1) - 1) (i, j) pairs.
+int dtw_align_dev(ss_dict* d, const double* d_qmfcc, const uint64_t* d_qoff, const uint64_t* h_qoff, size_t nq, const uint32_t* d_seg_idx,
+                  uint32_t* d_out_path, uint64_t* d_out_off, double* d_out_dist);
 int topk_merge_dev(ss_ctx* ctx, const uint32_t* d_idx, const double* d_dist, int nlists, size_t nq, int k,
                    uint32_t* d_out_idx, double* d_out_dist);
 }  // namespace ss
