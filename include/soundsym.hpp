@@ -308,6 +308,7 @@ class SoundDictionary {
    public:
     std::vector<std::shared_ptr<Sound>> sounds;
     int mode = SS_COSINE_REF;  // SS_DTW selects the DTW extension
+    uint32_t dtw_band = 0;     // Sakoe-Chiba radius of the SS_DTW distance and of align() (ss_dict_set_dtw_band; 0 = no band)
 
     explicit SoundDictionary(Context& ctx = Context::global()) : ctx_(&ctx) {}
     ~SoundDictionary() { ss_dict_destroy(dev_); }
@@ -418,14 +419,16 @@ class SoundDictionary {
 
    private:
     ss_dict* device() {
-        if (dev_) return dev_;
-        std::vector<uint64_t> off(sounds.size() + 1, 0);
-        std::vector<double> flat;
-        for (size_t i = 0; i < sounds.size(); i++) {
-            off[i + 1] = off[i] + sounds[i]->num_frames();
-            flat.insert(flat.end(), sounds[i]->mfccs().begin(), sounds[i]->mfccs().end());
+        if (!dev_) {
+            std::vector<uint64_t> off(sounds.size() + 1, 0);
+            std::vector<double> flat;
+            for (size_t i = 0; i < sounds.size(); i++) {
+                off[i + 1] = off[i] + sounds[i]->num_frames();
+                flat.insert(flat.end(), sounds[i]->mfccs().begin(), sounds[i]->mfccs().end());
+            }
+            ctx_->check(ss_dict_create(ctx_->get(), flat.data(), off.data(), sounds.size(), (int)NCOEFFS, 0, &dev_));
         }
-        ctx_->check(ss_dict_create(ctx_->get(), flat.data(), off.data(), sounds.size(), (int)NCOEFFS, 0, &dev_));
+        if (ss_dict_dtw_band(dev_) != dtw_band) ctx_->check(ss_dict_set_dtw_band(dev_, dtw_band));  // (add_segments drops dev_)
         return dev_;
     }
     Context* ctx_;

@@ -287,6 +287,21 @@ int ss_dict_debug_h2_scan(ss_dict* dict, const double* q_mfcc, const uint64_t* q
  * The results are identical by construction (every stage is followed by the f64 refine + certification); only the speed differs. */
 int ss_dict_set_scan(ss_dict* dict, int first_stage);
 
+/* Sakoe-Chiba band of the SS_DTW distance (DESIGN.md §3.1f), per dictionary. radius 0 (the default) = no band: every result is
+ * bit-identical to a dictionary that never set one. For radius r >= 1, cell (i, j) of a pair of Lq x Ld frames is inside the band iff
+ *     |i (Ld - 1) - j (Lq - 1)| <= r max(Lq - 1, Ld - 1)       (64-bit integers)
+ * - |i - j| <= r for equal lengths; otherwise the band follows the line from (0, 0) to (Lq-1, Ld-1), r counted in frames of the
+ * longer side. A cell outside the band has D = +inf and is never a predecessor; inside it the recurrence, the normalisation
+ * D(Lq-1, Ld-1) / (Lq + Ld), the (distance, index) order and the NaN rule are unchanged. The end cell is always reachable, and
+ * r >= min(Lq-1, Ld-1) covers the whole matrix. The band applies to SS_DTW matches (ss_dict_match, _dev, _sharded*) and to
+ * ss_dict_align[_dev]; SS_COSINE_REF, ss_dict_walk and the ss_dict_debug_* hooks ignore it. A pending SS_DTW match completes
+ * first, with the radius it started with. NULL -> SS_ERR_INVALID. With one rank per process every rank sets the radius of its own
+ * shard, and all ranks must set the same radius. */
+int ss_dict_set_dtw_band(ss_dict* dict, uint32_t radius);
+uint32_t ss_dict_dtw_band(const ss_dict* dict); /* 0 for NULL */
+/* the same on every shard of a single-process sharded dictionary */
+int ss_sharded_dict_set_dtw_band(ss_sharded_dict* dict, uint32_t radius);
+
 /* ss_resynth   SoundSequence::clone_from_dictionary sample assembly (src/sound.rs:451-472) + to_sound (:475-483):
  *              for target segment t copy min(len) samples of dictionary sound match_idx[t] and zero-pad to
  *              target_lens[t]; segments are concatenated into out_samples (capacity sum(target_lens)). */

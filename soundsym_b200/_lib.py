@@ -21,6 +21,7 @@ SYMBOLS = [
     "ss_symbols", "ss_gmm_train", "ss_vote_split", "ss_partition", "ss_dict_create", "ss_dict_destroy", "ss_dict_len", "ss_dict_match",
     "ss_queries_create", "ss_queries_destroy", "ss_dict_match_dev", "ss_topk_merge_dev", "ss_dict_last_work", "ss_dict_last_scan_kind",
     "ss_dict_last_uncertified", "ss_dict_last_tc_fallback", "ss_dict_last_exhaustive", "ss_queries_invalidate", "ss_dict_last_scan_ms", "ss_resynth", "ss_sequence_distances", "ss_dict_debug_tc_scan", "ss_dict_debug_h2_scan", "ss_dict_set_scan", "ss_dict_match_finish",
+    "ss_dict_set_dtw_band", "ss_dict_dtw_band", "ss_sharded_dict_set_dtw_band",
     "ss_dict_walk", "ss_dict_walk_dev", "ss_dict_align", "ss_dict_align_dev",
     "ss_shard_bounds", "ss_comm_unique_id", "ss_comm_create", "ss_comm_create_all", "ss_comm_destroy", "ss_comm_rank", "ss_comm_nranks",
     "ss_queries_create_sharded", "ss_dict_match_sharded_dev", "ss_dict_match_sharded", "ss_dict_create_sharded", "ss_sharded_dict_match",
@@ -113,6 +114,10 @@ def load():
     L.ss_dict_align_dev.argtypes = [vp, vp, vp, vp, sz, vp, vp]
     L.ss_dict_debug_h2_scan.argtypes = [vp, vp, vp, sz, vp, vp, P(C.c_float), P(C.c_float)]
     L.ss_dict_set_scan.argtypes = [vp, i]
+    L.ss_dict_set_dtw_band.argtypes = [vp, u32]
+    L.ss_dict_dtw_band.argtypes = [vp]
+    L.ss_dict_dtw_band.restype = u32
+    L.ss_sharded_dict_set_dtw_band.argtypes = [vp, u32]
     L.ss_shard_bounds.argtypes = [vp, sz, i, vp]
     L.ss_comm_unique_id.argtypes = [vp]
     L.ss_comm_create.argtypes = [vp, i, i, vp, P(vp)]

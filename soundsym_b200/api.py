@@ -304,6 +304,15 @@ class DeviceDictionary:
         """ss_dict_set_scan: 0 = packed-half tensor-core scan first (default), 1 = fp32-DP tensor-core scan, 2 = fp32 CUDA-core scan"""
         self.ctx.check(self.ctx.lib.ss_dict_set_scan(self.h, int(first_stage)))
 
+    def set_dtw_band(self, radius):
+        """ss_dict_set_dtw_band: Sakoe-Chiba radius of SS_DTW matches and align() (0 = no band, the default). For a shard of a
+        one-rank-per-process match (Comm.match), every rank must set the same radius."""
+        self.ctx.check(self.ctx.lib.ss_dict_set_dtw_band(self.h, _band(radius)))
+
+    @property
+    def dtw_band(self):
+        return int(self.ctx.lib.ss_dict_dtw_band(self.h))
+
     @property
     def last_scan_kind(self):
         return int(self.ctx.lib.ss_dict_last_scan_kind(self.h))
@@ -323,6 +332,13 @@ class DeviceDictionary:
     @property
     def last_exhaustive(self):
         return int(self.ctx.lib.ss_dict_last_exhaustive(self.h))
+
+
+def _band(radius):
+    r = int(radius)
+    if not 0 <= r <= 0xFFFFFFFF:
+        raise ValueError("dtw_band must be in 0..2**32-1 (got %d)" % r)
+    return r
 
 
 def shard_bounds(frame_offsets, nshards):
@@ -409,6 +425,10 @@ class ShardedDictionary:
 
     def __len__(self):
         return int(self.ctxs[0].lib.ss_sharded_dict_len(self.h))
+
+    def set_dtw_band(self, radius):
+        """ss_sharded_dict_set_dtw_band: the Sakoe-Chiba radius of every shard"""
+        self.ctxs[0].check(self.ctxs[0].lib.ss_sharded_dict_set_dtw_band(self.h, _band(radius)))
 
     def match(self, q_flat, q_frame_offsets, mode=SS_DTW, k=1, targets=None):
         q = np.ascontiguousarray(q_flat, dtype=np.float64)
@@ -587,11 +607,13 @@ def _read_wav_pcm(path):
 
 
 class SoundDictionary:
-    """src/sound.rs:288-371. `mode` selects the matcher: SS_COSINE_REF is the reference's, SS_DTW the extension."""
+    """src/sound.rs:288-371. `mode` selects the matcher: SS_COSINE_REF is the reference's, SS_DTW the extension.
+    `dtw_band`: Sakoe-Chiba radius of the SS_DTW distance and of align() (0 = no band; ss_dict_set_dtw_band)."""
 
-    def __init__(self, ctx=None, mode=SS_COSINE_REF):
+    def __init__(self, ctx=None, mode=SS_COSINE_REF, dtw_band=0):
         self.sounds = []
         self.mode = mode
+        self.dtw_band = _band(dtw_band)
         self._ctx = ctx or default_context()
         self._dev = None
 
@@ -656,6 +678,8 @@ class SoundDictionary:
             off[1:] = np.cumsum(lens)
             flat = np.concatenate([s.mfcc_arrays() for s in self.sounds], axis=0) if int(off[-1]) else np.zeros((0, NCOEFFS))
             self._dev = DeviceDictionary(self._ctx, flat, off, NCOEFFS)
+        if self._dev.dtw_band != self.dtw_band:  # a new device dictionary (add_segments drops it), or dtw_band was reassigned
+            self._dev.set_dtw_band(self.dtw_band)
         return self._dev
 
     def match_indices(self, sounds, targets=None, k=1):

@@ -450,6 +450,18 @@ int ss_dict_set_scan(ss_dict* d, int first_stage) {
     return SS_OK;
 }
 
+// Sakoe-Chiba band of the exact DTW (A10, DESIGN.md §3.1f). A pending SS_DTW match completes first, under the radius it
+// started with: its first stage already ran with that radius.
+int ss_dict_set_dtw_band(ss_dict* d, uint32_t radius) {
+    if (!d) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
+    SS_CUDA(d->ctx, cudaSetDevice(d->ctx->device));
+    SS_TRY(dtw_match_finish(d));
+    d->dtw_band = radius;
+    return SS_OK;
+}
+
+uint32_t ss_dict_dtw_band(const ss_dict* d) { return d ? d->dtw_band : 0; }
+
 static int debug_scan(ss_dict* d, const double* q_mfcc, const uint64_t* q_frame_offsets, size_t nq, float* out_scan, double* out_mu,
                       float* out_scale, float* out_s);
 

@@ -445,6 +445,12 @@ void ss_sharded_dict_destroy(ss_sharded_dict* sd) {
 }
 
 size_t ss_sharded_dict_len(const ss_sharded_dict* sd) { return sd ? sd->nseg : 0; }
+
+int ss_sharded_dict_set_dtw_band(ss_sharded_dict* sd, uint32_t radius) {
+    if (!sd) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
+    for (ss_dict* d : sd->shards) SS_TRY(ss_dict_set_dtw_band(d, radius));
+    return SS_OK;
+}
 int ss_sharded_dict_nshards(const ss_sharded_dict* sd) { return sd ? sd->n : 0; }
 
 int ss_sharded_dict_match(ss_sharded_dict* sd, const double* q_mfcc, const uint64_t* q_frame_offsets, size_t nq, int mode, const double* targets,

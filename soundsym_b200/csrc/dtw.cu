@@ -637,12 +637,39 @@ static int run_stage(ss_dict* d, ss_queries* q, int k, DtwStage s, bool timed, u
 // Sequences of more than 32 frames have no cheap second filter (the fp32-DP tensor-core scan stops at 32 frames, the CUDA-core
 // scan of ONE long query is a single warp's serial walk: 16 ms at config 5): below 2e8 cells the exhaustive stage is the
 // fastest way to finish (f64, measured 9e10 cells / s: 2 ms); a dozen such queries first take the wide packed-half pass.
+// Cells the banded strip kernel (exact.cu warp_dtw_exact_long<true>) visits for a pair of la x lb frames (la, lb >= 1): per strip of
+// 32 columns, the 32 x 32 step blocks from the one holding its first in-band row to the one in which lane 31 reaches its last.
+static uint64_t band_strip_cells(int la, int lb, uint32_t r) {
+    const int nsteps = la + 31;
+    uint64_t blocks = 0;
+    for (int s = 0; s < (lb + 31) / 32; s++) {
+        int lo, hi, lo_last, hi_last;
+        band_rows(32 * s, la, lb, r, &lo, &hi);
+        band_rows(std::min(32 * s + 31, lb - 1), la, lb, r, &lo_last, &hi_last);
+        blocks += (std::min(nsteps, hi_last + 32) - (lo & ~31) + 31) / 32;
+    }
+    return blocks * 32 * 32;
+}
+
 // ran_max_len: the longest query of the batch the last stage ran on; u: the uncertified queries of q.
+// With a band, a pair costs what the banded strip kernel visits (band_strip_cells), but never more than its Lq Ld cells.
 static bool exhaustive_is_cheaper(const ss_dict* d, uint32_t ran_max_len, const ss_queries* q, const std::vector<uint32_t>& u) {
     if (d->max_len <= 32 && ran_max_len <= 32) return false;
-    uint64_t rows = 0;
-    for (uint32_t i : u) rows += q->h_off[i + 1] - q->h_off[i];
-    return rows * d->total_frames <= 200000000ull;
+    const uint64_t limit = 200000000ull;
+    uint64_t cells = 0;
+    for (uint32_t i : u) {
+        const uint64_t lq = q->h_off[i + 1] - q->h_off[i];
+        if (!d->dtw_band || !lq) {
+            cells += lq * d->total_frames;
+            continue;
+        }
+        for (size_t s = 0; s < d->nseg && cells <= limit; s++) {
+            const uint64_t ld = d->h_off[s + 1] - d->h_off[s];
+            if (ld) cells += std::min<uint64_t>(lq * ld, band_strip_cells((int)lq, (int)ld, d->dtw_band));
+        }
+        if (cells > limit) return false;
+    }
+    return cells <= limit;
 }
 
 // the uncertified count of the stage that just ran travels to pinned host memory behind it; ev_done marks its arrival

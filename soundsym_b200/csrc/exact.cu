@@ -901,11 +901,15 @@ struct RescoreBound {
 // ---------------------------------------------------------------------------------------------------------------
 // `sa` holds the query's frames (staged once per slot, coalesced); lane j keeps dictionary frame j in registers (its 13 loads
 // are issued back to back: one memory latency per pair). cst = the pair's local costs, [row][lane].
+// BAND: cells outside the band of radius `band` (>= 1) are +inf, one integer test per cell against the lane's row range.
+template <bool BAND>
 __device__ __forceinline__ double warp_dtw_exact(const double* __restrict__ sa, int la, const double* __restrict__ b, int lb, int c, double* cst,
-                                                 int lane) {
+                                                 int lane, uint32_t band) {
     double br[SS_MAX_NCOEFFS];
 #pragma unroll
     for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = (k < c && lane < lb) ? b[(size_t)lane * c + k] : 0.0;
+    int blo = 0, bhi = 0;
+    if (BAND && la > 0 && lb > 0) band_rows(min(lane, lb - 1), la, lb, band, &blo, &bhi);
     __syncwarp();  // the previous pair's costs are no longer read
     for (int i = 0; i < la; i++) {
         double cost = 0.0;
@@ -930,7 +934,8 @@ __device__ __forceinline__ double warp_dtw_exact(const double* __restrict__ sa, 
             double m;
             if (i == 0 && lane == 0) m = 0.0;
             else m = fmin(fmin(up, left), diag);
-            cur = cst[i * 32 + lane] + m;
+            if (BAND && (i < blo || i > bhi)) cur = kInf;
+            else cur = cst[i * 32 + lane] + m;
             if (i == la - 1 && lane == lb - 1) result = cur;
         }
         recv_prev = recv;
@@ -939,13 +944,14 @@ __device__ __forceinline__ double warp_dtw_exact(const double* __restrict__ sa, 
     return (la && lb) ? result / (double)(la + lb) : kInf;
 }
 
+template <bool BAND>
 __global__ void __launch_bounds__(128)
 k_dtw_refine_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ qmfcc,
                   const uint64_t* __restrict__ qoff, int c, const uint32_t* __restrict__ group_qid, const uint32_t* __restrict__ cand_idx,
                   const float* __restrict__ cand_adist, uint32_t nslots, int kp, int k, uint32_t index_base, const float* __restrict__ max_na,
                   const float* __restrict__ max_nb, double eps, const float* __restrict__ slot_max_na, int bound_mode, double inv_s,
                   uint8_t* __restrict__ uncert_flag, uint32_t* __restrict__ out_idx, double* __restrict__ out_dist,
-                  unsigned long long* __restrict__ counters) {
+                  unsigned long long* __restrict__ counters, uint32_t band) {
     __shared__ double scost[4][32 * 32];
     __shared__ double squery[4][32 * SS_MAX_NCOEFFS];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -975,7 +981,7 @@ k_dtw_refine_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__
             if (bound.lower(adist) > kth) continue;  // provably outside the top-k
             extra++;
         }
-        const double e = warp_dtw_exact(squery[warp], la, dmfcc + doff[idx] * c, (int)(doff[idx + 1] - doff[idx]), c, scost[warp], lane);
+        const double e = warp_dtw_exact<BAND>(squery[warp], la, dmfcc + doff[idx] * c, (int)(doff[idx + 1] - doff[idx]), c, scost[warp], lane, band);
         if (lane == s) my_exact = e;
         if (s < k) kth = fmax(kth, e < kInf ? e : kInf);
     }
@@ -1026,9 +1032,14 @@ k_dtw_refine_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__
 //      value, left / diag = its left neighbour's values one / two steps earlier, by shuffle),
 // and the strip's last column travels to the next strip through `bnd` (global, one row of max query length per warp), IN
 // PLACE: lane 31 writes row t - 31 at the step lane 0 reads row t.
+// BAND: the strip's columns are inside the band for rows [rlo, rhi] at most (band_rows of its first and last column), so the
+// step blocks run from the one holding row rlo to the one in which lane 31 reaches row rhi, and only rows <= rhi get costs.
+// Cells outside the band inside those blocks are +inf by the per-cell test. Rows the strip never reaches are +inf for every
+// column of it: they go to the boundary row as +inf, for the next strip's lane 0.
 // ---------------------------------------------------------------------------------------------------------------
+template <bool BAND>
 __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__ a, int la, const double* __restrict__ b, int lb, int c,
-                                                      double* __restrict__ ring, double* bnd, int lane) {
+                                                      double* __restrict__ ring, double* bnd, int lane, uint32_t band) {
     if (!la || !lb) return kInf;
     double result = kInf;
     const int nstrips = (lb + 31) >> 5;
@@ -1040,10 +1051,19 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
 #pragma unroll
         for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = (k < c && colv) ? b[(size_t)col * c + k] : 0.0;
         double cur = kInf, recv_prev = kInf, bl_prev = kInf;
+        int blo = 0, bhi = 0, rhi = 0, t0b = 0, t0e = nsteps;
+        if (BAND) {
+            band_rows(min(col, lb - 1), la, lb, band, &blo, &bhi);
+            rhi = __shfl_sync(0xffffffffu, bhi, 31);
+            t0b = __shfl_sync(0xffffffffu, blo, 0) & ~31;
+            t0e = min(nsteps, rhi + 32);
+        }
         __syncwarp();  // the previous strip's boundary writes and ring reads are complete
-        for (int t0 = 0; t0 < nsteps; t0 += 32) {
+        if (BAND && lane == 0 && !first && t0b > 0) bl_prev = bnd[t0b - 1];  // D(t0b - 1, col0 - 1), the first step's diag
+        int t0 = t0b;
+        for (; t0 < t0e; t0 += 32) {
             // A: rows t0 .. t0 + 31 (ring slots of rows t0 - 64 .. t0 - 33, last read at step t0 - 2)
-            const int rows = min(32, la - t0);
+            const int rows = min(32, (BAND ? rhi + 1 : la) - t0);
             int r = 0;
             for (; r + 4 <= rows; r += 4) {  // four rows at a time: four independent accumulation chains
                 const double* ar = a + (size_t)(t0 + r) * c;
@@ -1089,7 +1109,8 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
                     double m;
                     if (first && i == 0 && lane == 0) m = 0.0;
                     else m = fmin(fmin(up, left), diag);
-                    cur = ring[(i & 63) * 32 + lane] + m;
+                    if (BAND && (i < blo || i > bhi)) cur = kInf;
+                    else cur = ring[(i & 63) * 32 + lane] + m;
                     if (last && i == la - 1 && col == lb - 1) result = cur;
                     if (!last && lane == 31) bnd[i] = cur;  // i = t - 31: behind every row lane 0 still has to read
                 }
@@ -1098,17 +1119,20 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
             }
             __syncwarp();
         }
+        if (BAND && !last)  // lane 31 stopped at row min(t0, nsteps) - 32
+            for (int r = max(0, min(t0, nsteps) - 31) + lane; r < la; r += 32) bnd[r] = kInf;
     }
     result = __shfl_sync(0xffffffffu, result, (lb - 1) & 31);
     return result / (double)(la + lb);
 }
 
 // one WARP per (slot, candidate) pair (grid-stride over the pairs; bnd: one row of bnd_stride doubles per warp)
+template <bool BAND>
 __global__ void __launch_bounds__(64)
 k_dtw_rescore_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ qmfcc,
                    const uint64_t* __restrict__ qoff, int c, const uint32_t* __restrict__ group_qid, const uint32_t* __restrict__ cand_idx,
                    uint32_t nt, int kp, int s_begin, int s_count, RescoreBound rb, double* __restrict__ bnd, uint32_t bnd_stride,
-                   double* __restrict__ exact, unsigned long long* __restrict__ counters) {
+                   double* __restrict__ exact, unsigned long long* __restrict__ counters, uint32_t band) {
     __shared__ double ring[2][64 * 32];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t gw = blockIdx.x * 2 + warp, nw = gridDim.x * 2;
@@ -1136,7 +1160,8 @@ k_dtw_rescore_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict_
             }
             if (lane == 0) atomicAdd(&counters[1], 1ull);
         }
-        const double e = warp_dtw_exact_long(qmfcc + qoff[qid] * c, la, dmfcc + doff[idx] * c, lb, c, ring[warp], bnd + (size_t)gw * bnd_stride, lane);
+        const double e =
+            warp_dtw_exact_long<BAND>(qmfcc + qoff[qid] * c, la, dmfcc + doff[idx] * c, lb, c, ring[warp], bnd + (size_t)gw * bnd_stride, lane, band);
         if (lane == 0) exact[pair] = e;
     }
 }
@@ -1152,13 +1177,14 @@ k_dtw_rescore_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict_
 // tensor-core scan was 1.5 of config 4's 39 ms, and a fixed ~0.5 ms of every shard's step at 8 GPUs).
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kSecondQueue = 192;  // entries a warp can queue for refinement; a query with more stays uncertified
+template <bool BAND>
 __global__ void __launch_bounds__(64)
 k_dtw_second_chance(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ qmfcc,
                     const uint64_t* __restrict__ qoff, int c, const uint32_t* __restrict__ group_qid, const uint32_t* __restrict__ cand_idx,
                     const unsigned long long* __restrict__ partial, uint32_t nlists, const unsigned long long* __restrict__ thr, uint32_t nslots,
                     int kp, int k, uint32_t index_base, const float* __restrict__ max_na, const float* __restrict__ max_nb, double eps,
                     const float* __restrict__ slot_max_na, int bound_mode, double inv_s, uint8_t* __restrict__ uncert_flag,
-                    uint32_t* __restrict__ out_idx, double* __restrict__ out_dist, unsigned long long* __restrict__ counters) {
+                    uint32_t* __restrict__ out_idx, double* __restrict__ out_dist, unsigned long long* __restrict__ counters, uint32_t band) {
     __shared__ double scost[2][32 * 32];
     __shared__ double squery[2][32 * SS_MAX_NCOEFFS];
     __shared__ uint32_t squeue[2][kSecondQueue];
@@ -1217,7 +1243,7 @@ k_dtw_second_chance(const double* __restrict__ dmfcc, const uint64_t* __restrict
     // ---- refine the queue (exact f64, the oracle's arithmetic), keeping the (distance, index) top-k --------------------------
     for (uint32_t e = 0; e < nqueued; e++) {
         const uint32_t idx = squeue[warp][e];
-        const double ex = warp_dtw_exact(squery[warp], la, dmfcc + doff[idx] * c, (int)(doff[idx + 1] - doff[idx]), c, scost[warp], lane);
+        const double ex = warp_dtw_exact<BAND>(squery[warp], la, dmfcc + doff[idx] * c, (int)(doff[idx + 1] - doff[idx]), c, scost[warp], lane, band);
         if (!(ex < kInf)) continue;
         if (n == k && !(ex < dv[k - 1] || (ex == dv[k - 1] && idx < iv[k - 1]))) continue;
         int pos = n < k ? n : k - 1;
@@ -1256,6 +1282,7 @@ k_dtw_second_chance(const double* __restrict__ dmfcc, const uint64_t* __restrict
 // 0.1 - 0.5 ms, so the queue is refined by the CTA's warps in parallel (each with its own cost ring and boundary row), then
 // thread 0 folds the results into the top-k and certifies.
 constexpr int kSecondWarps = 8;
+template <bool BAND>
 __global__ void __launch_bounds__(kSecondWarps * 32)
 k_dtw_second_chance_long(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ qmfcc,
                          const uint64_t* __restrict__ qoff, int c, const uint32_t* __restrict__ group_qid, const uint32_t* __restrict__ cand_idx,
@@ -1263,7 +1290,7 @@ k_dtw_second_chance_long(const double* __restrict__ dmfcc, const uint64_t* __res
                          uint32_t nslots, int kp, int k, uint32_t index_base, const float* __restrict__ max_na, const float* __restrict__ max_nb,
                          double eps, const float* __restrict__ slot_max_na, int bound_mode, double inv_s, int ld_max, double* __restrict__ bnd,
                          uint32_t bnd_stride, uint32_t bnd_rows_cap, uint8_t* __restrict__ uncert_flag, uint32_t* __restrict__ out_idx,
-                         double* __restrict__ out_dist, unsigned long long* __restrict__ counters) {
+                         double* __restrict__ out_dist, unsigned long long* __restrict__ counters, uint32_t band) {
     extern __shared__ __align__(16) unsigned char second_smem[];
     double* rings = reinterpret_cast<double*>(second_smem);                 // [warps][64 * 32]
     double* sexact = rings + kSecondWarps * 64 * 32;                         // [kSecondQueue]
@@ -1317,7 +1344,8 @@ k_dtw_second_chance_long(const double* __restrict__ dmfcc, const uint64_t* __res
     if (nqueued > (uint32_t)kSecondQueue) return;  // stays uncertified: the host re-runs it
     for (uint32_t e = warp; e < nqueued; e += kSecondWarps) {
         const uint32_t idx = squeue[e];
-        const double ex = warp_dtw_exact_long(a, la, dmfcc + doff[idx] * c, (int)(doff[idx + 1] - doff[idx]), c, rings + warp * 64 * 32, my_bnd, lane);
+        const double ex = warp_dtw_exact_long<BAND>(a, la, dmfcc + doff[idx] * c, (int)(doff[idx + 1] - doff[idx]), c, rings + warp * 64 * 32, my_bnd,
+                                                    lane, band);
         if (lane == 0) sexact[e] = ex;
     }
     __syncthreads();
@@ -1375,15 +1403,17 @@ int dtw_second_chance(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots,
         const uint32_t rows_cap = (uint32_t)std::max<uint64_t>(kSecondWarps, std::min<uint64_t>((uint64_t)nslots * kSecondWarps, (4ull << 20) / stride));
         SS_CUDA(ctx, d->d_second_bnd.reserve((size_t)rows_cap * stride));  // <= 32 MB of boundary rows
         const size_t smem = (size_t)kSecondWarps * 64 * 32 * sizeof(double) + kSecondQueue * (sizeof(double) + sizeof(uint32_t));
-        SS_CUDA(ctx, cudaFuncSetAttribute(k_dtw_second_chance_long, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_dtw_second_chance_long<<<nslots, kSecondWarps * 32, smem, ctx->stream>>>(
+        const auto kern = d->dtw_band ? k_dtw_second_chance_long<true> : k_dtw_second_chance_long<false>;
+        SS_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<nslots, kSecondWarps * 32, smem, ctx->stream>>>(
             d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d_slot_qid, d->d_cand_idx.p, d_partial, nlists, d_thr, nslots, kp, std::min(k, kp),
             d->index_base, d_max_na, d_max_nb, eps, d_slot_max_na, bound_mode, d->h2_bound_inv_s, (int)d->max_len, d->d_second_bnd.p, stride, rows_cap,
-            d_uncert_flag, d_out_idx, d_out_dist, d->d_counters.p);
+            d_uncert_flag, d_out_idx, d_out_dist, d->d_counters.p, d->dtw_band);
     } else {
-        k_dtw_second_chance<<<ceil_div(nslots, 2), 64, 0, ctx->stream>>>(
+        (d->dtw_band ? k_dtw_second_chance<true> : k_dtw_second_chance<false>)<<<ceil_div(nslots, 2), 64, 0, ctx->stream>>>(
             d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d_slot_qid, d->d_cand_idx.p, d_partial, nlists, d_thr, nslots, kp, std::min(k, kp),
-            d->index_base, d_max_na, d_max_nb, eps, d_slot_max_na, bound_mode, d->h2_bound_inv_s, d_uncert_flag, d_out_idx, d_out_dist, d->d_counters.p);
+            d->index_base, d_max_na, d_max_nb, eps, d_slot_max_na, bound_mode, d->h2_bound_inv_s, d_uncert_flag, d_out_idx, d_out_dist, d->d_counters.p,
+            d->dtw_band);
     }
     SS_LAUNCHED(ctx);
     return SS_OK;
@@ -1456,10 +1486,10 @@ int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslo
     SS_CUDA(ctx, cudaMemsetAsync(d->d_counters.p, 0, 4 * sizeof(unsigned long long), ctx->stream));
     if (!nslots || !d->ntiles) return SS_OK;
     if (d->max_len <= 32 && q->max_len <= 32) {  // one warp per query slot does the whole refine
-        k_dtw_refine_warp<<<ceil_div(nslots, 4), 128, 0, ctx->stream>>>(d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d_slot_qid,
-                                                                        d->d_cand_idx.p, d->d_cand_adist.p, nslots, kp, std::min(k, kp), d->index_base,
-                                                                        d_max_na, d_max_nb, eps, d_slot_max_na, bound_mode, d->h2_bound_inv_s,
-                                                                        d_uncert_flag, d_out_idx, d_out_dist, d->d_counters.p);
+        (d->dtw_band ? k_dtw_refine_warp<true> : k_dtw_refine_warp<false>)<<<ceil_div(nslots, 4), 128, 0, ctx->stream>>>(
+            d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d_slot_qid, d->d_cand_idx.p, d->d_cand_adist.p, nslots, kp, std::min(k, kp),
+            d->index_base, d_max_na, d_max_nb, eps, d_slot_max_na, bound_mode, d->h2_bound_inv_s, d_uncert_flag, d_out_idx, d_out_dist,
+            d->d_counters.p, d->dtw_band);
         SS_LAUNCHED(ctx);
         return SS_OK;
     }
@@ -1474,10 +1504,9 @@ int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslo
         RescoreBound rb = {phase ? d->d_cand_adist.p : nullptr, d_max_na, d_max_nb, d_slot_max_na, eps, bound_mode, std::min(k, kp), d->h2_bound_inv_s,
                            (int)d->max_len};
         const uint32_t nt = nslots * (uint32_t)s_count;
-        k_dtw_rescore_warp<<<std::min<uint32_t>(max_ctas, ceil_div(nt, 2)), 64, 0, ctx->stream>>>(d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c,
-                                                                                              d_slot_qid, d->d_cand_idx.p, nt, kp, s_begin, s_count, rb,
-                                                                                              d->d_rescore_rows.p, stride, d->d_cand_exact.p,
-                                                                                              d->d_counters.p);
+        (d->dtw_band ? k_dtw_rescore_warp<true> : k_dtw_rescore_warp<false>)<<<std::min<uint32_t>(max_ctas, ceil_div(nt, 2)), 64, 0, ctx->stream>>>(
+            d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d_slot_qid, d->d_cand_idx.p, nt, kp, s_begin, s_count, rb, d->d_rescore_rows.p,
+            stride, d->d_cand_exact.p, d->d_counters.p, d->dtw_band);
         SS_LAUNCHED(ctx);
     }
     k_dtw_finalize<<<ceil_div(nslots, 128), 128, 0, ctx->stream>>>(d->d_cand_idx.p, d->d_cand_adist.p, d->d_cand_exact.p, d_slot_qid, nslots, kp, k,
@@ -1491,10 +1520,11 @@ int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslo
 // exhaustive f64 DTW: (uncertified query u, every dictionary segment). One warp per pair (warp_dtw_exact_long); then one block
 // per query selects its top-k by (distance, index).
 // ---------------------------------------------------------------------------------------------------------------
+template <bool BAND>
 __global__ void __launch_bounds__(64)
 k_dtw_pairs_exact_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ qmfcc,
                        const uint64_t* __restrict__ qoff, int c, const uint32_t* __restrict__ qids, uint32_t nu, uint32_t nseg,
-                       double* __restrict__ bnd, uint32_t bnd_stride, double* __restrict__ exact) {
+                       double* __restrict__ bnd, uint32_t bnd_stride, double* __restrict__ exact, uint32_t band) {
     __shared__ double ring[2][64 * 32];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t gw = blockIdx.x * 2 + warp, nw = gridDim.x * 2;
@@ -1503,7 +1533,8 @@ k_dtw_pairs_exact_warp(const double* __restrict__ dmfcc, const uint64_t* __restr
         const uint32_t u = (uint32_t)(t / nseg), sidx = (uint32_t)(t % nseg);
         const uint32_t qid = qids[u];
         const int la = (int)(qoff[qid + 1] - qoff[qid]), lb = (int)(doff[sidx + 1] - doff[sidx]);
-        const double e = warp_dtw_exact_long(qmfcc + qoff[qid] * c, la, dmfcc + doff[sidx] * c, lb, c, ring[warp], bnd + (size_t)gw * bnd_stride, lane);
+        const double e =
+            warp_dtw_exact_long<BAND>(qmfcc + qoff[qid] * c, la, dmfcc + doff[sidx] * c, lb, c, ring[warp], bnd + (size_t)gw * bnd_stride, lane, band);
         if (lane == 0) exact[(size_t)u * nseg + sidx] = e;
     }
 }
@@ -1564,8 +1595,10 @@ int dtw_exhaustive_match(ss_dict* d, ss_queries* q, int k, const std::vector<uin
         const uint32_t nu = (uint32_t)std::min<size_t>(ubatch, subset.size() - u0);
         const uint64_t npairs = (uint64_t)nu * nseg;
         if (npairs) {
-            k_dtw_pairs_exact_warp<<<(unsigned)std::min<uint64_t>(max_ctas, (npairs + 1) / 2), 64, 0, ctx->stream>>>(
-                d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d->d_exh_qid.p + u0, nu, nseg, d->d_rescore_rows.p, stride, d->d_exh_dist.p);
+            (d->dtw_band ? k_dtw_pairs_exact_warp<true> : k_dtw_pairs_exact_warp<false>)<<<(unsigned)std::min<uint64_t>(max_ctas, (npairs + 1) / 2), 64, 0,
+                                                                                            ctx->stream>>>(
+                d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d->d_exh_qid.p + u0, nu, nseg, d->d_rescore_rows.p, stride, d->d_exh_dist.p,
+                d->dtw_band);
             SS_LAUNCHED(ctx);
         }
         k_dtw_select_exact<<<nu, 256, 0, ctx->stream>>>(d->d_exh_dist.p, nseg, k, d->d_exh_qid.p + u0, d->index_base, d_out_idx, d_out_dist);
@@ -1669,11 +1702,14 @@ __device__ __forceinline__ uint64_t align_dir(double up, double left, double dia
 }
 
 // warp_dtw_exact (same loads, same operations in the same order) + the directions of lane `lane`'s column in *dirs
+template <bool BAND>
 __device__ __forceinline__ double warp_dtw_align(const double* __restrict__ sa, int la, const double* __restrict__ b, int lb, int c, double* cst,
-                                                 int lane, uint64_t* dirs) {
+                                                 int lane, uint64_t* dirs, uint32_t band) {
     double br[SS_MAX_NCOEFFS];
 #pragma unroll
     for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = (k < c && lane < lb) ? b[(size_t)lane * c + k] : 0.0;
+    int blo = 0, bhi = 0;
+    if (BAND) band_rows(min(lane, lb - 1), la, lb, band, &blo, &bhi);
     for (int i = 0; i < la; i++) {
         double cost = 0.0;
 #pragma unroll
@@ -1699,7 +1735,8 @@ __device__ __forceinline__ double warp_dtw_align(const double* __restrict__ sa, 
             if (i == 0 && lane == 0) m = 0.0;
             else m = fmin(fmin(up, left), diag);
             w |= align_dir(up, left, diag, m) << (2 * i);
-            cur = cst[i * 32 + lane] + m;
+            if (BAND && (i < blo || i > bhi)) cur = kInf;
+            else cur = cst[i * 32 + lane] + m;
             if (i == la - 1 && lane == lb - 1) result = cur;
         }
         recv_prev = recv;
@@ -1710,7 +1747,8 @@ __device__ __forceinline__ double warp_dtw_align(const double* __restrict__ sa, 
 }
 
 // one warp per pair, both sides <= 32 frames (the other pairs are k_dtw_align_long's)
-__global__ void __launch_bounds__(128) k_dtw_align_warp(AlignArgs A) {
+template <bool BAND>
+__global__ void __launch_bounds__(128) k_dtw_align_warp(AlignArgs A, uint32_t band) {
     __shared__ double scost[4][32 * 32];
     __shared__ double squery[4][32 * SS_MAX_NCOEFFS];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1724,7 +1762,7 @@ __global__ void __launch_bounds__(128) k_dtw_align_warp(AlignArgs A) {
     for (int e = lane; e < la * c; e += 32) squery[warp][e] = a[e];
     __syncwarp();
     uint64_t dirs;
-    const double dist = warp_dtw_align(squery[warp], la, A.dmfcc + A.doff[s] * c, lb, c, scost[warp], lane, &dirs);
+    const double dist = warp_dtw_align<BAND>(squery[warp], la, A.dmfcc + A.doff[s] * c, lb, c, scost[warp], lane, &dirs, band);
     if (!(dist < kInf)) {  // NaN or inf: no path
         if (lane == 0) A.len[p] = 0, A.out_dist[p] = kInf;
         return;
@@ -1747,9 +1785,11 @@ __global__ void __launch_bounds__(128) k_dtw_align_warp(AlignArgs A) {
     if (lane == 0) A.len[p] = (uint64_t)n, A.out_dist[p] = dist;
 }
 
-// warp_dtw_exact_long (same loads, same operations in the same order) + the direction block `dir`, [strip][row / 32][lane]
+// warp_dtw_exact_long (same loads, same operations in the same order) + the direction block `dir`, [strip][row / 32][lane].
+// BAND: the same strip range; the words of row blocks outside it are not written, and no path cell reads them.
+template <bool BAND>
 __device__ __forceinline__ double warp_dtw_align_long(const double* __restrict__ a, int la, const double* __restrict__ b, int lb, int c,
-                                                      double* __restrict__ ring, double* bnd, uint64_t* __restrict__ dir, int lane) {
+                                                      double* __restrict__ ring, double* bnd, uint64_t* __restrict__ dir, int lane, uint32_t band) {
     double result = kInf;
     const int nstrips = (lb + 31) >> 5, nrb = (la + 31) >> 5;
     const int nsteps = la + 31;
@@ -1763,9 +1803,18 @@ __device__ __forceinline__ double warp_dtw_align_long(const double* __restrict__
         // at step t0 + r lane j is on row t0 + r - j: row block t0 / 32 - 1 (wprev) or t0 / 32 (wcur)
         uint64_t wprev = 0, wcur = 0;
         uint64_t* sdir = dir + (size_t)s * nrb * 32 + lane;
+        int blo = 0, bhi = 0, rhi = 0, t0b = 0, t0e = nsteps;
+        if (BAND) {
+            band_rows(min(col, lb - 1), la, lb, band, &blo, &bhi);
+            rhi = __shfl_sync(0xffffffffu, bhi, 31);
+            t0b = __shfl_sync(0xffffffffu, blo, 0) & ~31;
+            t0e = min(nsteps, rhi + 32);
+        }
         __syncwarp();
-        for (int t0 = 0; t0 < nsteps; t0 += 32) {
-            const int rows = min(32, la - t0);
+        if (BAND && lane == 0 && !first && t0b > 0) bl_prev = bnd[t0b - 1];
+        int t0 = t0b;
+        for (; t0 < t0e; t0 += 32) {
+            const int rows = min(32, (BAND ? rhi + 1 : la) - t0);
             int r = 0;
             for (; r + 4 <= rows; r += 4) {
                 const double* ar = a + (size_t)(t0 + r) * c;
@@ -1813,7 +1862,8 @@ __device__ __forceinline__ double warp_dtw_align_long(const double* __restrict__
                     const uint64_t bits = align_dir(up, left, diag, m) << (2 * (i & 31));
                     if (i < t0) wprev |= bits;
                     else wcur |= bits;
-                    cur = ring[(i & 63) * 32 + lane] + m;
+                    if (BAND && (i < blo || i > bhi)) cur = kInf;
+                    else cur = ring[(i & 63) * 32 + lane] + m;
                     if (last && i == la - 1 && col == lb - 1) result = cur;
                     if (!last && lane == 31) bnd[i] = cur;
                 }
@@ -1825,8 +1875,10 @@ __device__ __forceinline__ double warp_dtw_align_long(const double* __restrict__
             wprev = wcur;
             wcur = 0;
         }
-        const int rb_last = (nsteps - 1) >> 5;
+        const int rb_last = ((BAND ? t0 : nsteps) - 1) >> 5;
         if (rb_last < nrb) sdir[(size_t)rb_last * 32] = wprev;
+        if (BAND && !last)
+            for (int r = max(0, min(t0, nsteps) - 31) + lane; r < la; r += 32) bnd[r] = kInf;
     }
     result = __shfl_sync(0xffffffffu, result, (lb - 1) & 31);
     return result / (double)(la + lb);
@@ -1834,8 +1886,9 @@ __device__ __forceinline__ double warp_dtw_align_long(const double* __restrict__
 
 // one warp per pair of the wave [p0, p0 + np) that has a side longer than 32 frames; the pair's direction block and
 // boundary row are its own (dir_stride u64 words, bnd_stride doubles)
+template <bool BAND>
 __global__ void __launch_bounds__(64) k_dtw_align_long(AlignArgs A, uint32_t p0, uint32_t np, uint64_t* __restrict__ dir, uint64_t dir_stride,
-                                                       double* __restrict__ bnd, uint32_t bnd_stride) {
+                                                       double* __restrict__ bnd, uint32_t bnd_stride, uint32_t band) {
     __shared__ double ring[2][64 * 32];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t t = blockIdx.x * 2 + warp;
@@ -1846,8 +1899,8 @@ __global__ void __launch_bounds__(64) k_dtw_align_long(AlignArgs A, uint32_t p0,
     if (!align_pair(A, p, -1, &la, &lb, &s) || (la <= 32 && lb <= 32)) return;  // (lane -1: k_dtw_align_warp wrote those)
     const int c = A.c;
     uint64_t* my_dir = dir + (size_t)t * dir_stride;
-    const double dist = warp_dtw_align_long(A.qmfcc + A.qoff[p] * c, la, A.dmfcc + A.doff[s] * c, lb, c, ring[warp],
-                                            bnd + (size_t)t * bnd_stride, my_dir, lane);
+    const double dist = warp_dtw_align_long<BAND>(A.qmfcc + A.qoff[p] * c, la, A.dmfcc + A.doff[s] * c, lb, c, ring[warp],
+                                                  bnd + (size_t)t * bnd_stride, my_dir, lane, band);
     if (!(dist < kInf)) {
         if (lane == 0) A.len[p] = 0, A.out_dist[p] = kInf;
         return;
@@ -1938,11 +1991,13 @@ int dtw_align_dev(ss_dict* d, const double* d_qmfcc, const uint64_t* d_qoff, con
     SS_CUDA(ctx, cub::DeviceScan::InclusiveSum(nullptr, cub_bytes, d->d_align_len.p, d_out_off + 1, (int)nq, ctx->stream));
     SS_CUDA(ctx, d->d_align_cub.reserve(cub_bytes));
 
-    k_dtw_align_warp<<<ceil_div((long long)nq, 4), 128, 0, ctx->stream>>>(A);
+    (d->dtw_band ? k_dtw_align_warp<true> : k_dtw_align_warp<false>)<<<ceil_div((long long)nq, 4), 128, 0, ctx->stream>>>(A, d->dtw_band);
     SS_LAUNCHED(ctx);
     for (const Wave& w : waves) {
         const uint64_t dir_stride = (uint64_t)((w.lq + 31) / 32) * ((ld_max + 31) / 32) * 32;
-        k_dtw_align_long<<<ceil_div(w.np, 2), 64, 0, ctx->stream>>>(A, w.p0, w.np, d->d_align_dir.p, dir_stride, d->d_align_bnd.p, w.lq);
+        (d->dtw_band ? k_dtw_align_long<true> : k_dtw_align_long<false>)<<<ceil_div(w.np, 2), 64, 0, ctx->stream>>>(A, w.p0, w.np, d->d_align_dir.p,
+                                                                                                                 dir_stride, d->d_align_bnd.p, w.lq,
+                                                                                                                 d->dtw_band);
         SS_LAUNCHED(ctx);
     }
     SS_CUDA(ctx, cub::DeviceScan::InclusiveSum(d->d_align_cub.p, cub_bytes, d->d_align_len.p, d_out_off + 1, (int)nq, ctx->stream));

@@ -116,6 +116,7 @@ struct ss_dict {
     ss::DevBuf<int4> d_h2_desc;
     ss::DevBuf<unsigned long long> d_h2_timeline;  // SS_DTW_H2_TIMELINE measurement hook
     ss::DevBuf<unsigned long long> d_h2_thr;   // per query slot: running bound on the global KP-th key (dtw_h2.cu)
+    uint32_t dtw_band = 0;  // Sakoe-Chiba radius of the exact DTW stages and of ss_dict_align (ss_dict_set_dtw_band); 0 = no band
     int scan_pref = 0;  // test / A-B hook (ss_dict_set_scan): 0 = packed-half scan first, 1 = start at the fp32 tensor-core scan, 2 = fp32 CUDA-core scan, 3 = packed-half scan without its second chance
     // the last SS_DTW match is asynchronous up to its fallback decision: ss::dtw_match_finish waits for ev_done, reads the
     // uncertified count from pinned memory and runs the later stages for the queries that need them
@@ -237,6 +238,23 @@ struct TraceTimer {
         t0 = t1;
     }
 };
+
+// Sakoe-Chiba band (A10, DESIGN.md §3.1f): the rows [*lo, *hi] of column j (0 <= j < lb; la, lb >= 1) that lie inside the band
+// of radius r >= 1, |i (lb - 1) - j (la - 1)| <= r max(la - 1, lb - 1). Both ends are monotone in j. r is capped at max(la, lb),
+// beyond which the band covers the whole matrix anyway, so that the products stay inside 64 bits. The exact kernels (exact.cu)
+// and the host's cost estimate of the exhaustive stage (dtw.cu) use the same rows.
+__host__ __device__ __forceinline__ void band_rows(int j, int la, int lb, uint32_t r, int* lo, int* hi) {
+    const long long A = lb - 1, B = la - 1;
+    if (A == 0) {  // one column: every row
+        *lo = 0, *hi = la - 1;
+        return;
+    }
+    const long long rr = r < (uint32_t)(la > lb ? la : lb) ? r : (la > lb ? la : lb);
+    const long long w = rr * (A > B ? A : B), x = (long long)j * B;
+    *lo = x - w <= 0 ? 0 : (int)((x - w + A - 1) / A);
+    const long long h = (x + w) / A;
+    *hi = h < la - 1 ? (int)h : la - 1;
+}
 
 int dtw_dict_build(ss_dict* d);       // builds the fp32 stream + strip / tile tables (dtw.cu)
 int dtw_tc_dict_build(ss_dict* d);    // builds the fp16 UMMA tiles (dtw_tc.cu)
