@@ -1,8 +1,9 @@
 // examples/reconstruction.cpp — the flow of the reference's examples/reconstruction.rs (and, with --partition-only,
 // examples/partition.rs) written against include/soundsym.hpp:
-//   -s source.wav  -t target.wav  -o out.wav  -m model.bin  [--depth 3] [--threshold 4] [--dtw] [--partition-only]
+//   -s source.wav  -t target.wav  -o out.wav  -m model.bin  [--depth 3] [--threshold 4] [--dtw] [--warp] [--partition-only]
 // Partitioner::from_path(source).threshold(4).depth(3) -> train (model supplied) -> partition -> SoundDictionary::from_segments
-// -> partition the target with the source's model -> clone_from_dictionary -> to_sound -> write_file.
+// -> partition the target with the source's model -> clone_from_dictionary -> to_sound -> write_file. --warp fits every matched
+// sound to its target segment's timing along the DTW warping path (ss_resynth_warped) instead of zero-padding or cutting it.
 // Prints one JSON line with the segment counts, the match indices and checksums so that a test can compare it with the
 // golden fixtures.
 #include <cmath>
@@ -17,7 +18,7 @@ using namespace soundsym;
 int main(int argc, char** argv) {
     std::string src, tgt, out, model_path;
     size_t depth = 3, threshold = 4;  // examples/reconstruction.rs:44-45
-    bool dtw = false, partition_only = false, morph = false, matcher_loop = false;
+    bool dtw = false, partition_only = false, morph = false, matcher_loop = false, warp = false;
     size_t chain = 6;
     std::string dict_dir, query_dir, splits_dir;  // --matcher <dictionary dir> <query dir>: the flow of examples/matcher.rs
     for (int i = 1; i < argc; i++) {
@@ -30,6 +31,7 @@ int main(int argc, char** argv) {
         else if (a == "--depth") depth = std::stoul(next());
         else if (a == "--threshold") threshold = std::stoul(next());
         else if (a == "--dtw") dtw = true;
+        else if (a == "--warp") warp = true;
         else if (a == "--partition-only") partition_only = true;
         else if (a == "--matcher") dict_dir = next(), query_dir = next();
         else if (a == "--matcher-loop") dict_dir = next(), query_dir = next(), matcher_loop = true;
@@ -130,7 +132,7 @@ int main(int argc, char** argv) {
             return 0;
         }
         std::vector<uint32_t> idx;
-        Sound result = sequence.clone_from_dictionary_to_sound(*dictionary, &idx);
+        Sound result = sequence.clone_from_dictionary_to_sound(*dictionary, &idx, warp);
         if (!out.empty()) result.write_file(out);
         double sum = 0;
         for (double s : result.samples()) sum += s;

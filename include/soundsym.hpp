@@ -450,11 +450,23 @@ class SoundSequence {
     const std::vector<double>& distances() const { return distances_; }
 
     /// SoundSequence::clone_from_dictionary (src/sound.rs:451-472) + to_sound (:475-483): ONE batched match, then the
-    /// pad / truncate / concatenate on the GPU. Returns the assembled Sound.
-    Sound clone_from_dictionary_to_sound(SoundDictionary& dict, std::vector<uint32_t>* out_idx = nullptr) {
+    /// pad / truncate / concatenate on the GPU. Returns the assembled Sound. warp: each matched sound follows its target's
+    /// timing along the DTW warping path of the pair (SoundDictionary::align, with the dictionary's band, whichever matcher
+    /// chose it; then ss_resynth_warped) instead of being zero-padded or cut.
+    Sound clone_from_dictionary_to_sound(SoundDictionary& dict, std::vector<uint32_t>* out_idx = nullptr, bool warp = false) {
         std::vector<uint32_t> idx;
         std::vector<double> dist;
         dict.match_indices(sounds_, {}, 1, &idx, &dist);
+        std::vector<uint32_t> cells;
+        std::vector<uint64_t> poff(sounds_.size() + 1, 0);
+        if (warp) {
+            std::vector<std::vector<std::pair<uint32_t, uint32_t>>> paths;
+            dict.align(sounds_, idx, &paths, &dist);
+            for (size_t t = 0; t < paths.size(); t++) {
+                for (const auto& c : paths[t]) cells.insert(cells.end(), {c.first, c.second});
+                poff[t + 1] = poff[t] + paths[t].size();
+            }
+        }
         std::vector<uint64_t> doff(dict.sounds.size() + 1, 0), tlen(sounds_.size());
         std::vector<double> dsamples;
         for (size_t i = 0; i < dict.sounds.size(); i++) {
@@ -464,7 +476,11 @@ class SoundSequence {
         uint64_t total = 0;
         for (size_t i = 0; i < sounds_.size(); i++) total += (tlen[i] = sounds_[i]->samples().size());
         std::vector<double> out(total);
-        ctx_->check(ss_resynth(ctx_->get(), dsamples.data(), doff.data(), dict.sounds.size(), idx.data(), tlen.data(), sounds_.size(), out.data()));
+        if (warp)
+            ctx_->check(ss_resynth_warped(ctx_->get(), dsamples.data(), doff.data(), dict.sounds.size(), idx.data(), cells.data(), poff.data(), tlen.data(),
+                                          sounds_.size(), out.data()));
+        else
+            ctx_->check(ss_resynth(ctx_->get(), dsamples.data(), doff.data(), dict.sounds.size(), idx.data(), tlen.data(), sounds_.size(), out.data()));
         if (out_idx) *out_idx = idx;
         const double sr = sounds_.empty() ? 44100.0 : sounds_[0]->sample_rate();
         return Sound::from_samples(std::move(out), sr, std::nullopt, std::nullopt, *ctx_);

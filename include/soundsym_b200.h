@@ -307,6 +307,25 @@ int ss_sharded_dict_set_dtw_band(ss_sharded_dict* dict, uint32_t radius);
  *              target_lens[t]; segments are concatenated into out_samples (capacity sum(target_lens)). */
 int ss_resynth(ss_ctx* ctx, const double* dict_samples, const uint64_t* dict_sample_offsets, size_t ndict,
                const uint32_t* match_idx, const uint64_t* target_lens, size_t nseg, double* out_samples);
+/* ss_resynth_warped   ss_resynth along the DTW warping path of each match (no reference counterpart; spec A11, DESIGN.md §3.5), so
+ *              that every matched sound follows its target segment's timing instead of being zero-padded or cut. paths /
+ *              path_offsets are what ss_dict_align writes for the same segments and indices: (i, j) uint32 pairs, path t =
+ *              paths[2 path_offsets[t] .. 2 path_offsets[t+1]) (nseg + 1 offsets in pairs, path_offsets[0] = 0). With H = SS_HOP,
+ *              L = target_lens[t], m = match_idx[t] and X(p) = sample p of dictionary sound m (0.0 at or past its end):
+ *              - output block b (samples n = b H + r, 0 <= r < min(H, L - b H)) plays source frame j(b): the j of the first cell
+ *                of row b; for b >= Lq = 1 + the last cell's i, j(b) = j(Lq-1) + (b - Lq + 1); an empty path gives j(b) = b;
+ *              - with s_b = j(b) H (64-bit): out = X(s_b + r) if b = 0 or s_b = s_{b-1} + H, else the one-hop crossfade
+ *                X(s_{b-1} + H + r) (H - r) / H + X(s_b + r) r / H (exact dyadic weights; two products and a sum, each
+ *                rounded to nearest, no FMA).
+ *              A diagonal or empty path gives ss_resynth's samples bit for bit. Segments are concatenated into out_samples
+ *              (capacity sum(target_lens)). Host buffers, stream-synchronised on return; one kernel launch, none when
+ *              sum(target_lens) = 0. SS_ERR_INVALID (with a message) for a NULL buffer (paths may be NULL when every path is
+ *              empty), path offsets not monotone or not starting at 0, a non-empty path not starting at (0, 0), a step other
+ *              than (1, 0), (0, 1), (1, 1), or match_idx[t] >= ndict; nseg == 0 returns SS_OK and launches nothing; ndict == 0
+ *              gives SS_ERR_EMPTY_DICT. */
+int ss_resynth_warped(ss_ctx* ctx, const double* dict_samples, const uint64_t* dict_sample_offsets, size_t ndict,
+                      const uint32_t* match_idx, const uint32_t* paths, const uint64_t* path_offsets, const uint64_t* target_lens,
+                      size_t nseg, double* out_samples);
 
 /* cosine_sim_angular over consecutive mean-MFCC rows, SoundSequence::new (src/sound.rs:392-396, 62-69):
  * out_dist[i] = acos(clamp(cosine_sim(mean[i], mean[i+1]))) / pi with the reference's x < -1 -> 1 rule; nrows-1 outputs */

@@ -20,7 +20,7 @@ SYMBOLS = [
     "ss_ctx_launch_count", "ss_frame_count", "ss_decode_pcm", "ss_sound_analyze", "ss_sound_analyze_pcm", "ss_sound_analyze_batch", "ss_mfcc", "ss_max_power", "ss_mfcc_dev",
     "ss_symbols", "ss_gmm_train", "ss_vote_split", "ss_partition", "ss_dict_create", "ss_dict_destroy", "ss_dict_len", "ss_dict_match",
     "ss_queries_create", "ss_queries_destroy", "ss_dict_match_dev", "ss_topk_merge_dev", "ss_dict_last_work", "ss_dict_last_scan_kind",
-    "ss_dict_last_uncertified", "ss_dict_last_tc_fallback", "ss_dict_last_exhaustive", "ss_queries_invalidate", "ss_dict_last_scan_ms", "ss_resynth", "ss_sequence_distances", "ss_dict_debug_tc_scan", "ss_dict_debug_h2_scan", "ss_dict_set_scan", "ss_dict_match_finish",
+    "ss_dict_last_uncertified", "ss_dict_last_tc_fallback", "ss_dict_last_exhaustive", "ss_queries_invalidate", "ss_dict_last_scan_ms", "ss_resynth", "ss_resynth_warped", "ss_sequence_distances", "ss_dict_debug_tc_scan", "ss_dict_debug_h2_scan", "ss_dict_set_scan", "ss_dict_match_finish",
     "ss_dict_set_dtw_band", "ss_dict_dtw_band", "ss_sharded_dict_set_dtw_band",
     "ss_dict_walk", "ss_dict_walk_dev", "ss_dict_align", "ss_dict_align_dev",
     "ss_shard_bounds", "ss_comm_unique_id", "ss_comm_create", "ss_comm_create_all", "ss_comm_destroy", "ss_comm_rank", "ss_comm_nranks",
@@ -138,6 +138,7 @@ def load():
     L.ss_sharded_dict_nshards.argtypes = [vp]
     L.ss_dict_debug_tc_scan.argtypes = [vp, vp, vp, sz, vp, vp, P(C.c_float)]
     L.ss_resynth.argtypes = [vp, vp, vp, sz, vp, vp, sz, vp]
+    L.ss_resynth_warped.argtypes = [vp, vp, vp, sz, vp, vp, vp, vp, sz, vp]
     L.ss_sequence_distances.argtypes = [vp, vp, sz, i, vp]
     _lib = L
     return L

@@ -202,6 +202,23 @@ class Context:
         self.check(self.lib.ss_resynth(self.h, _ptr(ds), _ptr(do), do.shape[0] - 1, _ptr(mi), _ptr(tl), mi.shape[0], _ptr(out)))
         return out
 
+    def resynth_warped(self, dict_samples, dict_sample_offsets, match_idx, paths, path_offsets, target_lens):
+        """ss_resynth_warped: resynth along the DTW warping paths (A11, DESIGN.md §3.5). paths: uint32 [cells, 2] of (i, j),
+        path t = paths[path_offsets[t]:path_offsets[t + 1]] (what DeviceDictionary.align returns, concatenated)."""
+        ds = np.ascontiguousarray(dict_samples, dtype=np.float64)
+        do = np.ascontiguousarray(dict_sample_offsets, dtype=np.uint64)
+        mi = np.ascontiguousarray(match_idx, dtype=np.uint32)
+        pa = np.ascontiguousarray(paths, dtype=np.uint32).reshape(-1, 2)
+        po = np.ascontiguousarray(path_offsets, dtype=np.uint64)
+        tl = np.ascontiguousarray(target_lens, dtype=np.uint64)
+        if po.shape[0] != mi.shape[0] + 1 or tl.shape[0] != mi.shape[0]:
+            raise SoundsymError(_lib.SS_ERR_INVALID, "one path and one target length per segment (%d indices, %d path offsets, %d lengths)"
+                                % (mi.shape[0], po.shape[0], tl.shape[0]))
+        out = np.empty(int(tl.sum()), dtype=np.float64)
+        self.check(self.lib.ss_resynth_warped(self.h, _ptr(ds), _ptr(do), do.shape[0] - 1, _ptr(mi), _ptr(pa), _ptr(po), _ptr(tl), mi.shape[0],
+                                              _ptr(out)))
+        return out
+
     def sequence_distances(self, mean_rows):
         m = np.ascontiguousarray(mean_rows, dtype=np.float64)
         out = np.empty(max(m.shape[0] - 1, 0), dtype=np.float64)
@@ -727,9 +744,11 @@ class SoundSequence:
     def distances(self):
         return self._distances
 
-    def clone_from_dictionary(self, dictionary):
+    def clone_from_dictionary(self, dictionary, warp=False):
         """src/sound.rs:451-472: nearest dictionary sound per segment (ONE batched match), zero-padded / truncated to
-        the target segment's length on the GPU (ss_resynth)."""
+        the target segment's length on the GPU (ss_resynth). warp=True: each matched sound follows its target's timing along
+        the DTW warping path of the pair (dictionary.align, with the dictionary's band, whichever matcher chose it; then
+        ss_resynth_warped), and the output segments are analysed in one batch."""
         if not self._sounds:
             return SoundSequence([], self._ctx)
         idx, _ = dictionary.match_indices(self._sounds)
@@ -739,6 +758,8 @@ class SoundSequence:
         doff[1:] = np.cumsum(dlens)
         dsamples = np.concatenate([s.samples() for s in dictionary.sounds]) if int(doff[-1]) else np.zeros(0)
         tlens = np.array([len(s.samples()) for s in self._sounds], dtype=np.uint64)
+        if warp:
+            return self._clone_warped(dictionary, idx, dsamples, doff, tlens)
         out = self._ctx.resynth(dsamples, doff, idx, tlens)
         sounds, pos = [], 0
         for t, s in enumerate(self._sounds):
@@ -749,6 +770,24 @@ class SoundSequence:
             else:
                 sounds.append(Sound.from_samples(out[pos:pos + ln], s.sample_rate(), None, None, self._ctx))
             pos += ln
+        seq = SoundSequence(sounds, self._ctx)
+        seq._assembled = out
+        return seq
+
+    def _clone_warped(self, dictionary, idx, dsamples, doff, tlens):
+        sr = self._sounds[0].sample_rate()
+        if any(s.sample_rate() != sr for s in self._sounds):
+            raise ValueError("warped resynthesis analyses its output in one batch: every segment needs the same sample rate")
+        paths, _ = dictionary.align(self._sounds, idx)
+        poff = np.zeros(len(paths) + 1, dtype=np.uint64)
+        poff[1:] = np.cumsum([p.shape[0] for p in paths])
+        cells = np.concatenate(paths) if int(poff[-1]) else np.zeros((0, 2), dtype=np.uint32)
+        out = self._ctx.resynth_warped(dsamples, doff, idx, cells, poff, tlens)
+        ooff = np.zeros(len(tlens) + 1, dtype=np.uint64)
+        ooff[1:] = np.cumsum(tlens)
+        mfcc, foff, mp, mean = self._ctx.analyze_batch(out, ooff, sr, NCOEFFS)
+        sounds = [Sound(out[int(ooff[t]):int(ooff[t + 1])], sr, mfcc[int(foff[t]):int(foff[t + 1])], float(mp[t]), mean[t], None, self._ctx)
+                  for t in range(len(tlens))]
         seq = SoundSequence(sounds, self._ctx)
         seq._assembled = out
         return seq

@@ -6,6 +6,7 @@
 //   k_max_power    analyze_max_power: rectangular 128/64 frames, max RMS         src/sound.rs:244-256 (bit-exact fold)
 //   k_colsum_*     analyze_mean_mfccs                                            src/sound.rs:271-286
 //   k_resynth      clone_from_dictionary's pad / truncate + to_sound's concat   src/sound.rs:451-483
+//   k_resynth_warped  the same along the DTW warping path of each match (ss_resynth_warped; no reference counterpart, A11)
 //
 // k_mfcc: one warp per frame, all arithmetic in f64. The real 1024-point transform is done as a 512-point complex
 // Stockham FFT (three radix-8 passes, 2 butterflies per lane per pass, the first pass reading the windowed samples
@@ -62,6 +63,8 @@ struct SoundState {
     DevBuf<unsigned long long> d_maxbits;
     DevBuf<uint64_t> d_off_a, d_off_b, d_off_pf;
     DevBuf<uint32_t> d_idx;
+    DevBuf<uint64_t> d_path_off;  // ss_resynth_warped: path offsets (in cells) and (i, j) cells
+    DevBuf<uint2> d_path;
     // chunked ingest (ss_sound_analyze / _pcm on long inputs): the H2D copy of chunk k+1 runs on copy_stream while chunk k is
     // converted and analysed on the ctx stream
     cudaStream_t copy_stream = nullptr;
@@ -493,6 +496,53 @@ __global__ void k_resynth(const double* __restrict__ dict_samples, const uint64_
     }
 }
 
+// Resynthesis along the DTW warping path (ss_resynth_warped, DESIGN.md §3.5, A11): output block b (SS_HOP samples) of segment t
+// plays dictionary frame j(b) = the j of the first path cell of row b; past the path's last row the source runs on at unit speed.
+// Where j(b - 1) -> j(b) is not a unit step, the block crossfades linearly from where the previous block would have gone on.
+// Path cells are in forward order, so their i is non-decreasing and every row 0..Lq-1 occurs: the first cell of row b is the
+// lower bound of b in the segment's i values. The 32 lanes of a warp share b (SS_HOP is a multiple of 32) unless the warp
+// straddles two segments, so the search reads broadcast.
+__device__ __forceinline__ uint64_t warp_src_frame(const uint2* __restrict__ path, uint64_t p0, uint64_t p1, uint64_t b) {
+    if (p0 == p1) return b;  // empty path: the diagonal
+    const uint64_t lq = (uint64_t)path[p1 - 1].x + 1;
+    const uint64_t row = b < lq ? b : lq - 1;
+    uint64_t lo = p0, hi = p1 - 1;  // first cell with i >= row; row <= the last cell's i, so it lies in [p0, p1 - 1]
+    while (lo < hi) {
+        const uint64_t mid = (lo + hi) >> 1;
+        if ((uint64_t)path[mid].x < row) lo = mid + 1;
+        else hi = mid;
+    }
+    return (uint64_t)path[lo].y + (b - row);
+}
+
+__global__ void k_resynth_warped(const double* __restrict__ dict_samples, const uint64_t* __restrict__ dict_off,
+                                 const uint32_t* __restrict__ match_idx, const uint2* __restrict__ path, const uint64_t* __restrict__ path_off,
+                                 const uint64_t* __restrict__ out_off, size_t nseg, size_t total, double* __restrict__ out) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        size_t lo = 0, hi = nseg;  // last segment whose out_off <= i
+        while (hi - lo > 1) {
+            const size_t mid = (lo + hi) >> 1;
+            if (out_off[mid] <= i) lo = mid;
+            else hi = mid;
+        }
+        const uint64_t within = i - out_off[lo], b = within / SS_HOP, r = within % SS_HOP;
+        const uint32_t m = match_idx[lo];
+        const uint64_t base = dict_off[m], len = dict_off[m + 1] - base, p0 = path_off[lo], p1 = path_off[lo + 1];
+        auto x = [&](uint64_t p) { return p < len ? dict_samples[base + p] : 0.0; };
+        const uint64_t s = warp_src_frame(path, p0, p1, b) * SS_HOP;
+        const double a = x(s + r);
+        double v = a;
+        if (b > 0) {
+            const uint64_t prev = warp_src_frame(path, p0, p1, b - 1) * SS_HOP;
+            if (s != prev + SS_HOP) {  // not contiguous: c (H - r) / H + a r / H, weights exact, no FMA
+                const double c = x(prev + SS_HOP + r);
+                v = __dadd_rn(__dmul_rn(c, (double)(SS_HOP - r) * (1.0 / SS_HOP)), __dmul_rn(a, (double)r * (1.0 / SS_HOP)));
+            }
+        }
+        out[i] = v;
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 static int mfcc_launch(ss_ctx* ctx, const double* d_samples, size_t n, double sample_rate, int c, double* d_out, size_t frames) {
     if (!frames) return SS_OK;
@@ -790,6 +840,55 @@ int ss_resynth(ss_ctx* ctx, const double* dict_samples, const uint64_t* dict_sam
     SS_CUDA(ctx, st->d_mfcc.reserve(total));
     const int grid = (int)std::min<size_t>((total + 255) / 256, (size_t)ctx->sm_count * 16);
     k_resynth<<<grid, 256, 0, ctx->stream>>>(st->d_samples.p, st->d_off_a.p, st->d_idx.p, st->d_off_b.p, nseg, total, st->d_mfcc.p);
+    SS_LAUNCHED(ctx);
+    SS_CUDA(ctx, cudaMemcpyAsync(out_samples, st->d_mfcc.p, total * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return SS_OK;
+}
+
+int ss_resynth_warped(ss_ctx* ctx, const double* dict_samples, const uint64_t* dict_sample_offsets, size_t ndict, const uint32_t* match_idx,
+                      const uint32_t* paths, const uint64_t* path_offsets, const uint64_t* target_lens, size_t nseg, double* out_samples) {
+    if (!ctx) return set_error(nullptr, SS_ERR_INVALID, "ctx is NULL");
+    if (!nseg) return SS_OK;
+    if (!dict_sample_offsets || !match_idx || !path_offsets || !target_lens || !out_samples) return set_error(ctx, SS_ERR_INVALID, "NULL buffer");
+    if (!ndict) return set_error(ctx, SS_ERR_EMPTY_DICT, "resynthesis from an empty dictionary");
+    for (size_t i = 0; i < ndict; i++)
+        if (dict_sample_offsets[i + 1] < dict_sample_offsets[i]) return set_error(ctx, SS_ERR_INVALID, "dictionary offsets not monotone at %zu", i);
+    if (path_offsets[0] != 0) return set_error(ctx, SS_ERR_INVALID, "path_offsets[0] must be 0");
+    std::vector<uint64_t> out_off(nseg + 1, 0);
+    for (size_t t = 0; t < nseg; t++) {
+        if (match_idx[t] >= ndict) return set_error(ctx, SS_ERR_INVALID, "match_idx[%zu] = %u out of range", t, match_idx[t]);
+        if (path_offsets[t + 1] < path_offsets[t]) return set_error(ctx, SS_ERR_INVALID, "path offsets not monotone at %zu", t);
+        out_off[t + 1] = out_off[t] + target_lens[t];
+    }
+    const size_t cells = path_offsets[nseg];
+    if (cells && !paths) return set_error(ctx, SS_ERR_INVALID, "paths is NULL");
+    for (size_t t = 0; t < nseg; t++) {  // each path runs from (0, 0) in steps (1, 0), (0, 1) or (1, 1): what the kernel's search relies on
+        const uint64_t p0 = path_offsets[t], p1 = path_offsets[t + 1];
+        if (p0 == p1) continue;
+        if (paths[2 * p0] != 0 || paths[2 * p0 + 1] != 0) return set_error(ctx, SS_ERR_INVALID, "path %zu does not start at (0, 0)", t);
+        for (uint64_t e = p0 + 1; e < p1; e++) {
+            const uint32_t di = paths[2 * e] - paths[2 * e - 2], dj = paths[2 * e + 1] - paths[2 * e - 1];
+            if (di > 1 || dj > 1 || (di | dj) == 0)
+                return set_error(ctx, SS_ERR_INVALID, "path %zu: step %llu -> %llu is not (1, 0), (0, 1) or (1, 1)", t,
+                                 (unsigned long long)(e - 1 - p0), (unsigned long long)(e - p0));
+        }
+    }
+    const size_t total = out_off[nseg], dtotal = dict_sample_offsets[ndict];
+    if (!total) return SS_OK;
+    if (dtotal && !dict_samples) return set_error(ctx, SS_ERR_INVALID, "dict_samples is NULL");
+    SS_CUDA(ctx, cudaSetDevice(ctx->device));
+    SoundState* st = sound_state(ctx);
+    SS_TRY(upload(ctx, st->d_samples, dict_samples, dtotal));
+    SS_TRY(upload(ctx, st->d_off_a, dict_sample_offsets, ndict + 1));
+    SS_TRY(upload(ctx, st->d_off_b, out_off.data(), nseg + 1));
+    SS_TRY(upload(ctx, st->d_idx, match_idx, nseg));
+    SS_TRY(upload(ctx, st->d_path_off, path_offsets, nseg + 1));
+    SS_TRY(upload(ctx, st->d_path, reinterpret_cast<const uint2*>(paths), cells));
+    SS_CUDA(ctx, st->d_mfcc.reserve(total));
+    const int grid = (int)std::min<size_t>((total + 255) / 256, (size_t)ctx->sm_count * 16);
+    k_resynth_warped<<<grid, 256, 0, ctx->stream>>>(st->d_samples.p, st->d_off_a.p, st->d_idx.p, st->d_path.p, st->d_path_off.p, st->d_off_b.p, nseg,
+                                                    total, st->d_mfcc.p);
     SS_LAUNCHED(ctx);
     SS_CUDA(ctx, cudaMemcpyAsync(out_samples, st->d_mfcc.p, total * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
