@@ -101,7 +101,6 @@ __global__ void k_topk_merge_blocks(const unsigned char* __restrict__ blocks, si
                                     uint32_t* __restrict__ out_idx, double* __restrict__ out_dist) {
     const size_t qi = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (qi >= nq) return;
-    const double kInf = __longlong_as_double(0x7ff0000000000000ll);
     double dv[SS_MAX_TOPK];
     uint32_t iv[SS_MAX_TOPK];
     int n = 0;
@@ -111,23 +110,10 @@ __global__ void k_topk_merge_blocks(const unsigned char* __restrict__ blocks, si
         for (int s = 0; s < k; s++) {
             const double dd = dist[qi * k + s];
             const uint32_t ii = idx[qi * k + s];
-            if (ii == 0xFFFFFFFFu || dd != dd) continue;
-            if (n == k && !(dd < dv[k - 1] || (dd == dv[k - 1] && ii < iv[k - 1]))) continue;
-            int pos = n < k ? n : k - 1;
-            while (pos > 0 && (dd < dv[pos - 1] || (dd == dv[pos - 1] && ii < iv[pos - 1]))) {
-                dv[pos] = dv[pos - 1];
-                iv[pos] = iv[pos - 1];
-                pos--;
-            }
-            dv[pos] = dd;
-            iv[pos] = ii;
-            if (n < k) n++;
+            if (ii != 0xFFFFFFFFu && dd == dd) topk_push(dv, iv, n, k, dd, ii);  // as k_topk_merge (exact.cu)
         }
     }
-    for (int s = 0; s < k; s++) {
-        out_idx[qi * k + s] = s < n ? iv[s] : 0xFFFFFFFFu;
-        out_dist[qi * k + s] = s < n ? dv[s] : kInf;
-    }
+    topk_store(dv, iv, n, k, 0, out_idx + qi * k, out_dist + qi * k);
 }
 
 static size_t exchange_stride(size_t nq, int k) { return (nq * (size_t)k * 12 + 255) / 256 * 256; }

@@ -15,7 +15,6 @@
 //                     list could have entered it given the scan's error bound.
 #include <algorithm>
 #include <cmath>
-#include <cstring>
 #include <numeric>
 
 #include <chrono>
@@ -66,22 +65,6 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned by
                  "l"(src), "r"(bytes), "r"(smem_u32(bar))
                  : "memory");
 }
-
-// order-preserving float -> u32 (so packed (dist, idx) keys compare as integers, negatives included)
-__host__ __device__ __forceinline__ uint32_t f2ord(float f) {
-    uint32_t b;
-#ifdef __CUDA_ARCH__
-    b = __float_as_uint(f);
-#else
-    memcpy(&b, &f, 4);
-#endif
-    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-__device__ __forceinline__ float ord2f(uint32_t o) {
-    const uint32_t b = (o & 0x80000000u) ? (o & 0x7FFFFFFFu) : ~o;
-    return __uint_as_float(b);
-}
-constexpr unsigned long long kEmptyKey = 0xFFFFFFFFFFFFFFFFull;
 
 // ---------------------------------------------------------------------------------------------------------------
 // layout builders
@@ -372,7 +355,7 @@ __global__ void k_dtw_merge(const unsigned long long* __restrict__ partial, uint
 #pragma unroll
     for (int s = 0; s < KP; s++) {
         cand_idx[(size_t)slot * KP + s] = best[s] == kEmptyKey ? 0xFFFFFFFFu : (uint32_t)best[s];
-        cand_adist[(size_t)slot * KP + s] = best[s] == kEmptyKey ? __int_as_float(0x7f800000) : ord2f((uint32_t)(best[s] >> 32));
+        cand_adist[(size_t)slot * KP + s] = best[s] == kEmptyKey ? __int_as_float(0x7f800000) : key_dist(best[s]);
     }
 }
 
@@ -637,7 +620,7 @@ static int run_stage(ss_dict* d, ss_queries* q, int k, DtwStage s, bool timed, u
 // Sequences of more than 32 frames have no cheap second filter (the fp32-DP tensor-core scan stops at 32 frames, the CUDA-core
 // scan of ONE long query is a single warp's serial walk: 16 ms at config 5): below 2e8 cells the exhaustive stage is the
 // fastest way to finish (f64, measured 9e10 cells / s: 2 ms); a dozen such queries first take the wide packed-half pass.
-// Cells the banded strip kernel (exact.cu warp_dtw_exact_long<true>) visits for a pair of la x lb frames (la, lb >= 1): per strip of
+// Cells the banded strip kernel (exact.cu warp_dtw_exact_long with BAND) visits for a pair of la x lb frames (la, lb >= 1): per strip of
 // 32 columns, the 32 x 32 step blocks from the one holding its first in-band row to the one in which lane 31 reaches its last.
 static uint64_t band_strip_cells(int la, int lb, uint32_t r) {
     const int nsteps = la + 31;

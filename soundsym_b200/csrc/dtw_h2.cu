@@ -643,7 +643,7 @@ __global__ void __launch_bounds__(kH2Threads, 1) k_dtw_scan_h2(const H2Params p)
                             const float v = hsel ? __high2float(res[b]) : __low2float(res[b]);
                             // D16 / (S (Lq + Ld)); an overflowed path sum stays +inf and is never inserted
                             const float dist = __fdividef(v * p.inv_s, (float)(Lm + (uint32_t)h2_len_of(sc, e)));
-                            const unsigned long long key = ((unsigned long long)tc_f2ord(dist) << 32) | (uint32_t)seg;
+                            const unsigned long long key = ((unsigned long long)f2ord(dist) << 32) | (uint32_t)seg;
                             if (key < worst && dist == dist) {
                                 const bool full = cnt == KP;
                                 list[(full ? wpos : cnt) * kH2DpThreads] = key;
@@ -846,7 +846,7 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
                         if (seg >= 0) {
                             const float v = hsel ? __high2float(res[b]) : __low2float(res[b]);
                             const float dist = __fdividef(v * p.inv_s, (float)(Lm + (uint32_t)h2_len_of(sc, e)));
-                            const unsigned long long key = ((unsigned long long)tc_f2ord(dist) << 32) | (uint32_t)seg;
+                            const unsigned long long key = ((unsigned long long)f2ord(dist) << 32) | (uint32_t)seg;
                             if (key < worst && dist == dist) {
                                 const bool full = cnt == KP;
                                 list[(full ? wpos : cnt) * kH2PDpThreads] = key;

@@ -13,8 +13,6 @@
 
 namespace ss {
 
-constexpr double kInf = __builtin_huge_val();
-
 // ---------------------------------------------------------------------------------------------------------------
 // norm(me) = fold(0, |memo, item| item*item + memo)   src/sound.rs:36-38 — one thread per segment, sequential
 // ---------------------------------------------------------------------------------------------------------------
@@ -899,12 +897,19 @@ struct RescoreBound {
 // as an anti-diagonal wavefront: at step t lane j computes cell (t - j, j) from its own previous value (up), its left
 // neighbour's (one 64-bit shuffle) and the one it received a step earlier (diag).
 // ---------------------------------------------------------------------------------------------------------------
+// the alignment's record of which of its three neighbours a cell's min chose, as 2 bits (0 diag, 1 up, 2 left; ties in that
+// order), compared against the very value fmin(fmin(up, left), diag) returned
+__device__ __forceinline__ uint64_t align_dir(double up, double left, double diag, double m) {
+    return diag == m ? 0ull : (up == m ? 1ull : 2ull);
+}
+
 // `sa` holds the query's frames (staged once per slot, coalesced); lane j keeps dictionary frame j in registers (its 13 loads
 // are issued back to back: one memory latency per pair). cst = the pair's local costs, [row][lane].
 // BAND: cells outside the band of radius `band` (>= 1) are +inf, one integer test per cell against the lane's row range.
-template <bool BAND>
+// DIRS (the alignment, k_dtw_align_warp): *dirs = the directions of lane `lane`'s column, 2 bits per row (align_dir).
+template <bool BAND, bool DIRS = false>
 __device__ __forceinline__ double warp_dtw_exact(const double* __restrict__ sa, int la, const double* __restrict__ b, int lb, int c, double* cst,
-                                                 int lane, uint32_t band) {
+                                                 int lane, uint32_t band, uint64_t* dirs = nullptr) {
     double br[SS_MAX_NCOEFFS];
 #pragma unroll
     for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = (k < c && lane < lb) ? b[(size_t)lane * c + k] : 0.0;
@@ -923,6 +928,7 @@ __device__ __forceinline__ double warp_dtw_exact(const double* __restrict__ sa, 
     }
     __syncwarp();
     double cur = kInf, recv_prev = kInf, result = kInf;
+    uint64_t w = 0;
     for (int step = 0; step < la + lb - 1; step++) {
         const double recv = __shfl_up_sync(0xffffffffu, cur, 1);  // left neighbour's last cell = D(i, j-1)
         const int i = step - lane;
@@ -934,12 +940,14 @@ __device__ __forceinline__ double warp_dtw_exact(const double* __restrict__ sa, 
             double m;
             if (i == 0 && lane == 0) m = 0.0;
             else m = fmin(fmin(up, left), diag);
+            if constexpr (DIRS) w |= align_dir(up, left, diag, m) << (2 * i);
             if (BAND && (i < blo || i > bhi)) cur = kInf;
             else cur = cst[i * 32 + lane] + m;
             if (i == la - 1 && lane == lb - 1) result = cur;
         }
         recv_prev = recv;
     }
+    if constexpr (DIRS) *dirs = w;
     result = __shfl_sync(0xffffffffu, result, lb > 0 ? lb - 1 : 0);
     return (la && lb) ? result / (double)(la + lb) : kInf;
 }
@@ -993,22 +1001,11 @@ k_dtw_refine_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__
         const double dd = __shfl_sync(0xffffffffu, my_exact, s);
         const uint32_t ii = __shfl_sync(0xffffffffu, my_idx, s);
         if (lane != 0 || ii == 0xFFFFFFFFu || !(dd < kInf)) continue;
-        int pos = n;
-        while (pos > 0 && (dd < dv[pos - 1] || (dd == dv[pos - 1] && ii < iv[pos - 1]))) {
-            dv[pos] = dv[pos - 1];
-            iv[pos] = iv[pos - 1];
-            pos--;
-        }
-        dv[pos] = dd;
-        iv[pos] = ii;
-        n++;
+        topk_push(dv, iv, n, kMaxKeep, dd, ii);
     }
     const float worst = __shfl_sync(0xffffffffu, my_adist, kp - 1);
     if (lane == 0) {
-        for (int s = 0; s < k; s++) {
-            out_idx[(size_t)qid * k + s] = s < n ? iv[s] + index_base : 0xFFFFFFFFu;
-            out_dist[(size_t)qid * k + s] = s < n ? dv[s] : kInf;
-        }
+        topk_store(dv, iv, n, k, index_base, out_idx + (size_t)qid * k, out_dist + (size_t)qid * k);
         bool uncertified = false;  // see k_dtw_finalize
         // (bound_mode 2: a list that is not full does NOT mean every pair is in it - overflowed pairs read +inf and are never
         // inserted - so the bound is evaluated anyway, at its cap)
@@ -1036,10 +1033,14 @@ k_dtw_refine_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__
 // step blocks run from the one holding row rlo to the one in which lane 31 reaches row rhi, and only rows <= rhi get costs.
 // Cells outside the band inside those blocks are +inf by the per-cell test. Rows the strip never reaches are +inf for every
 // column of it: they go to the boundary row as +inf, for the next strip's lane 0.
+// DIRS (the alignment, k_dtw_align_long): per strip, lane j packs 32 rows of its column into a u64 and stores it to the
+// direction block `dir`, [strip][row / 32][lane], coalesced, once the whole warp has finished those rows. With BAND the words
+// of row blocks outside the strip's step range are not written, and no path cell reads them.
 // ---------------------------------------------------------------------------------------------------------------
-template <bool BAND>
+template <bool BAND, bool DIRS = false>
 __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__ a, int la, const double* __restrict__ b, int lb, int c,
-                                                      double* __restrict__ ring, double* bnd, int lane, uint32_t band) {
+                                                      double* __restrict__ ring, double* bnd, int lane, uint32_t band,
+                                                      uint64_t* __restrict__ dir = nullptr) {
     if (!la || !lb) return kInf;
     double result = kInf;
     const int nstrips = (lb + 31) >> 5;
@@ -1051,6 +1052,10 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
 #pragma unroll
         for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = (k < c && colv) ? b[(size_t)col * c + k] : 0.0;
         double cur = kInf, recv_prev = kInf, bl_prev = kInf;
+        // at step t0 + r lane j is on row t0 + r - j: row block t0 / 32 - 1 (wprev) or t0 / 32 (wcur)
+        uint64_t wprev = 0, wcur = 0;
+        const int nrb = (la + 31) >> 5;
+        uint64_t* sdir = dir + (size_t)s * nrb * 32 + lane;
         int blo = 0, bhi = 0, rhi = 0, t0b = 0, t0e = nsteps;
         if (BAND) {
             band_rows(min(col, lb - 1), la, lb, band, &blo, &bhi);
@@ -1109,6 +1114,11 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
                     double m;
                     if (first && i == 0 && lane == 0) m = 0.0;
                     else m = fmin(fmin(up, left), diag);
+                    if constexpr (DIRS) {
+                        const uint64_t bits = align_dir(up, left, diag, m) << (2 * (i & 31));
+                        if (i < t0) wprev |= bits;
+                        else wcur |= bits;
+                    }
                     if (BAND && (i < blo || i > bhi)) cur = kInf;
                     else cur = ring[(i & 63) * 32 + lane] + m;
                     if (last && i == la - 1 && col == lb - 1) result = cur;
@@ -1118,6 +1128,15 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
                 recv_prev = recv;
             }
             __syncwarp();
+            if constexpr (DIRS) {
+                if (t0 >= 32) sdir[(size_t)((t0 >> 5) - 1) * 32] = wprev;  // every lane is past that row block
+                wprev = wcur;
+                wcur = 0;
+            }
+        }
+        if constexpr (DIRS) {
+            const int rb_last = ((BAND ? t0 : nsteps) - 1) >> 5;
+            if (rb_last < nrb) sdir[(size_t)rb_last * 32] = wprev;
         }
         if (BAND && !last)  // lane 31 stopped at row min(t0, nsteps) - 32
             for (int r = max(0, min(t0, nsteps) - 31) + lane; r < la; r += 32) bnd[r] = kInf;
@@ -1177,6 +1196,56 @@ k_dtw_rescore_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict_
 // tensor-core scan was 1.5 of config 4's 39 ms, and a fixed ~0.5 ms of every shard's step at 8 GPUs).
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kSecondQueue = 192;  // entries a warp can queue for refinement; a query with more stays uncertified
+
+// The walk over slot `slot`'s slice lists by the calling warp: lists l0 + first, l0 + stride + first, .. (first = this lane's
+// first list). Every entry the bound cannot rule out against kth and the first pass did not refine (lane j's my_cand is
+// candidate j) goes to queue[atomicAdd(count, 1)]; entries past kSecondQueue are only counted.
+__device__ __forceinline__ void second_chance_walk(const unsigned long long* __restrict__ partial, uint32_t nlists, uint32_t nslots, uint32_t slot,
+                                                   int kp, const ScanBound& bound, double kth, uint32_t my_cand, uint32_t first, uint32_t stride,
+                                                   uint32_t* count, uint32_t* queue) {
+    for (uint32_t l0 = 0; l0 < nlists; l0 += stride) {
+        const uint32_t l = l0 + first;
+        for (int s = 0; s < kp; s++) {
+            unsigned long long key = kEmptyKey;
+            if (l < nlists) key = __ldg(partial + ((size_t)l * nslots + slot) * kp + s);
+            const bool want = key != kEmptyKey && !(bound.lower(key_dist(key)) > kth);
+            if (!__any_sync(0xffffffffu, want)) break;  // lists ascend: nothing further down any of these 32 lists qualifies
+            const uint32_t idx = (uint32_t)key;
+            bool seen = false;
+            for (int j = 0; j < kp; j++) seen |= __shfl_sync(0xffffffffu, my_cand, j) == idx;  // (all lanes take part)
+            if (want && !seen) {
+                const uint32_t pos = atomicAdd(count, 1u);
+                if (pos < (uint32_t)kSecondQueue) queue[pos] = idx;
+            }
+        }
+    }
+}
+
+// Certification against W = dist(thr): every pair outside the union of the slice lists has scan distance >= W (thr empty: no
+// CTA kept a full list, every finite pair is in the union, W = +inf). A certified query leaves the uncertified count.
+__device__ __forceinline__ void second_chance_certify(const ScanBound& bound, unsigned long long thr, double kth, uint32_t qid,
+                                                      uint8_t* __restrict__ uncert_flag, unsigned long long* __restrict__ counters) {
+    const float w = thr != kEmptyKey ? key_dist(thr) : __int_as_float(0x7f800000);
+    if (bound.lower(w) > kth) {
+        uncert_flag[qid] = 0;
+        atomicAdd(&counters[0], ~0ull);  // -1
+        atomicAdd(&counters[2], 1ull);
+    }
+}
+
+// the query's current top-k row (indices back to local ones)
+__device__ __forceinline__ void topk_load(const uint32_t* __restrict__ row_idx, const double* __restrict__ row_dist, int k, uint32_t index_base,
+                                          double* dv, uint32_t* iv, int& n) {
+    n = 0;
+    for (int s = 0; s < k; s++) {
+        const uint32_t ii = row_idx[s];
+        if (ii == 0xFFFFFFFFu) break;
+        iv[n] = ii - index_base;
+        dv[n] = row_dist[s];
+        n++;
+    }
+}
+
 template <bool BAND>
 __global__ void __launch_bounds__(64)
 k_dtw_second_chance(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ qmfcc,
@@ -1202,41 +1271,14 @@ k_dtw_second_chance(const double* __restrict__ dmfcc, const uint64_t* __restrict
     // current top-k (the k best of the merged list's kp candidates, exact)
     double dv[SS_MAX_TOPK];
     uint32_t iv[SS_MAX_TOPK];
-    int n = 0;
-    for (int s = 0; s < k; s++) {
-        const uint32_t ii = out_idx[(size_t)qid * k + s];
-        if (ii == 0xFFFFFFFFu) break;
-        iv[n] = ii - index_base;
-        dv[n] = out_dist[(size_t)qid * k + s];
-        n++;
-    }
-    double kth = n >= k ? dv[k - 1] : kInf;
+    int n;
+    topk_load(out_idx + (size_t)qid * k, out_dist + (size_t)qid * k, k, index_base, dv, iv, n);
+    const double kth = n >= k ? dv[k - 1] : kInf;
     const uint32_t my_cand = lane < kp ? cand_idx[(size_t)slot * kp + lane] : 0xFFFFFFFFu;  // already refined
     if (lane == 0) scount[warp] = 0;
     for (int e = lane; e < la * c; e += 32) squery[warp][e] = a[e];
     __syncwarp();
-    // ---- walk the slice lists: queue every entry the bound cannot rule out and the first pass did not refine ----------------
-    for (uint32_t l = lane; l < ((nlists + 31) & ~31u); l += 32) {
-        for (int s = 0; s < kp; s++) {
-            unsigned long long key = 0xFFFFFFFFFFFFFFFFull;
-            if (l < nlists) key = __ldg(partial + ((size_t)l * nslots + slot) * kp + s);
-            bool want = false;
-            if (key != 0xFFFFFFFFFFFFFFFFull) {
-                const uint32_t o = (uint32_t)(key >> 32);
-                const float dist = __uint_as_float((o & 0x80000000u) ? (o & 0x7FFFFFFFu) : ~o);
-                want = !(bound.lower(dist) > kth);
-            }
-            if (!__any_sync(0xffffffffu, want)) break;  // lists ascend: nothing further down any of these 32 lists qualifies
-            const uint32_t idx = (uint32_t)key;
-            bool seen = false;
-            for (int j = 0; j < kp; j++) seen |= __shfl_sync(0xffffffffu, my_cand, j) == idx;  // (all lanes take part)
-            want = want && !seen;
-            if (want) {
-                const uint32_t pos = atomicAdd(&scount[warp], 1u);
-                if (pos < (uint32_t)kSecondQueue) squeue[warp][pos] = idx;
-            }
-        }
-    }
+    second_chance_walk(partial, nlists, nslots, slot, kp, bound, kth, my_cand, lane, 32, &scount[warp], squeue[warp]);
     __syncwarp();
     const uint32_t nqueued = scount[warp];
     if (nqueued > (uint32_t)kSecondQueue) return;  // stays uncertified: the host re-runs it
@@ -1245,36 +1287,11 @@ k_dtw_second_chance(const double* __restrict__ dmfcc, const uint64_t* __restrict
         const uint32_t idx = squeue[warp][e];
         const double ex = warp_dtw_exact<BAND>(squery[warp], la, dmfcc + doff[idx] * c, (int)(doff[idx + 1] - doff[idx]), c, scost[warp], lane, band);
         if (!(ex < kInf)) continue;
-        if (n == k && !(ex < dv[k - 1] || (ex == dv[k - 1] && idx < iv[k - 1]))) continue;
-        int pos = n < k ? n : k - 1;
-        while (pos > 0 && (ex < dv[pos - 1] || (ex == dv[pos - 1] && idx < iv[pos - 1]))) {
-            dv[pos] = dv[pos - 1];
-            iv[pos] = iv[pos - 1];
-            pos--;
-        }
-        dv[pos] = ex;
-        iv[pos] = idx;
-        if (n < k) n++;
+        topk_push(dv, iv, n, k, ex, idx);
     }
-    kth = n >= k ? dv[k - 1] : kInf;
-    // ---- certify against W: every pair outside the union of the slice lists has scan distance >= W -------------------------
-    const unsigned long long t = thr[slot];
-    float w = __int_as_float(0x7f800000);  // no CTA kept a full list: every (finite) pair is in the union
-    if (t != 0xFFFFFFFFFFFFFFFFull) {
-        const uint32_t o = (uint32_t)(t >> 32);
-        w = __uint_as_float((o & 0x80000000u) ? (o & 0x7FFFFFFFu) : ~o);
-    }
-    const bool certified = bound.lower(w) > kth;
     if (lane == 0) {
-        for (int s = 0; s < k; s++) {
-            out_idx[(size_t)qid * k + s] = s < n ? iv[s] + index_base : 0xFFFFFFFFu;
-            out_dist[(size_t)qid * k + s] = s < n ? dv[s] : kInf;
-        }
-        if (certified) {
-            uncert_flag[qid] = 0;
-            atomicAdd(&counters[0], ~0ull);  // -1
-            atomicAdd(&counters[2], 1ull);
-        }
+        topk_store(dv, iv, n, k, index_base, out_idx + (size_t)qid * k, out_dist + (size_t)qid * k);
+        second_chance_certify(bound, thr[slot], n >= k ? dv[k - 1] : kInf, qid, uncert_flag, counters);
     }
 }
 
@@ -1313,32 +1330,10 @@ k_dtw_second_chance_long(const double* __restrict__ dmfcc, const uint64_t* __res
     const double* a = qmfcc + qoff[qid] * c;
     const int la = (int)(qoff[qid + 1] - qoff[qid]);
     const ScanBound bound = make_scan_bound(na, nb, eps, bound_mode, la, inv_s, ld_max);
-    double kth = out_idx[(size_t)qid * k + k - 1] != 0xFFFFFFFFu ? out_dist[(size_t)qid * k + k - 1] : kInf;
+    const double kth = out_idx[(size_t)qid * k + k - 1] != 0xFFFFFFFFu ? out_dist[(size_t)qid * k + k - 1] : kInf;
     const uint32_t my_cand = lane < kp ? cand_idx[(size_t)slot * kp + lane] : 0xFFFFFFFFu;  // already refined
-    // ---- walk the slice lists (32 lists per warp and round) ------------------------------------------------------------------
-    const uint32_t lround = kSecondWarps * 32;
-    for (uint32_t l0 = 0; l0 < nlists; l0 += lround) {
-        const uint32_t l = l0 + warp * 32 + lane;
-        for (int s = 0; s < kp; s++) {
-            unsigned long long key = 0xFFFFFFFFFFFFFFFFull;
-            if (l < nlists) key = __ldg(partial + ((size_t)l * nslots + slot) * kp + s);
-            bool want = false;
-            if (key != 0xFFFFFFFFFFFFFFFFull) {
-                const uint32_t o = (uint32_t)(key >> 32);
-                const float dist = __uint_as_float((o & 0x80000000u) ? (o & 0x7FFFFFFFu) : ~o);
-                want = !(bound.lower(dist) > kth);
-            }
-            if (!__any_sync(0xffffffffu, want)) break;  // lists ascend
-            const uint32_t idx = (uint32_t)key;
-            bool seen = false;
-            for (int j = 0; j < kp; j++) seen |= __shfl_sync(0xffffffffu, my_cand, j) == idx;
-            want = want && !seen;
-            if (want) {
-                const uint32_t pos = atomicAdd(&scount, 1u);
-                if (pos < (uint32_t)kSecondQueue) squeue[pos] = idx;
-            }
-        }
-    }
+    // 32 lists per warp and round
+    second_chance_walk(partial, nlists, nslots, slot, kp, bound, kth, my_cand, warp * 32 + lane, kSecondWarps * 32, &scount, squeue);
     __syncthreads();
     const uint32_t nqueued = scount;
     if (nqueued > (uint32_t)kSecondQueue) return;  // stays uncertified: the host re-runs it
@@ -1352,45 +1347,15 @@ k_dtw_second_chance_long(const double* __restrict__ dmfcc, const uint64_t* __res
     if (threadIdx.x != 0) return;
     double dv[SS_MAX_TOPK];
     uint32_t iv[SS_MAX_TOPK];
-    int n = 0;
-    for (int s = 0; s < k; s++) {
-        const uint32_t ii = out_idx[(size_t)qid * k + s];
-        if (ii == 0xFFFFFFFFu) break;
-        iv[n] = ii - index_base;
-        dv[n] = out_dist[(size_t)qid * k + s];
-        n++;
-    }
+    int n;
+    topk_load(out_idx + (size_t)qid * k, out_dist + (size_t)qid * k, k, index_base, dv, iv, n);
     for (uint32_t e = 0; e < nqueued; e++) {
-        const uint32_t idx = squeue[e];
         const double ex = sexact[e];
         if (!(ex < kInf)) continue;
-        if (n == k && !(ex < dv[k - 1] || (ex == dv[k - 1] && idx < iv[k - 1]))) continue;
-        int pos = n < k ? n : k - 1;
-        while (pos > 0 && (ex < dv[pos - 1] || (ex == dv[pos - 1] && idx < iv[pos - 1]))) {
-            dv[pos] = dv[pos - 1];
-            iv[pos] = iv[pos - 1];
-            pos--;
-        }
-        dv[pos] = ex;
-        iv[pos] = idx;
-        if (n < k) n++;
+        topk_push(dv, iv, n, k, ex, squeue[e]);
     }
-    kth = n >= k ? dv[k - 1] : kInf;
-    const unsigned long long t = thr[slot];
-    float w = __int_as_float(0x7f800000);
-    if (t != 0xFFFFFFFFFFFFFFFFull) {
-        const uint32_t o = (uint32_t)(t >> 32);
-        w = __uint_as_float((o & 0x80000000u) ? (o & 0x7FFFFFFFu) : ~o);
-    }
-    for (int s = 0; s < k; s++) {
-        out_idx[(size_t)qid * k + s] = s < n ? iv[s] + index_base : 0xFFFFFFFFu;
-        out_dist[(size_t)qid * k + s] = s < n ? dv[s] : kInf;
-    }
-    if (bound.lower(w) > kth) {
-        uncert_flag[qid] = 0;
-        atomicAdd(&counters[0], ~0ull);  // -1
-        atomicAdd(&counters[2], 1ull);
-    }
+    topk_store(dv, iv, n, k, index_base, out_idx + (size_t)qid * k, out_dist + (size_t)qid * k);
+    second_chance_certify(bound, thr[slot], n >= k ? dv[k - 1] : kInf, qid, uncert_flag, counters);
 }
 
 int dtw_second_chance(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, const unsigned long long* d_partial,
@@ -1436,20 +1401,9 @@ __global__ void k_dtw_finalize(const uint32_t* __restrict__ cand_idx, const floa
         const double dd = exact[(size_t)slot * kp + s];
         const uint32_t ii = cand_idx[(size_t)slot * kp + s];
         if (ii == 0xFFFFFFFFu || !(dd < kInf)) continue;
-        int pos = n;
-        while (pos > 0 && (dd < dv[pos - 1] || (dd == dv[pos - 1] && ii < iv[pos - 1]))) {
-            dv[pos] = dv[pos - 1];
-            iv[pos] = iv[pos - 1];
-            pos--;
-        }
-        dv[pos] = dd;
-        iv[pos] = ii;
-        n++;
+        topk_push(dv, iv, n, kMaxKeep, dd, ii);
     }
-    for (int s = 0; s < k; s++) {
-        out_idx[(size_t)qid * k + s] = s < n ? iv[s] + index_base : 0xFFFFFFFFu;
-        out_dist[(size_t)qid * k + s] = s < n ? dv[s] : kInf;
-    }
+    topk_store(dv, iv, n, k, index_base, out_idx + (size_t)qid * k, out_dist + (size_t)qid * k);
     // certification: every pair X outside the candidate list has scan distance >= the list's worst entry w, and
     //   bound_mode 0 (fp32 scan):  |scan - exact| <= E = eps (max|a|^2 + max|b|^2)            => exact(X) >= w - E
     //   bound_mode 1 (fp16 scan):  the scan is the DTW of the fp16-ROUNDED frames (products of fp16 values are exact in
@@ -1548,35 +1502,22 @@ k_dtw_select_exact(const double* __restrict__ exact, uint32_t nseg, int k, const
     double dv[SS_MAX_TOPK];
     uint32_t iv[SS_MAX_TOPK];
     int n = 0;
-    auto push = [&](double dd, uint32_t ii) {
-        if (!(dd < kInf)) return;
-        if (n == k && !(dd < dv[k - 1] || (dd == dv[k - 1] && ii < iv[k - 1]))) return;
-        int pos = n < k ? n : k - 1;
-        while (pos > 0 && (dd < dv[pos - 1] || (dd == dv[pos - 1] && ii < iv[pos - 1]))) {
-            dv[pos] = dv[pos - 1];
-            iv[pos] = iv[pos - 1];
-            pos--;
-        }
-        dv[pos] = dd;
-        iv[pos] = ii;
-        if (n < k) n++;
-    };
-    for (uint32_t s = t; s < nseg; s += 256) push(exact[(size_t)u * nseg + s], s);
-    for (int s = 0; s < k; s++) {
-        sd[t * SS_MAX_TOPK + s] = s < n ? dv[s] : kInf;
-        si[t * SS_MAX_TOPK + s] = s < n ? iv[s] : 0xFFFFFFFFu;
+    for (uint32_t s = t; s < nseg; s += 256) {
+        const double dd = exact[(size_t)u * nseg + s];
+        if (dd < kInf) topk_push(dv, iv, n, k, dd, s);
     }
+    topk_store(dv, iv, n, k, 0, si + t * SS_MAX_TOPK, sd + t * SS_MAX_TOPK);
     __syncthreads();
     if (t == 0) {
         n = 0;
         for (int w = 0; w < 256; w++)
-            for (int s = 0; s < k; s++)
-                if (si[w * SS_MAX_TOPK + s] != 0xFFFFFFFFu) push(sd[w * SS_MAX_TOPK + s], si[w * SS_MAX_TOPK + s]);
+            for (int s = 0; s < k; s++) {
+                const double dd = sd[w * SS_MAX_TOPK + s];
+                const uint32_t ii = si[w * SS_MAX_TOPK + s];
+                if (ii != 0xFFFFFFFFu && dd < kInf) topk_push(dv, iv, n, k, dd, ii);
+            }
         const uint32_t qid = qids[u];
-        for (int s = 0; s < k; s++) {
-            out_idx[(size_t)qid * k + s] = s < n ? iv[s] + index_base : 0xFFFFFFFFu;
-            out_dist[(size_t)qid * k + s] = s < n ? dv[s] : kInf;
-        }
+        topk_store(dv, iv, n, k, index_base, out_idx + (size_t)qid * k, out_dist + (size_t)qid * k);
     }
 }
 
@@ -1623,22 +1564,9 @@ __global__ void k_topk_merge(const uint32_t* __restrict__ idx, const double* __r
         for (int s = 0; s < k; s++) {
             const double dd = dist[((size_t)l * nq + qi) * k + s];
             const uint32_t ii = idx[((size_t)l * nq + qi) * k + s];
-            if (ii == 0xFFFFFFFFu || dd != dd) continue;
-            if (n == k && !(dd < dv[k - 1] || (dd == dv[k - 1] && ii < iv[k - 1]))) continue;
-            int pos = n < k ? n : k - 1;
-            while (pos > 0 && (dd < dv[pos - 1] || (dd == dv[pos - 1] && ii < iv[pos - 1]))) {
-                dv[pos] = dv[pos - 1];
-                iv[pos] = iv[pos - 1];
-                pos--;
-            }
-            dv[pos] = dd;
-            iv[pos] = ii;
-            if (n < k) n++;
+            if (ii != 0xFFFFFFFFu && dd == dd) topk_push(dv, iv, n, k, dd, ii);  // +inf entries that carry an index stay
         }
-    for (int s = 0; s < k; s++) {
-        out_idx[qi * k + s] = s < n ? iv[s] : 0xFFFFFFFFu;
-        out_dist[qi * k + s] = s < n ? dv[s] : kInf;
-    }
+    topk_store(dv, iv, n, k, 0, out_idx + qi * k, out_dist + qi * k);
 }
 
 int topk_merge_dev(ss_ctx* ctx, const uint32_t* d_idx, const double* d_dist, int nlists, size_t nq, int k, uint32_t* d_out_idx,
@@ -1652,14 +1580,13 @@ int topk_merge_dev(ss_ctx* ctx, const uint32_t* d_idx, const double* d_dist, int
 
 // ---------------------------------------------------------------------------------------------------------------
 // DTW alignment (ss_dict_align, spec in DESIGN.md §3.1e): the warping path of query p against dictionary segment seg_idx[p].
-// The recurrences below are warp_dtw_exact / warp_dtw_exact_long with one addition: every cell also records which of its
-// three neighbours the min chose, as 2 bits (0 diag, 1 up, 2 left; ties in that order), compared against the very value
-// fmin(fmin(up, left), diag) returned. D's bits are the refine's, so the path is the oracle's path cell for cell.
+// The recurrences are the refine's, warp_dtw_exact / warp_dtw_exact_long, instantiated with DIRS: every cell also records
+// which of its three neighbours the min chose (align_dir). D's bits are the refine's, so the path is the oracle's path cell
+// for cell.
 //   <= 32 x <= 32 (k_dtw_align_warp): lane j owns column j, whose 32 rows of directions fit in one u64 register; the
 //     backtrack is <= 63 steps of one shuffle of the current column's word.
-//   longer (k_dtw_align_long, waves of pairs): per strip, lane j packs 32 rows of its column into a u64 and stores it to the
-//     pair's direction block [strip][row / 32][lane], coalesced, once the whole warp has finished those rows. The backtrack
-//     loads one 32 x 32 tile (one coalesced u64 per lane) whenever the path enters it, then shuffles within it.
+//   longer (k_dtw_align_long, waves of pairs): the directions go to the pair's direction block [strip][row / 32][lane]. The
+//     backtrack loads one 32 x 32 tile (one coalesced u64 per lane) whenever the path enters it, then shuffles within it.
 // Paths are found from the end: cell s from the end goes to stage[last - s] of the pair's staging slot (last = its end),
 // so a path lands in forward order without knowing its length first. A scan of the lengths then gives the offsets and
 // k_dtw_align_compact packs the paths. Nothing is read back to the host.
@@ -1697,55 +1624,6 @@ __device__ __forceinline__ bool align_pair(const AlignArgs& A, uint32_t p, int l
     return false;
 }
 
-__device__ __forceinline__ uint64_t align_dir(double up, double left, double diag, double m) {
-    return diag == m ? 0ull : (up == m ? 1ull : 2ull);
-}
-
-// warp_dtw_exact (same loads, same operations in the same order) + the directions of lane `lane`'s column in *dirs
-template <bool BAND>
-__device__ __forceinline__ double warp_dtw_align(const double* __restrict__ sa, int la, const double* __restrict__ b, int lb, int c, double* cst,
-                                                 int lane, uint64_t* dirs, uint32_t band) {
-    double br[SS_MAX_NCOEFFS];
-#pragma unroll
-    for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = (k < c && lane < lb) ? b[(size_t)lane * c + k] : 0.0;
-    int blo = 0, bhi = 0;
-    if (BAND) band_rows(min(lane, lb - 1), la, lb, band, &blo, &bhi);
-    for (int i = 0; i < la; i++) {
-        double cost = 0.0;
-#pragma unroll
-        for (int k = 0; k < SS_MAX_NCOEFFS; k++)
-            if (k < c) {
-                const double dlt = sa[i * c + k] - br[k];
-                cost = cost + dlt * dlt;
-            }
-        cst[i * 32 + lane] = cost;
-    }
-    __syncwarp();
-    double cur = kInf, recv_prev = kInf, result = kInf;
-    uint64_t w = 0;
-    for (int step = 0; step < la + lb - 1; step++) {
-        const double recv = __shfl_up_sync(0xffffffffu, cur, 1);
-        const int i = step - lane;
-        const bool active = lane < lb && i >= 0 && i < la;
-        if (active) {
-            const double up = cur;
-            const double left = lane ? recv : kInf;
-            const double diag = lane ? recv_prev : kInf;
-            double m;
-            if (i == 0 && lane == 0) m = 0.0;
-            else m = fmin(fmin(up, left), diag);
-            w |= align_dir(up, left, diag, m) << (2 * i);
-            if (BAND && (i < blo || i > bhi)) cur = kInf;
-            else cur = cst[i * 32 + lane] + m;
-            if (i == la - 1 && lane == lb - 1) result = cur;
-        }
-        recv_prev = recv;
-    }
-    *dirs = w;
-    result = __shfl_sync(0xffffffffu, result, lb - 1);
-    return result / (double)(la + lb);
-}
-
 // one warp per pair, both sides <= 32 frames (the other pairs are k_dtw_align_long's)
 template <bool BAND>
 __global__ void __launch_bounds__(128) k_dtw_align_warp(AlignArgs A, uint32_t band) {
@@ -1762,7 +1640,7 @@ __global__ void __launch_bounds__(128) k_dtw_align_warp(AlignArgs A, uint32_t ba
     for (int e = lane; e < la * c; e += 32) squery[warp][e] = a[e];
     __syncwarp();
     uint64_t dirs;
-    const double dist = warp_dtw_align<BAND>(squery[warp], la, A.dmfcc + A.doff[s] * c, lb, c, scost[warp], lane, &dirs, band);
+    const double dist = warp_dtw_exact<BAND, true>(squery[warp], la, A.dmfcc + A.doff[s] * c, lb, c, scost[warp], lane, band, &dirs);
     if (!(dist < kInf)) {  // NaN or inf: no path
         if (lane == 0) A.len[p] = 0, A.out_dist[p] = kInf;
         return;
@@ -1785,105 +1663,6 @@ __global__ void __launch_bounds__(128) k_dtw_align_warp(AlignArgs A, uint32_t ba
     if (lane == 0) A.len[p] = (uint64_t)n, A.out_dist[p] = dist;
 }
 
-// warp_dtw_exact_long (same loads, same operations in the same order) + the direction block `dir`, [strip][row / 32][lane].
-// BAND: the same strip range; the words of row blocks outside it are not written, and no path cell reads them.
-template <bool BAND>
-__device__ __forceinline__ double warp_dtw_align_long(const double* __restrict__ a, int la, const double* __restrict__ b, int lb, int c,
-                                                      double* __restrict__ ring, double* bnd, uint64_t* __restrict__ dir, int lane, uint32_t band) {
-    double result = kInf;
-    const int nstrips = (lb + 31) >> 5, nrb = (la + 31) >> 5;
-    const int nsteps = la + 31;
-    for (int s = 0; s < nstrips; s++) {
-        const int col = 32 * s + lane;
-        const bool colv = col < lb, first = s == 0, last = s == nstrips - 1;
-        double br[SS_MAX_NCOEFFS];
-#pragma unroll
-        for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = (k < c && colv) ? b[(size_t)col * c + k] : 0.0;
-        double cur = kInf, recv_prev = kInf, bl_prev = kInf;
-        // at step t0 + r lane j is on row t0 + r - j: row block t0 / 32 - 1 (wprev) or t0 / 32 (wcur)
-        uint64_t wprev = 0, wcur = 0;
-        uint64_t* sdir = dir + (size_t)s * nrb * 32 + lane;
-        int blo = 0, bhi = 0, rhi = 0, t0b = 0, t0e = nsteps;
-        if (BAND) {
-            band_rows(min(col, lb - 1), la, lb, band, &blo, &bhi);
-            rhi = __shfl_sync(0xffffffffu, bhi, 31);
-            t0b = __shfl_sync(0xffffffffu, blo, 0) & ~31;
-            t0e = min(nsteps, rhi + 32);
-        }
-        __syncwarp();
-        if (BAND && lane == 0 && !first && t0b > 0) bl_prev = bnd[t0b - 1];
-        int t0 = t0b;
-        for (; t0 < t0e; t0 += 32) {
-            const int rows = min(32, (BAND ? rhi + 1 : la) - t0);
-            int r = 0;
-            for (; r + 4 <= rows; r += 4) {
-                const double* ar = a + (size_t)(t0 + r) * c;
-                double c0 = 0.0, c1 = 0.0, c2 = 0.0, c3 = 0.0;
-#pragma unroll
-                for (int k = 0; k < SS_MAX_NCOEFFS; k++)
-                    if (k < c) {
-                        const double d0 = ar[k] - br[k], d1 = ar[c + k] - br[k], d2 = ar[2 * c + k] - br[k], d3 = ar[3 * c + k] - br[k];
-                        c0 = c0 + d0 * d0;
-                        c1 = c1 + d1 * d1;
-                        c2 = c2 + d2 * d2;
-                        c3 = c3 + d3 * d3;
-                    }
-                double* dst = ring + ((t0 + r) & 63) * 32 + lane;
-                dst[0] = c0, dst[32] = c1, dst[64] = c2, dst[96] = c3;
-            }
-            for (; r < rows; r++) {
-                const double* ar = a + (size_t)(t0 + r) * c;
-                double cost = 0.0;
-#pragma unroll
-                for (int k = 0; k < SS_MAX_NCOEFFS; k++)
-                    if (k < c) {
-                        const double dlt = ar[k] - br[k];
-                        cost = cost + dlt * dlt;
-                    }
-                ring[((t0 + r) & 63) * 32 + lane] = cost;
-            }
-            __syncwarp();
-            const int steps = min(32, nsteps - t0);
-            double left_in = (lane == 0 && !first && t0 < la) ? bnd[t0] : kInf;
-            for (int r = 0; r < steps; r++) {
-                const int t = t0 + r;
-                const double recv = __shfl_up_sync(0xffffffffu, cur, 1);
-                const double left_now = left_in;
-                if (r + 1 < steps) left_in = (lane == 0 && !first && t + 1 < la) ? bnd[t + 1] : kInf;
-                const int i = t - lane;
-                const bool active = colv && i >= 0 && i < la;
-                if (active) {
-                    const double up = cur;
-                    const double left = lane ? recv : left_now;
-                    const double diag = lane ? recv_prev : bl_prev;
-                    double m;
-                    if (first && i == 0 && lane == 0) m = 0.0;
-                    else m = fmin(fmin(up, left), diag);
-                    const uint64_t bits = align_dir(up, left, diag, m) << (2 * (i & 31));
-                    if (i < t0) wprev |= bits;
-                    else wcur |= bits;
-                    if (BAND && (i < blo || i > bhi)) cur = kInf;
-                    else cur = ring[(i & 63) * 32 + lane] + m;
-                    if (last && i == la - 1 && col == lb - 1) result = cur;
-                    if (!last && lane == 31) bnd[i] = cur;
-                }
-                bl_prev = left_now;
-                recv_prev = recv;
-            }
-            __syncwarp();
-            if (t0 >= 32) sdir[(size_t)((t0 >> 5) - 1) * 32] = wprev;  // every lane is past that row block
-            wprev = wcur;
-            wcur = 0;
-        }
-        const int rb_last = ((BAND ? t0 : nsteps) - 1) >> 5;
-        if (rb_last < nrb) sdir[(size_t)rb_last * 32] = wprev;
-        if (BAND && !last)
-            for (int r = max(0, min(t0, nsteps) - 31) + lane; r < la; r += 32) bnd[r] = kInf;
-    }
-    result = __shfl_sync(0xffffffffu, result, (lb - 1) & 31);
-    return result / (double)(la + lb);
-}
-
 // one warp per pair of the wave [p0, p0 + np) that has a side longer than 32 frames; the pair's direction block and
 // boundary row are its own (dir_stride u64 words, bnd_stride doubles)
 template <bool BAND>
@@ -1899,8 +1678,8 @@ __global__ void __launch_bounds__(64) k_dtw_align_long(AlignArgs A, uint32_t p0,
     if (!align_pair(A, p, -1, &la, &lb, &s) || (la <= 32 && lb <= 32)) return;  // (lane -1: k_dtw_align_warp wrote those)
     const int c = A.c;
     uint64_t* my_dir = dir + (size_t)t * dir_stride;
-    const double dist = warp_dtw_align_long<BAND>(A.qmfcc + A.qoff[p] * c, la, A.dmfcc + A.doff[s] * c, lb, c, ring[warp],
-                                                  bnd + (size_t)t * bnd_stride, my_dir, lane, band);
+    const double dist = warp_dtw_exact_long<BAND, true>(A.qmfcc + A.qoff[p] * c, la, A.dmfcc + A.doff[s] * c, lb, c, ring[warp],
+                                                        bnd + (size_t)t * bnd_stride, lane, band, my_dir);
     if (!(dist < kInf)) {
         if (lane == 0) A.len[p] = 0, A.out_dist[p] = kInf;
         return;

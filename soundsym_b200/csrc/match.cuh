@@ -1,8 +1,9 @@
-// match.cuh — HBM-resident dictionary / query-batch handles shared by the DTW (dtw.cu) and cosine-ref (cosine.cu) matchers.
+// match.cuh — HBM-resident dictionary / query-batch handles shared by the DTW (dtw.cu) and cosine-ref (exact.cu) matchers.
 #pragma once
 #include <cuda_fp16.h>
 
 #include <chrono>
+#include <cstring>
 #include <map>
 #include <memory>
 
@@ -32,6 +33,48 @@ struct StripDesc {  // 16 B, read as int4
 struct TileDesc {  // 16 B, read as int4
     uint32_t frame_begin, nframes, strip_begin, nstrips;
 };
+
+constexpr double kInf = __builtin_huge_val();
+
+// ---- candidate keys: (ord(dist) << 32 | idx), so that keys compare as integers by (distance, index) ------------------------
+constexpr unsigned long long kEmptyKey = 0xFFFFFFFFFFFFFFFFull;  // an empty place of a candidate list
+
+// order-preserving float -> u32 (negatives included) and back
+__host__ __device__ __forceinline__ uint32_t f2ord(float f) {
+    uint32_t b;
+#ifdef __CUDA_ARCH__
+    b = __float_as_uint(f);
+#else
+    memcpy(&b, &f, 4);
+#endif
+    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+}
+__device__ __forceinline__ float ord2f(uint32_t o) { return __uint_as_float((o & 0x80000000u) ? (o & 0x7FFFFFFFu) : ~o); }
+__device__ __forceinline__ float key_dist(unsigned long long key) { return ord2f((uint32_t)(key >> 32)); }
+
+// ---- (distance, index) top-k lists: dv / iv ascending, n places taken --------------------------------------------------------
+// Inserts (dd, ii) into a list of at most `cap` places; when the list is full, the entry it pushes out (or itself) is dropped.
+// What may not enter a list at all (no index, NaN, +inf) is each caller's rule.
+__device__ __forceinline__ void topk_push(double* dv, uint32_t* iv, int& n, int cap, double dd, uint32_t ii) {
+    if (n == cap && !(dd < dv[cap - 1] || (dd == dv[cap - 1] && ii < iv[cap - 1]))) return;
+    int pos = n < cap ? n : cap - 1;
+    while (pos > 0 && (dd < dv[pos - 1] || (dd == dv[pos - 1] && ii < iv[pos - 1]))) {
+        dv[pos] = dv[pos - 1];
+        iv[pos] = iv[pos - 1];
+        pos--;
+    }
+    dv[pos] = dd;
+    iv[pos] = ii;
+    if (n < cap) n++;
+}
+// the first k places as a result row, indices + index_base; the places past n are (0xFFFFFFFF, +inf)
+__device__ __forceinline__ void topk_store(const double* dv, const uint32_t* iv, int n, int k, uint32_t index_base, uint32_t* out_idx,
+                                           double* out_dist) {
+    for (int s = 0; s < k; s++) {
+        out_idx[s] = s < n ? iv[s] + index_base : 0xFFFFFFFFu;
+        out_dist[s] = s < n ? dv[s] : kInf;
+    }
+}
 
 }  // namespace ss
 
@@ -270,7 +313,7 @@ int queries_check(ss_ctx* ctx, const double* q_mfcc, const uint64_t* q_frame_off
 int queries_prepare(ss_queries* q, const uint64_t* q_frame_offsets, size_t nq);
 int queries_fill(ss_queries* q, const double* q_mfcc, const uint64_t* q_frame_offsets, size_t nq);
 int fill_result(ss_ctx* ctx, uint32_t* d_idx, double* d_dist, size_t n);  // (inf, 0xFFFFFFFF) rows (exact.cu)
-int cosine_dict_build(ss_dict* d);    // per-segment norms (cosine.cu)
+int cosine_dict_build(ss_dict* d);    // per-segment norms (exact.cu)
 int cosine_queries_build(ss_queries* q);
 int cosine_match_dev(ss_dict* d, ss_queries* q, const double* d_targets, uint32_t* d_out_idx, double* d_out_dist);
 // SoundSequence::from_distances for SS_COSINE_REF: nsteps + 1 launches on the ctx stream, no host synchronisation (exact.cu)

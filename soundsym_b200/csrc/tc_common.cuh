@@ -166,16 +166,6 @@ __device__ __forceinline__ float tc_min3(float a, float b, float c) {
     return d;
 }
 
-__host__ __device__ __forceinline__ uint32_t tc_f2ord(float f) {
-    uint32_t b;
-#ifdef __CUDA_ARCH__
-    b = __float_as_uint(f);
-#else
-    memcpy(&b, &f, 4);
-#endif
-    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-
 // per-thread candidate list kept in shared memory as packed (ord(dist) << 32 | idx) keys, ascending; only the worst kept
 // key lives in a register for the per-pair test, so the hot loop pays two registers for the list
 // (STRIDE = number of DP threads of the kernel: entry s of a thread's list sits at list[s * STRIDE])
@@ -217,7 +207,7 @@ __device__ __forceinline__ void tc_sort_list(unsigned long long* list, int n) {
 }
 template <int KP, int STRIDE = kTcDpThreads>
 __device__ __forceinline__ void tc_insert(unsigned long long* list, unsigned long long& worst, float dist, uint32_t idx) {
-    const unsigned long long key = ((unsigned long long)tc_f2ord(dist) << 32) | idx;
+    const unsigned long long key = ((unsigned long long)f2ord(dist) << 32) | idx;
     if (key < worst && dist == dist) tc_insert_key<KP, STRIDE>(list, worst, key);
 }
 
@@ -302,10 +292,9 @@ __global__ void __launch_bounds__(256) k_tc_merge(const unsigned long long* __re
     const uint32_t slot = blockIdx.x * 8 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (slot >= nslots) return;
-    const unsigned long long EMPTY = 0xFFFFFFFFFFFFFFFFull;
     unsigned long long best[KP];
 #pragma unroll
-    for (int s = 0; s < KP; s++) best[s] = EMPTY;
+    for (int s = 0; s < KP; s++) best[s] = kEmptyKey;
     for (uint32_t l = lane; l < nlists; l += 32) {
         const ulonglong2* src = reinterpret_cast<const ulonglong2*>(partial + ((size_t)l * nslots + slot) * KP);
         unsigned long long key[KP];
@@ -333,26 +322,25 @@ __global__ void __launch_bounds__(256) k_tc_merge(const unsigned long long* __re
             }
         }
     }
-    unsigned long long mine = EMPTY;
+    unsigned long long mine = kEmptyKey;
 #pragma unroll
     for (int r = 0; r < KP; r++) {
         const uint32_t hi = (uint32_t)(best[0] >> 32), lo = (uint32_t)best[0];
         const uint32_t mhi = __reduce_min_sync(0xffffffffu, hi);
         const uint32_t mlo = __reduce_min_sync(0xffffffffu, hi == mhi ? lo : 0xFFFFFFFFu);
         const unsigned long long m = ((unsigned long long)mhi << 32) | mlo;
-        if (best[0] == m && m != EMPTY) {  // keys are unique (a segment sits in exactly one slice): one lane pops
+        if (best[0] == m && m != kEmptyKey) {  // keys are unique (a segment sits in exactly one slice): one lane pops
 #pragma unroll
             for (int s = 0; s + 1 < KP; s++) best[s] = best[s + 1];
-            best[KP - 1] = EMPTY;
+            best[KP - 1] = kEmptyKey;
         }
         if (lane == r) mine = m;
     }
     if (lane < KP) {
-        const bool empty = mine == EMPTY;
+        const bool empty = mine == kEmptyKey;
         cand_idx[(size_t)slot * KP + lane] = empty ? 0xFFFFFFFFu : (uint32_t)mine;
-        const uint32_t o = (uint32_t)(mine >> 32);
-        const uint32_t bits = (o & 0x80000000u) ? (o & 0x7FFFFFFFu) : ~o;
-        cand_adist[(size_t)slot * KP + lane] = empty ? __int_as_float(0x7f800000) : __uint_as_float(bits);
+        const float dist = key_dist(mine);
+        cand_adist[(size_t)slot * KP + lane] = empty ? __int_as_float(0x7f800000) : dist;
     }
 }
 
