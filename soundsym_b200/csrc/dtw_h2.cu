@@ -94,6 +94,10 @@ struct H2Params {
     // L << 32 | tiles} - [grid][8] u64, written by thread 0
     unsigned long long* timeline;
 };
+// this CTA's 8 timeline words (p.timeline != nullptr)
+__device__ __forceinline__ unsigned long long* h2_timeline_of(const H2Params& p) {
+    return p.timeline + ((size_t)(p.slice_begin * p.ngroups) + blockIdx.x) * 8;
+}
 __device__ __forceinline__ unsigned long long h2_now() {
     unsigned long long t;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
@@ -345,8 +349,13 @@ __device__ __forceinline__ void h2_step2(Cur& cur, __half2 (&d)[NB][4 * NG], __h
 // One dictionary tile for one thread (= one query x one slot = 2 NB segments). ra / rb: position of column len - 1 inside the
 // last 4-column group, for the band's first (low halves) and second (high halves) segment. res[b] = D(Lm - 1, len - 1) of both.
 // Cur: TcCursor (two TMEM buffers, k_dtw_scan_h2 / _long) or H2PipeCursor (one buffer per pipeline, k_dtw_scan_h2_2p).
-template <int NB, int NG, class Cur>
-__device__ __forceinline__ void h2_tile(uint32_t L, uint32_t lmin, uint32_t Lm, const int4& sc, Cur& cur, __half2 (&res)[NB]) {
+// before_capture runs once, after the capture-free steps (k_dtw_scan_h2_2p loads the tile's segment ids there).
+struct H2NoHook {
+    __device__ __forceinline__ void operator()() const {}
+};
+template <int NB, int NG, class Cur, class Hook = H2NoHook>
+__device__ __forceinline__ void h2_tile(uint32_t L, uint32_t lmin, uint32_t Lm, const int4& sc, Cur& cur, __half2 (&res)[NB],
+                                        Hook before_capture = Hook()) {
     __half2 d[NB][4 * NG];
 #pragma unroll
     for (int b = 0; b < NB; b++) {
@@ -359,13 +368,38 @@ __device__ __forceinline__ void h2_tile(uint32_t L, uint32_t lmin, uint32_t Lm, 
     const uint32_t ncap = min((lmin - 1) >> 1, nfull);   // steps before any query of the group can end
     uint32_t st = 0;
     if constexpr (std::is_same<Cur, H2PipeCursor>::value) {
-        // steps [0, ncap): no query of the group ends; one buffer, so every step has the same addresses
+        // steps [0, ncap): no query of the group ends; one buffer, so every step has the same addresses. NB = 1 runs two steps
+        // per iteration (the first step, the only one with D(-1, -1) = 0, before the loop): with one step per iteration ptxas
+        // made the home registers of d[] the second chunk's TMEM-load destination and copied every new row value back, 22 - 36
+        // moves per 80 - 128 band instructions; two steps let the row state and the loads trade registers (1 - 10 moves per
+        // two steps, tools/sass_step_mix.py). NB = 2 spills its per-slice state to local memory when unrolled and keeps one.
+        if constexpr (NB == 1) {
+            if (st < ncap) {
+                __half2 c0l[NB][4];
+                h2_step2<NB, NG>(cur, d, dinit, c0l);
+                dinit = h2_inf();
+                st++;
+            }
 #pragma unroll 1
-        for (; st < ncap; st++) {
-            __half2 c0l[NB][4];
-            h2_step2<NB, NG>(cur, d, dinit, c0l);
-            dinit = h2_inf();
+            for (; st + 2 <= ncap; st += 2) {
+                __half2 c0l[NB][4];
+                h2_step2<NB, NG>(cur, d, h2_inf(), c0l);
+                h2_step2<NB, NG>(cur, d, h2_inf(), c0l);
+            }
+            if (st < ncap) {
+                __half2 c0l[NB][4];
+                h2_step2<NB, NG>(cur, d, h2_inf(), c0l);
+                st++;
+            }
+        } else {
+#pragma unroll 1
+            for (; st < ncap; st++) {
+                __half2 c0l[NB][4];
+                h2_step2<NB, NG>(cur, d, dinit, c0l);
+                dinit = h2_inf();
+            }
         }
+        before_capture();
     } else {
         // steps [0, ncap): no query of the group ends; two per iteration on buffers 0, 1 with loop-invariant addresses
         if (st < ncap && cur.buf) {
@@ -711,6 +745,9 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
     uint64_t* t_full = bars + 1 + 2 * kH2Pipes * kTcStages;  // 17
     uint64_t* t_empty = t_full + kH2Pipes;                   // = t_full + 16 bytes (H2PipeCursor::release)
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(t_empty + kH2Pipes);
+    // the CTA's query group and slice, read back by the list merge at the end: held in registers through the slice, they
+    // pushed the NB = 1 kernel's two-step loop into local memory
+    uint32_t* cta_gs = reinterpret_cast<uint32_t*>(t_empty + kH2Pipes + 1);
     unsigned long long* topk = reinterpret_cast<unsigned long long*>(bars + 32);  // [KP][512]
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -727,7 +764,7 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
     const uint32_t L = glen & 0xFFFFu, lmin = glen >> 16;
     const uint32_t t0 = p.slice_tile[slice], t1 = p.slice_tile[slice + 1];
     const uint32_t ntiles = t1 - t0;
-    unsigned long long* tl = p.timeline ? p.timeline + ((size_t)(p.slice_begin * p.ngroups) + blockIdx.x) * 8 : nullptr;
+    unsigned long long* tl = p.timeline ? h2_timeline_of(p) : nullptr;
     if (tl && threadIdx.x == 0) {
         unsigned smid;
         asm("mov.u32 %0, %%smid;" : "=r"(smid));
@@ -735,6 +772,7 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
     }
 
     if (threadIdx.x == 0) {
+        cta_gs[0] = g, cta_gs[1] = slice;
         mb_init(a_full, 1);
         for (int s = 0; s < 2 * kH2Pipes * kTcStages; s++) mb_init(&bars[1 + s], 1);
         for (int s = 0; s < kH2Pipes; s++) mb_init(&t_full[s], 1), mb_init(&t_empty[s], kH2DpWarps);
@@ -811,31 +849,35 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
         const uint32_t Lm = p.slot_len[g * kTcM + m];  // this lane's own query length
         H2PipeCursor cur = {0u, s32(t_full + pipe), tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(pipe * kTcBufCols + slot * kH2SlotCols)};
         const uint32_t ntp = ntiles > (uint32_t)pipe ? (ntiles - pipe + 1) >> 1 : 0u;
-        // the NEXT tile's descriptors are fetched while the current tile is processed
-        const int4* dp = p.desc + ((size_t)(t0 + pipe) * kH2Slots + slot) * kH2DescInt4;
-        int4 na = make_int4(0, 0, 0, 0), nb = na, nc = na;
-        if (ntp) na = __ldg(dp), nb = __ldg(dp + 1), nc = __ldg(dp + 2);
+        // the NEXT tile's lengths and column groups are fetched while the current tile is processed; a tile's segment ids are
+        // only read after its last step and are loaded after its capture-free steps, so that those steps hold no descriptor
+        // registers beyond the lengths. The position is a 32-bit index into p.desc (its base stays in the constant bank): with
+        // a 64-bit pointer held through the slice, the NB = 1 two-step loop spilled to local memory (tools/sass_step_mix.py)
+        uint32_t di = ((t0 + pipe) * kH2Slots + slot) * kH2DescInt4;
+        int4 nc = make_int4(0, 0, 0, 0);
+        if (ntp) nc = __ldg(p.desc + di + 2);
         for (uint32_t n = 0; n < ntp; n++) {
-            const int4 sa = na, sb = nb, sc = nc;
-            dp += kH2Pipes * kH2Slots * kH2DescInt4;
-            if (n + 1 < ntp) na = __ldg(dp), nb = __ldg(dp + 1), nc = __ldg(dp + 2);
+            const int4 sc = nc;
+            const uint32_t dcur = di;
+            di += kH2Pipes * kH2Slots * kH2DescInt4;
+            if (n + 1 < ntp) nc = __ldg(p.desc + di + 2);
             const int ng = sc.z;
             __half2 res[NB];
+            int4 sa, sb;
+            const auto load_segs = [&] { sa = __ldg(p.desc + dcur), sb = __ldg(p.desc + dcur + 1); };
             if constexpr (NB == 1) {
                 switch (ng) {
-                    case 5: h2_tile<1, 5>(L, lmin, Lm, sc, cur, res); break;
-                    case 6: h2_tile<1, 6>(L, lmin, Lm, sc, cur, res); break;
-                    case 7: h2_tile<1, 7>(L, lmin, Lm, sc, cur, res); break;
-                    default: h2_tile<1, 8>(L, lmin, Lm, sc, cur, res); break;
+                    case 5: h2_tile<1, 5>(L, lmin, Lm, sc, cur, res, load_segs); break;
+                    case 6: h2_tile<1, 6>(L, lmin, Lm, sc, cur, res, load_segs); break;
+                    case 7: h2_tile<1, 7>(L, lmin, Lm, sc, cur, res, load_segs); break;
+                    default: h2_tile<1, 8>(L, lmin, Lm, sc, cur, res, load_segs); break;
                 }
-            } else if constexpr (NB == 2) {
-                if (ng == 3) h2_tile<2, 3>(L, lmin, Lm, sc, cur, res);
-                else h2_tile<2, 4>(L, lmin, Lm, sc, cur, res);
             } else {
-                if (ng == 1) h2_tile<4, 1>(L, lmin, Lm, sc, cur, res);
-                else h2_tile<4, 2>(L, lmin, Lm, sc, cur, res);
+                static_assert(NB == 2, "k_dtw_scan_h2_2p runs the NB = 1 and NB = 2 tiles");
+                if (ng == 3) h2_tile<2, 3>(L, lmin, Lm, sc, cur, res, load_segs);
+                else h2_tile<2, 4>(L, lmin, Lm, sc, cur, res, load_segs);
             }
-            if (tl && threadIdx.x == 0 && n + 1 == (ntp + 1) / 2) tl[6] = h2_now();  // (measurement: half of pipeline 0's tiles)
+            if (p.timeline && threadIdx.x == 0 && n + 1 == (ntp + 1) / 2) h2_timeline_of(p)[6] = h2_now();  // (measurement: half of pipeline 0's tiles)
             if (Lm) {
 #pragma unroll
                 for (int b = 0; b < NB; b++) {
@@ -867,7 +909,10 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
         worst = worst < thr0 ? worst : thr0;
         // the four lists of query m (threads m + 128 s, s = slot + 2 pipeline) are merged by thread m
         asm volatile("bar.sync 1, %0;" ::"n"(kH2PDpThreads) : "memory");
-        if (tl && threadIdx.x == 0) tl[2] = h2_now(), tl[5] = clock64() - tl[5];  // SM cycles of the DP phase (-> the SM clock under load)
+        if (p.timeline && threadIdx.x == 0) {  // (the pointer is re-derived here: held through the slice it took two of the DP warps' registers)
+            unsigned long long* t = h2_timeline_of(p);
+            t[2] = h2_now(), t[5] = clock64() - t[5];  // SM cycles of the DP phase (-> the SM clock under load)
+        }
         if (threadIdx.x < kTcM) {
             for (int o = 1; o < kH2Pipes * kH2Slots; o++) {
                 const unsigned long long* other = list + o * kTcM;
@@ -879,8 +924,9 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
                 }
             }
             const unsigned long long kept_worst = list[(KP - 1) * kH2PDpThreads];
-            if (kept_worst != 0xFFFFFFFFFFFFFFFFull && kept_worst < thr0) atomicMin(p.thr + g * kTcM + m, kept_worst);
-            unsigned long long* out = p.partial + ((size_t)slice * p.ngroups * kTcM + (size_t)g * kTcM + m) * KP;
+            const uint32_t gm = cta_gs[0] * kTcM + m;
+            if (kept_worst != 0xFFFFFFFFFFFFFFFFull && kept_worst < thr0) atomicMin(p.thr + gm, kept_worst);
+            unsigned long long* out = p.partial + ((size_t)cta_gs[1] * p.ngroups * kTcM + gm) * KP;
 #pragma unroll
             for (int s = 0; s < KP; s++) out[s] = list[s * kH2PDpThreads];
         }
