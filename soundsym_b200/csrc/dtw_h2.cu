@@ -32,6 +32,14 @@
 // one CTA, two pipelines of 8 DP warps + 1 producer warp that each own one 2-row TMEM buffer and take every other tile of the
 // slice, so that one pipeline's warps issue while the other's wait for their MMAs or close a tile (640 threads, setmaxnreg:
 // DP 112 registers, each step's columns pulled in two chunks).
+//
+// Code: the band recurrence (tc_band / tc_band_row over __half2), the capture-free step driver on the double-buffered cursor
+// (tc_steps), TMEM allocation and the CTA's exit (tc_tmem_alloc / tc_cta_exit), the producer lane (tc_produce), the merge
+// and write of a query's slot lists (tc_merge_store) and the launch (tc_launch_scan, tc_smem_bytes) come from tc_common.cuh,
+// shared with dtw_tc.cu's fp32 scan. This file keeps the packed loads and picks, the single-buffer cursor of the two
+// pipelines (H2PipeCursor) and its step loop in h2_tile, the strip of a long segment (h2_tile_strip), the helpers only its
+// kernels share (h2_cta_slice: CTA order; h2_timeline_open; h2_push_tile: a tile's results into the unsorted list), the
+// streamed-A producer of k_dtw_scan_h2_long, and the host side.
 #include <algorithm>
 #include <atomic>
 #include <type_traits>
@@ -103,6 +111,27 @@ __device__ __forceinline__ unsigned long long h2_now() {
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
     return t;
 }
+// the timeline's opening stamps (thread 0): start, SM, tile kind NB, group, group length and tiles of the slice
+__device__ __forceinline__ void h2_timeline_open(unsigned long long* tl, int nb, uint32_t g, uint32_t L, uint32_t ntiles) {
+    unsigned smid;
+    asm("mov.u32 %0, %%smid;" : "=r"(smid));
+    tl[0] = h2_now(), tl[4] = smid | ((unsigned long long)nb << 16) | ((unsigned long long)g << 32), tl[7] = ((unsigned long long)L << 32) | ntiles;
+}
+// CTA order of k_dtw_scan_h2 / _2p: the FIRST slice of every group, then the other slices group by group (longest groups first
+// in both parts). The slices of a group otherwise start together and none of them ever sees a sibling's threshold: with an
+// empty threshold a thread's list takes 8 (1 + ln(n / 8)) sorted insertions over the n pairs of its slice, whatever n - per
+// unit of work 5 times more on a 1/8 shard (ncu: 2.8 x the shared-memory wavefronts, + 5.7 % instructions, + 8 % cycles
+// per step). With the first slice's threshold published before most of the others start, ~KP pairs per slice pass.
+// Measured: 4.90 -> 4.85 ms on a 1/8 shard, 36.08 -> 35.97 ms at config 4 (the insertions were a part of the loss, not all
+// of it: profiles/r2_h2_cycles_per_tile_eighth_vs_full.txt). Restricting the order to the first launch measured the same.
+__device__ __forceinline__ void h2_cta_slice(const H2Params& p, uint32_t& g, uint32_t& slice) {
+    if (blockIdx.x < p.ngroups) {
+        g = blockIdx.x, slice = p.slice_begin;
+    } else {
+        const uint32_t r = blockIdx.x - p.ngroups;
+        g = r / (p.nslices - 1), slice = p.slice_begin + 1 + r % (p.nslices - 1);
+    }
+}
 
 // ---- packed TMEM loads: N registers <- 2 N adjacent columns ---------------------------------------------------------------
 template <int N>
@@ -154,7 +183,6 @@ __device__ __forceinline__ void h2_ld_row(uint32_t taddr, __half2 (&v)[4 * NG]) 
     if constexpr ((N & 4) != 0) h2_ld<4>(taddr + 2 * done, v + done);
 }
 
-__device__ __forceinline__ __half2 h2_min3(__half2 a, __half2 b, __half2 c) { return __hmin2(__hmin2(a, b), c); }  // one VHMNMX
 __device__ __forceinline__ __half2 h2_inf() {
     const uint32_t bits = 0x7C007C00u;
     return *reinterpret_cast<const __half2*>(&bits);
@@ -189,86 +217,6 @@ __device__ __forceinline__ __half2 h2_pick4(const __half2* v, int r) {
     return *reinterpret_cast<const __half2*>(&o);
 }
 
-// TWO rows (i, i + 1) of one band (two interleaved segments), row state in place: per half2 cell VHMNMX + HADD2.
-// c0l receives row i's values of the last 4-column group (row i + 1's stay in d[4 NG - 4 ..]).
-template <int NG>
-__device__ __forceinline__ void h2_band(const __half2 (&tm0)[4 * NG], const __half2 (&tm1)[4 * NG], __half2 (&d)[4 * NG], __half2 dinit, __half2 (&c0l)[4]) {
-    __half2 left0 = h2_inf(), diag0 = dinit, left1 = h2_inf();
-#pragma unroll
-    for (int j = 0; j < 4 * NG; j++) {
-        const __half2 up0 = d[j];
-        const __half2 c0 = __hadd2(tm0[j], h2_min3(left0, up0, diag0));
-        const __half2 c1 = __hadd2(tm1[j], h2_min3(left1, c0, left0));  // up = D(i, j), diag = D(i, j-1)
-        diag0 = up0;
-        left0 = c0;
-        left1 = c1;
-        d[j] = c1;
-        if (j >= 4 * (NG - 1)) c0l[j - 4 * (NG - 1)] = c0;
-    }
-}
-// the same band for one 32-column STRIP of a longer segment: the carries start from the previous strip's last column
-// (l0 = D(i, -1), dg0 = D(i-1, -1), l1 = D(i+1, -1)) and the strip's own last column comes back in o0 / o1
-template <int NG>
-__device__ __forceinline__ void h2_band_io(const __half2 (&tm0)[4 * NG], const __half2 (&tm1)[4 * NG], __half2 (&d)[4 * NG], __half2 l0, __half2 dg0,
-                                           __half2 l1, __half2 (&c0l)[4], __half2& o0, __half2& o1) {
-    __half2 left0 = l0, diag0 = dg0, left1 = l1;
-#pragma unroll
-    for (int j = 0; j < 4 * NG; j++) {
-        const __half2 up0 = d[j];
-        const __half2 c0 = __hadd2(tm0[j], h2_min3(left0, up0, diag0));
-        const __half2 c1 = __hadd2(tm1[j], h2_min3(left1, c0, left0));
-        diag0 = up0;
-        left0 = c0;
-        left1 = c1;
-        d[j] = c1;
-        if (j >= 4 * (NG - 1)) c0l[j - 4 * (NG - 1)] = c0;
-    }
-    o0 = left0, o1 = left1;
-}
-template <int NG>
-__device__ __forceinline__ void h2_band_row_io(const __half2 (&tm)[4 * NG], __half2 (&d)[4 * NG], __half2 l0, __half2 dg0, __half2& o0) {
-    __half2 left = l0, diag = dg0;
-#pragma unroll
-    for (int j = 0; j < 4 * NG; j++) {
-        const __half2 up = d[j];
-        const __half2 cur = __hadd2(tm[j], h2_min3(left, up, diag));
-        diag = up;
-        left = cur;
-        d[j] = cur;
-    }
-    o0 = left;
-}
-template <int NG>
-__device__ __forceinline__ void h2_band_row(const __half2 (&tm)[4 * NG], __half2 (&d)[4 * NG], __half2 dinit) {
-    __half2 left = h2_inf(), diag = dinit;
-#pragma unroll
-    for (int j = 0; j < 4 * NG; j++) {
-        const __half2 up = d[j];
-        const __half2 cur = __hadd2(tm[j], h2_min3(left, up, diag));
-        diag = up;
-        left = cur;
-        d[j] = cur;
-    }
-}
-
-// columns [J0, J1) of h2_band, the carries (left0, diag0, left1) passed in and out: the same operations in the same order,
-// so a band split into column chunks gives the bits of the whole band (tm0 / tm1 hold columns J0 ..)
-template <int NG, int J0, int J1>
-__device__ __forceinline__ void h2_band_cols(const __half2* tm0, const __half2* tm1, __half2 (&d)[4 * NG], __half2& left0, __half2& diag0,
-                                             __half2& left1, __half2 (&c0l)[4]) {
-#pragma unroll
-    for (int j = J0; j < J1; j++) {
-        const __half2 up0 = d[j];
-        const __half2 c0 = __hadd2(tm0[j - J0], h2_min3(left0, up0, diag0));
-        const __half2 c1 = __hadd2(tm1[j - J0], h2_min3(left1, c0, left0));
-        diag0 = up0;
-        left0 = c0;
-        left1 = c1;
-        d[j] = c1;
-        if (j >= 4 * (NG - 1)) c0l[j - 4 * (NG - 1)] = c0;
-    }
-}
-
 // consumer side of one pipeline's single 2-row TMEM buffer (k_dtw_scan_h2_2p): its "empty" barrier sits 16 bytes above its
 // "full" barrier, as in TcCursor, but the buffer and the barriers never change - only the parity flips
 struct H2PipeCursor {
@@ -295,20 +243,20 @@ __device__ __forceinline__ void h2_step2(Cur& cur, __half2 (&d)[NB][4 * NG], __h
     const uint32_t taddr = cur.taddr;
     if constexpr (std::is_same<Cur, H2PipeCursor>::value && NB == 1) {
         static_assert(NG >= 5, "NB = 1 tiles have 5..8 column groups");
-        __half2 left0 = h2_inf(), diag0 = dinit, left1 = h2_inf();
+        TcCarry<__half2> c = {h2_inf(), dinit, h2_inf()};
         {
             __half2 a0[16], a1[16];
             h2_ld_row<4>(taddr, a0);
             h2_ld_row<4>(taddr + kTcN, a1);
             tc_wait_ld();
-            h2_band_cols<NG, 0, 16>(a0, a1, d[0], left0, diag0, left1, c0l[0]);
+            tc_band<NG, 0, 16>(a0, a1, d[0], c, c0l[0]);
         }
         __half2 b0[4 * (NG - 4)], b1[4 * (NG - 4)];
         h2_ld_row<NG - 4>(taddr + 32, b0);
         h2_ld_row<NG - 4>(taddr + kTcN + 32, b1);
         tc_wait_ld();
         cur.release();
-        h2_band_cols<NG, 16, 4 * NG>(b0, b1, d[0], left0, diag0, left1, c0l[0]);
+        tc_band<NG, 16, 4 * NG>(b0, b1, d[0], c, c0l[0]);
     } else if constexpr (std::is_same<Cur, H2PipeCursor>::value) {
         constexpr int H = NB / 2;
         {
@@ -320,7 +268,10 @@ __device__ __forceinline__ void h2_step2(Cur& cur, __half2 (&d)[NB][4 * NG], __h
             }
             tc_wait_ld();
 #pragma unroll
-            for (int b = 0; b < H; b++) h2_band<NG>(tm0[b], tm1[b], d[b], dinit, c0l[b]);
+            for (int b = 0; b < H; b++) {
+                TcCarry<__half2> c = {h2_inf(), dinit, h2_inf()};
+                tc_band<NG, 0, 4 * NG>(tm0[b], tm1[b], d[b], c, c0l[b]);
+            }
         }
         __half2 tm0[H][4 * NG], tm1[H][4 * NG];
 #pragma unroll
@@ -331,7 +282,10 @@ __device__ __forceinline__ void h2_step2(Cur& cur, __half2 (&d)[NB][4 * NG], __h
         tc_wait_ld();
         cur.release();
 #pragma unroll
-        for (int b = 0; b < H; b++) h2_band<NG>(tm0[b], tm1[b], d[H + b], dinit, c0l[H + b]);
+        for (int b = 0; b < H; b++) {
+            TcCarry<__half2> c = {h2_inf(), dinit, h2_inf()};
+            tc_band<NG, 0, 4 * NG>(tm0[b], tm1[b], d[H + b], c, c0l[H + b]);
+        }
     } else {
         __half2 tm0[NB][4 * NG], tm1[NB][4 * NG];
 #pragma unroll
@@ -342,7 +296,10 @@ __device__ __forceinline__ void h2_step2(Cur& cur, __half2 (&d)[NB][4 * NG], __h
         tc_wait_ld();
         cur.release();
 #pragma unroll
-        for (int b = 0; b < NB; b++) h2_band<NG>(tm0[b], tm1[b], d[b], dinit, c0l[b]);
+        for (int b = 0; b < NB; b++) {
+            TcCarry<__half2> c = {h2_inf(), dinit, h2_inf()};
+            tc_band<NG, 0, 4 * NG>(tm0[b], tm1[b], d[b], c, c0l[b]);
+        }
     }
 }
 
@@ -401,34 +358,10 @@ __device__ __forceinline__ void h2_tile(uint32_t L, uint32_t lmin, uint32_t Lm, 
         }
         before_capture();
     } else {
-        // steps [0, ncap): no query of the group ends; two per iteration on buffers 0, 1 with loop-invariant addresses
-        if (st < ncap && cur.buf) {
+        st = tc_steps(cur, ncap, dinit, h2_inf(), [&](TcCursor& c, __half2 di) {  // no query of the group ends in steps [0, ncap)
             __half2 c0l[NB][4];
-            h2_step2<NB, NG>(cur, d, dinit, c0l);
-            dinit = h2_inf();
-            st++;
-        }
-        if (st + 2 <= ncap) {
-            const uint32_t full0 = cur.full, taddr0 = cur.taddr;
-            uint32_t par = cur.par;
-#pragma unroll 1
-            for (; st + 2 <= ncap; st += 2) {
-                __half2 c0l[NB][4];
-                TcCursor c0 = {0u, par, full0, taddr0, cur.full_sum, cur.taddr_sum};
-                h2_step2<NB, NG>(c0, d, dinit, c0l);
-                TcCursor c1 = {1u, par, full0 + 8u, taddr0 + (uint32_t)kTcBufCols, cur.full_sum, cur.taddr_sum};
-                h2_step2<NB, NG>(c1, d, h2_inf(), c0l);
-                dinit = h2_inf();
-                par ^= 1u;
-            }
-            cur.par = par;
-        }
-        if (st < ncap) {
-            __half2 c0l[NB][4];
-            h2_step2<NB, NG>(cur, d, dinit, c0l);
-            dinit = h2_inf();
-            st++;
-        }
+            h2_step2<NB, NG>(c, d, di, c0l);
+        });
     }
 #pragma unroll 1
     for (; st < nfull; st++) {  // only the last step or two of a tile: some query of the group can end here
@@ -454,7 +387,7 @@ __device__ __forceinline__ void h2_tile(uint32_t L, uint32_t lmin, uint32_t Lm, 
         cur.release();
 #pragma unroll
         for (int b = 0; b < NB; b++) {
-            h2_band_row<NG>(tm0[b], d[b], dinit);
+            tc_band_row<NG>(tm0[b], d[b], h2_inf(), dinit);
             const int ra = (h2_len_of(sc, 2 * b) - 1) & 3, rb = (h2_len_of(sc, 2 * b + 1) - 1) & 3;
             const __half2 e = h2_combine(h2_pick4(&d[b][4 * (NG - 1)], ra), h2_pick4(&d[b][4 * (NG - 1)], rb));
             res[b] = (L == Lm) ? e : res[b];
@@ -482,16 +415,17 @@ __device__ __forceinline__ void h2_tile_strip(uint32_t L, uint32_t lmin, uint32_
         if (IN) b0 = bnd[(size_t)(2 * st) * kStride], b1 = bnd[(size_t)(2 * st + 1) * kStride];  // issued ahead of the TMEM wait
         cur.wait();
         const uint32_t taddr = cur.taddr;
-        __half2 tm0[4 * NG], tm1[4 * NG], c0l[4], o0, o1;
+        __half2 tm0[4 * NG], tm1[4 * NG], c0l[4];
         h2_ld_row<NG>(taddr, tm0);
         h2_ld_row<NG>(taddr + kTcN, tm1);
         tc_wait_ld();
         cur.release();
-        h2_band_io<NG>(tm0, tm1, d, b0, prev_b, b1, c0l, o0, o1);
+        TcCarry<__half2> c = {b0, prev_b, b1};  // the previous strip's last column: D(i, -1), D(i-1, -1), D(i+1, -1)
+        tc_band<NG, 0, 4 * NG>(tm0, tm1, d, c, c0l);
         prev_b = IN ? b1 : h2_inf();
-        if (OUT) {
-            bnd[(size_t)(2 * st) * kStride] = o0;
-            bnd[(size_t)(2 * st + 1) * kStride] = o1;
+        if (OUT) {  // this strip's last column, for the next strip
+            bnd[(size_t)(2 * st) * kStride] = c.left0;
+            bnd[(size_t)(2 * st + 1) * kStride] = c.left1;
         } else if (st >= ncap) {
             const bool end0 = 2 * st + 1 == Lm, end1 = 2 * st + 2 == Lm;
             const __half2 e0 = h2_combine(h2_pick4(c0l, ra), h2_pick4(c0l, rb));
@@ -503,16 +437,52 @@ __device__ __forceinline__ void h2_tile_strip(uint32_t L, uint32_t lmin, uint32_
         __half2 b0 = h2_inf();
         if (IN) b0 = bnd[(size_t)(L - 1) * kStride];
         cur.wait();
-        __half2 tm0[4 * NG], o0;
+        __half2 tm0[4 * NG];
         h2_ld_row<NG>(cur.taddr, tm0);
         tc_wait_ld();
         cur.release();
-        h2_band_row_io<NG>(tm0, d, b0, prev_b, o0);
+        const __half2 o0 = tc_band_row<NG>(tm0, d, b0, prev_b);
         if (OUT) {
             bnd[(size_t)(L - 1) * kStride] = o0;
         } else {
             const __half2 e = h2_combine(h2_pick4(&d[4 * (NG - 1)], ra), h2_pick4(&d[4 * (NG - 1)], rb));
             res = (L == Lm) ? e : res;
+        }
+    }
+}
+
+// A tile's results res[b] (two segments per band) for query m of group g as candidates of this thread's list, kept UNSORTED
+// while the slice is scanned (see k_dtw_scan_h2): a key below `worst` goes to the next free place (cnt) or, once the list is
+// full, replaces its largest key (at wpos), and the new largest key and its place are found with KP independent loads.
+// DBG also stores every pair's scan distance.
+template <int KP, int STRIDE, int NB, bool DBG>
+__device__ __forceinline__ void h2_push_tile(const H2Params& p, uint32_t g, int m, uint32_t Lm, const int4& sa, const int4& sb, const int4& sc,
+                                             const __half2 (&res)[NB], unsigned long long* list, unsigned long long& worst, unsigned long long thr0,
+                                             int& cnt, int& wpos) {
+    if (Lm) {
+#pragma unroll
+        for (int b = 0; b < NB; b++) {
+#pragma unroll
+            for (int hsel = 0; hsel < 2; hsel++) {
+                const int e = 2 * b + hsel;
+                const int seg = h2_seg_of(sa, sb, e);
+                if (seg >= 0) {
+                    const float v = hsel ? __high2float(res[b]) : __low2float(res[b]);
+                    // D16 / (S (Lq + Ld)); an overflowed path sum stays +inf and is never inserted
+                    const float dist = __fdividef(v * p.inv_s, (float)(Lm + (uint32_t)h2_len_of(sc, e)));
+                    const unsigned long long key = ((unsigned long long)f2ord(dist) << 32) | (uint32_t)seg;
+                    if (key < worst && dist == dist) {
+                        const bool full = cnt == KP;
+                        list[(full ? wpos : cnt) * STRIDE] = key;
+                        cnt += full ? 0 : 1;
+                        if (cnt == KP) {
+                            tc_list_max<KP, STRIDE>(list, worst, wpos);
+                            worst = worst < thr0 ? worst : thr0;
+                        }
+                    }
+                    if constexpr (DBG) p.dbg[(size_t)(g * kTcM + m) * p.dbg_nseg + seg] = dist;
+                }
+            }
         }
     }
 }
@@ -535,31 +505,15 @@ __global__ void __launch_bounds__(kH2Threads, 1) k_dtw_scan_h2(const H2Params p)
     unsigned long long* topk = reinterpret_cast<unsigned long long*>(bars + 32);  // [KP][256]
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    // CTA order: the FIRST slice of every group, then the other slices group by group (longest groups first in both parts).
-    // The slices of a group otherwise start together and none of them ever sees a sibling's threshold: with an empty
-    // threshold a thread's list takes 8 (1 + ln(n / 8)) sorted insertions over the n pairs of its slice, whatever n - per
-    // unit of work 5 times more on a 1/8 shard (ncu: 2.8 x the shared-memory wavefronts, + 5.7 % instructions, + 8 % cycles
-    // per step). With the first slice's threshold published before most of the others start, ~KP pairs per slice pass.
-    // Measured: 4.90 -> 4.85 ms on a 1/8 shard, 36.08 -> 35.97 ms at config 4 (the insertions were a part of the loss, not all
-    // of it: profiles/r2_h2_cycles_per_tile_eighth_vs_full.txt). Restricting the order to the first launch measured the same.
     uint32_t g, slice;
-    if (blockIdx.x < p.ngroups) {
-        g = blockIdx.x, slice = p.slice_begin;
-    } else {
-        const uint32_t r = blockIdx.x - p.ngroups;
-        g = r / (p.nslices - 1), slice = p.slice_begin + 1 + r % (p.nslices - 1);
-    }
+    h2_cta_slice(p, g, slice);
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // the next tile kind's launch may start filling SMs
     const uint32_t glen = p.group_len[g];
     const uint32_t L = glen & 0xFFFFu, lmin = glen >> 16;
     const uint32_t t0 = p.slice_tile[slice], t1 = p.slice_tile[slice + 1];
     const uint32_t ntiles = t1 - t0;
-    unsigned long long* tl = p.timeline ? p.timeline + ((size_t)(p.slice_begin * p.ngroups) + blockIdx.x) * 8 : nullptr;
-    if (tl && threadIdx.x == 0) {
-        unsigned smid;
-        asm("mov.u32 %0, %%smid;" : "=r"(smid));
-        tl[0] = h2_now(), tl[4] = smid | ((unsigned long long)NB << 16) | ((unsigned long long)g << 32), tl[7] = ((unsigned long long)L << 32) | ntiles;
-    }
+    unsigned long long* tl = p.timeline ? h2_timeline_of(p) : nullptr;
+    if (tl && threadIdx.x == 0) h2_timeline_open(tl, NB, g, L, ntiles);
 
     if (threadIdx.x == 0) {
         mb_init(a_full, 1);
@@ -567,57 +521,12 @@ __global__ void __launch_bounds__(kH2Threads, 1) k_dtw_scan_h2(const H2Params p)
         for (int s = 0; s < 2; s++) mb_init(&t_full[s], 1), mb_init(&t_empty[s], kH2DpWarps);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == kH2DpWarps) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tc_tmem_alloc(warp == kH2DpWarps, tmem_slot);
     if (tl && threadIdx.x == 0) tl[1] = h2_now(), tl[5] = clock64();
     if (warp == kH2DpWarps) {
         if (lane == 0 && ntiles) {
-            // ---- producer: TMA + MMA issue ---------------------------------------------------------------------------------
-            const uint32_t bars_s = s32(bars), sA_s = s32(sA), sB_s = s32(sB);
-            const uint32_t a_full_s = bars_s, b_full_s = bars_s + 8, b_empty_s = bars_s + 8 + 8 * kTcStages, t_full_s = bars_s + 80,
-                           t_empty_s = bars_s + 96;
-            mbs_expect_tx(a_full_s, L * kTcATileBytes);
-            tmas_g2s(sA_s, p.a_blocks + p.group_off[g], L * kTcATileBytes, a_full_s);
-            const unsigned char* tile_src = p.tiles + (size_t)t0 * kTcBTileBytes;
-            for (uint32_t n = 0; n < ntiles && n < (uint32_t)kTcStages; n++) {
-                mbs_expect_tx(b_full_s + 8 * n, kTcBTileBytes);
-                tmas_g2s(sB_s + n * kTcBTileBytes, tile_src + (size_t)n * kTcBTileBytes, kTcBTileBytes, b_full_s + 8 * n);
-            }
-            tile_src += (size_t)kTcStages * kTcBTileBytes;
-            mbs_wait_sleep(a_full_s, 0);
-            // f16 x f16 -> F16 accumulator (c_format = 0), K-major both, N = 128, M = 128
-            const uint32_t idesc = (0u << 4) | ((uint32_t)(kTcN >> 3) << 17) | ((uint32_t)(kTcM >> 4) << 24);
-            const uint64_t adesc0 = tc_smem_desc_s<kTcM>(sA_s);
-            uint32_t cnt = 0, stage = 0, sphase = 0;
-            for (uint32_t n = 0; n < ntiles; n++) {
-                mbs_wait_sleep(b_full_s + 8 * stage, sphase);
-                const uint64_t bdesc = tc_smem_desc_s<kTcN>(sB_s + stage * kTcBTileBytes);
-                uint64_t adesc = adesc0;
-                for (uint32_t row = 0; row < L; row += 2, cnt++) {
-                    const uint32_t buf = cnt & 1;
-                    if (cnt >= 2) mbs_wait_sleep(t_empty_s + 8 * buf, ((cnt >> 1) - 1) & 1);
-                    tc_fence_after();
-                    const uint32_t tm = tmem_base + buf * kTcBufCols;
-                    tc_mma_f16(tm, adesc, bdesc, idesc);
-                    if (row + 1 < L) tc_mma_f16(tm + kTcN, adesc + (kTcATileBytes >> 4), bdesc, idesc);
-                    tcs_commit(t_full_s + 8 * buf);
-                    adesc += 2 * (kTcATileBytes >> 4);
-                }
-                tcs_commit(b_empty_s + 8 * stage);
-                if (n + kTcStages < ntiles) {
-                    mbs_wait_sleep(b_empty_s + 8 * stage, sphase);
-                    mbs_expect_tx(b_full_s + 8 * stage, kTcBTileBytes);
-                    tmas_g2s(sB_s + stage * kTcBTileBytes, tile_src, kTcBTileBytes, b_full_s + 8 * stage);
-                    tile_src += kTcBTileBytes;
-                }
-                if (++stage == (uint32_t)kTcStages) stage = 0, sphase ^= 1;
-            }
+            const uint32_t bars_s = s32(bars);
+            tc_produce<1>(p, g, L, t0, ntiles, 0, kTcIdescF16, s32(sA), s32(sB), bars_s, bars_s + 8, bars_s + 80, tmem_base);
         }
     } else {
         // ---- DP warps ---------------------------------------------------------------------------------------------------
@@ -666,32 +575,7 @@ __global__ void __launch_bounds__(kH2Threads, 1) k_dtw_scan_h2(const H2Params p)
                 else h2_tile<4, 2>(L, lmin, Lm, sc, cur, res);
             }
             if (tl && threadIdx.x == 0 && n + 1 == (ntiles + 1) / 2) tl[6] = h2_now();  // (measurement: the slice's half-way mark)
-            if (Lm) {
-#pragma unroll
-                for (int b = 0; b < NB; b++) {
-#pragma unroll
-                    for (int hsel = 0; hsel < 2; hsel++) {
-                        const int e = 2 * b + hsel;
-                        const int seg = h2_seg_of(sa, sb, e);
-                        if (seg >= 0) {
-                            const float v = hsel ? __high2float(res[b]) : __low2float(res[b]);
-                            // D16 / (S (Lq + Ld)); an overflowed path sum stays +inf and is never inserted
-                            const float dist = __fdividef(v * p.inv_s, (float)(Lm + (uint32_t)h2_len_of(sc, e)));
-                            const unsigned long long key = ((unsigned long long)f2ord(dist) << 32) | (uint32_t)seg;
-                            if (key < worst && dist == dist) {
-                                const bool full = cnt == KP;
-                                list[(full ? wpos : cnt) * kH2DpThreads] = key;
-                                cnt += full ? 0 : 1;
-                                if (cnt == KP) {
-                                    tc_list_max<KP, kH2DpThreads>(list, worst, wpos);
-                                    worst = worst < thr0 ? worst : thr0;
-                                }
-                            }
-                            if constexpr (DBG) p.dbg[(size_t)(g * kTcM + m) * p.dbg_nseg + seg] = dist;
-                        }
-                    }
-                }
-            }
+            h2_push_tile<KP, kH2DpThreads, NB, DBG>(p, g, m, Lm, sa, sb, sc, res, list, worst, thr0, cnt, wpos);
         }
         tc_sort_list<KP, kH2DpThreads>(list, cnt);  // (the places beyond cnt still hold the initial +inf keys)
         worst = list[(KP - 1) * kH2DpThreads];
@@ -699,28 +583,12 @@ __global__ void __launch_bounds__(kH2Threads, 1) k_dtw_scan_h2(const H2Params p)
         // the two slots' lists of query m (threads m, m + 128) are merged by the slot-0 thread
         asm volatile("bar.sync 1, %0;" ::"n"(kH2DpThreads) : "memory");
         if (tl && threadIdx.x == 0) tl[2] = h2_now(), tl[5] = clock64() - tl[5];  // SM cycles of the DP phase (-> the SM clock under load)
-        if (slot == 0) {
-            const unsigned long long* other = list + kTcM;
-            for (int s = 0; s < KP; s++) {  // ascending: stop at the first key that does not make the cut
-                const unsigned long long key = other[s * kH2DpThreads];
-                if (key >= worst) break;
-                tc_insert_key<KP, kH2DpThreads>(list, worst, key);
-                worst = worst < thr0 ? worst : thr0;
-            }
-            const unsigned long long kept_worst = list[(KP - 1) * kH2DpThreads];
-            if (kept_worst != 0xFFFFFFFFFFFFFFFFull && kept_worst < thr0) atomicMin(p.thr + g * kTcM + m, kept_worst);
-            unsigned long long* out = p.partial + ((size_t)slice * p.ngroups * kTcM + (size_t)g * kTcM + m) * KP;
-#pragma unroll
-            for (int s = 0; s < KP; s++) out[s] = list[s * kH2DpThreads];
-        }
+        if (slot == 0)
+            tc_merge_store<KP, kH2DpThreads, kH2Slots, true>(list, worst, thr0, [&] {
+                return TcListDst{p.thr + g * kTcM + m, p.partial + ((size_t)slice * p.ngroups * kTcM + (size_t)g * kTcM + m) * KP};
+            });
     }
-    if constexpr (NB != 1) asm volatile("griddepcontrol.wait;" ::: "memory");  // see k_dtw_scan_tc: not complete before the launch ahead is
-    tc_fence_before();
-    __syncthreads();
-    if (warp == kH2DpWarps) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
+    tc_cta_exit<NB != 1>(warp == kH2DpWarps, tmem_base);  // the NB = 2 and 4 launches are the dependent ones
     if (tl && threadIdx.x == 0) tl[3] = h2_now();
 }
 
@@ -751,25 +619,15 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
     unsigned long long* topk = reinterpret_cast<unsigned long long*>(bars + 32);  // [KP][512]
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    // CTA order as in k_dtw_scan_h2: the first slice of every group, then the others
     uint32_t g, slice;
-    if (blockIdx.x < p.ngroups) {
-        g = blockIdx.x, slice = p.slice_begin;
-    } else {
-        const uint32_t r = blockIdx.x - p.ngroups;
-        g = r / (p.nslices - 1), slice = p.slice_begin + 1 + r % (p.nslices - 1);
-    }
+    h2_cta_slice(p, g, slice);
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // the next tile kind's launch may start filling SMs
     const uint32_t glen = p.group_len[g];
     const uint32_t L = glen & 0xFFFFu, lmin = glen >> 16;
     const uint32_t t0 = p.slice_tile[slice], t1 = p.slice_tile[slice + 1];
     const uint32_t ntiles = t1 - t0;
     unsigned long long* tl = p.timeline ? h2_timeline_of(p) : nullptr;
-    if (tl && threadIdx.x == 0) {
-        unsigned smid;
-        asm("mov.u32 %0, %%smid;" : "=r"(smid));
-        tl[0] = h2_now(), tl[4] = smid | ((unsigned long long)NB << 16) | ((unsigned long long)g << 32), tl[7] = ((unsigned long long)L << 32) | ntiles;
-    }
+    if (tl && threadIdx.x == 0) h2_timeline_open(tl, NB, g, L, ntiles);
 
     if (threadIdx.x == 0) {
         cta_gs[0] = g, cta_gs[1] = slice;
@@ -778,62 +636,15 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
         for (int s = 0; s < kH2Pipes; s++) mb_init(&t_full[s], 1), mb_init(&t_empty[s], kH2DpWarps);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == kH2PDpWarps) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tc_tmem_alloc(warp == kH2PDpWarps, tmem_slot);
     if (tl && threadIdx.x == 0) tl[1] = h2_now(), tl[5] = clock64();
     if (warp >= kH2PDpWarps) {
         asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kH2PRegsProd));
         const uint32_t pipe = (uint32_t)(warp - kH2PDpWarps);
         const uint32_t ntp = ntiles > pipe ? (ntiles - pipe + 1) >> 1 : 0u;  // this pipeline's tiles: t0 + pipe, t0 + pipe + 2, ..
         if (pipe < (uint32_t)kH2Pipes && lane == 0 && ntp) {
-            // ---- producer of pipeline `pipe`: its B ring (TMA), its MMAs; producer 0 also copies the A block ---------------
-            const uint32_t bars_s = s32(bars), sA_s = s32(sA), sB_s = s32(sB) + pipe * (kTcStages * kTcBTileBytes);
-            const uint32_t a_full_s = bars_s, b_full_s = bars_s + 8 + pipe * (16 * kTcStages), b_empty_s = b_full_s + 8 * kTcStages,
-                           t_full_s = s32(t_full) + 8 * pipe, t_empty_s = t_full_s + 16;
-            if (pipe == 0) {
-                mbs_expect_tx(a_full_s, L * kTcATileBytes);
-                tmas_g2s(sA_s, p.a_blocks + p.group_off[g], L * kTcATileBytes, a_full_s);
-            }
-            constexpr size_t kStride = (size_t)kH2Pipes * kTcBTileBytes;  // this pipeline's next tile
-            const unsigned char* tile_src = p.tiles + (size_t)(t0 + pipe) * kTcBTileBytes;
-            for (uint32_t n = 0; n < ntp && n < (uint32_t)kTcStages; n++) {
-                mbs_expect_tx(b_full_s + 8 * n, kTcBTileBytes);
-                tmas_g2s(sB_s + n * kTcBTileBytes, tile_src + n * kStride, kTcBTileBytes, b_full_s + 8 * n);
-            }
-            tile_src += kTcStages * kStride;
-            mbs_wait_sleep(a_full_s, 0);
-            // f16 x f16 -> F16 accumulator (c_format = 0), K-major both, N = 128, M = 128
-            const uint32_t idesc = (0u << 4) | ((uint32_t)(kTcN >> 3) << 17) | ((uint32_t)(kTcM >> 4) << 24);
-            const uint64_t adesc0 = tc_smem_desc_s<kTcM>(sA_s);
-            const uint32_t tm = tmem_base + pipe * kTcBufCols;
-            uint32_t cnt = 0, stage = 0, sphase = 0;
-            for (uint32_t n = 0; n < ntp; n++) {
-                mbs_wait_sleep(b_full_s + 8 * stage, sphase);
-                const uint64_t bdesc = tc_smem_desc_s<kTcN>(sB_s + stage * kTcBTileBytes);
-                uint64_t adesc = adesc0;
-                for (uint32_t row = 0; row < L; row += 2, cnt++) {
-                    if (cnt >= 1) mbs_wait_sleep(t_empty_s, (cnt - 1) & 1);  // the pipeline's 8 DP warps have pulled the last step
-                    tc_fence_after();
-                    tc_mma_f16(tm, adesc, bdesc, idesc);
-                    if (row + 1 < L) tc_mma_f16(tm + kTcN, adesc + (kTcATileBytes >> 4), bdesc, idesc);
-                    tcs_commit(t_full_s);
-                    adesc += 2 * (kTcATileBytes >> 4);
-                }
-                tcs_commit(b_empty_s + 8 * stage);
-                if (n + kTcStages < ntp) {
-                    mbs_wait_sleep(b_empty_s + 8 * stage, sphase);
-                    mbs_expect_tx(b_full_s + 8 * stage, kTcBTileBytes);
-                    tmas_g2s(sB_s + stage * kTcBTileBytes, tile_src, kTcBTileBytes, b_full_s + 8 * stage);
-                    tile_src += kStride;
-                }
-                if (++stage == (uint32_t)kTcStages) stage = 0, sphase ^= 1;
-            }
+            const uint32_t bars_s = s32(bars);  // producer of pipeline `pipe`: its B ring, its MMAs; producer 0 also copies the A block
+            tc_produce<kH2Pipes>(p, g, L, t0, ntp, pipe, kTcIdescF16, s32(sA), s32(sB), bars_s, bars_s + 8, s32(t_full), tmem_base);
         }
     } else {
         // ---- DP warps ---------------------------------------------------------------------------------------------------
@@ -878,31 +689,7 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
                 else h2_tile<2, 4>(L, lmin, Lm, sc, cur, res, load_segs);
             }
             if (p.timeline && threadIdx.x == 0 && n + 1 == (ntp + 1) / 2) h2_timeline_of(p)[6] = h2_now();  // (measurement: half of pipeline 0's tiles)
-            if (Lm) {
-#pragma unroll
-                for (int b = 0; b < NB; b++) {
-#pragma unroll
-                    for (int hsel = 0; hsel < 2; hsel++) {
-                        const int e = 2 * b + hsel;
-                        const int seg = h2_seg_of(sa, sb, e);
-                        if (seg >= 0) {
-                            const float v = hsel ? __high2float(res[b]) : __low2float(res[b]);
-                            const float dist = __fdividef(v * p.inv_s, (float)(Lm + (uint32_t)h2_len_of(sc, e)));
-                            const unsigned long long key = ((unsigned long long)f2ord(dist) << 32) | (uint32_t)seg;
-                            if (key < worst && dist == dist) {
-                                const bool full = cnt == KP;
-                                list[(full ? wpos : cnt) * kH2PDpThreads] = key;
-                                cnt += full ? 0 : 1;
-                                if (cnt == KP) {
-                                    tc_list_max<KP, kH2PDpThreads>(list, worst, wpos);
-                                    worst = worst < thr0 ? worst : thr0;
-                                }
-                            }
-                            if constexpr (DBG) p.dbg[(size_t)(g * kTcM + m) * p.dbg_nseg + seg] = dist;
-                        }
-                    }
-                }
-            }
+            h2_push_tile<KP, kH2PDpThreads, NB, DBG>(p, g, m, Lm, sa, sb, sc, res, list, worst, thr0, cnt, wpos);
         }
         tc_sort_list<KP, kH2PDpThreads>(list, cnt);  // (the places beyond cnt still hold the initial +inf keys)
         worst = list[(KP - 1) * kH2PDpThreads];
@@ -913,31 +700,13 @@ __global__ void __launch_bounds__(kH2PThreads, 1) k_dtw_scan_h2_2p(const H2Param
             unsigned long long* t = h2_timeline_of(p);
             t[2] = h2_now(), t[5] = clock64() - t[5];  // SM cycles of the DP phase (-> the SM clock under load)
         }
-        if (threadIdx.x < kTcM) {
-            for (int o = 1; o < kH2Pipes * kH2Slots; o++) {
-                const unsigned long long* other = list + o * kTcM;
-                for (int s = 0; s < KP; s++) {  // ascending: stop at the first key that does not make the cut
-                    const unsigned long long key = other[s * kH2PDpThreads];
-                    if (key >= worst) break;
-                    tc_insert_key<KP, kH2PDpThreads>(list, worst, key);
-                    worst = worst < thr0 ? worst : thr0;
-                }
-            }
-            const unsigned long long kept_worst = list[(KP - 1) * kH2PDpThreads];
-            const uint32_t gm = cta_gs[0] * kTcM + m;
-            if (kept_worst != 0xFFFFFFFFFFFFFFFFull && kept_worst < thr0) atomicMin(p.thr + gm, kept_worst);
-            unsigned long long* out = p.partial + ((size_t)cta_gs[1] * p.ngroups * kTcM + gm) * KP;
-#pragma unroll
-            for (int s = 0; s < KP; s++) out[s] = list[s * kH2PDpThreads];
-        }
+        if (threadIdx.x < kTcM)
+            tc_merge_store<KP, kH2PDpThreads, kH2Pipes * kH2Slots, true>(list, worst, thr0, [&] {
+                const uint32_t gm = cta_gs[0] * kTcM + m;
+                return TcListDst{p.thr + gm, p.partial + ((size_t)cta_gs[1] * p.ngroups * kTcM + gm) * KP};
+            });
     }
-    if constexpr (NB != 1) asm volatile("griddepcontrol.wait;" ::: "memory");  // see k_dtw_scan_tc: not complete before the launch ahead is
-    tc_fence_before();
-    __syncthreads();
-    if (warp == kH2PDpWarps) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
+    tc_cta_exit<NB != 1>(warp == kH2PDpWarps, tmem_base);
     if (tl && threadIdx.x == 0) tl[3] = h2_now();
 }
 
@@ -976,14 +745,7 @@ __global__ void __launch_bounds__(kH2Threads, 1) k_dtw_scan_h2_long(const H2Para
         for (int s = 0; s < 2; s++) mb_init(&t_full[s], 1), mb_init(&t_empty[s], kH2DpWarps);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == kH2DpWarps) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tc_tmem_alloc(warp == kH2DpWarps, tmem_slot);
     if (warp == kH2DpWarps) {
         if (lane == 0 && ntiles) {
             // ---- producer: TMA + MMA issue. The group's A block (L rows) lives in a ring of 4 pieces of 8 rows. Up to 32 rows it
@@ -1010,8 +772,7 @@ __global__ void __launch_bounds__(kH2Threads, 1) k_dtw_scan_h2_long(const H2Para
                 tmas_g2s(sB_s + n * kTcBTileBytes, tile_src + (size_t)n * kTcBTileBytes, kTcBTileBytes, b_full_s + 8 * n);
             }
             tile_src += (size_t)kTcStages * kTcBTileBytes;
-            // f16 x f16 -> F16 accumulator (c_format = 0), K-major both, N = 128, M = 128
-            const uint32_t idesc = (0u << 4) | ((uint32_t)(kTcN >> 3) << 17) | ((uint32_t)(kTcM >> 4) << 24);
+            const uint32_t idesc = kTcIdescF16;
             uint32_t cnt = 0, stage = 0, sphase = 0, use_n = 0;
             for (uint32_t n = 0; n < ntiles; n++) {
                 mbs_wait_sleep(b_full_s + 8 * stage, sphase);
@@ -1133,28 +894,12 @@ __global__ void __launch_bounds__(kH2Threads, 1) k_dtw_scan_h2_long(const H2Para
         }
         // the two slots' lists of query m (threads m, m + 128) are merged by the slot-0 thread
         asm volatile("bar.sync 1, %0;" ::"n"(kH2DpThreads) : "memory");
-        if (slot == 0) {
-            const unsigned long long* other = list + kTcM;
-            for (int s = 0; s < KP; s++) {  // ascending: stop at the first key that does not make the cut
-                const unsigned long long key = other[s * kH2DpThreads];
-                if (key >= worst) break;
-                tc_insert_key<KP, kH2DpThreads>(list, worst, key);
-                worst = worst < thr0 ? worst : thr0;
-            }
-            const unsigned long long kept_worst = list[(KP - 1) * kH2DpThreads];
-            if (kept_worst != 0xFFFFFFFFFFFFFFFFull && kept_worst < thr0) atomicMin(p.thr + g * kTcM + m, kept_worst);
-            unsigned long long* out = p.partial + ((size_t)slice * p.ngroups * kTcM + (size_t)g * kTcM + m) * KP;
-#pragma unroll
-            for (int s = 0; s < KP; s++) out[s] = list[s * kH2DpThreads];
-        }
+        if (slot == 0)
+            tc_merge_store<KP, kH2DpThreads, kH2Slots, true>(list, worst, thr0, [&] {
+                return TcListDst{p.thr + g * kTcM + m, p.partial + ((size_t)slice * p.ngroups * kTcM + (size_t)g * kTcM + m) * KP};
+            });
     }
-    if constexpr (NB != 1) asm volatile("griddepcontrol.wait;" ::: "memory");  // see k_dtw_scan_tc: not complete before the launch ahead is
-    tc_fence_before();
-    __syncthreads();
-    if (warp == kH2DpWarps) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
+    tc_cta_exit<NB != 1>(warp == kH2DpWarps, tmem_base);  // the NB = 2 and 4 launches are the dependent ones
 }
 
 __global__ void k_h2_nsmid(uint32_t* out) {
@@ -1383,31 +1128,10 @@ static int h2_launch_kind(ss_ctx* ctx, H2Params p, uint32_t slice_begin, uint32_
     p.nslices = nslices;
     // KP = 8 (k <= 2) runs the two-pipeline kernel for NB = 1 and 2. Its 32-entry lists (H2_WIDE, k > 2) would need 128 KB of
     // shared memory, and NB = 4 does not fit its 112 DP registers without spilling: both keep the one-pipeline kernel.
-    void (*kern)(H2Params);
-    unsigned threads = kH2Threads;
-    if constexpr (LONG) {
-        kern = k_dtw_scan_h2_long<KP, NB, DBG>;
-    } else if constexpr (KP == kH2Kp && NB != 4) {
-        kern = k_dtw_scan_h2_2p<KP, NB, DBG>;
-        threads = kH2PThreads;
-        smem = (size_t)p.max_len * kTcATileBytes + kH2Pipes * kTcStages * kTcBTileBytes + 32 * 8 + (size_t)KP * kH2PDpThreads * 8 + 1024;
-    } else {
-        kern = k_dtw_scan_h2<KP, NB, DBG>;
-    }
-    SS_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(p.ngroups * nslices);
-    cfg.blockDim = dim3(threads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = ctx->stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = dependent ? 1 : 0;
-    SS_CUDA(ctx, cudaLaunchKernelEx(&cfg, kern, p));
-    SS_LAUNCHED(ctx);
-    return SS_OK;
+    if constexpr (LONG) return tc_launch_scan(ctx, k_dtw_scan_h2_long<KP, NB, DBG>, p, kH2Threads, smem, dependent);
+    else if constexpr (KP == kH2Kp && NB != 4)
+        return tc_launch_scan(ctx, k_dtw_scan_h2_2p<KP, NB, DBG>, p, kH2PThreads, tc_smem_bytes(p.max_len, kH2Pipes, KP, kH2PDpThreads), dependent);
+    else return tc_launch_scan(ctx, k_dtw_scan_h2<KP, NB, DBG>, p, kH2Threads, smem, dependent);
 }
 
 // eta of the bound (true units, per normalised distance): fp16 subnormal roundings of the S-scaled operands and sums
@@ -1500,9 +1224,9 @@ static int h2_plan(ss_dict* d, ss_queries* q, int kp, H2Plan* plan) {
             p.bnd = d->d_h2_bnd.p;
         }
         p.eta = (float)h2_eta(d) * 1.0001f;
-        plan->smem = (size_t)kH2ARing * kTcATileBytes + kTcStages * kTcBTileBytes + 32 * 8 + (size_t)kp * kH2DpThreads * 8 + 1024;
+        plan->smem = tc_smem_bytes(kH2ARing, 1, kp, kH2DpThreads);
     } else {
-        plan->smem = (size_t)q->max_len * kTcATileBytes + kTcStages * kTcBTileBytes + 32 * 8 + (size_t)kp * kH2DpThreads * 8 + 1024;
+        plan->smem = tc_smem_bytes(q->max_len, 1, kp, kH2DpThreads);
     }
     return SS_OK;
 }

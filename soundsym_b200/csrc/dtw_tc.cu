@@ -25,6 +25,9 @@
 // advances together - the step's fixed cost is then paid once for both; the two tile kinds are separate instantiations.
 // Queries are grouped 128 at a time in length order; a group's queries may differ in length by a row or two (shorter ones
 // are zero-padded and every lane captures its result at its own last row).
+// What this file keeps: the fp32 TMEM loads, the DP step and tile of one segment (tc_step2, tc_tile) or of a pair of short
+// segments (tc_dp_band_pair, tc_step2_pair, tc_tile_pair), the kernel and its host side. The band recurrence, the step
+// driver, the CTA skeleton, the producer, the list merge and the launch are tc_common.cuh's, shared with dtw_h2.cu.
 #include <cuda_fp16.h>
 
 #include <algorithm>
@@ -178,43 +181,6 @@ __device__ __forceinline__ void tc_ld_row(uint32_t taddr, float (&v)[4 * NG]) {
     }
 }
 
-// TWO rows (i, i+1) of one segment slot in column-major order, row state updated in place: cell (i, j) reads d[j]
-// (row i-1) and feeds cell (i+1, j), which overwrites d[j]. Two independent dependency chains per thread (ILP 2), no
-// register copies, no guards: per cell FMNMX3 + FADD. The column count 4*NG is a compile-time constant. The band also
-// hands back row i's values of the last 4-column group (c0l; row i+1's are d[4 NG - 4 ..]): the column len - 1 lies in
-// that group, and the caller picks D(i, len-1) / D(i+1, len-1) from them only in the steps where a query can end.
-struct TcCarry {  // what a band carries from column j-1 to column j: D(i, j-1), D(i-1, j-1), D(i+1, j-1)
-    float left0, diag0, left1;
-};
-// columns [J0, J1) of the band; tm0 / tm1 hold the costs of those columns only
-template <int NG, int J0, int J1, int W>
-__device__ __forceinline__ void tc_dp_band_cols(const float (&tm0)[W], const float (&tm1)[W], float (&d)[4 * NG], TcCarry& c, float (&c0l)[4]) {
-#pragma unroll
-    for (int j = J0; j < J1; j++) {
-        const float up0 = d[j];
-        const float c0 = tm0[j - J0] + tc_min3(c.left0, up0, c.diag0);
-        const float c1 = tm1[j - J0] + tc_min3(c.left1, c0, c.left0);  // up = D(i, j), diag = D(i, j-1)
-        c.diag0 = up0;
-        c.left0 = c0;
-        c.left1 = c1;
-        d[j] = c1;
-        if (j >= 4 * (NG - 1)) c0l[j - 4 * (NG - 1)] = c0;
-    }
-}
-// a single trailing row (odd group length), in place
-template <int NG>
-__device__ __forceinline__ void tc_dp_row_ng(const float (&tm)[4 * NG], float (&d)[4 * NG], float dinit) {
-    const float INF = __int_as_float(0x7f800000);
-    float left = INF, diag = dinit;
-#pragma unroll
-    for (int j = 0; j < 4 * NG; j++) {
-        const float up = d[j];
-        const float cur = tm[j] + tc_min3(left, up, diag);
-        diag = up;
-        left = cur;
-        d[j] = cur;
-    }
-}
 __device__ __forceinline__ float tc_pick4(const float* v, int r) { return r == 0 ? v[0] : (r == 1 ? v[1] : (r == 2 ? v[2] : v[3])); }
 
 // one pipeline step for one thread: wait for the step's MMAs, pull this slot's columns of both rows into registers, hand
@@ -223,7 +189,7 @@ template <int NG>
 __device__ __forceinline__ void tc_step2(TcCursor& cur, float (&d)[4 * NG], float dinit, float (&c0l)[4]) {
     const float INF = __int_as_float(0x7f800000);
     cur.wait();
-    TcCarry c = {INF, dinit, INF};  // dinit = 0 on the first row of the pair (the virtual D(-1,-1)), +inf after
+    TcCarry<float> c = {INF, dinit, INF};  // dinit = 0 on the first row of the pair (the virtual D(-1,-1)), +inf after
     if constexpr (kTcChunked && NG > 4) {
         // 112-register budget: the step's costs come in two column chunks (16 + the rest), each two rows; the compiler
         // starts the second chunk's loads while the first is being consumed
@@ -233,7 +199,7 @@ __device__ __forceinline__ void tc_step2(TcCursor& cur, float (&d)[4 * NG], floa
             tc_ld<16>(taddr, a0);
             tc_ld<16>(taddr + kTcN, a1);
             tc_wait_ld();
-            tc_dp_band_cols<NG, 0, 16, 16>(a0, a1, d, c, c0l);
+            tc_band<NG, 0, 16>(a0, a1, d, c, c0l);
         }
         constexpr int W2 = NG <= 6 ? 8 : 16;  // the remaining 4 NG - 16 columns, loaded as x8 or x16
         float b0[W2], b1[W2];
@@ -241,14 +207,14 @@ __device__ __forceinline__ void tc_step2(TcCursor& cur, float (&d)[4 * NG], floa
         tc_ld<W2>(taddr + kTcN + 16, b1);
         tc_wait_ld();
         cur.release();
-        tc_dp_band_cols<NG, 16, 4 * NG, W2>(b0, b1, d, c, c0l);
+        tc_band<NG, 16, 4 * NG>(b0, b1, d, c, c0l);
     } else {
         float tm0[4 * NG], tm1[4 * NG];
         tc_ld_row<NG>(cur.taddr, tm0);
         tc_ld_row<NG>(cur.taddr + kTcN, tm1);
         tc_wait_ld();
         cur.release();
-        tc_dp_band_cols<NG, 0, 4 * NG, 4 * NG>(tm0, tm1, d, c, c0l);
+        tc_band<NG, 0, 4 * NG>(tm0, tm1, d, c, c0l);
     }
 }
 
@@ -265,37 +231,10 @@ __device__ __forceinline__ float tc_tile(uint32_t L, uint32_t lmin, uint32_t Lm,
     const uint32_t nfull = L >> 1;           // steps that carry two rows
     const uint32_t ncap = min((lmin - 1) >> 1, nfull);   // steps before any query of the group can end
     const int r = (len - 1) & 3;             // where column len - 1 sits in the last 4-column group
-    uint32_t st = 0;
-    // no query of the group ends in steps [0, ncap). They run two per iteration on buffer 0 then buffer 1, from cursors
-    // rebuilt out of loop invariants - barrier and TMEM addresses are then constants of the loop and only the parity flips
-    // (once per pair) - after one plain step if the tile happens to start on buffer 1.
-    if (st < ncap && cur.buf) {
+    uint32_t st = tc_steps(cur, ncap, dinit, INF, [&](TcCursor& c, float di) {  // no query of the group ends in steps [0, ncap)
         float c0l[4];
-        tc_step2<NG>(cur, d, dinit, c0l);
-        dinit = INF;
-        st++;
-    }
-    if (st + 2 <= ncap) {
-        const uint32_t full0 = cur.full, taddr0 = cur.taddr;
-        uint32_t par = cur.par;
-#pragma unroll 1
-        for (; st + 2 <= ncap; st += 2) {
-            float c0l[4];
-            TcCursor c0 = {0u, par, full0, taddr0, cur.full_sum, cur.taddr_sum};
-            tc_step2<NG>(c0, d, dinit, c0l);
-            TcCursor c1 = {1u, par, full0 + 8u, taddr0 + (uint32_t)kTcBufCols, cur.full_sum, cur.taddr_sum};
-            tc_step2<NG>(c1, d, INF, c0l);
-            dinit = INF;
-            par ^= 1u;
-        }
-        cur.par = par;
-    }
-    if (st < ncap) {
-        float c0l[4];
-        tc_step2<NG>(cur, d, dinit, c0l);
-        dinit = INF;
-        st++;
-    }
+        tc_step2<NG>(c, d, di, c0l);
+    });
 #pragma unroll 1
     for (; st < nfull; st++) {  // only the last step or two of a tile
         float c0l[4];
@@ -310,7 +249,7 @@ __device__ __forceinline__ float tc_tile(uint32_t L, uint32_t lmin, uint32_t Lm,
         tc_ld_row<NG>(cur.taddr, tm0);
         tc_wait_ld();
         cur.release();
-        tc_dp_row_ng<NG>(tm0, d, dinit);
+        tc_band_row<NG>(tm0, d, INF, dinit);
         res = (L == Lm) ? tc_pick4(&d[4 * (NG - 1)], r) : res;
     }
     return res;
@@ -375,35 +314,10 @@ __device__ __forceinline__ void tc_tile_pair(uint32_t L, uint32_t lmin, uint32_t
     float dinit = 0.f;
     const uint32_t nfull = L >> 1;
     const uint32_t ncap = min((lmin - 1) >> 1, nfull);
-    uint32_t st = 0;
-    // steps [0, ncap): no query of the group ends; two per iteration on buffers 0, 1 with loop-invariant addresses (tc_tile)
-    if (st < ncap && cur.buf) {
+    uint32_t st = tc_steps(cur, ncap, dinit, INF, [&](TcCursor& c, float di) {  // no query of the group ends in steps [0, ncap)
         float e0A, e0B;
-        tc_step2_pair<NG, false>(cur, dA, dB, dinit, lenA, lenB, e0A, e0B);
-        dinit = INF;
-        st++;
-    }
-    if (st + 2 <= ncap) {
-        const uint32_t full0 = cur.full, taddr0 = cur.taddr;
-        uint32_t par = cur.par;
-#pragma unroll 1
-        for (; st + 2 <= ncap; st += 2) {
-            float e0A, e0B;
-            TcCursor c0 = {0u, par, full0, taddr0, cur.full_sum, cur.taddr_sum};
-            tc_step2_pair<NG, false>(c0, dA, dB, dinit, lenA, lenB, e0A, e0B);
-            TcCursor c1 = {1u, par, full0 + 8u, taddr0 + (uint32_t)kTcBufCols, cur.full_sum, cur.taddr_sum};
-            tc_step2_pair<NG, false>(c1, dA, dB, INF, lenA, lenB, e0A, e0B);
-            dinit = INF;
-            par ^= 1u;
-        }
-        cur.par = par;
-    }
-    if (st < ncap) {
-        float e0A, e0B;
-        tc_step2_pair<NG, false>(cur, dA, dB, dinit, lenA, lenB, e0A, e0B);
-        dinit = INF;
-        st++;
-    }
+        tc_step2_pair<NG, false>(c, dA, dB, di, lenA, lenB, e0A, e0B);
+    });
 #pragma unroll 1
     for (; st < nfull; st++) {  // only the last step or two of a tile
         float e0A = INF, e0B = INF;
@@ -420,8 +334,8 @@ __device__ __forceinline__ void tc_tile_pair(uint32_t L, uint32_t lmin, uint32_t
         tc_ld_row<NG>(cur.taddr + kTcPairCol, b0);
         tc_wait_ld();
         cur.release();
-        tc_dp_row_ng<NG>(a0, dA, dinit);
-        tc_dp_row_ng<NG>(b0, dB, dinit);
+        tc_band_row<NG>(a0, dA, INF, dinit);
+        tc_band_row<NG>(b0, dB, INF, dinit);
         resA = (L == Lm) ? tc_pick_n<4 * NG>(dA, lenA - 1) : resA;
         resB = (L == Lm) ? tc_pick_n<4 * NG>(dB, lenB - 1) : resB;
     }
@@ -463,14 +377,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_dtw_scan_tc(const TcParams p)
         for (int s = 0; s < 2; s++) mb_init(&t_full[s], 1), mb_init(&t_empty[s], kTcDpWarps);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == kTcDpWarps) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tc_tmem_alloc(warp == kTcDpWarps, tmem_slot);
     // register re-distribution between warpgroups (setmaxnreg): the producer's warpgroup (one working lane, three idle
     // warps) hands registers to the three DP warpgroups, whose band loop keeps 32 + 64 values live per thread
     if (warp >= kTcDpWarps) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kTcRegsProd));
@@ -478,45 +385,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_dtw_scan_tc(const TcParams p)
         // idle warps of the producer's warpgroup
     } else if (warp == kTcDpWarps) {
         if (lane == 0 && ntiles) {
-            // ---- producer: TMA + MMA issue (32-bit shared addresses and running counters: it lives in kTcRegsProd registers)
-            const uint32_t bars_s = s32(bars), sA_s = s32(sA), sB_s = s32(sB);
-            const uint32_t a_full_s = bars_s, b_full_s = bars_s + 8, b_empty_s = bars_s + 8 + 8 * kTcStages, t_full_s = bars_s + 80,
-                           t_empty_s = bars_s + 96;
-            mbs_expect_tx(a_full_s, L * kTcATileBytes);
-            tmas_g2s(sA_s, p.a_blocks + p.group_off[g], L * kTcATileBytes, a_full_s);
-            const unsigned char* tile_src = p.tiles + (size_t)t0 * kTcBTileBytes;
-            for (uint32_t n = 0; n < ntiles && n < (uint32_t)kTcStages; n++) {
-                mbs_expect_tx(b_full_s + 8 * n, kTcBTileBytes);
-                tmas_g2s(sB_s + n * kTcBTileBytes, tile_src + (size_t)n * kTcBTileBytes, kTcBTileBytes, b_full_s + 8 * n);
-            }
-            tile_src += (size_t)kTcStages * kTcBTileBytes;  // the next tile to fetch
-            mbs_wait_sleep(a_full_s, 0);
-            const uint32_t idesc = (1u << 4) | ((uint32_t)(kTcN >> 3) << 17) | ((uint32_t)(kTcM >> 4) << 24);  // f16 x f16 -> f32, K-major
-            const uint64_t adesc0 = tc_smem_desc_s<kTcM>(sA_s);
-            uint32_t cnt = 0, stage = 0, sphase = 0;
-            for (uint32_t n = 0; n < ntiles; n++) {
-                mbs_wait_sleep(b_full_s + 8 * stage, sphase);
-                const uint64_t bdesc = tc_smem_desc_s<kTcN>(sB_s + stage * kTcBTileBytes);
-                uint64_t adesc = adesc0;  // advances by one A tile (4 KB = 256 descriptor units) per row
-                for (uint32_t row = 0; row < L; row += 2, cnt++) {
-                    const uint32_t buf = cnt & 1;
-                    if (cnt >= 2) mbs_wait_sleep(t_empty_s + 8 * buf, ((cnt >> 1) - 1) & 1);
-                    tc_fence_after();
-                    const uint32_t tm = tmem_base + buf * kTcBufCols;
-                    tc_mma_f16(tm, adesc, bdesc, idesc);
-                    if (row + 1 < L) tc_mma_f16(tm + kTcN, adesc + (kTcATileBytes >> 4), bdesc, idesc);
-                    tcs_commit(t_full_s + 8 * buf);
-                    adesc += 2 * (kTcATileBytes >> 4);
-                }
-                tcs_commit(b_empty_s + 8 * stage);
-                if (n + kTcStages < ntiles) {  // refill this stage once its MMAs have completed
-                    mbs_wait_sleep(b_empty_s + 8 * stage, sphase);
-                    mbs_expect_tx(b_full_s + 8 * stage, kTcBTileBytes);
-                    tmas_g2s(sB_s + stage * kTcBTileBytes, tile_src, kTcBTileBytes, b_full_s + 8 * stage);
-                    tile_src += kTcBTileBytes;
-                }
-                if (++stage == (uint32_t)kTcStages) stage = 0, sphase ^= 1;
-            }
+            const uint32_t bars_s = s32(bars);
+            tc_produce<1>(p, g, L, t0, ntiles, 0, kTcIdescF32, s32(sA), s32(sB), bars_s, bars_s + 8, bars_s + 80, tmem_base);
         }
     } else {
         // ---- DP warps ---------------------------------------------------------------------------------------------------
@@ -575,30 +445,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_dtw_scan_tc(const TcParams p)
         // the four slots' lists of query m (threads m, m + 128, m + 256, m + 384) are merged by the slot-0 thread: one list per
         // (slice, query) leaves the CTA
         asm volatile("bar.sync 1, %0;" ::"n"(kTcDpThreads) : "memory");
-        if (slot == 0) {
-            for (int o = 1; o < kTcSlots; o++) {
-                const unsigned long long* other = list + o * kTcM;
-                for (int s = 0; s < KP; s++) {  // ascending: stop at the first key that does not make the cut
-                    const unsigned long long key = other[s * kTcDpThreads];
-                    if (key >= worst) break;
-                    tc_insert_key<KP>(list, worst, key);
-                }
-            }
-            unsigned long long* out = p.partial + ((size_t)slice * p.ngroups * kTcM + (size_t)g * kTcM + m) * KP;
-#pragma unroll
-            for (int s = 0; s < KP; s++) out[s] = list[s * kTcDpThreads];
-        }
+        if (slot == 0)
+            tc_merge_store<KP, kTcDpThreads, kTcSlots, false>(list, worst, 0, [&] {
+                return TcListDst{nullptr, p.partial + ((size_t)slice * p.ngroups * kTcM + (size_t)g * kTcM + m) * KP};
+            });
     }
-    // a dependent launch may finish its own work before the launch ahead of it has: it must not be seen as complete (the
-    // merge kernel is ordered after THIS grid) until that one is, so every CTA waits for it on the way out. By then all of
-    // the earlier grid's CTAs are at least resident, so nothing is held up; a no-op for a normal launch.
-    if constexpr (PAIRED) asm volatile("griddepcontrol.wait;" ::: "memory");
-    tc_fence_before();
-    __syncthreads();
-    if (warp == kTcDpWarps) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
+    tc_cta_exit<PAIRED>(warp == kTcDpWarps, tmem_base);  // the paired launch is the dependent one
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -774,20 +626,7 @@ static int tc_launch_kind(ss_ctx* ctx, TcParams p, uint32_t slice_begin, uint32_
     if (!nslices) return SS_OK;
     p.slice_begin = slice_begin;
     p.nslices = nslices;
-    SS_CUDA(ctx, cudaFuncSetAttribute(k_dtw_scan_tc<KP, PAIRED, DBG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(p.ngroups * nslices);
-    cfg.blockDim = dim3(kTcThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = ctx->stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;  // may start while the previous scan launch is still draining
-    cfg.attrs = attr;
-    cfg.numAttrs = dependent ? 1 : 0;
-    SS_CUDA(ctx, cudaLaunchKernelEx(&cfg, k_dtw_scan_tc<KP, PAIRED, DBG>, p));
-    SS_LAUNCHED(ctx);
-    return SS_OK;
+    return tc_launch_scan(ctx, k_dtw_scan_tc<KP, PAIRED, DBG>, p, kTcThreads, smem, dependent);
 }
 // slices [0, nsingle) hold single-segment tiles, [nsingle, nslices) paired ones
 template <int KP>
@@ -870,7 +709,7 @@ static int tc_plan(ss_dict* d, ss_queries* q, int kp, TcPlan* plan) {
     plan->nsingle = nsingle;
     plan->nslices = nslices;
     plan->nslots = nslots;
-    plan->smem = (size_t)q->max_len * kTcATileBytes + kTcStages * kTcBTileBytes + 32 * 8 + (size_t)kp * kTcDpThreads * 8 + 1024;
+    plan->smem = tc_smem_bytes(q->max_len, 1, kp, kTcDpThreads);
     return SS_OK;
 }
 

@@ -1,6 +1,9 @@
 // tc_common.cuh — what the two tensor-core DTW scans (dtw_tc.cu: fp32 DP, dtw_h2.cu: packed-half DP) share: tile geometry,
-// the PTX wrappers (mbarrier, bulk TMA, tcgen05.mma / commit / fences, UMMA descriptors), the packed candidate keys and the
-// consumer-side cursor over the double-buffered TMEM accumulators.
+// the PTX wrappers (mbarrier, bulk TMA, tcgen05.mma / commit / fences, UMMA descriptors), the packed candidate keys, and the
+// pieces every scan kernel is built from: the DP band recurrence over float or __half2 (tc_band, tc_band_row), the consumer-side
+// cursor over the double-buffered TMEM accumulators and the step driver of a tile's capture-free steps (TcCursor, tc_steps), the
+// CTA skeleton (tc_tmem_alloc, tc_cta_exit), the producer lane (tc_produce), the merge and write of a query's slot lists
+// (tc_merge_store), and on the host the launch (tc_launch_scan) and the shared-memory size (tc_smem_bytes).
 #pragma once
 #include <cuda_fp16.h>
 
@@ -27,6 +30,10 @@ constexpr int kTcRegsDp = 112, kTcRegsProd = 32;
 constexpr bool kTcChunked = true;
 constexpr int kTcThreads = (kTcDpWarps + 4) * 32;    // 640
 constexpr int kTcDpThreads = kTcDpWarps * 32;
+// instruction descriptors of the scans' MMA: f16 x f16, K-major both, N = 128, M = 128, into an fp32 (c_format = 1) or an
+// F16 (c_format = 0) accumulator
+constexpr uint32_t kTcIdescF32 = (1u << 4) | ((uint32_t)(kTcN >> 3) << 17) | ((uint32_t)(kTcM >> 4) << 24);
+constexpr uint32_t kTcIdescF16 = (0u << 4) | ((uint32_t)(kTcN >> 3) << 17) | ((uint32_t)(kTcM >> 4) << 24);
 
 // byte offset of element (row, k) inside a ROWS x 16 fp16 K-major no-swizzle UMMA tile: core matrix = 8 rows x 16 B;
 // SBO (between 8-row groups) = 128 B, LBO (between the two K chunks) = ROWS / 8 * 128 B
@@ -165,6 +172,53 @@ __device__ __forceinline__ float tc_min3(float a, float b, float c) {
     asm("min.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
     return d;
 }
+__device__ __forceinline__ __half2 tc_min3(__half2 a, __half2 b, __half2 c) { return __hmin2(__hmin2(a, b), c); }  // one VHMNMX
+__device__ __forceinline__ float tc_add(float a, float b) { return a + b; }
+__device__ __forceinline__ __half2 tc_add(__half2 a, __half2 b) { return __hadd2(a, b); }
+
+// ---------------------------------------------------------------------------------------------------------------
+// the DP band, over float (dtw_tc.cu) or __half2 (dtw_h2.cu: two segments per register)
+// ---------------------------------------------------------------------------------------------------------------
+// what a band carries from column j-1 to column j: D(i, j-1), D(i-1, j-1), D(i+1, j-1)
+template <class T>
+struct TcCarry {
+    T left0, diag0, left1;
+};
+// TWO rows (i, i+1) of a band over columns [J0, J1), row state updated in place: cell (i, j) reads d[j] (row i-1) and feeds
+// cell (i+1, j), which overwrites d[j]. Two independent dependency chains per thread, no register copies, no guards: per cell
+// one three-input min and one add. tm0 / tm1 hold the costs of columns J0 .. J1 - 1 of the two rows. The carries come in and
+// go out through c, so a band split into column chunks (or a strip of a longer band) does the same operations in the same
+// order as the whole band. c0l receives row i's values of the last 4-column group (row i+1's are d[4 NG - 4 ..]): the
+// column len - 1 lies in that group, and the caller picks D(i, len-1) / D(i+1, len-1) from them in the steps where a query
+// can end.
+template <int NG, int J0, int J1, class T>
+__device__ __forceinline__ void tc_band(const T* tm0, const T* tm1, T (&d)[4 * NG], TcCarry<T>& c, T (&c0l)[4]) {
+#pragma unroll
+    for (int j = J0; j < J1; j++) {
+        const T up0 = d[j];
+        const T c0 = tc_add(tm0[j - J0], tc_min3(c.left0, up0, c.diag0));
+        const T c1 = tc_add(tm1[j - J0], tc_min3(c.left1, c0, c.left0));  // up = D(i, j), diag = D(i, j-1)
+        c.diag0 = up0;
+        c.left0 = c0;
+        c.left1 = c1;
+        d[j] = c1;
+        if (j >= 4 * (NG - 1)) c0l[j - 4 * (NG - 1)] = c0;
+    }
+}
+// a single row of a band, in place (the odd last row of a tile): carries D(i, -1) = left, D(i-1, -1) = diag in; returns the
+// row's last column, the left carry of whatever follows
+template <int NG, class T>
+__device__ __forceinline__ T tc_band_row(const T* tm, T (&d)[4 * NG], T left, T diag) {
+#pragma unroll
+    for (int j = 0; j < 4 * NG; j++) {
+        const T up = d[j];
+        const T cur = tc_add(tm[j], tc_min3(left, up, diag));
+        diag = up;
+        left = cur;
+        d[j] = cur;
+    }
+    return left;
+}
 
 // per-thread candidate list kept in shared memory as packed (ord(dist) << 32 | idx) keys, ascending; only the worst kept
 // key lives in a register for the per-pair test, so the hot loop pays two registers for the list
@@ -234,6 +288,155 @@ struct TcCursor {
         taddr = taddr_sum - taddr;
     }
 };
+
+// Steps [0, ncap) of a tile on the double-buffered cursor, the ones in which no query of the group ends. They run two per
+// iteration on buffer 0 then buffer 1, from cursors rebuilt out of loop invariants - barrier and TMEM addresses are then
+// constants of the loop and only the parity flips (once per pair) - after one plain step if the tile happens to start on
+// buffer 1. step(cursor, dinit) is one pipeline step; dinit = D(i-1, -1) of its first row: the caller's value for the tile's
+// first step (the virtual D(-1, -1) = 0), inf after; dinit is left at inf once a step has run. Returns the next step (ncap).
+template <class T, class Step>
+__device__ __forceinline__ uint32_t tc_steps(TcCursor& cur, uint32_t ncap, T& dinit, T inf, Step step) {
+    uint32_t st = 0;
+    if (st < ncap && cur.buf) {
+        step(cur, dinit);
+        dinit = inf;
+        st++;
+    }
+    if (st + 2 <= ncap) {
+        const uint32_t full0 = cur.full, taddr0 = cur.taddr;
+        uint32_t par = cur.par;
+#pragma unroll 1
+        for (; st + 2 <= ncap; st += 2) {
+            TcCursor c0 = {0u, par, full0, taddr0, cur.full_sum, cur.taddr_sum};
+            step(c0, dinit);
+            TcCursor c1 = {1u, par, full0 + 8u, taddr0 + (uint32_t)kTcBufCols, cur.full_sum, cur.taddr_sum};
+            step(c1, inf);
+            dinit = inf;
+            par ^= 1u;
+        }
+        cur.par = par;
+    }
+    if (st < ncap) {
+        step(cur, dinit);
+        dinit = inf;
+        st++;
+    }
+    return st;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// CTA skeleton of the scan kernels
+// ---------------------------------------------------------------------------------------------------------------
+// all 512 TMEM columns, allocated by the warp alloc_warp into *slot; every thread returns with their base address (the
+// mbarriers must be initialised before: the __syncthreads here publishes them too)
+__device__ __forceinline__ uint32_t tc_tmem_alloc(bool alloc_warp, uint32_t* slot) {
+    if (alloc_warp) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(slot)), "r"(512u) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    return *slot;
+}
+// the CTA's way out: the allocating warp hands TMEM back once every thread is done with it. DEPENDENT: the launch may have
+// started early (programmatic dependent launch) and may finish its own work before the launch ahead of it has: it must not
+// be seen as complete (the merge kernel is ordered after THIS grid) until that one is, so every CTA waits for it on the
+// way out. By then all of the earlier grid's CTAs are at least resident, so nothing is held up.
+template <bool DEPENDENT>
+__device__ __forceinline__ void tc_cta_exit(bool alloc_warp, uint32_t tmem_base) {
+    if constexpr (DEPENDENT) asm volatile("griddepcontrol.wait;" ::: "memory");
+    tc_fence_before();
+    __syncthreads();
+    if (alloc_warp) {
+        tc_fence_after();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    }
+}
+
+// The producer lane of pipeline `pipe` of a scan CTA: bulk-TMA copies and MMA issue. It lives in kTcRegsProd registers, so it
+// keeps 32-bit shared addresses and running counters only. Pipeline 0's producer copies the group's A block (L rows) into
+// sA_s; every producer waits for it. The ntiles B tiles t0 + pipe, t0 + pipe + PIPES, .. stream through the pipeline's ring of
+// kTcStages tiles (the rings from sB_s on, one per pipeline; per pipeline b_full[kTcStages], b_empty[kTcStages] barriers from
+// b_full_s on); per tile, one step per two query rows: two MMAs and one commit to the step's t_full barrier (t_empty 16
+// bytes above; one per pipeline from t_full_s on). PIPES = 1: the steps alternate between the TMEM buffers tmem_base and
+// tmem_base + kTcBufCols; PIPES = 2: every step goes to the pipeline's one buffer, tmem_base + pipe kTcBufCols.
+template <int PIPES, class Params>
+__device__ __forceinline__ void tc_produce(const Params& p, uint32_t g, uint32_t L, uint32_t t0, uint32_t ntiles, uint32_t pipe, uint32_t idesc,
+                                           uint32_t sA_s, uint32_t sB_s, uint32_t a_full_s, uint32_t b_full_s, uint32_t t_full_s, uint32_t tmem_base) {
+    constexpr uint32_t kBufs = PIPES == 1 ? 2 : 1;  // TMEM buffers the steps go round
+    constexpr size_t kStride = (size_t)PIPES * kTcBTileBytes;  // from one of this producer's tiles to the next
+    sB_s += pipe * (kTcStages * kTcBTileBytes);
+    b_full_s += pipe * (16 * kTcStages);
+    t_full_s += 8 * pipe;
+    const uint32_t b_empty_s = b_full_s + 8 * kTcStages, t_empty_s = t_full_s + 16;
+    if (pipe == 0) {
+        mbs_expect_tx(a_full_s, L * kTcATileBytes);
+        tmas_g2s(sA_s, p.a_blocks + p.group_off[g], L * kTcATileBytes, a_full_s);
+    }
+    const unsigned char* tile_src = p.tiles + (size_t)(t0 + pipe) * kTcBTileBytes;
+    for (uint32_t n = 0; n < ntiles && n < (uint32_t)kTcStages; n++) {
+        mbs_expect_tx(b_full_s + 8 * n, kTcBTileBytes);
+        tmas_g2s(sB_s + n * kTcBTileBytes, tile_src + n * kStride, kTcBTileBytes, b_full_s + 8 * n);
+    }
+    tile_src += kTcStages * kStride;  // the next tile to fetch
+    mbs_wait_sleep(a_full_s, 0);
+    const uint64_t adesc0 = tc_smem_desc_s<kTcM>(sA_s);
+    const uint32_t tm = tmem_base + pipe * kTcBufCols;
+    uint32_t cnt = 0, stage = 0, sphase = 0;
+    for (uint32_t n = 0; n < ntiles; n++) {
+        mbs_wait_sleep(b_full_s + 8 * stage, sphase);
+        const uint64_t bdesc = tc_smem_desc_s<kTcN>(sB_s + stage * kTcBTileBytes);
+        uint64_t adesc = adesc0;  // advances by one A tile (4 KB = 256 descriptor units) per row
+        for (uint32_t row = 0; row < L; row += 2, cnt++) {
+            const uint32_t buf = cnt % kBufs;
+            if (cnt >= kBufs) mbs_wait_sleep(t_empty_s + 8 * buf, (cnt / kBufs - 1) & 1);  // the DP warps have pulled the step before
+            tc_fence_after();
+            const uint32_t tmb = tm + buf * kTcBufCols;
+            tc_mma_f16(tmb, adesc, bdesc, idesc);
+            if (row + 1 < L) tc_mma_f16(tmb + kTcN, adesc + (kTcATileBytes >> 4), bdesc, idesc);
+            tcs_commit(t_full_s + 8 * buf);
+            adesc += 2 * (kTcATileBytes >> 4);
+        }
+        tcs_commit(b_empty_s + 8 * stage);
+        if (n + kTcStages < ntiles) {  // refill this stage once its MMAs have completed
+            mbs_wait_sleep(b_empty_s + 8 * stage, sphase);
+            mbs_expect_tx(b_full_s + 8 * stage, kTcBTileBytes);
+            tmas_g2s(sB_s + stage * kTcBTileBytes, tile_src, kTcBTileBytes, b_full_s + 8 * stage);
+            tile_src += kStride;
+        }
+        if (++stage == (uint32_t)kTcStages) stage = 0, sphase ^= 1;
+    }
+}
+
+// The end of a slice for the thread that owns query m's first list: the other NLISTS - 1 lists of the query (list + o kTcM,
+// each ascending) are merged into its own ascending list, which then leaves the CTA as the (slice, query) partial dst().out.
+// THR (packed-half scans): `worst` never rises above the query's threshold thr0, and a kept worst key below it is published
+// to the query's threshold word dst().thr. dst is evaluated once the lists are merged, so that what it reads (k_dtw_scan_h2_2p:
+// its group and slice, from shared memory) is not held through the merge.
+struct TcListDst {
+    unsigned long long* thr;
+    unsigned long long* out;
+};
+template <int KP, int STRIDE, int NLISTS, bool THR, class Dst>
+__device__ __forceinline__ void tc_merge_store(unsigned long long* list, unsigned long long worst, unsigned long long thr0, Dst dst) {
+    for (int o = 1; o < NLISTS; o++) {
+        const unsigned long long* other = list + o * kTcM;
+        for (int s = 0; s < KP; s++) {  // ascending: stop at the first key that does not make the cut
+            const unsigned long long key = other[s * STRIDE];
+            if (key >= worst) break;
+            tc_insert_key<KP, STRIDE>(list, worst, key);
+            if constexpr (THR) worst = worst < thr0 ? worst : thr0;
+        }
+    }
+    const TcListDst to = dst();
+    if constexpr (THR) {
+        const unsigned long long kept_worst = list[(KP - 1) * STRIDE];
+        if (kept_worst != 0xFFFFFFFFFFFFFFFFull && kept_worst < thr0) atomicMin(to.thr, kept_worst);
+    }
+#pragma unroll
+    for (int s = 0; s < KP; s++) to.out[s] = list[s * STRIDE];
+}
 
 // one thread per (group g = blockIdx.x, row i = blockIdx.y, query m): A_i[m, :] = [-2 (a_i - mu) (13), s, s, rd(|a_i|^2 / s)],
 // written as the two 16-byte K chunks of row m (K-major core matrices). slot_max_na (per query: max |a_i|^2 over its rows)
@@ -342,6 +545,34 @@ __global__ void __launch_bounds__(256) k_tc_merge(const unsigned long long* __re
         const float dist = key_dist(mine);
         cand_adist[(size_t)slot * KP + lane] = empty ? __int_as_float(0x7f800000) : dist;
     }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// host side of the scan launches
+// ---------------------------------------------------------------------------------------------------------------
+// dynamic shared memory of a scan CTA: a_rows A tiles, b_rings B-tile rings, the barriers, kp candidate keys per DP thread,
+// and the slack of the 128-byte alignment
+static inline size_t tc_smem_bytes(uint32_t a_rows, int b_rings, int kp, int dp_threads) {
+    return (size_t)a_rows * kTcATileBytes + b_rings * kTcStages * kTcBTileBytes + 32 * 8 + (size_t)kp * dp_threads * 8 + 1024;
+}
+// one scan launch of p.ngroups x p.nslices CTAs. dependent: it may start while the previous scan launch is still draining
+// (programmatic dependent launch; the launches write disjoint candidate lists and none reads another's output)
+template <class Params>
+static int tc_launch_scan(ss_ctx* ctx, void (*kern)(Params), const Params& p, unsigned threads, size_t smem, bool dependent) {
+    SS_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(p.ngroups * p.nslices);
+    cfg.blockDim = dim3(threads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = ctx->stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = dependent ? 1 : 0;
+    SS_CUDA(ctx, cudaLaunchKernelEx(&cfg, kern, p));
+    SS_LAUNCHED(ctx);
+    return SS_OK;
 }
 
 }  // namespace ss
