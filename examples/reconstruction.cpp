@@ -1,6 +1,7 @@
 // examples/reconstruction.cpp — the flow of the reference's examples/reconstruction.rs (and, with --partition-only,
 // examples/partition.rs) written against include/soundsym.hpp:
 //   -s source.wav  -t target.wav  -o out.wav  -m model.bin  [--depth 3] [--threshold 4] [--dtw] [--warp] [--partition-only]
+//   --matcher dict_dir query_dir [--dtw] [--locate]
 // Partitioner::from_path(source).threshold(4).depth(3) -> train (model supplied) -> partition -> SoundDictionary::from_segments
 // -> partition the target with the source's model -> clone_from_dictionary -> to_sound -> write_file. --warp fits every matched
 // sound to its target segment's timing along the DTW warping path (ss_resynth_warped) instead of zero-padding or cutting it.
@@ -18,7 +19,7 @@ using namespace soundsym;
 int main(int argc, char** argv) {
     std::string src, tgt, out, model_path;
     size_t depth = 3, threshold = 4;  // examples/reconstruction.rs:44-45
-    bool dtw = false, partition_only = false, morph = false, matcher_loop = false, warp = false;
+    bool dtw = false, partition_only = false, morph = false, matcher_loop = false, warp = false, locate = false;
     size_t chain = 6;
     std::string dict_dir, query_dir, splits_dir;  // --matcher <dictionary dir> <query dir>: the flow of examples/matcher.rs
     for (int i = 1; i < argc; i++) {
@@ -35,6 +36,7 @@ int main(int argc, char** argv) {
         else if (a == "--partition-only") partition_only = true;
         else if (a == "--matcher") dict_dir = next(), query_dir = next();
         else if (a == "--matcher-loop") dict_dir = next(), query_dir = next(), matcher_loop = true;
+        else if (a == "--locate") locate = true;
         else if (a == "--morph") morph = true;
         else if (a == "--chain") chain = std::stoul(next());
         else if (a == "--write-splits") splits_dir = next();
@@ -67,6 +69,21 @@ int main(int argc, char** argv) {
             long long sum = 0;
             for (int16_t v : concat) sum += v;
             printf("], \"concat_len\": %zu, \"concat_sum\": %lld}\n", concat.size(), sum);
+            return 0;
+        }
+        if (!dict_dir.empty() && locate) {
+            // --matcher <dictionary dir> <query dir> --locate: where inside the dictionary files every query file occurs
+            // (SoundDictionary::locate, k = 1), as [query, dictionary sound, first frame, last frame, cost]
+            auto dictionary = SoundDictionary::from_path(dict_dir);
+            auto queries = SoundDictionary::from_path(query_dir);
+            std::vector<uint32_t> idx, first, last;
+            std::vector<double> cost;
+            dictionary->locate(queries->sounds, 1, &idx, &first, &last, &cost);
+            printf("{\"located\": [");
+            for (size_t i = 0; i < queries->sounds.size(); i++)
+                printf("%s[\"%s\", \"%s\", %u, %u, %.17g]", i ? "," : "", queries->sounds[i]->name.value_or("").c_str(),
+                       idx[i] < dictionary->sounds.size() ? dictionary->sounds[idx[i]]->name.value_or("").c_str() : "", first[i], last[i], cost[i]);
+            printf("]}\n");
             return 0;
         }
         if (!dict_dir.empty()) {

@@ -413,6 +413,23 @@ class SoundDictionary {
         for (size_t p = 0; p < queries.size(); p++)
             for (uint64_t e = poff[p]; e < poff[p + 1]; e++) (*paths)[p].emplace_back(cells[2 * e], cells[2 * e + 1]);
     }
+    /// where inside the dictionary sounds each query occurs (subsequence DTW, ss_dict_locate): the k best dictionary sounds by
+    /// (cost, index), and in each the frames start..end (inclusive) the query fits best, at the unnormalised DTW cost; all
+    /// queries.size() x k. Frame t of a sound begins at its sample t * SS_HOP (the add_segments convention), so the located
+    /// passage is samples [start * SS_HOP, end * SS_HOP + SS_BIN) of sounds[idx]. Works in either mode; dtw_band does not apply.
+    void locate(const std::vector<std::shared_ptr<Sound>>& queries, int k, std::vector<uint32_t>* idx, std::vector<uint32_t>* start,
+                std::vector<uint32_t>* end, std::vector<double>* cost) {
+        ss_dict* d = device();
+        std::vector<uint64_t> off(queries.size() + 1, 0);
+        std::vector<double> flat;
+        for (size_t i = 0; i < queries.size(); i++) {
+            off[i + 1] = off[i] + queries[i]->num_frames();
+            flat.insert(flat.end(), queries[i]->mfccs().begin(), queries[i]->mfccs().end());
+        }
+        const size_t n = queries.size() * (size_t)std::max(k, 0);
+        idx->assign(n, 0), start->assign(n, 0), end->assign(n, 0), cost->assign(n, 0.0);
+        ctx_->check(ss_dict_locate(d, flat.data(), off.data(), queries.size(), k, idx->data(), start->data(), end->data(), cost->data()));
+    }
     /// SoundDictionary::match_sound (src/sound.rs:346-348)
     std::shared_ptr<Sound> match_sound(const std::shared_ptr<Sound>& other) { return at_distance(1.0, other); }
     Context& context() const { return *ctx_; }

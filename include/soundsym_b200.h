@@ -197,6 +197,29 @@ int ss_dict_align(ss_dict* dict, const double* q_mfcc, const uint64_t* q_frame_o
  * query lengths and Ld_max, so the count is known before the call); nq == 0 launches nothing. */
 int ss_dict_align_dev(ss_dict* dict, ss_queries* q, const uint32_t* d_seg_idx, uint32_t* d_out_path, size_t path_capacity,
                       uint64_t* d_out_path_offsets, double* d_out_dist);
+/* ss_dict_locate   subsequence DTW (no reference counterpart; spec A12, DESIGN.md §3.1g): WHERE inside a dictionary segment each query
+ *              fits best, the query free to start and end at any frame of it. For a query of Lq frames and a segment of Ld frames,
+ *              c(i, j) is A8's local cost (same operations, same order) and
+ *                  S(0, j) = c(0, j);   S(i, j) = c(i, j) + fmin(fmin(S(i-1, j), S(i, j-1)), S(i-1, j-1))   (i >= 1)
+ *              with a missing neighbour (j = 0) +inf and NaN counting as +inf. The start column st(0, j) = j travels along the
+ *              neighbour the min chose (ss_dict_align's rule: diag if it equals the min, else up if it does, else left). The end e
+ *              is the smallest j whose S(Lq-1, j) is the minimum of the finite values of row Lq-1; the pair's hit is
+ *              (cost = S(Lq-1, e), start = st(Lq-1, e), end = e), cost UNNORMALISED; no finite value, empty query or empty
+ *              segment: no hit. One hit per (query, segment); the k best across segments by (cost, index) ascending,
+ *              indices + index_base; unfilled slots (idx, start, end, cost) = (0xFFFFFFFF, 0xFFFFFFFF, 0xFFFFFFFF, +inf).
+ *              cost / (Lq + end - start + 1) is ss_dict_match's SS_DTW distance of the query against frames start..end
+ *              of the segment bit for bit, and ss_dict_align's path on that span is the backtrack of S from (Lq-1, end): the span
+ *              can feed ss_dict_align and ss_resynth_warped unchanged (dictionary samples offset by start * SS_HOP).
+ *              out_*: nq x k; start / end are frame indices within the segment, end inclusive; any output other than out_idx may
+ *              be NULL. The Sakoe-Chiba band does not apply. k outside 1..SS_MAX_TOPK or a NULL input -> SS_ERR_INVALID; an
+ *              empty dictionary -> SS_ERR_EMPTY_DICT. A pending SS_DTW match completes first; the ss_dict_last_* readers still
+ *              describe the last MATCH. Host buffers, stream-synchronised on return. */
+int ss_dict_locate(ss_dict* dict, const double* q_mfcc, const uint64_t* q_frame_offsets, size_t nq, int k, uint32_t* out_idx,
+                   uint32_t* out_start, uint32_t* out_end, double* out_cost);
+/* the same on device pointers, asynchronous on the ctx stream (no host synchronisation besides completing a pending SS_DTW match).
+ * Launches: 3 per batch of B = max(1, min(nq, floor(2^24 / nseg))) queries, i.e. 3 ceil(nq / B); nq == 0 launches nothing. */
+int ss_dict_locate_dev(ss_dict* dict, ss_queries* q, int k, uint32_t* d_out_idx, uint32_t* d_out_start, uint32_t* d_out_end,
+                       double* d_out_cost);
 int ss_topk_merge_dev(ss_ctx* ctx, const uint32_t* d_idx, const double* d_dist, int nlists, size_t nq, int k,
                       uint32_t* d_out_idx, double* d_out_dist);
 /* drops the cached device layouts of a query batch so that the next match rebuilds them (bench.py calls this every

@@ -294,6 +294,19 @@ class DeviceDictionary:
         self.ctx.check(self.ctx.lib.ss_dict_align(self.h, _ptr(q), _ptr(qo), nq, _ptr(seg), _ptr(path), cap, _ptr(poff), _ptr(dist)))
         return [path[int(poff[p]):int(poff[p + 1])].copy() for p in range(nq)], dist
 
+    def locate(self, q_flat, q_frame_offsets, k=1):
+        """ss_dict_locate: subsequence DTW (spec A12, DESIGN.md §3.1g), where inside a segment each query fits best -> (idx u32
+        [nq, k], start u32 [nq, k], end u32 [nq, k], cost f64 [nq, k]); start / end are frames of the segment, end inclusive,
+        cost is unnormalised. The k best (cost, index) hits, one per segment; unfilled slots (0xFFFFFFFF, 0xFFFFFFFF,
+        0xFFFFFFFF, inf). The band does not apply."""
+        q = np.ascontiguousarray(q_flat, dtype=np.float64)
+        qo = np.ascontiguousarray(q_frame_offsets, dtype=np.uint64)
+        nq = qo.shape[0] - 1
+        idx, start, end = (np.empty((nq, k), dtype=np.uint32) for _ in range(3))
+        cost = np.empty((nq, k), dtype=np.float64)
+        self.ctx.check(self.ctx.lib.ss_dict_locate(self.h, _ptr(q), _ptr(qo), nq, int(k), _ptr(idx), _ptr(start), _ptr(end), _ptr(cost)))
+        return idx, start, end, cost
+
     def debug_tc_scan(self, q_flat, q_frame_offsets):
         """ss_dict_debug_tc_scan: raw tensor-core scan distance of every (query, segment) pair -> (scan f32 [nq, nseg],
         mean frame f64 [16], norm scale)."""
@@ -716,6 +729,18 @@ class SoundDictionary:
         off[1:] = np.cumsum(lens)
         flat = np.concatenate([s.mfcc_arrays() for s in sounds], axis=0) if int(off[-1]) else np.zeros((0, NCOEFFS))
         return self._device().align(flat, off, indices)
+
+    def locate(self, sounds, k=1):
+        """where inside the dictionary sounds each sound occurs (subsequence DTW, ss_dict_locate) -> (idx, start, end, cost),
+        each [n, k]: the k best dictionary sounds by (cost, index), and in each the frames start..end (inclusive) the sound
+        fits best, at the unnormalised DTW cost. Frames map to samples as in add_segments: frame t of a sound begins at its
+        sample t * HOP, so the located passage is samples [start * HOP, end * HOP + BIN) of dictionary sound idx. Works in
+        either mode, and dtw_band does not apply."""
+        lens = np.array([s.num_frames() for s in sounds], dtype=np.uint64)
+        off = np.zeros(len(lens) + 1, dtype=np.uint64)
+        off[1:] = np.cumsum(lens)
+        flat = np.concatenate([s.mfcc_arrays() for s in sounds], axis=0) if int(off[-1]) else np.zeros((0, NCOEFFS))
+        return self._device().locate(flat, off, k)
 
     def at_distance(self, distance, other):
         """src/sound.rs:351-370 (always Some)."""

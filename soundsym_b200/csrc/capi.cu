@@ -441,6 +441,61 @@ int ss_dict_align(ss_dict* d, const double* q_mfcc, const uint64_t* q_frame_offs
     return rc;
 }
 
+// Subsequence DTW (A12, DESIGN.md §3.1g). Like an alignment it takes no matcher state: a pending SS_DTW match completes first,
+// and the ss_dict_last_* counters stay as the last match left them. The band does not apply.
+int ss_dict_locate_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, uint32_t* d_out_start, uint32_t* d_out_end, double* d_out_cost) {
+    if (!d || !q) return set_error(d ? d->ctx : nullptr, SS_ERR_INVALID, "dict / queries is NULL");
+    ss_ctx* ctx = d->ctx;
+    if (q->ctx != ctx) return set_error(ctx, SS_ERR_INVALID, "dict and queries belong to different contexts");
+    if (q->c != d->c) return set_error(ctx, SS_ERR_INVALID, "ncoeffs mismatch: dict %d, queries %d", d->c, q->c);
+    if (d->nseg == 0) return set_error(ctx, SS_ERR_EMPTY_DICT, "locate in an empty dictionary");
+    if (k < 1 || k > SS_MAX_TOPK) return set_error(ctx, SS_ERR_INVALID, "k must be in 1..%d (got %d)", SS_MAX_TOPK, k);
+    if (q->nq && !d_out_idx) return set_error(ctx, SS_ERR_INVALID, "d_out_idx is NULL");
+    SS_CUDA(ctx, cudaSetDevice(ctx->device));
+    SS_TRY(dtw_match_finish(d));  // a pending SS_DTW match shares the exhaustive stage's tables
+    return dtw_locate_dev(d, q, k, d_out_idx, d_out_start, d_out_end, d_out_cost);
+}
+
+int ss_dict_locate(ss_dict* d, const double* q_mfcc, const uint64_t* q_frame_offsets, size_t nq, int k, uint32_t* out_idx, uint32_t* out_start,
+                   uint32_t* out_end, double* out_cost) {
+    if (!d) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
+    ss_ctx* ctx = d->ctx;
+    if (d->nseg == 0) return set_error(ctx, SS_ERR_EMPTY_DICT, "locate in an empty dictionary");
+    if (k < 1 || k > SS_MAX_TOPK) return set_error(ctx, SS_ERR_INVALID, "k must be in 1..%d (got %d)", SS_MAX_TOPK, k);
+    if (nq && !out_idx) return set_error(ctx, SS_ERR_INVALID, "out_idx is NULL");
+    SS_TRY(queries_check(ctx, q_mfcc, q_frame_offsets, nq, d->c));
+    SS_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (!d->scratch_q) {
+        d->scratch_q = new (std::nothrow) ss_queries();
+        if (!d->scratch_q) return set_error(ctx, SS_ERR_NOMEM, "out of host memory");
+        d->scratch_q->ctx = ctx;
+        d->scratch_q->c = d->c;
+    }
+    ss_queries* q = d->scratch_q;
+    auto body = [&]() -> int {
+        SS_TRY(dtw_match_finish(d));
+        SS_TRY(queries_fill(q, q_mfcc, q_frame_offsets, nq));
+        const size_t n = nq * (size_t)k;
+        SS_CUDA(ctx, d->d_locate_idx.reserve(n));
+        if (out_start) SS_CUDA(ctx, d->d_locate_start.reserve(n));
+        if (out_end) SS_CUDA(ctx, d->d_locate_end.reserve(n));
+        if (out_cost) SS_CUDA(ctx, d->d_locate_cost.reserve(n));
+        SS_TRY(dtw_locate_dev(d, q, k, d->d_locate_idx.p, out_start ? d->d_locate_start.p : nullptr, out_end ? d->d_locate_end.p : nullptr,
+                              out_cost ? d->d_locate_cost.p : nullptr));
+        if (n) {  // ONE blocking point per call
+            SS_CUDA(ctx, cudaMemcpyAsync(out_idx, d->d_locate_idx.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+            if (out_start) SS_CUDA(ctx, cudaMemcpyAsync(out_start, d->d_locate_start.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+            if (out_end) SS_CUDA(ctx, cudaMemcpyAsync(out_end, d->d_locate_end.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+            if (out_cost) SS_CUDA(ctx, cudaMemcpyAsync(out_cost, d->d_locate_cost.p, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        }
+        SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        return SS_OK;
+    };
+    const int rc = body();
+    if (rc != SS_OK) cudaStreamSynchronize(ctx->stream);
+    return rc;
+}
+
 int ss_dict_set_scan(ss_dict* d, int first_stage) {
     if (!d) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
     if (first_stage < 0 || first_stage > 3) return set_error(d->ctx, SS_ERR_INVALID, "first_stage must be 0, 1, 2 or 3");

@@ -5,6 +5,7 @@
 //   DTW refine           the oracle's f64 recurrence (ASSUMPTIONS.h A8) on the candidates the fp32 scan kept
 //   top-k merge          (distance, index) lexicographic merge of per-shard lists
 //   DTW alignment        the refine's recurrence with the direction of every cell kept, then the backtrack (DESIGN.md §3.1e)
+//   DTW locate           the refine's recurrence with the query free to start and end anywhere in a segment (DESIGN.md §3.1g)
 #include <cub/cub.cuh>
 
 #include <algorithm>
@@ -1036,13 +1037,20 @@ k_dtw_refine_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__
 // DIRS (the alignment, k_dtw_align_long): per strip, lane j packs 32 rows of its column into a u64 and stores it to the
 // direction block `dir`, [strip][row / 32][lane], coalesced, once the whole warp has finished those rows. With BAND the words
 // of row blocks outside the strip's step range are not written, and no path cell reads them.
+// SUBSEQ (subsequence DTW, k_dtw_locate_pairs, A12 in DESIGN.md §3.1g): row 0 takes m = 0 on every column, and a u32 start column
+// travels beside every value - up is the lane's own, left comes by shuffle, diag is the one received a step earlier, and the
+// boundary row gets a parallel row of starts `bst`, written in place like `bnd`. Every lane keeps its best (S, column, start) of
+// row la - 1 (strict '<': its smallest column among equal values), one warp reduction by (S, column) ends the pair. Returns the
+// UNNORMALISED S of the hit (+inf: none) and *span = (start, end). BAND and DIRS must be false.
 // ---------------------------------------------------------------------------------------------------------------
-template <bool BAND, bool DIRS = false>
+template <bool BAND, bool DIRS = false, bool SUBSEQ = false>
 __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__ a, int la, const double* __restrict__ b, int lb, int c,
                                                       double* __restrict__ ring, double* bnd, int lane, uint32_t band,
-                                                      uint64_t* __restrict__ dir = nullptr) {
+                                                      uint64_t* __restrict__ dir = nullptr, uint32_t* bst = nullptr, uint2* span = nullptr) {
+    static_assert(!(SUBSEQ && (BAND || DIRS)), "the subsequence recurrence has no band and no directions");
     if (!la || !lb) return kInf;
     double result = kInf;
+    uint32_t best_col = 0xFFFFFFFFu, best_st = 0xFFFFFFFFu;  // SUBSEQ: the lane's best cell of row la - 1
     const int nstrips = (lb + 31) >> 5;
     const int nsteps = la + 31;
     for (int s = 0; s < nstrips; s++) {
@@ -1052,6 +1060,7 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
 #pragma unroll
         for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = (k < c && colv) ? b[(size_t)col * c + k] : 0.0;
         double cur = kInf, recv_prev = kInf, bl_prev = kInf;
+        uint32_t cur_st = 0, recv_st_prev = 0, bl_st_prev = 0;  // SUBSEQ: the starts of cur, recv_prev, bl_prev
         // at step t0 + r lane j is on row t0 + r - j: row block t0 / 32 - 1 (wprev) or t0 / 32 (wcur)
         uint64_t wprev = 0, wcur = 0;
         const int nrb = (la + 31) >> 5;
@@ -1100,11 +1109,19 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
             // B: steps t0 .. t0 + 31
             const int steps = min(32, nsteps - t0);
             double left_in = (lane == 0 && !first && t0 < la) ? bnd[t0] : kInf;  // D(t, col0 - 1), fetched one step ahead
+            uint32_t left_st_in = 0;
+            if constexpr (SUBSEQ) left_st_in = (lane == 0 && !first && t0 < la) ? bst[t0] : 0u;
             for (int r = 0; r < steps; r++) {
                 const int t = t0 + r;
                 const double recv = __shfl_up_sync(0xffffffffu, cur, 1);  // left neighbour's last cell = D(i, col - 1)
                 const double left_now = left_in;
                 if (r + 1 < steps) left_in = (lane == 0 && !first && t + 1 < la) ? bnd[t + 1] : kInf;
+                uint32_t recv_st = 0, left_st_now = 0;
+                if constexpr (SUBSEQ) {
+                    recv_st = __shfl_up_sync(0xffffffffu, cur_st, 1);
+                    left_st_now = left_st_in;
+                    if (r + 1 < steps) left_st_in = (lane == 0 && !first && t + 1 < la) ? bst[t + 1] : 0u;
+                }
                 const int i = t - lane;
                 const bool active = colv && i >= 0 && i < la;
                 if (active) {
@@ -1112,8 +1129,20 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
                     const double left = lane ? recv : left_now;
                     const double diag = lane ? recv_prev : bl_prev;
                     double m;
-                    if (first && i == 0 && lane == 0) m = 0.0;
-                    else m = fmin(fmin(up, left), diag);
+                    if constexpr (SUBSEQ) {
+                        if (i == 0) {
+                            m = 0.0;
+                            cur_st = (uint32_t)col;
+                        } else {
+                            m = fmin(fmin(up, left), diag);
+                            // align_dir's choice: diag, else up (cur_st stays), else left
+                            if (diag == m) cur_st = lane ? recv_st_prev : bl_st_prev;
+                            else if (!(up == m)) cur_st = lane ? recv_st : left_st_now;
+                        }
+                    } else {
+                        if (first && i == 0 && lane == 0) m = 0.0;
+                        else m = fmin(fmin(up, left), diag);
+                    }
                     if constexpr (DIRS) {
                         const uint64_t bits = align_dir(up, left, diag, m) << (2 * (i & 31));
                         if (i < t0) wprev |= bits;
@@ -1121,11 +1150,17 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
                     }
                     if (BAND && (i < blo || i > bhi)) cur = kInf;
                     else cur = ring[(i & 63) * 32 + lane] + m;
-                    if (last && i == la - 1 && col == lb - 1) result = cur;
-                    if (!last && lane == 31) bnd[i] = cur;  // i = t - 31: behind every row lane 0 still has to read
+                    if constexpr (SUBSEQ) {
+                        if (i == la - 1 && cur < result) result = cur, best_col = (uint32_t)col, best_st = cur_st;
+                        if (!last && lane == 31) bnd[i] = cur, bst[i] = cur_st;
+                    } else {
+                        if (last && i == la - 1 && col == lb - 1) result = cur;
+                        if (!last && lane == 31) bnd[i] = cur;  // i = t - 31: behind every row lane 0 still has to read
+                    }
                 }
                 bl_prev = left_now;
                 recv_prev = recv;
+                if constexpr (SUBSEQ) bl_st_prev = left_st_now, recv_st_prev = recv_st;
             }
             __syncwarp();
             if constexpr (DIRS) {
@@ -1140,6 +1175,15 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
         }
         if (BAND && !last)  // lane 31 stopped at row min(t0, nsteps) - 32
             for (int r = max(0, min(t0, nsteps) - 31) + lane; r < la; r += 32) bnd[r] = kInf;
+    }
+    if constexpr (SUBSEQ) {
+        for (int o = 16; o; o >>= 1) {  // (S, column) minimum; +inf / NaN never entered a lane's best
+            const double od = __shfl_xor_sync(0xffffffffu, result, o);
+            const uint32_t oc = __shfl_xor_sync(0xffffffffu, best_col, o), os = __shfl_xor_sync(0xffffffffu, best_st, o);
+            if (od < result || (od == result && oc < best_col)) result = od, best_col = oc, best_st = os;
+        }
+        *span = make_uint2(best_st, best_col);
+        return result;
     }
     result = __shfl_sync(0xffffffffu, result, (lb - 1) & 31);
     return result / (double)(la + lb);
@@ -1547,6 +1591,88 @@ int dtw_exhaustive_match(ss_dict* d, ss_queries* q, int k, const std::vector<uin
     }
     SS_CUDA(ctx, cudaMemsetAsync(d->d_counters.p, 0, sizeof(unsigned long long), ctx->stream));  // everything is exact now
     SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // `subset` is read by the async copy above
+    return SS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// subsequence DTW (ss_dict_locate, A12 in DESIGN.md §3.1g): every query against every segment, where the query may start and
+// end anywhere in the segment. The exhaustive stage's shape with the SUBSEQ recurrence: one warp per (query, segment) pair
+// writes the pair's unnormalised cost (+inf: no hit) into an f64 table that k_dtw_select_exact reads as it is, and its
+// (start | end << 32) into a parallel u64 table; k_dtw_locate_spans then fills start / end of the selected slots by index.
+// ---------------------------------------------------------------------------------------------------------------
+// pairs of the queries [u0, u0 + nu) x nseg; bnd: one slot of 2 bnd_stride doubles per warp (the D row, then the row of starts).
+// The warp of pair (u, 0) also writes qids[u] = u0 + u, the output row k_dtw_select_exact stores query u of the batch to.
+__global__ void __launch_bounds__(64)
+k_dtw_locate_pairs(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ qmfcc,
+                   const uint64_t* __restrict__ qoff, int c, uint32_t u0, uint32_t nu, uint32_t nseg, double* __restrict__ bnd,
+                   uint32_t bnd_stride, uint32_t* __restrict__ qids, double* __restrict__ cost, uint64_t* __restrict__ span) {
+    __shared__ double ring[2][64 * 32];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t gw = blockIdx.x * 2 + warp, nw = gridDim.x * 2;
+    double* row = bnd + (size_t)gw * 2 * bnd_stride;
+    const uint64_t npairs = (uint64_t)nu * nseg;
+    for (uint64_t t = gw; t < npairs; t += nw) {  // warp-uniform; consecutive warps take consecutive segments of one query
+        const uint32_t u = (uint32_t)(t / nseg), sidx = (uint32_t)(t % nseg);
+        const uint32_t qid = u0 + u;
+        const int la = (int)(qoff[qid + 1] - qoff[qid]), lb = (int)(doff[sidx + 1] - doff[sidx]);
+        uint2 sp = make_uint2(0xFFFFFFFFu, 0xFFFFFFFFu);
+        const double e = warp_dtw_exact_long<false, false, true>(qmfcc + qoff[qid] * c, la, dmfcc + doff[sidx] * c, lb, c, ring[warp], row, lane,
+                                                                 0, nullptr, reinterpret_cast<uint32_t*>(row + bnd_stride), &sp);
+        if (lane == 0) {
+            cost[t] = e;
+            span[t] = (uint64_t)sp.x | (uint64_t)sp.y << 32;
+            if (sidx == 0) qids[u] = qid;
+        }
+    }
+}
+
+// slot s of query u0 + u: (start, end) of the segment k_dtw_select_exact put there; an unfilled slot is (0xFFFFFFFF, 0xFFFFFFFF)
+__global__ void __launch_bounds__(256)
+k_dtw_locate_spans(const uint64_t* __restrict__ span, uint32_t nseg, uint32_t u0, uint32_t nu, int k, uint32_t index_base,
+                   const uint32_t* __restrict__ out_idx, uint32_t* __restrict__ out_start, uint32_t* __restrict__ out_end) {
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= nu * (uint32_t)k) return;
+    const uint32_t u = t / (uint32_t)k;
+    const size_t o = (size_t)u0 * k + t;
+    const uint32_t idx = out_idx[o];
+    const uint64_t sp = idx == 0xFFFFFFFFu ? ~0ull : span[(size_t)u * nseg + (idx - index_base)];
+    if (out_start) out_start[o] = (uint32_t)sp;
+    if (out_end) out_end[o] = (uint32_t)(sp >> 32);
+}
+
+// queries per batch: the two tables take 16 B per pair, at most 256 MB (more only when one query alone needs it)
+static uint32_t locate_batch(uint32_t nq, uint32_t nseg) {
+    return (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(nq, (16ull << 20) / std::max<uint32_t>(nseg, 1)));
+}
+
+int dtw_locate_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, uint32_t* d_out_start, uint32_t* d_out_end, double* d_out_cost) {
+    ss_ctx* ctx = d->ctx;
+    const uint32_t nseg = (uint32_t)d->nseg, nq = (uint32_t)q->nq;
+    if (!nq) return SS_OK;
+    const uint32_t ubatch = locate_batch(nq, nseg);
+    if (!d_out_cost) {  // k_dtw_select_exact always stores costs
+        SS_CUDA(ctx, d->d_locate_cost.reserve((size_t)nq * k));
+        d_out_cost = d->d_locate_cost.p;
+    }
+    SS_CUDA(ctx, d->d_exh_qid.reserve(ubatch));
+    SS_CUDA(ctx, d->d_exh_dist.reserve((size_t)ubatch * nseg));
+    SS_CUDA(ctx, d->d_locate_span.reserve((size_t)ubatch * nseg));
+    const uint32_t stride = (std::max<uint32_t>(q->max_len, 1) + 15) & ~15u;
+    const uint32_t max_ctas = (uint32_t)ctx->sm_count * 6;
+    SS_CUDA(ctx, d->d_rescore_rows.reserve((size_t)max_ctas * 2 * 2 * stride));
+    for (uint32_t u0 = 0; u0 < nq; u0 += ubatch) {
+        const uint32_t nu = std::min(ubatch, nq - u0);
+        const uint64_t npairs = (uint64_t)nu * nseg;
+        k_dtw_locate_pairs<<<(unsigned)std::min<uint64_t>(max_ctas, (npairs + 1) / 2), 64, 0, ctx->stream>>>(
+            d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, u0, nu, nseg, d->d_rescore_rows.p, stride, d->d_exh_qid.p, d->d_exh_dist.p,
+            d->d_locate_span.p);
+        SS_LAUNCHED(ctx);
+        k_dtw_select_exact<<<nu, 256, 0, ctx->stream>>>(d->d_exh_dist.p, nseg, k, d->d_exh_qid.p, d->index_base, d_out_idx, d_out_cost);
+        SS_LAUNCHED(ctx);
+        k_dtw_locate_spans<<<ceil_div((long long)nu * k, 256), 256, 0, ctx->stream>>>(d->d_locate_span.p, nseg, u0, nu, k, d->index_base, d_out_idx,
+                                                                                      d_out_start, d_out_end);
+        SS_LAUNCHED(ctx);
+    }
     return SS_OK;
 }
 

@@ -201,6 +201,11 @@ struct ss_dict {
     ss::DevBuf<double> d_align_q, d_align_dist;
     ss::DevBuf<uint64_t> d_align_qoff, d_align_off;
     ss::DevBuf<uint32_t> d_align_seg, d_align_path;
+    // ss_dict_locate (exact.cu dtw_locate_dev): the (start | end << 32) table beside the cost table d_exh_dist, the costs when
+    // the caller wants none; then the host-buffer entry point's inputs and outputs
+    ss::DevBuf<uint64_t> d_locate_span;
+    ss::DevBuf<double> d_locate_cost;
+    ss::DevBuf<uint32_t> d_locate_idx, d_locate_start, d_locate_end;
     ~ss_dict();
 };
 
@@ -324,6 +329,9 @@ int cosine_walk_dev(ss_dict* d, const double* d_start, const uint64_t* d_start_o
 // hold sum over non-empty queries of (Lq + max(longest segment, 1) - 1) (i, j) pairs.
 int dtw_align_dev(ss_dict* d, const double* d_qmfcc, const uint64_t* d_qoff, const uint64_t* h_qoff, size_t nq, const uint32_t* d_seg_idx,
                   uint32_t* d_out_path, uint64_t* d_out_off, double* d_out_dist);
+// subsequence DTW (A12, DESIGN.md §3.1g): every query of q against every segment, the k best hits by (cost, index); start / end /
+// cost may be NULL. 3 launches per batch of locate_batch(nq, nseg) queries on the ctx stream, no host synchronisation (exact.cu)
+int dtw_locate_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, uint32_t* d_out_start, uint32_t* d_out_end, double* d_out_cost);
 int topk_merge_dev(ss_ctx* ctx, const uint32_t* d_idx, const double* d_dist, int nlists, size_t nq, int k,
                    uint32_t* d_out_idx, double* d_out_dist);
 }  // namespace ss
