@@ -1,10 +1,12 @@
 // examples/reconstruction.cpp — the flow of the reference's examples/reconstruction.rs (and, with --partition-only,
 // examples/partition.rs) written against include/soundsym.hpp:
-//   -s source.wav  -t target.wav  -o out.wav  -m model.bin  [--depth 3] [--threshold 4] [--dtw] [--warp] [--partition-only]
+//   -s source.wav  -t target.wav  -o out.wav  -m model.bin  [--depth 3] [--threshold 4] [--dtw | --dtw-target] [--warp] [--partition-only]
 //   --matcher dict_dir query_dir [--dtw] [--locate]
 // Partitioner::from_path(source).threshold(4).depth(3) -> train (model supplied) -> partition -> SoundDictionary::from_segments
 // -> partition the target with the source's model -> clone_from_dictionary -> to_sound -> write_file. --warp fits every matched
 // sound to its target segment's timing along the DTW warping path (ss_resynth_warped) instead of zero-padding or cutting it.
+// --dtw-target matches in SS_DTW_TARGET mode; with --morph its target distances are DTW distances, spread over the range the
+// flow's own nearest-match distances span.
 // Prints one JSON line with the segment counts, the match indices and checksums so that a test can compare it with the
 // golden fixtures.
 #include <cmath>
@@ -19,7 +21,7 @@ using namespace soundsym;
 int main(int argc, char** argv) {
     std::string src, tgt, out, model_path;
     size_t depth = 3, threshold = 4;  // examples/reconstruction.rs:44-45
-    bool dtw = false, partition_only = false, morph = false, matcher_loop = false, warp = false, locate = false;
+    bool dtw = false, dtw_target = false, partition_only = false, morph = false, matcher_loop = false, warp = false, locate = false;
     size_t chain = 6;
     std::string dict_dir, query_dir, splits_dir;  // --matcher <dictionary dir> <query dir>: the flow of examples/matcher.rs
     for (int i = 1; i < argc; i++) {
@@ -32,6 +34,7 @@ int main(int argc, char** argv) {
         else if (a == "--depth") depth = std::stoul(next());
         else if (a == "--threshold") threshold = std::stoul(next());
         else if (a == "--dtw") dtw = true;
+        else if (a == "--dtw-target") dtw_target = true;
         else if (a == "--warp") warp = true;
         else if (a == "--partition-only") partition_only = true;
         else if (a == "--matcher") dict_dir = next(), query_dir = next();
@@ -118,7 +121,7 @@ int main(int argc, char** argv) {
             return 0;
         }
         auto dictionary = SoundDictionary::from_segments(*source, splits);
-        dictionary->mode = dtw ? SS_DTW : SS_COSINE_REF;
+        dictionary->mode = dtw_target ? SS_DTW_TARGET : (dtw ? SS_DTW : SS_COSINE_REF);
 
         auto target = std::make_shared<Sound>(Sound::from_path(tgt));
         partitioner.sound = target;
@@ -135,11 +138,31 @@ int main(int argc, char** argv) {
             };
             std::vector<double> distances(segments.size());
             for (size_t i = 0; i < distances.size(); i++) distances[i] = -1e-4 + 2e-4 * (double)i / (double)std::max<size_t>(distances.size() - 1, 1);
-            SoundSequence morphed = sequence.morph_to(distances, *dictionary);
             std::vector<double> steps(chain);
             for (size_t i = 0; i < chain; i++) steps[i] = (i % 2 ? -1.0 : 1.0) * 5e-5 * (double)(i + 1) / (double)chain;
+            if (dtw_target) {
+                // DTW distances from [lo, 2 hi], lo / hi the smallest / largest nearest-match distance of the target's segments
+                std::vector<uint32_t> nidx;
+                std::vector<double> ndist;
+                dictionary->match_indices(segments, {}, 1, &nidx, &ndist);
+                double lo = INFINITY, hi = 0.0;
+                for (double v : ndist)
+                    if (std::isfinite(v)) lo = std::min(lo, v), hi = std::max(hi, v);
+                if (!(lo <= hi)) lo = hi = 0.0;
+                for (size_t i = 0; i < distances.size(); i++) distances[i] = lo + (2.0 * hi - lo) * (double)i / (double)std::max<size_t>(distances.size() - 1, 1);
+                for (size_t i = 0; i < chain; i++) steps[i] = lo + (2.0 * hi - lo) * (double)(i + 1) / (double)chain;
+            }
+            SoundSequence morphed = sequence.morph_to(distances, *dictionary);
             SoundSequence chained = SoundSequence::from_distances(steps, segments.at(0), *dictionary);
-            printf("{\"morph\": [");
+            printf("{");
+            if (dtw_target) {
+                printf("\"targets\": [");
+                for (size_t i = 0; i < distances.size(); i++) printf("%s%.17g", i ? "," : "", distances[i]);
+                printf("], \"steps\": [");
+                for (size_t i = 0; i < chain; i++) printf("%s%.17g", i ? "," : "", steps[i]);
+                printf("], ");
+            }
+            printf("\"morph\": [");
             for (size_t i = 0; i < morphed.sounds().size(); i++) printf("%s%lld", i ? "," : "", index_of(morphed.sounds()[i]));
             printf("], \"chain\": [");
             for (size_t i = 1; i < chained.sounds().size(); i++) printf("%s%lld", i > 1 ? "," : "", index_of(chained.sounds()[i]));

@@ -307,7 +307,7 @@ class Sound {
 class SoundDictionary {
    public:
     std::vector<std::shared_ptr<Sound>> sounds;
-    int mode = SS_COSINE_REF;  // SS_DTW selects the DTW extension
+    int mode = SS_COSINE_REF;  // SS_DTW selects the DTW extension, SS_DTW_TARGET its at_distance (the DTW distance closest to a target)
     uint32_t dtw_band = 0;     // Sakoe-Chiba radius of the SS_DTW distance and of align() (ss_dict_set_dtw_band; 0 = no band)
 
     explicit SoundDictionary(Context& ctx = Context::global()) : ctx_(&ctx) {}
@@ -359,7 +359,7 @@ class SoundDictionary {
         return d;
     }
 
-    /// batched at_distance: (indices, distances) for every query; targets empty -> 1.0 (match_sound)
+    /// batched at_distance: (indices, distances) for every query; targets empty -> 1.0 (match_sound), 0.0 in SS_DTW_TARGET mode
     void match_indices(const std::vector<std::shared_ptr<Sound>>& queries, const std::vector<double>& targets, int k, std::vector<uint32_t>* idx,
                        std::vector<double>* dist) {
         ss_dict* d = device();
@@ -430,8 +430,9 @@ class SoundDictionary {
         idx->assign(n, 0), start->assign(n, 0), end->assign(n, 0), cost->assign(n, 0.0);
         ctx_->check(ss_dict_locate(d, flat.data(), off.data(), queries.size(), k, idx->data(), start->data(), end->data(), cost->data()));
     }
-    /// SoundDictionary::match_sound (src/sound.rs:346-348)
-    std::shared_ptr<Sound> match_sound(const std::shared_ptr<Sound>& other) { return at_distance(1.0, other); }
+    /// SoundDictionary::match_sound (src/sound.rs:346-348). The reference's 1.0 is cosine's perfect similarity; in SS_DTW_TARGET
+    /// mode the perfect distance is 0.0, so there match_sound is at_distance(0.0) (the nearest sound, as in SS_DTW).
+    std::shared_ptr<Sound> match_sound(const std::shared_ptr<Sound>& other) { return at_distance(mode == SS_DTW_TARGET ? 0.0 : 1.0, other); }
     Context& context() const { return *ctx_; }
 
    private:
@@ -518,7 +519,8 @@ class SoundSequence {
         return SoundSequence(std::move(out), *ctx_);
     }
     /// SoundSequence::from_distances (src/sound.rs:405-417): a chain, step t matches the sound step t - 1 returned.
-    /// SS_COSINE_REF runs it on the device in one call; SS_DTW (whose at_distance ignores the target) keeps the nq = 1 loop.
+    /// SS_COSINE_REF runs it on the device in one call; the DTW modes keep the nq = 1 loop (SS_DTW's at_distance ignores the
+    /// target, SS_DTW_TARGET's takes it).
     static SoundSequence from_distances(const std::vector<double>& distances, std::shared_ptr<Sound> start, SoundDictionary& dict) {
         std::vector<std::shared_ptr<Sound>> sounds{std::move(start)};
         if (!distances.empty() && dict.mode == SS_COSINE_REF) {

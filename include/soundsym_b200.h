@@ -49,7 +49,8 @@ typedef enum ss_status {
 
 typedef enum ss_match_mode {
     SS_COSINE_REF = 0, /* the reference's matcher: cosine_sim + at_distance, src/sound.rs:23-38, 351-370 (bit-exact f64) */
-    SS_DTW = 1         /* north-star extension (no reference counterpart): DTW, spec in oracle/ASSUMPTIONS.h A8 */
+    SS_DTW = 1,        /* north-star extension (no reference counterpart): DTW, spec in oracle/ASSUMPTIONS.h A8 */
+    SS_DTW_TARGET = 2  /* at_distance with the DTW distance: the k sounds whose SS_DTW distance is closest to a target (A13) */
 } ss_match_mode;
 
 typedef struct ss_ctx ss_ctx;         /* device + stream + workspace */
@@ -142,7 +143,14 @@ int ss_partition(ss_ctx* ctx, const double* mfcc, size_t frames, const ss_gmm* m
  * ss_dict_match    SoundDictionary::at_distance (src/sound.rs:351-370) for a batch of queries; targets == NULL means
  *                  1.0 = match_sound (src/sound.rs:346-348). SS_COSINE_REF: k must be 1, out_dist = |sim - target|
  *                  (2.0 and index index_base if nothing is < 2.0, as the reference's fold). SS_DTW: the k best
- *                  (distance, index) ascending, ties to the lowest index; unfilled slots (inf, 0xFFFFFFFF).
+ *                  (distance, index) ascending, ties to the lowest index; unfilled slots (inf, 0xFFFFFFFF); targets are
+ *                  ignored. SS_DTW_TARGET (spec A13, DESIGN.md §3.1h): with D the SS_DTW distance of the pair (its recurrence,
+ *                  normalisation, band and NaN rule) and t the query's target, the key is e = fabs(D - t) in f64; the k best
+ *                  (e, index) ascending, ties to the lowest index, out_dist = e (as SS_COSINE_REF's |sim - target|), unfilled
+ *                  slots (inf, 0xFFFFFFFF), k in 1..SS_MAX_TOPK. targets == NULL means t = 0 for every query, and then the
+ *                  results equal SS_DTW's bit for bit. A non-finite target -> SS_ERR_INVALID (the _dev entry points take
+ *                  finite targets as a precondition). The ss_dict_last_* readers describe the match as for SS_DTW; the
+ *                  ss_dict_set_scan preference does not apply (the match always starts at the fp32 CUDA-core scan).
  *                  out_idx / out_dist: nq x k.
  * ss_queries_*     the same in two steps with the queries kept in HBM (bench.py's kernel-only number; multi-GPU).
  * ss_topk_merge_dev merges `nlists` per-shard results (as gathered from all ranks, list-major [nlists][nq][k]) into the
@@ -164,7 +172,7 @@ void ss_queries_destroy(ss_queries* q);
  * fallback stage (fp32 scan / exhaustive f64) is only known once the refine has run, so the results in d_out_* are final after
  * ss_dict_match_finish(dict) - which waits for that one event and, in the rare case, runs the fallback for the queries
  * concerned. The ss_dict_last_* readers, the next match on the same dictionary and ss_dict_match_sharded* call it
- * themselves; `q` must stay alive until then. */
+ * themselves; `q` must stay alive until then, and so must SS_DTW_TARGET's d_targets (nq finite f64, or NULL). */
 int ss_dict_match_dev(ss_dict* dict, ss_queries* q, int mode, const double* d_targets, int k, uint32_t* d_out_idx,
                       double* d_out_dist);
 int ss_dict_match_finish(ss_dict* dict);

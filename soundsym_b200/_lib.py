@@ -10,7 +10,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SS_B200_LIB") or os.path.join(_HERE, "libsoundsym_b200.so")  # override: development A/B builds
 
 SS_OK, SS_ERR_INVALID, SS_ERR_CUDA, SS_ERR_NOMEM, SS_ERR_NOT_TRAINED, SS_ERR_EMPTY_DICT, SS_ERR_TOO_FEW_ROWS = 0, -1, -2, -3, -4, -5, -6
-SS_COSINE_REF, SS_DTW = 0, 1
+SS_COSINE_REF, SS_DTW, SS_DTW_TARGET = 0, 1, 2
 SS_MAX_TOPK = 8
 SS_COMM_ID_BYTES = 128
 

@@ -16,7 +16,7 @@ import struct
 import numpy as np
 
 from . import _lib
-from ._lib import SS_COSINE_REF, SS_DTW, SoundsymError
+from ._lib import SS_COSINE_REF, SS_DTW, SS_DTW_TARGET, SoundsymError
 
 NCOEFFS, NCLUSTERS, HOP, BIN = 12, 26, 256, 1024  # src/lib.rs:22-25
 
@@ -637,7 +637,8 @@ def _read_wav_pcm(path):
 
 
 class SoundDictionary:
-    """src/sound.rs:288-371. `mode` selects the matcher: SS_COSINE_REF is the reference's, SS_DTW the extension.
+    """src/sound.rs:288-371. `mode` selects the matcher: SS_COSINE_REF is the reference's, SS_DTW the extension, and
+    SS_DTW_TARGET the extension's at_distance: the sounds whose SS_DTW distance is closest to each target (A13).
     `dtw_band`: Sakoe-Chiba radius of the SS_DTW distance and of align() (0 = no band; ss_dict_set_dtw_band)."""
 
     def __init__(self, ctx=None, mode=SS_COSINE_REF, dtw_band=0):
@@ -748,8 +749,9 @@ class SoundDictionary:
         return self.sounds[int(idx[0, 0])]
 
     def match_sound(self, other):
-        """src/sound.rs:346-348."""
-        return self.at_distance(1.0, other)
+        """src/sound.rs:346-348. The reference's 1.0 is cosine's perfect similarity; in SS_DTW_TARGET mode the perfect
+        distance is 0.0, so there match_sound is at_distance(0.0) (the nearest sound, as in SS_DTW)."""
+        return self.at_distance(0.0 if self.mode == SS_DTW_TARGET else 1.0, other)
 
 
 class SoundSequence:
@@ -848,7 +850,8 @@ class SoundSequence:
     @classmethod
     def from_distances(cls, distances, start, dictionary):
         """src/sound.rs:405-417: a chain, step t matches the sound step t - 1 returned. SS_COSINE_REF runs it on the device
-        in one call (ss_dict_walk); in SS_DTW mode at_distance ignores the target, so that mode keeps the nq = 1 loop."""
+        in one call (ss_dict_walk); the DTW modes keep the nq = 1 loop (SS_DTW's at_distance ignores the target,
+        SS_DTW_TARGET's takes it)."""
         sounds = [start]
         distances = list(distances)
         if distances and dictionary.mode == SS_COSINE_REF:

@@ -70,6 +70,13 @@ int queries_check(ss_ctx* ctx, const double* q_mfcc, const uint64_t* q_frame_off
     return SS_OK;
 }
 
+// SS_DTW_TARGET's host-buffer targets: every one finite (the _dev entry points take that as a precondition)
+int targets_check(ss_ctx* ctx, int mode, const double* targets, size_t nq) {
+    if (mode != SS_DTW_TARGET || !targets) return SS_OK;
+    for (size_t i = 0; i < nq; i++)
+        if (!std::isfinite(targets[i])) return set_error(ctx, SS_ERR_INVALID, "targets[%zu] = %g is not finite", i, targets[i]);
+    return SS_OK;
+}
 
 }  // namespace ss
 
@@ -265,6 +272,7 @@ int ss_dict_match_dev(ss_dict* d, ss_queries* q, int mode, const double* d_targe
         return cosine_match_dev(d, q, d_targets, d_out_idx, d_out_dist);
     }
     if (mode == SS_DTW) return dtw_match_dev(d, q, k, d_out_idx, d_out_dist);
+    if (mode == SS_DTW_TARGET) return dtw_match_dev(d, q, k, d_out_idx, d_out_dist, /*target=*/true, d_targets);
     return set_error(ctx, SS_ERR_INVALID, "unknown match mode %d", mode);
 }
 
@@ -276,6 +284,7 @@ int ss_dict_match(ss_dict* d, const double* q_mfcc, const uint64_t* q_frame_offs
     if (k < 1 || k > SS_MAX_TOPK) return set_error(ctx, SS_ERR_INVALID, "k must be in 1..%d (got %d)", SS_MAX_TOPK, k);
     if (nq && (!out_idx || !out_dist)) return set_error(ctx, SS_ERR_INVALID, "output pointers are NULL");
     SS_TRY(queries_check(ctx, q_mfcc, q_frame_offsets, nq, d->c));
+    SS_TRY(targets_check(ctx, mode, targets, nq));
     SS_CUDA(ctx, cudaSetDevice(ctx->device));
     if (!d->scratch_q) {
         d->scratch_q = new (std::nothrow) ss_queries();
@@ -291,7 +300,7 @@ int ss_dict_match(ss_dict* d, const double* q_mfcc, const uint64_t* q_frame_offs
         tt.lap("ss_dict_match: queries_fill");
         SS_CUDA(ctx, d->d_res_idx.reserve(nq * (size_t)k));
         SS_CUDA(ctx, d->d_res_dist.reserve(nq * (size_t)k));
-        const bool use_targets = targets && mode == SS_COSINE_REF;
+        const bool use_targets = targets && (mode == SS_COSINE_REF || mode == SS_DTW_TARGET);
         if (use_targets) SS_TRY(upload(ctx, d->d_res_targets, targets, nq));
         SS_TRY(ss_dict_match_dev(d, q, mode, use_targets ? d->d_res_targets.p : nullptr, k, d->d_res_idx.p, d->d_res_dist.p));
         tt.lap("ss_dict_match: first stage");
@@ -304,7 +313,7 @@ int ss_dict_match(ss_dict* d, const double* q_mfcc, const uint64_t* q_frame_offs
                 SS_CUDA(ctx, cudaMemcpyAsync(out_dist, d->d_res_dist.p, nq * (size_t)k * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
             }
             SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-            if (pass || mode != SS_DTW) break;
+            if (pass || mode == SS_COSINE_REF) break;
             SS_TRY(dtw_match_finish(d));
             if (!d->last_tc_fallback && !d->last_exhaustive) break;
         }

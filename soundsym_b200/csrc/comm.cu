@@ -356,6 +356,7 @@ int ss_dict_match_sharded(ss_dict* d, ss_comm* cm, const double* q_mfcc, const u
     if (mode == SS_COSINE_REF && k != 1) return set_error(ctx, SS_ERR_INVALID, "SS_COSINE_REF returns one match per query (k must be 1, got %d)", k);
     if (nq && (!out_idx || !out_dist)) return set_error(ctx, SS_ERR_INVALID, "output pointers are NULL");
     SS_TRY(queries_check(ctx, q_mfcc, q_frame_offsets, nq, d->c));
+    SS_TRY(targets_check(ctx, mode, targets, nq));
     SS_CUDA(ctx, cudaSetDevice(ctx->device));
     if (!cm->scratch_q) {
         cm->scratch_q = new (std::nothrow) ss_queries();
@@ -369,7 +370,7 @@ int ss_dict_match_sharded(ss_dict* d, ss_comm* cm, const double* q_mfcc, const u
         SS_TRY(queries_fill_sharded(cm, q, q_mfcc, q_frame_offsets, nq));
         SS_CUDA(ctx, cm->d_out_idx.reserve(std::max<size_t>(nq * (size_t)k, 1)));
         SS_CUDA(ctx, cm->d_out_dist.reserve(std::max<size_t>(nq * (size_t)k, 1)));
-        const bool use_targets = targets && mode == SS_COSINE_REF;
+        const bool use_targets = targets && (mode == SS_COSINE_REF || mode == SS_DTW_TARGET);
         if (use_targets) SS_TRY(upload(ctx, cm->d_targets, targets, nq));
         SS_TRY(match_sharded_dev(d, cm, q, mode, use_targets ? cm->d_targets.p : nullptr, k, cm->d_out_idx.p, cm->d_out_dist.p));
         if (nq) {

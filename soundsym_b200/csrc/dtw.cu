@@ -13,6 +13,8 @@
 //   3. k_dtw_rescore_warp  f64, direct (a-b)^2, unfused — the oracle's arithmetic — on the KP candidates only.
 //   4. k_dtw_finalize sorts by (distance, index), writes the top-k, and certifies that no pair outside the candidate
 //                     list could have entered it given the scan's error bound.
+// SS_DTW_TARGET (DESIGN.md §3.1h) runs the same four steps with the scan's TARGET form: it keeps the pairs of smallest
+// lower bound on e = |D - t| instead of smallest scan distance, under the dictionary's band, and 3. / 4. rank by exact e.
 #include <algorithm>
 #include <cmath>
 #include <numeric>
@@ -155,12 +157,39 @@ struct ScanParams {
     float* scratch;               // per CTA: scratch_rows x 128 floats (strip boundary columns of multi-strip segments)
     uint32_t scratch_rows;
 };
+// what the TARGET scans (SS_DTW_TARGET) read besides: the targets in the caller's query order (NULL: t = 0), the lanes' query
+// ids, the batch's and the shard's largest frame norms (the per-cell error of E), the Sakoe-Chiba radius (0: no band)
+struct ScanTarget {
+    const double* targets;
+    const uint32_t* group_qid;
+    const float* max_na;
+    const float* max_nb;
+    uint32_t band;
+};
+
+// The TARGET scan's key of a pair (DESIGN.md §3.1h): a lower bound on e = |D - t| for a pair of ncells = Lq + Ld - 1 path cells
+// at most whose scan distance is s, max(0, |s - t| - E), E = (g |s| + (1 + g) ec) / (1 - g) with g = gamma_{ncells+1} of fp32 and
+// ec = kScanCellEps (max|a|^2 + max|b|^2) the error of one computed local cost. The f64 evaluation of E is covered by the factor
+// 1.001, |s - t| and the subtraction of E round down, and so does the conversion to float. A NaN / inf scan distance stays what it
+// is: such a pair is never a candidate, as in SS_DTW.
+constexpr double kScanCellEps = 4e-6;
+__device__ __forceinline__ float target_key(float s, double t, double ec, uint32_t ncells) {
+    const double sd = (double)s;
+    if (!(fabs(sd) < __longlong_as_double(0x7ff0000000000000ll))) return s;
+    const double nu = (double)(ncells + 1) * 0x1p-24, g = nu / (1.0 - nu);
+    const double e = 1.001 * (g * fabs(sd) + (1.0 + g) * ec) / (1.0 - g);
+    const double lo = __dsub_rd(sd >= t ? __dsub_rd(sd, t) : __dsub_rd(t, sd), e);
+    return lo > 0.0 ? __double2float_rd(lo) : 0.f;
+}
 
 constexpr int kTileFloats = kTileFrames * kSlots;
 constexpr int kScanSmemBytes = kStages * kTileFloats * 4 + kStages * 8 + kStages * 4 + 4;
 
-template <int RB, int KP>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, RB <= 2 ? 4 : 3) k_dtw_scan(const ScanParams p) {
+// TARGET: the SS_DTW_TARGET form. Each lane reads its query's target; a pair's key is target_key, not the scan distance, and
+// under a band (p.band != 0) cells outside it are +inf by one 64-bit integer test per cell (A10's rule, warp-uniform: the
+// lanes of a warp share Lq and the segment).
+template <int RB, int KP, bool TARGET = false>
+__global__ void __launch_bounds__(kWarpsPerCta * 32, RB <= 2 ? 4 : 3) k_dtw_scan(const ScanParams p, const ScanTarget tg) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     float* stage_buf = reinterpret_cast<float*>(smem_raw);
     uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + kStages * kTileFloats * 4);
@@ -201,6 +230,13 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, RB <= 2 ? 4 : 3) k_dtw_scan
     uint32_t ki[KP];
 #pragma unroll
     for (int s = 0; s < KP; s++) kd[s] = INF, ki[s] = 0xFFFFFFFFu;
+    double tq = 0.0, ec = 0.0;
+    uint32_t col_next = 0;  // TARGET: the first column of the segment's next strip
+    if constexpr (TARGET) {
+        const uint32_t qid = tg.group_qid[g * 32 + lane];
+        tq = (tg.targets && qid != 0xFFFFFFFFu) ? tg.targets[qid] : 0.0;
+        ec = kScanCellEps * ((double)tg.max_na[0] + (double)tg.max_nb[0]);
+    }
 
     for (uint32_t t = t0; t < t1; ++t) {
         const uint32_t n = t - t0;
@@ -214,6 +250,18 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, RB <= 2 ? 4 : 3) k_dtw_scan
             const int len = sd.z & 0xFFFF;
             const bool first = (sd.z >> 16) & 1, last = (sd.z >> 17) & 1;
             const float* bs = sb + ((uint32_t)sd.x - (uint32_t)td.x) * kSlots;
+            // TARGET under a band: cell (i, col0 + j) is inside iff |i A - (col0 + j) B| <= bw (band_rows' test)
+            long long bA = 0, bB = 0, bw = 0;
+            uint32_t col0 = 0;
+            bool banded = false;
+            if constexpr (TARGET) {
+                col0 = first ? 0 : col_next;
+                col_next = col0 + (uint32_t)len;
+                banded = tg.band != 0;
+                bA = (long long)sd.w - 1, bB = (long long)Lq - 1;
+                const long long lmax = max((long long)Lq, (long long)sd.w);
+                bw = min((long long)tg.band, lmax) * max(bA, bB);
+            }
 
             float dprev[kStrip];
 #pragma unroll
@@ -266,7 +314,13 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, RB <= 2 ? 4 : 3) k_dtw_scan
                             acc = ffma2(a[r][6], b3, acc);  // (a_12 b_12, 1 * |b|^2)
                             const float c = lo32(acc) + hi32(acc);
                             const float m = min3f(leftv[r], upv, diag);
-                            const float cur = c + m;
+                            float cur = c + m;
+                            if constexpr (TARGET) {
+                                if (banded) {
+                                    const long long x = (long long)(i0 + r) * bA - (long long)(col0 + j) * bB;
+                                    if (x < -bw || x > bw) cur = INF;
+                                }
+                            }
                             diag = leftv[r];
                             leftv[r] = cur;
                             upv = cur;
@@ -286,7 +340,8 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, RB <= 2 ? 4 : 3) k_dtw_scan
 #pragma unroll
                 for (int r = 1; r < RB; r++)
                     if (r == rstar) res = leftv[r];
-                const float dist = res * (1.0f / (float)(Lq + (uint32_t)sd.w));
+                float dist = res * (1.0f / (float)(Lq + (uint32_t)sd.w));
+                if constexpr (TARGET) dist = target_key(dist, tq, ec, Lq + (uint32_t)sd.w - 1);
                 if (dist < kd[KP - 1]) {
                     kd[KP - 1] = dist;
                     ki[KP - 1] = (uint32_t)sd.y;
@@ -363,14 +418,12 @@ __global__ void k_dtw_merge(const unsigned long long* __restrict__ partial, uint
 
 // exact f64 kernels live in exact.cu (compiled with --fmad=false)
 namespace ss {
-int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, double eps,
-                         const float* d_max_na, const float* d_max_nb, const float* d_slot_max_na, int bound_mode, uint8_t* d_uncert_flag,
-                         uint32_t* d_out_idx, double* d_out_dist);
 bool dtw_tc_applies(const ss_dict* d, const ss_queries* q);
 int dtw_tc_match_dev(ss_dict* d, ss_queries* q, int k, bool timed, uint32_t* d_out_idx, double* d_out_dist);
 bool dtw_h2_applies(const ss_dict* d, const ss_queries* q);
 int dtw_h2_match_dev(ss_dict* d, ss_queries* q, int k, bool wide, bool second_chance, bool timed, uint32_t* d_out_idx, double* d_out_dist);
-int dtw_exhaustive_match(ss_dict* d, ss_queries* q, int k, const std::vector<uint32_t>& subset, uint32_t* d_out_idx, double* d_out_dist);
+int dtw_exhaustive_match(ss_dict* d, ss_queries* q, int k, const std::vector<uint32_t>& subset, uint32_t* d_out_idx, double* d_out_dist,
+                         bool target = false, const double* d_targets = nullptr);
 }
 
 namespace ss {
@@ -486,12 +539,12 @@ int dtw_queries_build(ss_queries* q) {
 constexpr int kScanRB = 4;     // query rows per pass of k_dtw_scan (DESIGN.md §3.1c)
 constexpr int kScanWaves = 8;  // the fp32 scan's grid: about this many waves at 4 CTAs / SM
 
-template <int KP>
-static int launch_scan_merge(ss_dict* d, const ScanParams& p, uint32_t grid, uint32_t nslots, bool timed) {
+template <int KP, bool TARGET>
+static int launch_scan_merge(ss_dict* d, const ScanParams& p, const ScanTarget& tg, uint32_t grid, uint32_t nslots, bool timed) {
     ss_ctx* ctx = d->ctx;
     if (timed) SS_CUDA(ctx, cudaEventRecord(d->ev_scan0, ctx->stream));
-    SS_CUDA(ctx, cudaFuncSetAttribute(k_dtw_scan<kScanRB, KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, kScanSmemBytes));
-    k_dtw_scan<kScanRB, KP><<<grid, kWarpsPerCta * 32, kScanSmemBytes, ctx->stream>>>(p);
+    SS_CUDA(ctx, cudaFuncSetAttribute(k_dtw_scan<kScanRB, KP, TARGET>, cudaFuncAttributeMaxDynamicSharedMemorySize, kScanSmemBytes));
+    k_dtw_scan<kScanRB, KP, TARGET><<<grid, kWarpsPerCta * 32, kScanSmemBytes, ctx->stream>>>(p, tg);
     SS_LAUNCHED(ctx);
     if (timed) {
         SS_CUDA(ctx, cudaEventRecord(d->ev_scan1, ctx->stream));
@@ -502,8 +555,10 @@ static int launch_scan_merge(ss_dict* d, const ScanParams& p, uint32_t grid, uin
     return SS_OK;
 }
 
-// the fp32 CUDA-core scan of batch q, its f64 refine and certification (any sequence length)
-static int dtw_fp32_match(ss_dict* d, ss_queries* q, int k, bool timed, uint32_t* d_out_idx, double* d_out_dist) {
+// the fp32 CUDA-core scan of batch q, its f64 refine and certification (any sequence length). target: the SS_DTW_TARGET form,
+// d_targets in q's order (NULL: t = 0)
+static int dtw_fp32_match(ss_dict* d, ss_queries* q, int k, bool timed, uint32_t* d_out_idx, double* d_out_dist, bool target = false,
+                          const double* d_targets = nullptr) {
     ss_ctx* ctx = d->ctx;
     SS_TRY(dtw_queries_build(q));
     const int kp = k <= 2 ? 4 : (k <= 6 ? 8 : 16);  // candidates kept per query by the scan
@@ -555,17 +610,19 @@ static int dtw_fp32_match(ss_dict* d, ss_queries* q, int k, bool timed, uint32_t
             SS_CUDA(ctx, d->d_scratch.reserve((size_t)grid * p.scratch_rows * 128));
             p.scratch = d->d_scratch.p;
         }
+        const ScanTarget tg = {d_targets, q->d_group_qid.p, q->d_max_norm.p, d->d_max_norm.p, d->dtw_band};
         if (!d->ev_scan0) {
             SS_CUDA(ctx, cudaEventCreate(&d->ev_scan0));
             SS_CUDA(ctx, cudaEventCreate(&d->ev_scan1));
         }
-        if (kp == 4) SS_TRY(launch_scan_merge<4>(d, p, grid, nslots, timed));
-        else if (kp == 8) SS_TRY(launch_scan_merge<8>(d, p, grid, nslots, timed));
-        else SS_TRY(launch_scan_merge<16>(d, p, grid, nslots, timed));
+        if (kp == 4) SS_TRY((target ? launch_scan_merge<4, true> : launch_scan_merge<4, false>)(d, p, tg, grid, nslots, timed));
+        else if (kp == 8) SS_TRY((target ? launch_scan_merge<8, true> : launch_scan_merge<8, false>)(d, p, tg, grid, nslots, timed));
+        else SS_TRY((target ? launch_scan_merge<16, true> : launch_scan_merge<16, false>)(d, p, tg, grid, nslots, timed));
     }
-    // fp32 scan: |error| of a normalised distance <= 4e-6 (max|a|^2 + max|b|^2)  (14 roundings of 2^-24 on terms <= 2(|a|^2+|b|^2))
+    // fp32 scan: |error| of a normalised distance <= 4e-6 (max|a|^2 + max|b|^2)  (14 roundings of 2^-24 on terms <= 2(|a|^2+|b|^2);
+    // the running sum along the path is not counted: DESIGN.md §3.1h). The TARGET keys carry their own bound.
     return dtw_rescore_finalize(d, q, k, kp, nslots, q->d_group_qid.p, 4e-6, q->d_max_norm.p, d->d_max_norm.p, nullptr, 0, q->d_uncert_flag.p,
-                                d_out_idx, d_out_dist);
+                                d_out_idx, d_out_dist, target, d_targets);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -689,21 +746,26 @@ static int read_uncertified(ss_dict* d, const ss_queries* ran, const std::vector
     return SS_OK;
 }
 
-int dtw_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist) {
+// target (SS_DTW_TARGET, DESIGN.md §3.1h): the cascade is FP32 -> EXHAUSTIVE, the scan's TARGET form first whatever ss_dict_set_scan
+// chose (the tensor-core scans' bounds are one-sided or too wide); d_targets (q's order, NULL: t = 0) is read until dtw_match_finish.
+int dtw_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist, bool target, const double* d_targets) {
     ss_ctx* ctx = d->ctx;
     if (k < 1 || k > SS_MAX_TOPK) return set_error(ctx, SS_ERR_INVALID, "k must be in 1..%d (got %d)", SS_MAX_TOPK, k);
     SS_TRY(dtw_match_finish(d));  // the previous match shares this dictionary's workspaces
     SS_CUDA(ctx, q->d_uncert_flag.reserve(std::max<size_t>(q->nq, 1)));
     SS_CUDA(ctx, cudaMemsetAsync(q->d_uncert_flag.p, 0, std::max<size_t>(q->nq, 1), ctx->stream));
-    const DtwStage first = first_stage(d, q);
+    const DtwStage first = target ? DtwStage::FP32 : first_stage(d, q);
     d->last_scan_kind = first == DtwStage::H2 ? 1 : (first == DtwStage::TC ? 2 : 3);
     d->last_work = d->total_frames * q->total_frames;
     d->last_tc_fallback = 0;
     d->last_exhaustive = 0;
     d->last_uncertified = q->nq;  // no row is final before dtw_match_finish
-    SS_TRY(run_stage(d, q, k, first, /*timed=*/true, d_out_idx, d_out_dist));
+    if (target) SS_TRY(dtw_fp32_match(d, q, k, /*timed=*/true, d_out_idx, d_out_dist, true, d_targets));
+    else SS_TRY(run_stage(d, q, k, first, /*timed=*/true, d_out_idx, d_out_dist));
     SS_TRY(post_counters(d));
     d->pending.active = true;
+    d->pending.target = target;
+    d->pending.d_targets = d_targets;
     d->pending.first = first;
     d->pending.q = q;
     d->pending.k = k;
@@ -785,7 +847,7 @@ static int run_later_stages(ss_dict* d) {
     while (!u.empty()) {
         if (s == DtwStage::FP32 || exhaustive_is_cheaper(d, ran_max_len, q, u)) {
             d->last_exhaustive += u.size();
-            SS_TRY(dtw_exhaustive_match(d, q, k, u, out_idx, out_dist));
+            SS_TRY(dtw_exhaustive_match(d, q, k, u, out_idx, out_dist, d->pending.target, d->pending.d_targets));
             u.clear();
             trace(DtwStage::EXHAUSTIVE);
             break;

@@ -49,10 +49,6 @@
 
 namespace ss {
 
-int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, double eps,
-                         const float* d_max_na, const float* d_max_nb, const float* d_slot_max_na, int bound_mode, uint8_t* d_uncert_flag,
-                         uint32_t* d_out_idx, double* d_out_dist);
-
 int dtw_second_chance(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, const unsigned long long* d_partial,
                       uint32_t nlists, const unsigned long long* d_thr, double eps, const float* d_max_na, const float* d_max_nb,
                       const float* d_slot_max_na, int bound_mode, uint8_t* d_uncert_flag, uint32_t* d_out_idx, double* d_out_dist);

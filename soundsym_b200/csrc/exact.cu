@@ -1190,12 +1190,14 @@ __device__ __forceinline__ double warp_dtw_exact_long(const double* __restrict__
 }
 
 // one WARP per (slot, candidate) pair (grid-stride over the pairs; bnd: one row of bnd_stride doubles per warp)
-template <bool BAND>
+// TARGET (SS_DTW_TARGET, DESIGN.md §3.1h): `exact` holds e = |D - t| (targets in the caller's query order, NULL: t = 0), and a
+// candidate's key is already a lower bound on its e, compared with the k-th exact e as it is.
+template <bool BAND, bool TARGET = false>
 __global__ void __launch_bounds__(64)
 k_dtw_rescore_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const double* __restrict__ qmfcc,
                    const uint64_t* __restrict__ qoff, int c, const uint32_t* __restrict__ group_qid, const uint32_t* __restrict__ cand_idx,
                    uint32_t nt, int kp, int s_begin, int s_count, RescoreBound rb, double* __restrict__ bnd, uint32_t bnd_stride,
-                   double* __restrict__ exact, unsigned long long* __restrict__ counters, uint32_t band) {
+                   double* __restrict__ exact, unsigned long long* __restrict__ counters, uint32_t band, const double* __restrict__ targets) {
     __shared__ double ring[2][64 * 32];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t gw = blockIdx.x * 2 + warp, nw = gridDim.x * 2;
@@ -1217,14 +1219,17 @@ k_dtw_rescore_warp(const double* __restrict__ dmfcc, const uint64_t* __restrict_
                 kth = fmax(kth, e);
             }
             const double na = rb.slot_max_na ? (double)rb.slot_max_na[slot] : (double)rb.max_na[0];
-            if (scan_lower_bound(rb.cand_adist[pair], na, (double)rb.max_nb[0], rb.eps, rb.bound_mode, la, rb.inv_s, rb.ld_max) > kth) {
+            const double lower = TARGET ? (double)rb.cand_adist[pair]
+                                        : scan_lower_bound(rb.cand_adist[pair], na, (double)rb.max_nb[0], rb.eps, rb.bound_mode, la, rb.inv_s, rb.ld_max);
+            if (lower > kth) {
                 if (lane == 0) exact[pair] = kInf;  // provably outside the top-k
                 continue;
             }
             if (lane == 0) atomicAdd(&counters[1], 1ull);
         }
-        const double e =
+        double e =
             warp_dtw_exact_long<BAND>(qmfcc + qoff[qid] * c, la, dmfcc + doff[idx] * c, lb, c, ring[warp], bnd + (size_t)gw * bnd_stride, lane, band);
+        if constexpr (TARGET) e = fabs(e - (targets ? targets[qid] : 0.0));
         if (lane == 0) exact[pair] = e;
     }
 }
@@ -1428,6 +1433,9 @@ int dtw_second_chance(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots,
     return SS_OK;
 }
 
+// TARGET: `exact` holds e = |D - t| and the candidate keys are lower bounds on e (the SS_DTW_TARGET scan): the list's worst key
+// bounds every pair outside it, with the same strict rule
+template <bool TARGET = false>
 __global__ void k_dtw_finalize(const uint32_t* __restrict__ cand_idx, const float* __restrict__ cand_adist,
                                const double* __restrict__ exact, const uint32_t* __restrict__ group_qid, uint32_t nslots, int kp,
                                int k, uint32_t index_base, const float* __restrict__ max_na, const float* __restrict__ max_nb, double eps,
@@ -1458,12 +1466,13 @@ __global__ void k_dtw_finalize(const uint32_t* __restrict__ cand_idx, const floa
     const float worst = cand_adist[(size_t)slot * kp + kp - 1];
     bool uncertified = false;
     // (bound_mode 2 / 3: a list that is not full does NOT mean every pair is in it - an overflowed pair reads +inf)
-    if (bound_mode >= 2 || worst < __int_as_float(0x7f800000)) {
+    if ((!TARGET && bound_mode >= 2) || worst < __int_as_float(0x7f800000)) {
         const double kth = n >= k ? dv[k - 1] : kInf;
         const double na = slot_max_na ? (double)slot_max_na[slot] : (double)max_na[0];
         const double nb = (double)max_nb[0];
         double lower;
-        lower = scan_lower_bound(worst, na, nb, eps, bound_mode, (int)(qoff[qid + 1] - qoff[qid]), inv_s, ld_max);
+        if constexpr (TARGET) lower = (double)worst;
+        else lower = scan_lower_bound(worst, na, nb, eps, bound_mode, (int)(qoff[qid + 1] - qoff[qid]), inv_s, ld_max);
         uncertified = !(lower > kth);
         if (uncertified) atomicAdd(&counters[0], 1ull);
     }
@@ -1472,7 +1481,7 @@ __global__ void k_dtw_finalize(const uint32_t* __restrict__ cand_idx, const floa
 
 int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, double eps,
                          const float* d_max_na, const float* d_max_nb, const float* d_slot_max_na, int bound_mode, uint8_t* d_uncert_flag,
-                         uint32_t* d_out_idx, double* d_out_dist) {
+                         uint32_t* d_out_idx, double* d_out_dist, bool target, const double* d_targets) {
     ss_ctx* ctx = d->ctx;
     // queries without a frame never reach a slot: their rows keep (inf, 0xFFFFFFFF). Only launched when such queries exist.
     if (q->nq && q->nonempty < q->nq) {
@@ -1483,7 +1492,7 @@ int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslo
     SS_CUDA(ctx, d->d_counters.reserve(4));
     SS_CUDA(ctx, cudaMemsetAsync(d->d_counters.p, 0, 4 * sizeof(unsigned long long), ctx->stream));
     if (!nslots || !d->ntiles) return SS_OK;
-    if (d->max_len <= 32 && q->max_len <= 32) {  // one warp per query slot does the whole refine
+    if (!target && d->max_len <= 32 && q->max_len <= 32) {  // one warp per query slot does the whole refine
         (d->dtw_band ? k_dtw_refine_warp<true> : k_dtw_refine_warp<false>)<<<ceil_div(nslots, 4), 128, 0, ctx->stream>>>(
             d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d_slot_qid, d->d_cand_idx.p, d->d_cand_adist.p, nslots, kp, std::min(k, kp),
             d->index_base, d_max_na, d_max_nb, eps, d_slot_max_na, bound_mode, d->h2_bound_inv_s, d_uncert_flag, d_out_idx, d_out_dist,
@@ -1502,12 +1511,14 @@ int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslo
         RescoreBound rb = {phase ? d->d_cand_adist.p : nullptr, d_max_na, d_max_nb, d_slot_max_na, eps, bound_mode, std::min(k, kp), d->h2_bound_inv_s,
                            (int)d->max_len};
         const uint32_t nt = nslots * (uint32_t)s_count;
-        (d->dtw_band ? k_dtw_rescore_warp<true> : k_dtw_rescore_warp<false>)<<<std::min<uint32_t>(max_ctas, ceil_div(nt, 2)), 64, 0, ctx->stream>>>(
+        const auto kern = target ? (d->dtw_band ? k_dtw_rescore_warp<true, true> : k_dtw_rescore_warp<false, true>)
+                                 : (d->dtw_band ? k_dtw_rescore_warp<true> : k_dtw_rescore_warp<false>);
+        kern<<<std::min<uint32_t>(max_ctas, ceil_div(nt, 2)), 64, 0, ctx->stream>>>(
             d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, d_slot_qid, d->d_cand_idx.p, nt, kp, s_begin, s_count, rb, d->d_rescore_rows.p,
-            stride, d->d_cand_exact.p, d->d_counters.p, d->dtw_band);
+            stride, d->d_cand_exact.p, d->d_counters.p, d->dtw_band, d_targets);
         SS_LAUNCHED(ctx);
     }
-    k_dtw_finalize<<<ceil_div(nslots, 128), 128, 0, ctx->stream>>>(d->d_cand_idx.p, d->d_cand_adist.p, d->d_cand_exact.p, d_slot_qid, nslots, kp, k,
+    (target ? k_dtw_finalize<true> : k_dtw_finalize<false>)<<<ceil_div(nslots, 128), 128, 0, ctx->stream>>>(d->d_cand_idx.p, d->d_cand_adist.p, d->d_cand_exact.p, d_slot_qid, nslots, kp, k,
                                                                   d->index_base, d_max_na, d_max_nb, eps, d_slot_max_na, bound_mode, d->h2_bound_inv_s,
                                                                   (int)d->max_len, q->d_off.p, d_uncert_flag, d_out_idx, d_out_dist, d->d_counters.p);
     SS_LAUNCHED(ctx);
@@ -1537,17 +1548,22 @@ k_dtw_pairs_exact_warp(const double* __restrict__ dmfcc, const uint64_t* __restr
     }
 }
 
+// TARGET (SS_DTW_TARGET): selects by (|D - t|, index), t = targets[qids[u]] (targets NULL: t = 0)
+template <bool TARGET = false>
 __global__ void __launch_bounds__(256)
 k_dtw_select_exact(const double* __restrict__ exact, uint32_t nseg, int k, const uint32_t* __restrict__ qids, uint32_t index_base,
-                   uint32_t* __restrict__ out_idx, double* __restrict__ out_dist) {
+                   uint32_t* __restrict__ out_idx, double* __restrict__ out_dist, const double* __restrict__ targets) {
     __shared__ double sd[256 * SS_MAX_TOPK];
     __shared__ uint32_t si[256 * SS_MAX_TOPK];
     const uint32_t u = blockIdx.x, t = threadIdx.x;
     double dv[SS_MAX_TOPK];
     uint32_t iv[SS_MAX_TOPK];
     int n = 0;
+    double tq = 0.0;
+    if constexpr (TARGET) tq = targets ? targets[qids[u]] : 0.0;
     for (uint32_t s = t; s < nseg; s += 256) {
-        const double dd = exact[(size_t)u * nseg + s];
+        double dd = exact[(size_t)u * nseg + s];
+        if constexpr (TARGET) dd = fabs(dd - tq);
         if (dd < kInf) topk_push(dv, iv, n, k, dd, s);
     }
     topk_store(dv, iv, n, k, 0, si + t * SS_MAX_TOPK, sd + t * SS_MAX_TOPK);
@@ -1565,7 +1581,8 @@ k_dtw_select_exact(const double* __restrict__ exact, uint32_t nseg, int k, const
     }
 }
 
-int dtw_exhaustive_match(ss_dict* d, ss_queries* q, int k, const std::vector<uint32_t>& subset, uint32_t* d_out_idx, double* d_out_dist) {
+int dtw_exhaustive_match(ss_dict* d, ss_queries* q, int k, const std::vector<uint32_t>& subset, uint32_t* d_out_idx, double* d_out_dist,
+                         bool target, const double* d_targets) {
     ss_ctx* ctx = d->ctx;
     const uint32_t nseg = (uint32_t)d->nseg;
     const uint64_t budget = 32ull << 20;  // doubles of the distance table (256 MB)
@@ -1586,7 +1603,8 @@ int dtw_exhaustive_match(ss_dict* d, ss_queries* q, int k, const std::vector<uin
                 d->dtw_band);
             SS_LAUNCHED(ctx);
         }
-        k_dtw_select_exact<<<nu, 256, 0, ctx->stream>>>(d->d_exh_dist.p, nseg, k, d->d_exh_qid.p + u0, d->index_base, d_out_idx, d_out_dist);
+        (target ? k_dtw_select_exact<true> : k_dtw_select_exact<false>)<<<nu, 256, 0, ctx->stream>>>(d->d_exh_dist.p, nseg, k, d->d_exh_qid.p + u0,
+                                                                                                   d->index_base, d_out_idx, d_out_dist, d_targets);
         SS_LAUNCHED(ctx);
     }
     SS_CUDA(ctx, cudaMemsetAsync(d->d_counters.p, 0, sizeof(unsigned long long), ctx->stream));  // everything is exact now
@@ -1667,7 +1685,7 @@ int dtw_locate_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, uint32
             d->d_mfcc.p, d->d_off.p, q->d_mfcc.p, q->d_off.p, d->c, u0, nu, nseg, d->d_rescore_rows.p, stride, d->d_exh_qid.p, d->d_exh_dist.p,
             d->d_locate_span.p);
         SS_LAUNCHED(ctx);
-        k_dtw_select_exact<<<nu, 256, 0, ctx->stream>>>(d->d_exh_dist.p, nseg, k, d->d_exh_qid.p, d->index_base, d_out_idx, d_out_cost);
+        k_dtw_select_exact<<<nu, 256, 0, ctx->stream>>>(d->d_exh_dist.p, nseg, k, d->d_exh_qid.p, d->index_base, d_out_idx, d_out_cost, nullptr);
         SS_LAUNCHED(ctx);
         k_dtw_locate_spans<<<ceil_div((long long)nu * k, 256), 256, 0, ctx->stream>>>(d->d_locate_span.p, nseg, u0, nu, k, d->index_base, d_out_idx,
                                                                                       d_out_start, d_out_end);

@@ -170,6 +170,8 @@ struct ss_dict {
         int k = 0;
         uint32_t* d_out_idx = nullptr;
         double* d_out_dist = nullptr;
+        bool target = false;                  // SS_DTW_TARGET
+        const double* d_targets = nullptr;    // its targets, q's order (NULL: t = 0)
     } pending;
     unsigned long long* h_counters = nullptr;  // pinned, 4 entries: [0] uncertified queries, [1] extra candidates refined
     cudaEvent_t ev_done = nullptr;
@@ -309,12 +311,20 @@ int dtw_tc_dict_build(ss_dict* d);    // builds the fp16 UMMA tiles (dtw_tc.cu)
 int dtw_queries_build(ss_queries* q); // builds the lane layout (dtw.cu)
 int dtw_tc_queries_group(ss_queries* q);  // length-sorted groups of 128 for the tensor-core scan (dtw_tc.cu); no-op for long queries
 // asynchronous on the ctx stream up to the fallback decision; dtw_match_finish completes it (a no-op when nothing is pending)
-int dtw_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist);
+// target: SS_DTW_TARGET (DESIGN.md §3.1h), d_targets in q's order (NULL: t = 0), read until dtw_match_finish
+int dtw_match_dev(ss_dict* d, ss_queries* q, int k, uint32_t* d_out_idx, double* d_out_dist, bool target = false,
+                  const double* d_targets = nullptr);
 int dtw_match_finish(ss_dict* d);
+// the f64 refine and certification of a filter stage's candidate lists (exact.cu); target: the SS_DTW_TARGET form, whose
+// candidate keys (d_cand_adist) are already lower bounds on e = |D - t|
+int dtw_rescore_finalize(ss_dict* d, ss_queries* q, int k, int kp, uint32_t nslots, const uint32_t* d_slot_qid, double eps,
+                         const float* d_max_na, const float* d_max_nb, const float* d_slot_max_na, int bound_mode, uint8_t* d_uncert_flag,
+                         uint32_t* d_out_idx, double* d_out_dist, bool target = false, const double* d_targets = nullptr);
 int dtw_h2_dict_build(ss_dict* d);    // builds the interleaved fp16 tiles of the packed-half scan (dtw_h2.cu; after dtw_tc_dict_build)
 int dtw_h2_debug_scan(ss_dict* d, ss_queries* q, float* d_out, std::vector<uint32_t>* slot_qid, double* mu16, float* scale, float* s_out);
 int dtw_tc_debug_scan(ss_dict* d, ss_queries* q, float* d_out, std::vector<uint32_t>* slot_qid, double* mu16, float* scale);
 int queries_check(ss_ctx* ctx, const double* q_mfcc, const uint64_t* q_frame_offsets, size_t nq, int ncoeffs);  // capi.cu
+int targets_check(ss_ctx* ctx, int mode, const double* targets, size_t nq);  // capi.cu: SS_DTW_TARGET's targets are finite
 int queries_prepare(ss_queries* q, const uint64_t* q_frame_offsets, size_t nq);
 int queries_fill(ss_queries* q, const double* q_mfcc, const uint64_t* q_frame_offsets, size_t nq);
 int fill_result(ss_ctx* ctx, uint32_t* d_idx, double* d_dist, size_t n);  // (inf, 0xFFFFFFFF) rows (exact.cu)
