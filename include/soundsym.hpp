@@ -389,6 +389,13 @@ class SoundDictionary {
         dist->assign(distances.size(), 0.0);
         ctx_->check(ss_dict_walk(d, start.mfccs().data(), start.num_frames(), distances.data(), distances.size(), idx->data(), dist->data()));
     }
+    /// the same chain for SS_DTW_TARGET (ss_dict_walk_dtw): a step with no result gives (0xFFFFFFFF, inf), and so does every later one
+    void walk_dtw(const Sound& start, const std::vector<double>& distances, std::vector<uint32_t>* idx, std::vector<double>* dist) {
+        ss_dict* d = device();
+        idx->assign(distances.size(), 0);
+        dist->assign(distances.size(), 0.0);
+        ctx_->check(ss_dict_walk_dtw(d, start.mfccs().data(), start.num_frames(), distances.data(), distances.size(), idx->data(), dist->data()));
+    }
     /// DTW warping path (ss_dict_align) of queries[p] against sounds[indices[p]] (indices as match_indices returns them;
     /// 0xFFFFFFFF -> empty path, inf): (*paths)[p] holds (frame of the query, frame of the dictionary sound) pairs in order.
     /// Works in either mode: the path is the SS_DTW one whatever matcher chose the indices.
@@ -519,15 +526,19 @@ class SoundSequence {
         return SoundSequence(std::move(out), *ctx_);
     }
     /// SoundSequence::from_distances (src/sound.rs:405-417): a chain, step t matches the sound step t - 1 returned.
-    /// SS_COSINE_REF runs it on the device in one call; the DTW modes keep the nq = 1 loop (SS_DTW's at_distance ignores the
-    /// target, SS_DTW_TARGET's takes it).
+    /// SS_COSINE_REF runs it on the device in one call, and so does SS_DTW_TARGET (a step with no result throws
+    /// std::out_of_range); SS_DTW keeps the nq = 1 loop (its at_distance ignores the target).
     static SoundSequence from_distances(const std::vector<double>& distances, std::shared_ptr<Sound> start, SoundDictionary& dict) {
         std::vector<std::shared_ptr<Sound>> sounds{std::move(start)};
-        if (!distances.empty() && dict.mode == SS_COSINE_REF) {
+        if (!distances.empty() && (dict.mode == SS_COSINE_REF || dict.mode == SS_DTW_TARGET)) {
             std::vector<uint32_t> idx;
             std::vector<double> dist;
-            dict.walk(*sounds[0], distances, &idx, &dist);
-            for (uint32_t i : idx) sounds.push_back(dict.sounds[i]);
+            if (dict.mode == SS_COSINE_REF) dict.walk(*sounds[0], distances, &idx, &dist);
+            else dict.walk_dtw(*sounds[0], distances, &idx, &dist);
+            for (size_t t = 0; t < idx.size(); t++) {
+                if (idx[t] >= dict.sounds.size()) throw std::out_of_range("from_distances: step " + std::to_string(t) + " has no result");
+                sounds.push_back(dict.sounds[idx[t]]);
+            }
         } else {
             for (double d : distances) sounds.push_back(dict.at_distance(d, sounds.back()));
         }

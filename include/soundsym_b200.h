@@ -187,6 +187,20 @@ int ss_dict_walk(ss_dict* dict, const double* start_mfcc, size_t start_frames, c
  * `start` holds exactly one query */
 int ss_dict_walk_dev(ss_dict* dict, ss_queries* start, const double* d_distances, size_t nsteps, uint32_t* d_out_idx,
                      double* d_out_dist);
+/* SoundSequence::from_distances for SS_DTW_TARGET (DESIGN.md §3.1i), on the device: step t's (out_idx[t], out_dist[t]) equals
+ * ss_dict_match(dict, query_t, 1, SS_DTW_TARGET, &distances[t], 1, ...) bit for bit (A13: e = fabs(D - t) under the dictionary's
+ * band, indices include index_base); query_0 is the start sound, query_{t+1} the segment out_idx[t] - index_base. A step with
+ * no result (every e NaN or +inf) writes (0xFFFFFFFF, +inf), and every later step, which runs from an empty query, does too.
+ * distances == NULL means t = 0 at every step: SS_DTW's nq = 1 chain. A non-finite target -> SS_ERR_INVALID. Checks and ordering
+ * as ss_dict_walk: a pending SS_DTW match completes first, the ss_dict_last_* readers are untouched, ss_dict_set_scan does not
+ * apply (every step is exact f64 DTW against every segment). nsteps == 0 returns SS_OK and launches nothing. Host buffers, one
+ * blocking point. */
+int ss_dict_walk_dtw(ss_dict* dict, const double* start_mfcc, size_t start_frames, const double* distances, size_t nsteps,
+                     uint32_t* out_idx, double* out_dist);
+/* the same on device pointers, asynchronous on the ctx stream: exactly nsteps kernel launches, no host synchronisation besides
+ * completing a pending SS_DTW match; `start` holds exactly one query; d_distances (nsteps finite f64, or NULL) */
+int ss_dict_walk_dtw_dev(ss_dict* dict, ss_queries* start, const double* d_distances, size_t nsteps, uint32_t* d_out_idx,
+                         double* d_out_dist);
 /* DTW warping path of query p against dictionary segment seg_idx[p] (an index as ss_dict_match
  * reports it, index_base included; 0xFFFFFFFF -> empty path, inf). out_path: (i, j) uint32 pairs, compacted; path p is
  * out_path[out_path_offsets[p] .. out_path_offsets[p+1]) (nq + 1 offsets, in pairs). out_dist[p] is bit-equal to ss_dict_match's

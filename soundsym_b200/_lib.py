@@ -22,7 +22,7 @@ SYMBOLS = [
     "ss_queries_create", "ss_queries_destroy", "ss_dict_match_dev", "ss_topk_merge_dev", "ss_dict_last_work", "ss_dict_last_scan_kind",
     "ss_dict_last_uncertified", "ss_dict_last_tc_fallback", "ss_dict_last_exhaustive", "ss_queries_invalidate", "ss_dict_last_scan_ms", "ss_resynth", "ss_resynth_warped", "ss_sequence_distances", "ss_dict_debug_tc_scan", "ss_dict_debug_h2_scan", "ss_dict_set_scan", "ss_dict_match_finish",
     "ss_dict_set_dtw_band", "ss_dict_dtw_band", "ss_sharded_dict_set_dtw_band",
-    "ss_dict_walk", "ss_dict_walk_dev", "ss_dict_align", "ss_dict_align_dev", "ss_dict_locate", "ss_dict_locate_dev",
+    "ss_dict_walk", "ss_dict_walk_dev", "ss_dict_walk_dtw", "ss_dict_walk_dtw_dev", "ss_dict_align", "ss_dict_align_dev", "ss_dict_locate", "ss_dict_locate_dev",
     "ss_shard_bounds", "ss_comm_unique_id", "ss_comm_create", "ss_comm_create_all", "ss_comm_destroy", "ss_comm_rank", "ss_comm_nranks",
     "ss_queries_create_sharded", "ss_dict_match_sharded_dev", "ss_dict_match_sharded", "ss_dict_create_sharded", "ss_sharded_dict_match",
     "ss_sharded_dict_destroy", "ss_sharded_dict_len", "ss_sharded_dict_nshards",
@@ -110,6 +110,8 @@ def load():
     L.ss_dict_match_finish.argtypes = [vp]
     L.ss_dict_walk.argtypes = [vp, vp, sz, vp, sz, vp, vp]
     L.ss_dict_walk_dev.argtypes = [vp, vp, vp, sz, vp, vp]
+    L.ss_dict_walk_dtw.argtypes = [vp, vp, sz, vp, sz, vp, vp]
+    L.ss_dict_walk_dtw_dev.argtypes = [vp, vp, vp, sz, vp, vp]
     L.ss_dict_align.argtypes = [vp, vp, vp, sz, vp, vp, sz, vp, vp]
     L.ss_dict_align_dev.argtypes = [vp, vp, vp, vp, sz, vp, vp]
     L.ss_dict_locate.argtypes = [vp, vp, vp, sz, i, vp, vp, vp, vp]

@@ -277,6 +277,18 @@ class DeviceDictionary:
         self.ctx.check(self.ctx.lib.ss_dict_walk(self.h, _ptr(s), s.shape[0], _ptr(t), n, _ptr(idx), _ptr(dist)))
         return idx, dist
 
+    def walk_dtw(self, start_mfcc, distances=None, nsteps=None):
+        """ss_dict_walk_dtw: SoundSequence::from_distances for SS_DTW_TARGET on the device -> (idx u32 [n], dist f64 [n]); step t
+        matches the segment step t - 1 returned (step 0: start_mfcc) at target distances[t]. distances=None: t = 0 at each of
+        `nsteps` steps (SS_DTW's chain). A step with no result gives (0xFFFFFFFF, inf), and so does every later one."""
+        s = np.ascontiguousarray(start_mfcc, dtype=np.float64).reshape(-1, self.ncoeffs)
+        t = None if distances is None else np.ascontiguousarray(distances, dtype=np.float64).reshape(-1)
+        n = t.shape[0] if t is not None else int(nsteps or 0)
+        idx = np.empty(n, dtype=np.uint32)
+        dist = np.empty(n, dtype=np.float64)
+        self.ctx.check(self.ctx.lib.ss_dict_walk_dtw(self.h, _ptr(s), s.shape[0], _ptr(t), n, _ptr(idx), _ptr(dist)))
+        return idx, dist
+
     def align(self, q_flat, q_frame_offsets, seg_idx):
         """ss_dict_align: the DTW warping path (DESIGN.md §3.1e) of query p against segment seg_idx[p] (an index as
         match reports it; 0xFFFFFFFF -> empty path, inf) -> (paths: list of uint32 [n, 2] arrays of (i, j), dist f64 [nq])."""
@@ -850,13 +862,15 @@ class SoundSequence:
     @classmethod
     def from_distances(cls, distances, start, dictionary):
         """src/sound.rs:405-417: a chain, step t matches the sound step t - 1 returned. SS_COSINE_REF runs it on the device
-        in one call (ss_dict_walk); the DTW modes keep the nq = 1 loop (SS_DTW's at_distance ignores the target,
-        SS_DTW_TARGET's takes it)."""
+        in one call (ss_dict_walk), and so does SS_DTW_TARGET (ss_dict_walk_dtw; a step with no result raises IndexError
+        there, as at_distance does); SS_DTW keeps the nq = 1 loop (its at_distance ignores the target)."""
         sounds = [start]
         distances = list(distances)
-        if distances and dictionary.mode == SS_COSINE_REF:
-            idx, _ = dictionary._device().walk(start.mfcc_arrays(), distances)
-            sounds += [dictionary.sounds[int(i)] for i in idx]
+        if distances and dictionary.mode in (SS_COSINE_REF, SS_DTW_TARGET):
+            dev = dictionary._device()
+            walk = dev.walk if dictionary.mode == SS_COSINE_REF else dev.walk_dtw
+            idx, _ = walk(start.mfcc_arrays(), distances)
+            sounds += [dictionary.sounds[int(i)] for i in idx]  # (0xFFFFFFFF: IndexError at that step)
         else:
             for d in distances:
                 sounds.append(dictionary.at_distance(d, sounds[-1]))

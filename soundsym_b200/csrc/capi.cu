@@ -374,6 +374,58 @@ int ss_dict_walk(ss_dict* d, const double* start_mfcc, size_t start_frames, cons
     return rc;
 }
 
+// SoundSequence::from_distances for SS_DTW_TARGET (DESIGN.md §3.1i), with ss_dict_walk's checks and ordering. The walk is exact
+// f64 DTW against every segment, so ss_dict_set_scan does not apply; the band does.
+int ss_dict_walk_dtw_dev(ss_dict* d, ss_queries* start, const double* d_distances, size_t nsteps, uint32_t* d_out_idx, double* d_out_dist) {
+    if (!d) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
+    ss_ctx* ctx = d->ctx;
+    if (nsteps && (!d_out_idx || !d_out_dist)) return set_error(ctx, SS_ERR_INVALID, "output pointers are NULL");
+    if (d->nseg == 0) return set_error(ctx, SS_ERR_EMPTY_DICT, "walk over an empty dictionary");
+    if (!start) return set_error(ctx, SS_ERR_INVALID, "start is NULL");
+    if (start->ctx != ctx) return set_error(ctx, SS_ERR_INVALID, "dict and start belong to different contexts");
+    if (start->c != d->c) return set_error(ctx, SS_ERR_INVALID, "ncoeffs mismatch: dict %d, start %d", d->c, start->c);
+    if (start->nq != 1) return set_error(ctx, SS_ERR_INVALID, "start must hold exactly one query (got %zu)", start->nq);
+    if (nsteps > 0xFFFFFFFFull) return set_error(ctx, SS_ERR_INVALID, "too many steps");
+    if (!nsteps) return SS_OK;
+    SS_CUDA(ctx, cudaSetDevice(ctx->device));
+    SS_TRY(dtw_match_finish(d));  // a pending SS_DTW match completes first, as before a cosine walk
+    return dtw_walk_dev(d, start->d_mfcc.p, start->d_off.p, start->h_off[1], d_distances, nsteps, d_out_idx, d_out_dist);
+}
+
+int ss_dict_walk_dtw(ss_dict* d, const double* start_mfcc, size_t start_frames, const double* distances, size_t nsteps, uint32_t* out_idx,
+                     double* out_dist) {
+    if (!d) return set_error(nullptr, SS_ERR_INVALID, "dict is NULL");
+    ss_ctx* ctx = d->ctx;
+    if (nsteps && (!out_idx || !out_dist)) return set_error(ctx, SS_ERR_INVALID, "output pointers are NULL");
+    if (d->nseg == 0) return set_error(ctx, SS_ERR_EMPTY_DICT, "walk over an empty dictionary");
+    if (start_frames && !start_mfcc) return set_error(ctx, SS_ERR_INVALID, "start_mfcc is NULL");
+    if (start_frames > 0x7FFFFFFFull / (uint64_t)d->c) return set_error(ctx, SS_ERR_INVALID, "start sound too long");
+    if (nsteps > 0xFFFFFFFFull) return set_error(ctx, SS_ERR_INVALID, "too many steps");
+    SS_TRY(targets_check(ctx, SS_DTW_TARGET, distances, nsteps));
+    if (!nsteps) return SS_OK;
+    SS_CUDA(ctx, cudaSetDevice(ctx->device));
+    auto body = [&]() -> int {
+        SS_TRY(dtw_match_finish(d));
+        d->h_walk_off[0] = 0;
+        d->h_walk_off[1] = start_frames;
+        SS_TRY(upload(ctx, d->d_walk_start, start_mfcc, start_frames * (size_t)d->c));
+        SS_TRY(upload(ctx, d->d_walk_off, d->h_walk_off, 2));
+        if (distances) SS_TRY(upload(ctx, d->d_walk_targets, distances, nsteps));
+        SS_CUDA(ctx, d->d_walk_idx.reserve(nsteps));
+        SS_CUDA(ctx, d->d_walk_dist.reserve(nsteps));
+        SS_TRY(dtw_walk_dev(d, d->d_walk_start.p, d->d_walk_off.p, start_frames, distances ? d->d_walk_targets.p : nullptr, nsteps, d->d_walk_idx.p,
+                            d->d_walk_dist.p));
+        // ONE blocking point per call
+        SS_CUDA(ctx, cudaMemcpyAsync(out_idx, d->d_walk_idx.p, nsteps * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+        SS_CUDA(ctx, cudaMemcpyAsync(out_dist, d->d_walk_dist.p, nsteps * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        SS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        return SS_OK;
+    };
+    const int rc = body();
+    if (rc != SS_OK) cudaStreamSynchronize(ctx->stream);
+    return rc;
+}
+
 // DTW warping paths (DESIGN.md §3.1e). Alignment takes indices, not a matcher: it works whatever mode the dictionary was last
 // matched in. Like a walk it first completes a pending SS_DTW match, has its own workspaces and leaves the ss_dict_last_*
 // counters as the last match left them.

@@ -1613,6 +1613,193 @@ int dtw_exhaustive_match(ss_dict* d, ss_queries* q, int k, const std::vector<uin
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// SoundSequence::from_distances for SS_DTW_TARGET on the device (DESIGN.md §3.1i): step t is ss_dict_match(query_t, nq = 1,
+// SS_DTW_TARGET, distances[t], k = 1), query_{t+1} = the segment step t returned. From step 1 on the query is a dictionary
+// segment already in HBM, and an exact f64 DTW of one query against every segment needs no filter and no certification, so
+// the chain runs as one launch per step with no host decision in between - k_cosine_walk_step's skeleton: CTAs grid-stride
+// over the (length, index) order d_cos_seg, each keeps its (e, index) minimum, and the last CTA to finish (atomic ticket)
+// reduces the partials and writes the step's result and the next step's query. No CTA ever waits for another.
+// The query's length is the same for the whole grid, so the mapping branch is uniform:
+//   short pairs (query and segment <= 32 frames): SEGMENTS on lanes, the query broadcast from shared memory. A lane holds its
+//     segment's DP column of Lq <= 32 doubles in registers and walks the segment's frames; consecutive lanes take consecutive
+//     positions of the length order, so the lanes of a warp run (almost) the same number of columns;
+//   every other pair: one warp per pair (warp_dtw_exact_long, the exhaustive stage's recurrence), the positions past the
+//     short ones (the order is by length, so the long segments are its tail), or all of them for a query of > 32 frames.
+// Both compute A8's operations in A8's order (dlt = a - b, cost = cost + dlt * dlt from 0.0; D(0, 0) = cost + 0.0;
+// D(i, j) = cost + fmin(fmin(up, left), diag), a missing neighbour +inf; +inf outside the band; D / (Lq + Ld); an empty side
+// +inf), then e = fabs(D - t): every step's (index, e) is the bits of the nq = 1 match.
+constexpr int kDtwWalkWarps = 2;                      // warps per CTA (a 16 KB cost ring each for the warp path)
+constexpr int kDtwWalkThreads = 32 * kDtwWalkWarps;
+constexpr int kDtwWalkCtasPerSm = 4;                  // 2 warps per SM sub-partition: up to 255 registers a thread (6 CTAs spilled at 168)
+constexpr int kDtwWalkShort = 32;                     // frames of the longest pair side the lane path takes
+
+// (e, index) minimum of the walk: seed (+inf, none); only e < +inf enters (NaN and +inf are never a result), a smaller e wins,
+// an equal one with a smaller index
+__device__ __forceinline__ void dtw_walk_min(double& bd, uint32_t& bi, double e, uint32_t i) {
+    if (e < kInf && (e < bd || (e == bd && i < bi))) {
+        bd = e;
+        bi = i;
+    }
+}
+
+__device__ __forceinline__ void dtw_walk_block_min(double& bd, uint32_t& bi) {
+    __shared__ double sd[kDtwWalkWarps];
+    __shared__ uint32_t si[kDtwWalkWarps];
+#pragma unroll
+    for (int o = 16; o; o >>= 1) dtw_walk_min(bd, bi, __shfl_xor_sync(0xffffffffu, bd, o), __shfl_xor_sync(0xffffffffu, bi, o));
+    __syncthreads();  // (sd / si are reused by the last CTA's second reduction)
+    if ((threadIdx.x & 31) == 0) sd[threadIdx.x >> 5] = bd, si[threadIdx.x >> 5] = bi;
+    __syncthreads();
+    if (threadIdx.x == 0)
+        for (int w = 1; w < kDtwWalkWarps; w++) dtw_walk_min(bd, bi, sd[w], si[w]);
+}
+
+// A8's D of a query of la <= 32 frames (sa: shared memory, broadcast) against a segment of lb <= 32 frames (b: global memory)
+// by one thread: column j of D lives in col[], cell (i, j) takes up = D(i-1, j) (this column's previous row), left = col[i]
+// (= D(i, j-1)) and diag = D(i-1, j-1) (the previous row's old value)
+template <bool BAND>
+__device__ __forceinline__ double lane_dtw_exact(const double* __restrict__ sa, int la, const double* __restrict__ b, int lb, int c, uint32_t band) {
+    double col[kDtwWalkShort];
+#pragma unroll
+    for (int i = 0; i < kDtwWalkShort; i++) col[i] = kInf;
+    for (int j = 0; j < lb; j++) {
+        // (every load in bounds and unconditional, the coefficient test after it: a load behind `k < c` waited for the previous
+        // one, one memory latency per coefficient)
+        double br[SS_MAX_NCOEFFS];
+#pragma unroll
+        for (int k = 0; k < SS_MAX_NCOEFFS; k++) br[k] = __ldg(b + (size_t)j * c + min(k, c - 1));
+        int blo = 0, bhi = 0;
+        if (BAND) band_rows(j, la, lb, band, &blo, &bhi);
+        double up = kInf, diag = kInf;
+#pragma unroll
+        for (int i = 0; i < kDtwWalkShort; i++) {
+            if (i < la) {
+                double cost = 0.0;
+#pragma unroll
+                for (int k = 0; k < SS_MAX_NCOEFFS; k++)
+                    if (k < c) {
+                        const double dlt = sa[i * c + k] - br[k];
+                        cost = cost + dlt * dlt;
+                    }
+                const double left = col[i];
+                double m;
+                if (i == 0 && j == 0) m = 0.0;
+                else m = fmin(fmin(up, left), diag);
+                double v;
+                if (BAND && (i < blo || i > bhi)) v = kInf;
+                else v = cost + m;
+                diag = left;
+                col[i] = v;
+                up = v;
+            }
+        }
+    }
+    double r = kInf;
+#pragma unroll
+    for (int i = 0; i < kDtwWalkShort; i++)
+        if (i == la - 1) r = col[i];  // (a register, not a local-memory index)
+    return (la && lb) ? r / (double)(la + lb) : kInf;
+}
+
+template <bool BAND>
+__global__ void __launch_bounds__(kDtwWalkThreads, kDtwWalkCtasPerSm)
+k_dtw_walk_step(const double* __restrict__ dmfcc, const uint64_t* __restrict__ doff, const uint4* __restrict__ cseg, uint32_t nseg,
+                uint32_t nshort, int c, const double* __restrict__ start, const uint64_t* __restrict__ start_off,
+                const double* __restrict__ targets, uint32_t step, uint32_t index_base, uint32_t band, double* __restrict__ bnd,
+                uint32_t bnd_stride, double* __restrict__ part_dist, uint32_t* __restrict__ part_idx,
+                uint32_t* __restrict__ state /* [0] ticket, [1] query of the next step (none: an empty query) */,
+                uint32_t* __restrict__ out_idx, double* __restrict__ out_dist) {
+    __shared__ double ring[kDtwWalkWarps][64 * 32];
+    __shared__ double sq[kDtwWalkShort * SS_MAX_NCOEFFS];
+    __shared__ bool last;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    // the query: the start sound at step 0, else the segment the previous step returned (written by its last CTA)
+    const double* qp = start;
+    int lq = 0;
+    if (step == 0) {
+        qp = start + start_off[0] * c;
+        lq = (int)(start_off[1] - start_off[0]);
+    } else if (state[1] != kCosNone) {
+        const uint32_t s = state[1];
+        qp = dmfcc + doff[s] * c;
+        lq = (int)(doff[s + 1] - doff[s]);
+    }
+    const double t = targets ? targets[step] : 0.0;
+    double bd = kInf;
+    uint32_t bi = kCosNone;
+    if (lq > 0) {  // (an empty query has no result: every e is +inf)
+        uint32_t long_begin = 0;
+        if (lq <= kDtwWalkShort) {
+            for (int e = threadIdx.x; e < lq * c; e += kDtwWalkThreads) sq[e] = qp[e];
+            __syncthreads();
+            for (uint32_t pos = blockIdx.x * kDtwWalkThreads + threadIdx.x; pos < nshort; pos += gridDim.x * kDtwWalkThreads) {
+                const uint4 dsc = __ldg(&cseg[pos]);
+                const double D = lane_dtw_exact<BAND>(sq, lq, dmfcc + (((uint64_t)dsc.y << 32) | dsc.x) * c, (int)dsc.z, c, band);
+                dtw_walk_min(bd, bi, fabs(D - t), dsc.w);
+            }
+            long_begin = nshort;
+        }
+        const uint32_t gw = blockIdx.x * kDtwWalkWarps + warp;
+        for (uint32_t pos = long_begin + gw; pos < nseg; pos += gridDim.x * kDtwWalkWarps) {  // warp-uniform
+            const uint4 dsc = __ldg(&cseg[pos]);
+            const double D = warp_dtw_exact_long<BAND>(qp, lq, dmfcc + (((uint64_t)dsc.y << 32) | dsc.x) * c, (int)dsc.z, c, ring[warp],
+                                                       bnd + (size_t)gw * bnd_stride, lane, band);
+            if (lane == 0) dtw_walk_min(bd, bi, fabs(D - t), dsc.w);
+        }
+    }
+    dtw_walk_block_min(bd, bi);
+    if (threadIdx.x == 0) {
+        part_dist[blockIdx.x] = bd;
+        part_idx[blockIdx.x] = bi;
+        __threadfence();
+        last = atomicAdd(&state[0], 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (!last) return;
+    // the last CTA: every other CTA's partial is visible (its fence came before its ticket)
+    __threadfence();
+    bd = kInf;
+    bi = kCosNone;
+    for (uint32_t b = threadIdx.x; b < gridDim.x; b += kDtwWalkThreads) dtw_walk_min(bd, bi, __ldcg(&part_dist[b]), __ldcg(&part_idx[b]));
+    dtw_walk_block_min(bd, bi);
+    if (threadIdx.x == 0) {
+        out_idx[step] = bi != kCosNone ? bi + index_base : 0xFFFFFFFFu;  // no result: SS_DTW_TARGET's unfilled slot
+        out_dist[step] = bd;
+        state[1] = bi;
+        state[0] = 0;
+    }
+}
+
+int dtw_walk_dev(ss_dict* d, const double* d_start, const uint64_t* d_start_off, uint64_t start_frames, const double* d_targets, size_t nsteps,
+                 uint32_t* d_out_idx, double* d_out_dist) {
+    ss_ctx* ctx = d->ctx;
+    if (!nsteps) return SS_OK;
+    const uint32_t nseg = (uint32_t)d->nseg;
+    // the length order's segments of <= 32 frames come first
+    const uint32_t nshort = (uint32_t)(std::partition_point(d->h_cos_seg.begin(), d->h_cos_seg.end(),
+                                                            [](const uint4& s) { return s.z <= (uint32_t)kDtwWalkShort; }) -
+                                       d->h_cos_seg.begin());
+    // enough CTAs for one segment per lane, or one pair per warp when the query is long; at most one wave
+    const uint32_t want = std::max<uint32_t>(ceil_div(nshort, kDtwWalkThreads), ceil_div((long long)nseg, kDtwWalkWarps));
+    const uint32_t grid = (uint32_t)std::max<long long>(1, std::min<long long>(want, (long long)ctx->sm_count * kDtwWalkCtasPerSm));
+    // warp_dtw_exact_long's boundary row: one row of the longest query per warp
+    const uint32_t stride = (uint32_t)((std::max<uint64_t>(std::max<uint64_t>(start_frames, d->max_len), 1) + 15) & ~15ull);
+    SS_CUDA(ctx, d->d_walk_part_dist.reserve(grid));
+    SS_CUDA(ctx, d->d_walk_part_idx.reserve(grid));
+    SS_CUDA(ctx, d->d_walk_state.reserve(2));
+    SS_CUDA(ctx, d->d_walk_bnd.reserve((size_t)grid * kDtwWalkWarps * stride));
+    SS_CUDA(ctx, cudaMemsetAsync(d->d_walk_state.p, 0, 2 * sizeof(uint32_t), ctx->stream));
+    auto kern = d->dtw_band ? k_dtw_walk_step<true> : k_dtw_walk_step<false>;
+    for (size_t t = 0; t < nsteps; t++) {
+        kern<<<grid, kDtwWalkThreads, 0, ctx->stream>>>(d->d_mfcc.p, d->d_off.p, d->d_cos_seg.p, nseg, nshort, d->c, d_start, d_start_off, d_targets,
+                                                        (uint32_t)t, d->index_base, d->dtw_band, d->d_walk_bnd.p, stride, d->d_walk_part_dist.p,
+                                                        d->d_walk_part_idx.p, d->d_walk_state.p, d_out_idx, d_out_dist);
+        SS_LAUNCHED(ctx);
+    }
+    return SS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // subsequence DTW (ss_dict_locate, A12 in DESIGN.md §3.1g): every query against every segment, where the query may start and
 // end anywhere in the segment. The exhaustive stage's shape with the SUBSEQ recurrence: one warp per (query, segment) pair
 // writes the pair's unnormalised cost (+inf: no hit) into an f64 table that k_dtw_select_exact reads as it is, and its

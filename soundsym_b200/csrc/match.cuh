@@ -188,7 +188,8 @@ struct ss_dict {
     ss::DevBuf<double> d_res_dist, d_res_targets;
     // ss_dict_walk (exact.cu cosine_walk_dev): its own buffers, so that a walk never touches a match's workspaces or the
     // last_* counters. state = {ticket of the last-CTA reduction, local index of the next step's query}
-    ss::DevBuf<double> d_walk_part_dist, d_walk_qnorm;
+    // (ss_dict_walk_dtw, exact.cu dtw_walk_dev, shares them and adds the boundary rows of its warp-per-pair path)
+    ss::DevBuf<double> d_walk_part_dist, d_walk_qnorm, d_walk_bnd;
     ss::DevBuf<uint32_t> d_walk_part_idx, d_walk_state;
     ss::DevBuf<double> d_walk_start, d_walk_targets, d_walk_dist;  // host-buffer entry point: start frames, targets, results
     ss::DevBuf<uint64_t> d_walk_off;
@@ -334,6 +335,10 @@ int cosine_match_dev(ss_dict* d, ss_queries* q, const double* d_targets, uint32_
 // SoundSequence::from_distances for SS_COSINE_REF: nsteps + 1 launches on the ctx stream, no host synchronisation (exact.cu)
 int cosine_walk_dev(ss_dict* d, const double* d_start, const uint64_t* d_start_off, const double* d_targets, size_t nsteps,
                     uint32_t* d_out_idx, double* d_out_dist);
+// SoundSequence::from_distances for SS_DTW_TARGET (DESIGN.md §3.1i): nsteps launches on the ctx stream, no host synchronisation
+// (exact.cu). d_targets NULL: t = 0; start_frames: the start query's length (sizes the boundary rows)
+int dtw_walk_dev(ss_dict* d, const double* d_start, const uint64_t* d_start_off, uint64_t start_frames, const double* d_targets, size_t nsteps,
+                 uint32_t* d_out_idx, double* d_out_dist);
 // the DTW warping path (DESIGN.md §3.1e) of query p (frames d_qoff[p] .. d_qoff[p+1], h_qoff its host copy) against segment
 // d_seg_idx[p]: 1 + (waves of long pairs) + 2 launches on the ctx stream, no host synchronisation (exact.cu). d_out_path must
 // hold sum over non-empty queries of (Lq + max(longest segment, 1) - 1) (i, j) pairs.
